@@ -21,6 +21,15 @@ unsigned long long g_launch_count = 0;
 
 using namespace biu;
 
+// `esz` of the layer entry points: 2 = bf16, 4 = fp32, BIU_ESZ_FP16 = fp16 -> storage bytes and fp16 flag
+static int layer_format(int esz, int* bytes, int* f16) {
+  BIU_REQUIRE(esz == 2 || esz == 4 || esz == BIU_ESZ_FP16, "unknown element code esz=%d (2 = bf16, %d = fp16, 4 = fp32)",
+              esz, BIU_ESZ_FP16);
+  *bytes = esz == 4 ? 4 : 2;
+  *f16 = esz == BIU_ESZ_FP16 ? 1 : 0;
+  return 0;
+}
+
 struct biu_net {
   Net* n;
 };
@@ -34,7 +43,7 @@ biu_net* biu_net_create(int kind, int n_filter, int in_channels, int n_heads, co
                         const int* head_acts, const char* const* head_names, int siam_mode, int use_interpolation,
                         int precision) {
   if (kind < 0 || kind > 8) { set_error("unknown network kind %d", kind); return nullptr; }
-  if (precision < 0 || precision > 2) { set_error("unknown precision %d", precision); return nullptr; }
+  if (precision < 0 || precision > 3) { set_error("unknown precision %d", precision); return nullptr; }
   if (n_heads < 1 || !head_channels || !head_acts) { set_error("at least one output head is required"); return nullptr; }
   Net* n = new Net();
   n->kind = kind; n->nf = n_filter; n->in_ch = in_channels; n->precision = precision;
@@ -183,7 +192,8 @@ int biu_conv_tc(int esz, const void* in, int in_ctot, int in_coff, int cin, int 
                 void* out, int out_ctot, int out_coff, void* stream) {
   ConvTcArgs a;
   memset(&a, 0, sizeof(a));
-  a.esz = esz; a.in = in; a.in_ctot = in_ctot; a.in_coff = in_coff; a.cin = cin;
+  if (int rc = layer_format(esz, &a.esz, &a.f16)) return rc;
+  a.in = in; a.in_ctot = in_ctot; a.in_coff = in_coff; a.cin = cin;
   a.W = W; a.H = H; a.D = D; a.B = B; a.kw = kw; a.kh = kh; a.kd = kd;
   a.wgt = wgt; a.n_total = cout; a.mode = EPI_CONV; a.slope = slope; a.scale = scale; a.shift = shift;
   a.out = out; a.out_ctot = out_ctot; a.out_coff = out_coff;
@@ -193,7 +203,8 @@ int biu_up_tc(int esz, const void* in, int in_ctot, int in_coff, int cin, int B,
               const void* wgt, int cout, const float* bias_rep, void* out, int out_ctot, int out_coff, void* stream) {
   ConvTcArgs a;
   memset(&a, 0, sizeof(a));
-  a.esz = esz; a.in = in; a.in_ctot = in_ctot; a.in_coff = in_coff; a.cin = cin;
+  if (int rc = layer_format(esz, &a.esz, &a.f16)) return rc;
+  a.in = in; a.in_ctot = in_ctot; a.in_coff = in_coff; a.cin = cin;
   a.W = W; a.H = H; a.D = D; a.B = B; a.kw = a.kh = a.kd = 1;
   a.wgt = wgt; a.n_total = (dims == 3 ? 8 : 4) * cout; a.mode = EPI_UP; a.slope = 1.f; a.scale = bias_rep;
   a.shift = bias_rep; a.out = out; a.out_ctot = out_ctot; a.out_coff = out_coff; a.up_cout = cout; a.up_dims = dims;
@@ -204,7 +215,8 @@ int biu_conv_direct(int esz, const void* in, int in_ctot, int in_coff, int cin, 
                     void* out, int out_ctot, int out_coff, void* stream) {
   DirectConvArgs a;
   memset(&a, 0, sizeof(a));
-  a.esz = esz; a.in = in; a.in_ctot = in_ctot; a.in_coff = in_coff; a.cin = cin;
+  if (int rc = layer_format(esz, &a.esz, &a.f16)) return rc;
+  a.in = in; a.in_ctot = in_ctot; a.in_coff = in_coff; a.cin = cin;
   a.W = W; a.H = H; a.D = D; a.B = B; a.kw = kw; a.kh = kh; a.kd = kd;
   a.wgt = wgt; a.cout = cout; a.slope = slope; a.scale = scale; a.shift = shift;
   a.out = out; a.out_ctot = out_ctot; a.out_coff = out_coff;
@@ -214,7 +226,8 @@ int biu_pool2(int esz, const void* in, int in_ctot, int in_coff, int c, int B, i
               int mode, void* out, int out_ctot, int out_coff, void* stream) {
   PoolArgs a;
   memset(&a, 0, sizeof(a));
-  a.esz = esz; a.in = in; a.in_ctot = in_ctot; a.in_coff = in_coff; a.c = c; a.W = W; a.H = H; a.D = D; a.B = B;
+  if (int rc = layer_format(esz, &a.esz, &a.f16)) return rc;
+  a.in = in; a.in_ctot = in_ctot; a.in_coff = in_coff; a.c = c; a.W = W; a.H = H; a.D = D; a.B = B;
   a.dims = dims; a.mode = mode; a.out = out; a.out_ctot = out_ctot; a.out_coff = out_coff;
   return launch_pool2(a, (cudaStream_t)stream);
 }

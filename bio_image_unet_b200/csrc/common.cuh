@@ -7,6 +7,7 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
 #include <stdio.h>
 
@@ -47,6 +48,15 @@ static __device__ unsigned int g_device_fault = 0;
 // ----------------------------------------------------------------------------------------------
 __host__ __device__ inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 __host__ __device__ inline long long ceil_div_ll(long long a, long long b) { return (a + b - 1) / b; }
+
+// ----------------------------------------------------------------------------------------------
+// Element formats of the activations and tcgen05 operands. bf16 and fp32 / tf32 are coded by their byte size (the `esz`
+// of the layer C-ABI, the template argument of the kernels); fp16 is a second 2-byte format with a code of its own.
+// ----------------------------------------------------------------------------------------------
+enum ElemFmt { FMT_BF16 = 2, FMT_F16 = 3, FMT_TF32 = 4 };
+__host__ __device__ constexpr int fmt_esz(int fmt) { return fmt == FMT_TF32 ? 4 : 2; }
+// A / B format field of the tcgen05 instruction descriptor (make_idesc)
+__host__ __device__ constexpr uint32_t fmt_idesc(int fmt) { return fmt == FMT_F16 ? 0u : (fmt == FMT_BF16 ? 1u : 2u); }
 
 #ifdef __CUDACC__
 
@@ -221,7 +231,7 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr, uint32_t sbo_
 }
 
 // Instruction descriptor, kind::f16 / kind::tf32, K-major A and B, fp32 accumulate, M = 128 (256 for a CTA pair).
-//   fmt: 0 = f16, 1 = bf16, 2 = tf32
+//   fmt: 0 = f16, 1 = bf16, 2 = tf32 (fmt_idesc)
 __device__ __forceinline__ uint32_t make_idesc(uint32_t fmt, uint32_t n, uint32_t m = 128u) {
   return (1u << 4) | (fmt << 7) | (fmt << 10) | ((n >> 3) << 17) | ((m >> 4) << 24);
 }
@@ -263,6 +273,27 @@ __device__ __forceinline__ void tc_commit2(uint64_t* bar) {
           smem_u32(bar)),
       "h"((uint16_t)3)
       : "memory");
+}
+
+// Two floats -> one 32-bit pair of a 2-byte format (a in the low half), each rounded to nearest even.
+template <int FMT>
+__device__ __forceinline__ uint32_t pack_half2(float a, float b) {
+  if (FMT == FMT_F16) {
+    __half2 h2 = __floats2half2_rn(a, b);
+    return *reinterpret_cast<uint32_t*>(&h2);
+  }
+  __nv_bfloat162 b2 = __floats2bfloat162_rn(a, b);
+  return *reinterpret_cast<uint32_t*>(&b2);
+}
+// Element-wise maximum of two 32-bit pairs of a 2-byte format.
+template <int FMT>
+__device__ __forceinline__ uint32_t max_half2(uint32_t a, uint32_t b) {
+  if (FMT == FMT_F16) {
+    __half2 m = __hmax2(*reinterpret_cast<__half2*>(&a), *reinterpret_cast<__half2*>(&b));
+    return *reinterpret_cast<uint32_t*>(&m);
+  }
+  __nv_bfloat162 m = __hmax2(*reinterpret_cast<__nv_bfloat162*>(&a), *reinterpret_cast<__nv_bfloat162*>(&b));
+  return *reinterpret_cast<uint32_t*>(&m);
 }
 
 #endif  // __CUDACC__

@@ -100,8 +100,9 @@ __device__ __forceinline__ HaloTile halo_decode(const ConvHaloParams& p, int t) 
 }
 
 // tcgen05.mma with a compile-time accumulate flag (no predicate register to materialise per instruction)
-template <int ESZ, int ACC, bool CTA2 = false>
+template <int FMT, int ACC, bool CTA2 = false>
 __device__ __forceinline__ void tc_mma_imm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc) {
+  constexpr int ESZ = fmt_esz(FMT);               // 2: kind::f16 (bf16 and fp16 operands), 4: kind::tf32
   if (CTA2) {                           // one MMA of M = 256 over the CTA pair (issued by the leader CTA only)
     if (ESZ == 2) {
       asm volatile(
@@ -144,9 +145,10 @@ __device__ __forceinline__ void tc_mma_imm(uint32_t tmem_d, uint64_t adesc, uint
 }
 
 // predicated single-lane issue from warp-uniform code
-template <int ESZ>
+template <int FMT>
 __device__ __forceinline__ void tc_mma_pred(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
                                             uint32_t accumulate, uint32_t issue) {
+  constexpr int ESZ = fmt_esz(FMT);
   if (ESZ == 2) {
     asm volatile(
         "{\n"
@@ -227,14 +229,11 @@ __device__ __forceinline__ void tmem_wait_regs(uint32_t (&r)[32]) {
 // Work units = (MMA tile j, chunk of CW accumulator columns); the two warp groups take alternate units. With the
 // fused head a thread needs the whole channel row of its pixel, so there the groups alternate MMA tiles instead.
 // ---------------------------------------------------------------------------------------------------------------
-template <int ESZ>
+template <int FMT>
 __device__ __forceinline__ void epi_store16(char* dst, const float (&v)[16], uint32_t (&w)[8]) {
-  if (ESZ == 2) {
+  if (fmt_esz(FMT) == 2) {
 #pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      __nv_bfloat162 b2 = __floats2bfloat162_rn(v[2 * i], v[2 * i + 1]);
-      w[i] = *reinterpret_cast<uint32_t*>(&b2);
-    }
+    for (int i = 0; i < 8; ++i) w[i] = pack_half2<FMT>(v[2 * i], v[2 * i + 1]);
     if (dst != nullptr) {
       uint4* d4 = reinterpret_cast<uint4*>(dst);
       d4[0] = make_uint4(w[0], w[1], w[2], w[3]);
@@ -249,12 +248,13 @@ __device__ __forceinline__ void epi_store16(char* dst, const float (&v)[16], uin
   }
 }
 
-template <int ESZ, int CW, int MODE, bool POOL>
+template <int FMT, int CW, int MODE, bool POOL>
 __device__ __forceinline__ void halo_epi_chunk(const ConvHaloParams& p, const uint32_t (&acc)[32], const float* s_sc,
                                                const float* s_sh, const float* s_hw, char* out_px, char* pool_px,
                                                int n, float (&hacc)[kMaxHead], int up_plane_elems, int up_row_elems,
                                                uint32_t stage, char* tr_ptr, long long tr_row_bytes, int tr_px_bytes,
                                                uint32_t tr_mask, int lane) {
+  constexpr int ESZ = fmt_esz(FMT);
   // s_sc / s_sh / s_hw already point at the first channel of this chunk; out_px at the thread's pixel (channel of
   // the chunk for CONV, channel 0 of the output pixel (2y, 2x) for UP); nullptr = masked pixel.
   // stage != 0 (CW = 32, one destination pixel per thread): the 64 / 128 bytes of every pixel go through a
@@ -311,10 +311,7 @@ __device__ __forceinline__ void halo_epi_chunk(const ConvHaloParams& p, const ui
     if (CW == 32 && stage != 0) {
       if (ESZ == 2) {
 #pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          __nv_bfloat162 b2 = __floats2bfloat162_rn(v[2 * i], v[2 * i + 1]);
-          w[i] = *reinterpret_cast<uint32_t*>(&b2);
-        }
+        for (int i = 0; i < 8; ++i) w[i] = pack_half2<FMT>(v[2 * i], v[2 * i + 1]);
         const uint32_t sw = (uint32_t)(lane >> 1) & 3u, row = stage + (uint32_t)lane * 64u;
         asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(row + (((2u * q) ^ sw) << 4)), "r"(w[0]), "r"(w[1]),
                      "r"(w[2]), "r"(w[3]) : "memory");
@@ -333,21 +330,16 @@ __device__ __forceinline__ void halo_epi_chunk(const ConvHaloParams& p, const ui
       const int nn = n + q * 16;
       const int qd = nn / p.up_cout, co = nn - qd * p.up_cout;
       const int off = (qd >> 2) * up_plane_elems + ((qd >> 1) & 1) * up_row_elems + (qd & 1) * p.out_ctot + co;
-      epi_store16<ESZ>(out_px ? out_px + (long long)off * ESZ : nullptr, v, w);
+      epi_store16<FMT>(out_px ? out_px + (long long)off * ESZ : nullptr, v, w);
     } else {
-      epi_store16<ESZ>(out_px ? out_px + q * 16 * ESZ : nullptr, v, w);
+      epi_store16<FMT>(out_px ? out_px + q * 16 * ESZ : nullptr, v, w);
     }
     if (POOL) {                                       // MaxPool2d(2) of the stored (rounded) values: x pairs are
       if (ESZ == 2) {                                 // lanes ^1, y pairs lanes ^8 (pixel = (lane >> 3, lane & 7))
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
-          __nv_bfloat162 mx = *reinterpret_cast<__nv_bfloat162*>(&w[i]);
-          uint32_t o = __shfl_xor_sync(0xffffffffu, w[i], 1);
-          mx = __hmax2(mx, *reinterpret_cast<__nv_bfloat162*>(&o));
-          const uint32_t mm = *reinterpret_cast<uint32_t*>(&mx);
-          o = __shfl_xor_sync(0xffffffffu, mm, 8);
-          mx = __hmax2(mx, *reinterpret_cast<__nv_bfloat162*>(&o));
-          w[i] = *reinterpret_cast<uint32_t*>(&mx);
+          const uint32_t mm = max_half2<FMT>(w[i], __shfl_xor_sync(0xffffffffu, w[i], 1));
+          w[i] = max_half2<FMT>(mm, __shfl_xor_sync(0xffffffffu, mm, 8));
         }
         if (pool_px != nullptr) {
           uint4* d4 = reinterpret_cast<uint4*>(pool_px + q * 16 * ESZ);
@@ -388,11 +380,12 @@ __device__ __forceinline__ void halo_epi_chunk(const ConvHaloParams& p, const ui
   }
 }
 
-template <int ESZ, int CW, int MODE, bool POOL, bool CTA2>
+template <int FMT, int CW, int MODE, bool POOL, bool CTA2>
 __device__ __forceinline__ void halo_epilogue(const ConvHaloParams& p, uint32_t tmem_base, uint32_t acc_cols,
                                               uint64_t* acc_full, uint64_t* acc_empty, const float* s_scale,
                                               const float* s_shift, const float* s_headw, uint32_t stage_base,
                                               int warp, int lane) {
+  constexpr int ESZ = fmt_esz(FMT);
   const int grp = warp & 3;                      // TMEM lane quarter
   const int egrp = (warp - 4) >> 2;              // epilogue group 0 / 1
   const int m = grp * 32 + lane;                 // accumulator row: pixel (m >> 3, m & 7) of each MMA tile
@@ -493,7 +486,7 @@ __device__ __forceinline__ void halo_epilogue(const ConvHaloParams& p, uint32_t 
           tr = tr0 + j * j_bytes + c * CW * ESZ;
         }
       }
-      halo_epi_chunk<ESZ, CW, MODE, POOL>(p, acc, sc_n0 + c * CW, sh_n0 + c * CW, s_headw + c * CW, o, po,
+      halo_epi_chunk<FMT, CW, MODE, POOL>(p, acc, sc_n0 + c * CW, sh_n0 + c * CW, s_headw + c * CW, o, po,
                                           tl.n0 + c * CW, hacc, up_plane_elems, up_row_elems, stage, tr, tr_row_bytes,
                                           tr_px_bytes, tr_mask, lane);
       if (MODE == EPI_HEAD && c == nchunks - 1) {
@@ -540,7 +533,7 @@ __device__ __forceinline__ void halo_epilogue(const ConvHaloParams& p, uint32_t 
   }
 }
 
-template <int ESZ, int KS, int MT, bool CTA2>
+template <int FMT, int KS, int MT, bool CTA2>
 __global__ void __launch_bounds__(kHaloThreads, 1) conv_halo_kernel(const __grid_constant__ CUtensorMap tmA,
                                                                     const __grid_constant__ CUtensorMap tmB,
                                                                     const ConvHaloParams p) {
@@ -688,7 +681,7 @@ __global__ void __launch_bounds__(kHaloThreads, 1) conv_halo_kernel(const __grid
     // compile-time so the MT*KS MMAs of a tap are straight-line code with immediate descriptor offsets.
     const bool issue = !BIU_DBG(p, 2);
     const uint32_t layout = rb == 128 ? 2u : (rb == 64 ? 4u : 6u);
-    const uint32_t idesc = make_idesc(ESZ == 2 ? 1u : 2u, (uint32_t)p.n_blk, CTA2 ? 256u : 128u);
+    const uint32_t idesc = make_idesc(fmt_idesc(FMT), (uint32_t)p.n_blk, CTA2 ? 256u : 128u);
     // Descriptors: only the 14-bit start-address field (address >> 4) changes between MMAs and it never carries
     // out of the field (shared memory < 256 KB).
     const uint64_t a_desc0 = make_smem_desc(smem_base, (uint32_t)pw * rb, layout);
@@ -732,15 +725,15 @@ __global__ void __launch_bounds__(kHaloThreads, 1) conv_halo_kernel(const __grid
                 for (int j = 0; j < MT; ++j)
 #pragma unroll
                   for (int k = 0; k < KS; ++k) {
-                    if (k == 0) tc_mma_imm<ESZ, 0, CTA2>(tacc + j * n_blk, ad0 + (j * j_step + 2 * k), bd0 + 2 * k, idesc);
-                    else tc_mma_imm<ESZ, 1, CTA2>(tacc + j * n_blk, ad0 + (j * j_step + 2 * k), bd0 + 2 * k, idesc);
+                    if (k == 0) tc_mma_imm<FMT, 0, CTA2>(tacc + j * n_blk, ad0 + (j * j_step + 2 * k), bd0 + 2 * k, idesc);
+                    else tc_mma_imm<FMT, 1, CTA2>(tacc + j * n_blk, ad0 + (j * j_step + 2 * k), bd0 + 2 * k, idesc);
                   }
               } else {
 #pragma unroll
                 for (int j = 0; j < MT; ++j)
 #pragma unroll
                   for (int k = 0; k < KS; ++k)
-                    tc_mma_imm<ESZ, 1, CTA2>(tacc + j * n_blk, ad0 + (j * j_step + 2 * k), bd0 + 2 * k, idesc);
+                    tc_mma_imm<FMT, 1, CTA2>(tacc + j * n_blk, ad0 + (j * j_step + 2 * k), bd0 + 2 * k, idesc);
               }
             }
             if (!p.b_resident && elect_one()) { if (CTA2) tc_commit2(&b_empty[bs]); else tc_commit(&b_empty[bs]); }
@@ -757,7 +750,7 @@ __global__ void __launch_bounds__(kHaloThreads, 1) conv_halo_kernel(const __grid
   } else if (warp >= 4) {
     // ======================================= epilogue =======================================
 #define BIU_EPI(CW, MODE, POOL) \
-    halo_epilogue<ESZ, CW, MODE, POOL, CTA2>(p, tmem_base, acc_cols, acc_full, acc_empty, s_scale, s_shift, s_headw, stage_base, warp, lane)
+    halo_epilogue<FMT, CW, MODE, POOL, CTA2>(p, tmem_base, acc_cols, acc_full, acc_empty, s_scale, s_shift, s_headw, stage_base, warp, lane)
     if (p.n_blk % 32 == 0) {
       if (p.mode == EPI_CONV) { if (p.pool_out != nullptr) BIU_EPI(32, EPI_CONV, true); else BIU_EPI(32, EPI_CONV, false); }
       else if (p.mode == EPI_UP) BIU_EPI(32, EPI_UP, false);
@@ -776,10 +769,13 @@ __global__ void __launch_bounds__(kHaloThreads, 1) conv_halo_kernel(const __grid
   if (warp == 1) { if (CTA2) tmem_dealloc2(tmem_base, ncols); else tmem_dealloc(tmem_base, ncols); }
 }
 
-// Host-side dispatch over the (k-steps per chunk, MMA tiles per work item) instantiations of one element size;
-// defined in conv_halo_bf16.cu / conv_halo_tf32.cu through BIU_DEFINE_HALO_DISPATCH so the two compile in parallel.
+// Host-side dispatch over the (k-steps per chunk, MMA tiles per work item) instantiations of one element format;
+// defined in conv_halo_bf16.cu / conv_halo_f16.cu / conv_halo_tf32.cu through BIU_DEFINE_HALO_DISPATCH so they compile in
+// parallel.
 int halo_dispatch_bf16(const CUtensorMap& tmA, const CUtensorMap& tmB, const ConvHaloParams& p, int grid, int smem,
                        cudaStream_t stream);
+int halo_dispatch_f16(const CUtensorMap& tmA, const CUtensorMap& tmB, const ConvHaloParams& p, int grid, int smem,
+                      cudaStream_t stream);
 int halo_dispatch_tf32(const CUtensorMap& tmA, const CUtensorMap& tmB, const ConvHaloParams& p, int grid, int smem,
                        cudaStream_t stream);
 
@@ -826,6 +822,7 @@ int halo_dispatch_tf32(const CUtensorMap& tmA, const CUtensorMap& tmB, const Con
 // Co-resident CTA pairs of the 2-CTA kernel with `smem` bytes of dynamic shared memory (0: no cluster launch possible).
 // The kernel is persistent with a static tile stride, so its grid must not exceed what is resident at once.
 int halo_max_pairs_bf16(int ks, int mt, int smem);
+int halo_max_pairs_f16(int ks, int mt, int smem);
 int halo_max_pairs_tf32(int ks, int mt, int smem);
 
 #define BIU_HALO_PAIRS(E, K, M)                                                                                    \

@@ -1,4 +1,4 @@
-// Row-streaming 3x3(x3) convolution for NARROW layers (Cout <= 32; 2D bf16 also Cout = 64) on tcgen05: the dy taps
+// Row-streaming 3x3(x3) convolution for NARROW layers (Cout <= 32; 2D bf16 / fp16 also Cout = 64) on tcgen05: the dy taps
 // are folded into N.
 //
 // Why: with M = 128 the tensor core fetches its operands from shared memory at ~85 B/clk (measured,
@@ -76,8 +76,8 @@ struct ConvRowsParams {
   int acc_mode;
   float* acc_scratch;
   // FIRST mode (first block of the 2D nets, one uint8 input channel): the three dx taps are the K dimension. An A-ring row
-  // is one pixel's {in[x-1], in[x], in[x+1], 0...} (32 bytes: bf16 K = 16 / tf32 K = 8) and is WRITTEN BY THE PRODUCER
-  // WARP itself from the planar uint8 tile (integers 0..255 are exact in bf16 / tf32; the 1/255 of unet/predict.py:192 is
+  // is one pixel's {in[x-1], in[x], in[x+1], 0...} (32 bytes: bf16 / fp16 K = 16, tf32 K = 8) and is WRITTEN BY THE
+  // PRODUCER WARP itself from the planar uint8 tile (integers 0..255 are exact in all three; the 1/255 of unet/predict.py:192 is
   // folded into the fp32 scale), so one MMA of N = 3 * Cout per input row does the whole block: w_taps = 1.
   int first;
   const uint8_t* first_in;       // [B][H][W] uint8
@@ -249,10 +249,11 @@ __device__ __forceinline__ RowsItem rows_decode(const ConvRowsParams& p, int t) 
 }
 
 // Epilogue of all work items for one warp. CP = padded output channels (all of them are handled by this warp).
-template <int ESZ, int CP, int MODE, bool POOL, int SBW = 64>
+template <int FMT, int CP, int MODE, bool POOL, int SBW = 64>
 __device__ __forceinline__ void rows_epilogue(const ConvRowsParams& p, uint32_t tmem_base, uint64_t* t_full,
                                               uint64_t* t_empty, const float* s_scale, const float* s_shift,
                                               const float* s_headw, uint8_t* stage, int warp, int lane) {
+  constexpr int ESZ = fmt_esz(FMT);
   constexpr int PXB = CP * ESZ;                  // bytes of one output pixel
   constexpr int HC = CP > 32 ? 32 : CP;          // TMEM columns per drain (64-channel rows are drained in two halves)
   constexpr int NH = CP / HC;
@@ -355,7 +356,7 @@ __device__ __forceinline__ void rows_epilogue(const ConvRowsParams& p, uint32_t 
     const int vrows = it.rows + 4;               // virtual output rows: 2 dummies, rows real ones, 2 dummies
 
     const unsigned long long slope2 = pack_f32x2(p.slope, p.slope);
-    // BatchNorm + LeakyReLU of one drained row, packed in the storage format (bf16 pairs / tf32-rounded floats)
+    // BatchNorm + LeakyReLU of one drained row, packed in the storage format (bf16 / fp16 pairs, tf32-rounded floats)
     auto activate = [&](const uint32_t (&e)[HC], uint32_t (&w)[NW], int hh) {     // channels hh * HC .. hh * HC + HC - 1
       constexpr int NWH = HC * ESZ / 4;
 #pragma unroll
@@ -373,9 +374,8 @@ __device__ __forceinline__ void rows_epilogue(const ConvRowsParams& p, uint32_t 
 #pragma unroll
         for (int k = 0; k < 4; ++k) a[k] = fmaxf(a[k], u[k]);        // LeakyReLU for 0 <= slope <= 1
         if (ESZ == 2) {
-          __nv_bfloat162 b0 = __floats2bfloat162_rn(a[0], a[1]), b1 = __floats2bfloat162_rn(a[2], a[3]);
-          w[(hh * NWH + 2 * i4) % NW] = *reinterpret_cast<uint32_t*>(&b0);
-          w[(hh * NWH + 2 * i4 + 1) % NW] = *reinterpret_cast<uint32_t*>(&b1);
+          w[(hh * NWH + 2 * i4) % NW] = pack_half2<FMT>(a[0], a[1]);
+          w[(hh * NWH + 2 * i4 + 1) % NW] = pack_half2<FMT>(a[2], a[3]);
         } else {
 #pragma unroll
           for (int k = 0; k < 4; ++k) w[(hh * NWH + 4 * i4 + k) % NW] = __float_as_uint(round_tf32(a[k]));
@@ -518,16 +518,10 @@ __device__ __forceinline__ void rows_epilogue(const ConvRowsParams& p, uint32_t 
           if (ESZ == 2) {                          // (plane mode, MaxPool3d(2): the pair is a z pair, y pairs are lanes ^ 8)
 #pragma unroll
             for (int i = 0; i < NW; ++i) {
-              __nv_bfloat162 mx = __hmax2(*reinterpret_cast<__nv_bfloat162*>(&w0[i]), *reinterpret_cast<__nv_bfloat162*>(&w1[i]));
-              uint32_t mine = *reinterpret_cast<uint32_t*>(&mx);
-              uint32_t ot = __shfl_xor_sync(0xffffffffu, mine, 1);
-              mx = __hmax2(mx, *reinterpret_cast<const __nv_bfloat162*>(&ot));
-              if (plane) {
-                mine = *reinterpret_cast<uint32_t*>(&mx);
-                ot = __shfl_xor_sync(0xffffffffu, mine, 8);
-                mx = __hmax2(mx, *reinterpret_cast<const __nv_bfloat162*>(&ot));
-              }
-              w0[i] = *reinterpret_cast<uint32_t*>(&mx);
+              uint32_t mx = max_half2<FMT>(w0[i], w1[i]);
+              mx = max_half2<FMT>(mx, __shfl_xor_sync(0xffffffffu, mx, 1));
+              if (plane) mx = max_half2<FMT>(mx, __shfl_xor_sync(0xffffffffu, mx, 8));
+              w0[i] = mx;
             }
           } else {
 #pragma unroll
@@ -551,10 +545,11 @@ __device__ __forceinline__ void rows_epilogue(const ConvRowsParams& p, uint32_t 
   }
 }
 
-template <int ESZ, int KS>
+template <int FMT, int KS>
 __global__ void __launch_bounds__(kRowsThreads, 1) conv_rows_kernel(const __grid_constant__ CUtensorMap tmA,
                                                                     const __grid_constant__ CUtensorMap tmW,
                                                                     const ConvRowsParams p) {
+  constexpr int ESZ = fmt_esz(FMT);
   extern __shared__ uint8_t smem_raw[];
   __shared__ uint64_t a_full[kRowsMaxASlots], a_empty[kRowsMaxASlots];
   __shared__ uint64_t t_full[kRowsMaxTSlots], t_empty[kRowsMaxTSlots];
@@ -661,8 +656,7 @@ __global__ void __launch_bounds__(kRowsThreads, 1) conv_rows_kernel(const __grid
           const int r = 4 * lane + j;                             // 32B swizzle: 16-byte chunk ^ ((r >> 2) & 1)
           uint8_t* row = slot + r * 32 + (((r >> 2) & 1) << 4);
           if (ESZ == 2) {
-            __nv_bfloat162 lo = __floats2bfloat162_rn(v[j], v[j + 1]), hi = __floats2bfloat162_rn(v[j + 2], 0.f);
-            *reinterpret_cast<uint2*>(row) = make_uint2(*reinterpret_cast<uint32_t*>(&lo), *reinterpret_cast<uint32_t*>(&hi));
+            *reinterpret_cast<uint2*>(row) = make_uint2(pack_half2<FMT>(v[j], v[j + 1]), pack_half2<FMT>(v[j + 2], 0.f));
           } else {
             *reinterpret_cast<float4*>(row) = make_float4(v[j], v[j + 1], v[j + 2], 0.f);
           }
@@ -732,7 +726,7 @@ __global__ void __launch_bounds__(kRowsThreads, 1) conv_rows_kernel(const __grid
     // ====================================== MMA issuer ======================================
     const int pipe = warp >> 1;
     const uint32_t layout = rb == 128 ? 2u : (rb == 64 ? 4u : 6u);
-    const uint32_t fmt = ESZ == 2 ? 1u : 2u;
+    const uint32_t fmt = fmt_idesc(FMT);
     const uint32_t idesc3 = make_idesc(fmt, (uint32_t)(3 * p.cp));      // whole folded tile
     const uint32_t idesc2 = make_idesc(fmt, (uint32_t)(2 * p.cp));      // split MMAs where the three slots wrap
     const uint32_t idesc1 = make_idesc(fmt, (uint32_t)p.cp);
@@ -824,20 +818,20 @@ __global__ void __launch_bounds__(kRowsThreads, 1) conv_rows_kernel(const __grid
                       const uint64_t ad = ad0 + ((dy * 10 + dx) * px_step + 2 * k);
                       const uint64_t wd = wd0 + ((dy * 3 + dx) * wdx_step + 2 * k);
                       if (wrap <= 0) {
-                        tc_mma_imm<ESZ, 1>(tcol, ad, wd, idesc3);
+                        tc_mma_imm<FMT, 1>(tcol, ad, wd, idesc3);
                       } else {
-                        tc_mma_imm<ESZ, 1>(tcol, ad, wd, n_lo);
-                        tc_mma_imm<ESZ, 1>(tmem_pipe, ad, wd + w_hi, n_hi);
+                        tc_mma_imm<FMT, 1>(tcol, ad, wd, n_lo);
+                        tc_mma_imm<FMT, 1>(tmem_pipe, ad, wd + w_hi, n_hi);
                       }
                     }
               }
             } else if (p.first) {
               if (!dbg_nomma && elect_one()) {                     // dx is the K dimension: one MMA per input row
                 if (wrap <= 0) {
-                  tc_mma_imm<ESZ, 1>(tcol, ad0, wd0, idesc3);
+                  tc_mma_imm<FMT, 1>(tcol, ad0, wd0, idesc3);
                 } else {
-                  tc_mma_imm<ESZ, 1>(tcol, ad0, wd0, wrap == 1 ? idesc2 : idesc1);
-                  tc_mma_imm<ESZ, 1>(tmem_pipe, ad0, wd0 + (uint32_t)(3 - wrap) * wrow_step, wrap == 1 ? idesc1 : idesc2);
+                  tc_mma_imm<FMT, 1>(tcol, ad0, wd0, wrap == 1 ? idesc2 : idesc1);
+                  tc_mma_imm<FMT, 1>(tmem_pipe, ad0, wd0 + (uint32_t)(3 - wrap) * wrow_step, wrap == 1 ? idesc1 : idesc2);
                 }
               }
             } else if (!dbg_nomma && elect_one()) {
@@ -846,7 +840,7 @@ __global__ void __launch_bounds__(kRowsThreads, 1) conv_rows_kernel(const __grid
                 for (int dx = 0; dx < 3; ++dx)
 #pragma unroll
                   for (int k = 0; k < KS; ++k)
-                    tc_mma_imm<ESZ, 1>(tcol, ad0 + (dx * px_step + 2 * k), wd0 + (dx * wdx_step + 2 * k), idesc3);
+                    tc_mma_imm<FMT, 1>(tcol, ad0 + (dx * px_step + 2 * k), wd0 + (dx * wdx_step + 2 * k), idesc3);
               } else {
                 const uint32_t n_lo = wrap == 1 ? idesc2 : idesc1;        // slots before the wrap
                 const uint32_t n_hi = wrap == 1 ? idesc1 : idesc2;        // slots continuing at slot 0
@@ -855,8 +849,8 @@ __global__ void __launch_bounds__(kRowsThreads, 1) conv_rows_kernel(const __grid
                 for (int dx = 0; dx < 3; ++dx)
 #pragma unroll
                   for (int k = 0; k < KS; ++k) {
-                    tc_mma_imm<ESZ, 1>(tcol, ad0 + (dx * px_step + 2 * k), wd0 + (dx * wdx_step + 2 * k), n_lo);
-                    tc_mma_imm<ESZ, 1>(tmem_pipe, ad0 + (dx * px_step + 2 * k), wd0 + (w_hi + dx * wdx_step + 2 * k), n_hi);
+                    tc_mma_imm<FMT, 1>(tcol, ad0 + (dx * px_step + 2 * k), wd0 + (dx * wdx_step + 2 * k), n_lo);
+                    tc_mma_imm<FMT, 1>(tmem_pipe, ad0 + (dx * px_step + 2 * k), wd0 + (w_hi + dx * wdx_step + 2 * k), n_hi);
                   }
               }
             }
@@ -874,11 +868,11 @@ __global__ void __launch_bounds__(kRowsThreads, 1) conv_rows_kernel(const __grid
   } else if (warp >= 4) {
     // ======================================= epilogue =======================================
 #define BIU_REPI(CP, MODE, POOL) \
-    rows_epilogue<ESZ, CP, MODE, POOL>(p, tmem_base, t_full, t_empty, s_scale, s_shift, s_headw, stage, warp, lane)
-    if (p.cp == 64) {                                  // plan_rows: bf16, 2D, EPI_CONV only
+    rows_epilogue<FMT, CP, MODE, POOL>(p, tmem_base, t_full, t_empty, s_scale, s_shift, s_headw, stage, warp, lane)
+    if (p.cp == 64) {                                  // plan_rows: 2-byte formats, 2D, EPI_CONV only
       if (ESZ == 2) {
 #define BIU_REPI64(POOL, SBW) \
-        rows_epilogue<ESZ, 64, EPI_CONV, POOL, SBW>(p, tmem_base, t_full, t_empty, s_scale, s_shift, s_headw, stage, warp, lane)
+        rows_epilogue<FMT, 64, EPI_CONV, POOL, SBW>(p, tmem_base, t_full, t_empty, s_scale, s_shift, s_headw, stage, warp, lane)
         if (p.stage_px == 32) { if (p.pool_out != nullptr) BIU_REPI64(true, 32); else BIU_REPI64(false, 32); }
         else { if (p.pool_out != nullptr) BIU_REPI64(true, 64); else BIU_REPI64(false, 64); }
 #undef BIU_REPI64
@@ -902,6 +896,8 @@ __global__ void __launch_bounds__(kRowsThreads, 1) conv_rows_kernel(const __grid
 
 int rows_dispatch_bf16(const CUtensorMap& tmA, const CUtensorMap& tmW, const ConvRowsParams& p, int grid, int smem,
                        cudaStream_t stream);
+int rows_dispatch_f16(const CUtensorMap& tmA, const CUtensorMap& tmW, const ConvRowsParams& p, int grid, int smem,
+                      cudaStream_t stream);
 int rows_dispatch_tf32(const CUtensorMap& tmA, const CUtensorMap& tmW, const ConvRowsParams& p, int grid, int smem,
                        cudaStream_t stream);
 

@@ -47,7 +47,11 @@ void choose_box(int W, int H, int D, int B, int* lbw, int* lbh, int* lbd, int* l
   *lbw = lw; *lbh = lh; *lbd = ld; *lbb = lb;
 }
 
-static int encode_act_map(CUtensorMap* tm, const void* base, int esz, int C, int W, int H, int D, int B, int ctot,
+static CUtensorMapDataType tma_dtype(int esz, int f16) {
+  return esz == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : (f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16);
+}
+
+static int encode_act_map(CUtensorMap* tm, const void* base, int esz, int f16, int C, int W, int H, int D, int B, int ctot,
                           int ck, int bw, int bh, int bd, int bb) {
   EncodeTiledFn enc = get_encode_fn();
   BIU_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled entry point not available");
@@ -59,7 +63,7 @@ static int encode_act_map(CUtensorMap* tm, const void* base, int esz, int C, int
   const int rb = ck * esz;
   CUtensorMapSwizzle sw = rb == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
                                     : (rb == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
-  CUresult r = enc(tm, esz == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5,
+  CUresult r = enc(tm, tma_dtype(esz, f16), 5,
                    const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   BIU_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled(activations) failed with %d (C=%d W=%d H=%d D=%d B=%d ctot=%d ck=%d)",
@@ -67,7 +71,7 @@ static int encode_act_map(CUtensorMap* tm, const void* base, int esz, int C, int
   return 0;
 }
 
-static int encode_wgt_map(CUtensorMap* tm, const void* base, int esz, int cin, int ntotal, int taps, int ck,
+static int encode_wgt_map(CUtensorMap* tm, const void* base, int esz, int f16, int cin, int ntotal, int taps, int ck,
                           int n_blk) {
   EncodeTiledFn enc = get_encode_fn();
   BIU_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled entry point not available");
@@ -78,7 +82,7 @@ static int encode_wgt_map(CUtensorMap* tm, const void* base, int esz, int cin, i
   const int rb = ck * esz;
   CUtensorMapSwizzle sw = rb == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
                                     : (rb == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
-  CUresult r = enc(tm, esz == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3,
+  CUresult r = enc(tm, tma_dtype(esz, f16), 3,
                    const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   BIU_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled(weights) failed with %d (cin=%d n=%d taps=%d ck=%d nblk=%d)",
@@ -95,6 +99,7 @@ int pick_ck(int cin, int esz) {
 
 bool conv_tc_supported(const ConvTcArgs& a) {
   if (a.esz != 2 && a.esz != 4) return false;
+  if (a.f16 && a.esz != 2) return false;
   if (pick_ck(a.cin, a.esz) == 0) return false;
   if (a.n_total % 16 != 0) return false;
   if (a.in_ctot % (16 / a.esz) != 0 || a.in_coff % (16 / a.esz) != 0) return false;
@@ -225,12 +230,13 @@ static bool halo_try_cta2(const ConvTcArgs& a, int n_blk, HaloPlan* out, int* pa
   if (!pl.ok) return false;
   const long long per_block = (long long)ceil_div(a.W, 8 * pl.mt) * ceil_div(a.H, 16) * a.D * a.B;
   if (per_block < 2 || (per_block & 1)) return false;
-  static int cache[2][3][4];                               // [esz][ks index][mt index] -> pairs + 1 for the largest smem seen
-  static int cache_smem[2][3][4];
+  static int cache[3][3][4];                               // [format][ks index][mt index] -> pairs + 1 for the largest smem seen
+  static int cache_smem[3][3][4];
   const int ks = pl.ck * a.esz / 32, ki = ks == 4 ? 2 : (ks == 2 ? 1 : 0), mi = pl.mt == 8 ? 3 : (pl.mt == 4 ? 2 : (pl.mt == 2 ? 1 : 0));
-  const int ei = a.esz == 2 ? 0 : 1;
+  const int ei = a.esz == 4 ? 2 : (a.f16 ? 1 : 0);
   if (cache[ei][ki][mi] == 0 || cache_smem[ei][ki][mi] < pl.smem) {
-    const int n = a.esz == 2 ? halo_max_pairs_bf16(ks, pl.mt, pl.smem) : halo_max_pairs_tf32(ks, pl.mt, pl.smem);
+    const int n = a.esz == 4 ? halo_max_pairs_tf32(ks, pl.mt, pl.smem)
+                             : (a.f16 ? halo_max_pairs_f16(ks, pl.mt, pl.smem) : halo_max_pairs_bf16(ks, pl.mt, pl.smem));
     cache[ei][ki][mi] = n + 1;
     cache_smem[ei][ki][mi] = pl.smem;
   }
@@ -272,9 +278,9 @@ static int launch_conv_halo(const ConvTcArgs& a, int n_blk, const HaloPlan& pl, 
 
   CUtensorMap tmA, tmB;
   const char* in_base = reinterpret_cast<const char*>(a.in) + (size_t)a.in_coff * a.esz;
-  if (int rc = encode_act_map(&tmA, in_base, a.esz, a.cin, a.W, a.H, a.D, a.B, a.in_ctot, pl.ck, 8 * pl.mt + 2 * p.halo, 2, 1, 1))
+  if (int rc = encode_act_map(&tmA, in_base, a.esz, a.f16, a.cin, a.W, a.H, a.D, a.B, a.in_ctot, pl.ck, 8 * pl.mt + 2 * p.halo, 2, 1, 1))
     return rc;
-  if (int rc = encode_wgt_map(&tmB, a.wgt, a.esz, a.cin, a.n_total, p.halo ? 9 * a.kd : 1, pl.ck, pl.cta2 ? n_blk / 2 : n_blk))
+  if (int rc = encode_wgt_map(&tmB, a.wgt, a.esz, a.f16, a.cin, a.n_total, p.halo ? 9 * a.kd : 1, pl.ck, pl.cta2 ? n_blk / 2 : n_blk))
     return rc;
   int grid = p.total_tiles < sm_count() ? p.total_tiles : sm_count();
   if (pl.cta2) {                                           // whole pairs, all of them resident at once
@@ -284,9 +290,10 @@ static int launch_conv_halo(const ConvTcArgs& a, int n_blk, const HaloPlan& pl, 
     grid = 2 * pairs;
   }
   BIU_REQUIRE(pl.mt == 1 || pl.mt == 2 || pl.mt == 4 || pl.mt == 8, "halo kernel: mt must be 1, 2, 4 or 8 (got %d)", pl.mt);
-  // the kernel instantiations live in their own translation units (conv_halo_bf16.cu / conv_halo_tf32.cu)
-  if (int rc = a.esz == 2 ? halo_dispatch_bf16(tmA, tmB, p, grid, pl.smem, stream)
-                          : halo_dispatch_tf32(tmA, tmB, p, grid, pl.smem, stream))
+  // the kernel instantiations live in their own translation units (conv_halo_bf16.cu / _f16.cu / _tf32.cu)
+  if (int rc = a.esz == 4 ? halo_dispatch_tf32(tmA, tmB, p, grid, pl.smem, stream)
+                          : (a.f16 ? halo_dispatch_f16(tmA, tmB, p, grid, pl.smem, stream)
+                                   : halo_dispatch_bf16(tmA, tmB, p, grid, pl.smem, stream)))
     return rc;
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
@@ -324,7 +331,7 @@ static RowsPlan plan_rows(const ConvTcArgs& a) {
   if (rows_disabled() || halo_disabled() || a.wgt_fold == nullptr) return pl;
   if (a.mode != EPI_CONV && a.mode != EPI_HEAD) return pl;
   if (a.kw != 3 || a.kh != 3 || (a.kd != 1 && a.kd != 3)) return pl;
-  // N of the folded MMA = 3 * Cout = 48 or 96; 192 (Cout = 64) for 2D bf16 blocks: 8 TMEM slots, one pipeline
+  // N of the folded MMA = 3 * Cout = 48 or 96; 192 (Cout = 64) for 2D bf16 / fp16 blocks: 8 TMEM slots, one pipeline
   const bool wide = a.n_total == 64 && a.esz == 2 && a.kd == 1 && a.mode == EPI_CONV && !rows_no_wide();
   if (a.n_total != 16 && a.n_total != 32 && !wide) return pl;
   if (a.W < 128) return pl;                                  // one MMA tile = 128 consecutive pixels of a row
@@ -405,14 +412,15 @@ static int launch_conv_rows(const ConvTcArgs& a, const RowsPlan& pl, cudaStream_
   p.out_val = a.out_val; p.out_u8 = a.out_u8;
   CUtensorMap tmA, tmW;
   const char* in_base = reinterpret_cast<const char*>(a.in) + (size_t)a.in_coff * a.esz;
-  if (int rc = pl.plane ? encode_act_map(&tmA, in_base, a.esz, a.cin, a.W, a.H, a.D, a.B, a.in_ctot, pl.ck, 10, 18, 1, 1)
-                        : encode_act_map(&tmA, in_base, a.esz, a.cin, a.W, a.H, a.D, a.B, a.in_ctot, pl.ck, kRowsPx, 1, 1, 1))
+  if (int rc = pl.plane ? encode_act_map(&tmA, in_base, a.esz, a.f16, a.cin, a.W, a.H, a.D, a.B, a.in_ctot, pl.ck, 10, 18, 1, 1)
+                        : encode_act_map(&tmA, in_base, a.esz, a.f16, a.cin, a.W, a.H, a.D, a.B, a.in_ctot, pl.ck, kRowsPx, 1, 1, 1))
     return rc;
-  if (int rc = encode_wgt_map(&tmW, pl.plane ? a.wgt_fold_z : a.wgt_fold, a.esz, a.cin, 3 * a.n_total, a.kd * 3, pl.ck, 3 * a.n_total))
+  if (int rc = encode_wgt_map(&tmW, pl.plane ? a.wgt_fold_z : a.wgt_fold, a.esz, a.f16, a.cin, 3 * a.n_total, a.kd * 3, pl.ck, 3 * a.n_total))
     return rc;
   const int grid = p.total_items < sm_count_cached() ? p.total_items : sm_count_cached();
-  if (int rc = a.esz == 2 ? rows_dispatch_bf16(tmA, tmW, p, grid, pl.smem, stream)
-                          : rows_dispatch_tf32(tmA, tmW, p, grid, pl.smem, stream))
+  if (int rc = a.esz == 4 ? rows_dispatch_tf32(tmA, tmW, p, grid, pl.smem, stream)
+                          : (a.f16 ? rows_dispatch_f16(tmA, tmW, p, grid, pl.smem, stream)
+                                   : rows_dispatch_bf16(tmA, tmW, p, grid, pl.smem, stream)))
     return rc;
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
@@ -430,7 +438,8 @@ static bool first_rows_enabled() {
 }
 bool conv_first_rows_supported(const FirstRowsArgs& a) {
   if (!first_rows_enabled() || rows_disabled() || halo_disabled()) return false;
-  if (a.wgt == nullptr || (a.n_total != 16 && a.n_total != 32) || (a.esz != 2 && a.esz != 4)) return false;
+  if (a.wgt == nullptr || (a.n_total != 16 && a.n_total != 32) || (a.esz != 2 && a.esz != 4) || (a.f16 && a.esz != 2))
+    return false;
   return a.W >= 128 && a.H >= 1 && a.out_ctot % 8 == 0 && a.out_coff % 8 == 0;
 }
 int launch_conv_first_rows(const FirstRowsArgs& a, cudaStream_t stream) {
@@ -462,10 +471,11 @@ int launch_conv_first_rows(const FirstRowsArgs& a, cudaStream_t stream) {
   p.mode = EPI_CONV; p.slope = a.slope; p.scale = a.scale; p.shift = a.shift;
   p.out = a.out; p.out_ctot = a.out_ctot; p.out_coff = a.out_coff;
   CUtensorMap tmW;
-  if (int rc = encode_wgt_map(&tmW, a.wgt, a.esz, p.ck, nfold, 1, p.ck, nfold)) return rc;
+  if (int rc = encode_wgt_map(&tmW, a.wgt, a.esz, a.f16, p.ck, nfold, 1, p.ck, nfold)) return rc;
   const int grid = p.total_items < sm_count_cached() ? p.total_items : sm_count_cached();
-  if (int rc = a.esz == 2 ? rows_dispatch_bf16(tmW, tmW, p, grid, smem, stream)        // no activation map: the rows are
-                          : rows_dispatch_tf32(tmW, tmW, p, grid, smem, stream))       // built in the kernel
+  if (int rc = a.esz == 4 ? rows_dispatch_tf32(tmW, tmW, p, grid, smem, stream)        // no activation map: the rows are
+                          : (a.f16 ? rows_dispatch_f16(tmW, tmW, p, grid, smem, stream)  // built in the kernel
+                                   : rows_dispatch_bf16(tmW, tmW, p, grid, smem, stream)))
     return rc;
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
@@ -651,13 +661,20 @@ int launch_conv_tc(const ConvTcArgs& a, cudaStream_t stream) {
 
   CUtensorMap tmA, tmB;
   const char* in_base = reinterpret_cast<const char*>(a.in) + (size_t)a.in_coff * a.esz;
-  if (int rc = encode_act_map(&tmA, in_base, a.esz, a.cin, a.W, a.H, a.D, a.B, a.in_ctot, p.ck, 1 << p.lbw,
+  if (int rc = encode_act_map(&tmA, in_base, a.esz, a.f16, a.cin, a.W, a.H, a.D, a.B, a.in_ctot, p.ck, 1 << p.lbw,
                               1 << p.lbh, 1 << p.lbd, 1 << p.lbb))
     return rc;
-  if (int rc = encode_wgt_map(&tmB, a.wgt, a.esz, a.cin, a.n_total, a.kw * a.kh * a.kd, p.ck, n_blk)) return rc;
+  if (int rc = encode_wgt_map(&tmB, a.wgt, a.esz, a.f16, a.cin, a.n_total, a.kw * a.kh * a.kd, p.ck, n_blk)) return rc;
 
   dim3 grid(p.tiles_w * p.tiles_h * p.tiles_d * p.tiles_b, a.n_total / n_blk);
-  if (a.esz == 2) {
+  if (a.esz == 2 && a.f16) {
+    static int max_set = 0;
+    if (smem > max_set) {
+      BIU_CHECK_CUDA(cudaFuncSetAttribute(conv_tc_kernel<FMT_F16>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+      max_set = smem;
+    }
+    conv_tc_kernel<FMT_F16><<<grid, 192, smem, stream>>>(tmA, tmB, p);
+  } else if (a.esz == 2) {
     static int max_set = 0;
     if (smem > max_set) {
       BIU_CHECK_CUDA(cudaFuncSetAttribute(conv_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));

@@ -35,7 +35,7 @@ struct ConvTcParams {
   float slope;
   const float* scale;                        // [n_total]
   const float* shift;                        // [n_total]
-  void* out;                                 // NHWC destination (bf16 or fp32); may be null in EPI_HEAD
+  void* out;                                 // NHWC destination (bf16 / fp16 or fp32); may be null in EPI_HEAD
   int out_ctot, out_coff;
   int up_cout, up_dims;                      // EPI_UP
   int head_n;                                // EPI_HEAD
@@ -61,10 +61,11 @@ __device__ __forceinline__ float round_tf32(float v) {
   return __uint_as_float(u);
 }
 
-template <int ESZ>
+template <int FMT>
 __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CUtensorMap tmA,
                                                       const __grid_constant__ CUtensorMap tmB,
                                                       const ConvTcParams p) {
+  constexpr int ESZ = fmt_esz(FMT);
   extern __shared__ uint8_t smem_raw[];
   __shared__ uint64_t full_bar[kMaxStages];
   __shared__ uint64_t empty_bar[kMaxStages];
@@ -150,7 +151,7 @@ __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CU
     if (elect_one()) {
       const uint32_t layout = p.row_bytes == 128 ? 2u : (p.row_bytes == 64 ? 4u : 6u);
       const uint32_t sbo = 8u * p.row_bytes;
-      const uint32_t idesc = make_idesc(ESZ == 2 ? 1u : 2u, (uint32_t)p.n_blk);
+      const uint32_t idesc = make_idesc(fmt_idesc(FMT), (uint32_t)p.n_blk);
       const int ksteps = p.row_bytes / 32;
       for (int kb = 0; kb < num_kb; ++kb) {
         const int s = kb % p.stages;
@@ -230,11 +231,8 @@ __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CU
         if (ESZ == 2) {
           uint32_t w[8];
 #pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            __nv_bfloat162 b2 = __floats2bfloat162_rn(v[2 * i], v[2 * i + 1]);
-            w[i] = *reinterpret_cast<uint32_t*>(&b2);
-          }
-          uint4* dst = reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(p.out) + off);
+          for (int i = 0; i < 8; ++i) w[i] = pack_half2<FMT>(v[2 * i], v[2 * i + 1]);
+          uint4* dst = reinterpret_cast<uint4*>(reinterpret_cast<uint16_t*>(p.out) + off);
           dst[0] = make_uint4(w[0], w[1], w[2], w[3]);
           dst[1] = make_uint4(w[4], w[5], w[6], w[7]);
         } else {

@@ -4,13 +4,20 @@
 #include "common.cuh"
 #include "launch.h"
 
+#include <type_traits>
+
 namespace biu {
+
+// element format of an activation storage type
+template <typename T>
+constexpr int fmt_of = sizeof(T) == 4 ? FMT_TF32 : (std::is_same<T, __half>::value ? FMT_F16 : FMT_BF16);
 
 template <typename T> __device__ __forceinline__ float ld_act(const T* p);
 template <> __device__ __forceinline__ float ld_act<float>(const float* p) { return __ldg(p); }
 template <> __device__ __forceinline__ float ld_act<__nv_bfloat16>(const __nv_bfloat16* p) {
   return __bfloat162float(*p);
 }
+template <> __device__ __forceinline__ float ld_act<__half>(const __half* p) { return __half2float(*p); }
 __device__ __forceinline__ float to_tf32(float v) {
   uint32_t u;
   asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(u) : "f"(v));
@@ -23,11 +30,12 @@ template <> __device__ __forceinline__ void st_act<float>(float* p, float v, int
 template <> __device__ __forceinline__ void st_act<__nv_bfloat16>(__nv_bfloat16* p, float v, int) {
   *p = __float2bfloat16_rn(v);
 }
+template <> __device__ __forceinline__ void st_act<__half>(__half* p, float v, int) { *p = __float2half_rn(v); }
 
 // ------------------------------------------------------------------------------------------------
 // First block: Conv(k=3,pad=1) on a planar few-channel input + folded BN + LeakyReLU (unet/unet.py:20,54-60;
 // unet3d/unet3d.py:24). u8 tiles are converted as float32(u8)/255 (unet/predict.py:192). One thread per
-// (pixel, 8 output channels): 16-byte bf16 stores; weights staged in shared memory.
+// (pixel, 8 output channels): 16-byte bf16 / fp16 stores; weights staged in shared memory.
 // ------------------------------------------------------------------------------------------------
 template <typename TIN, typename TOUT>
 __global__ void __launch_bounds__(256) first_conv_kernel(FirstConvArgs a) {
@@ -157,10 +165,7 @@ __global__ void __launch_bounds__(256) first_conv1_kernel(FirstConvArgs a) {
       if (sizeof(TOUT) == 2) {
         uint32_t w[4];
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          __nv_bfloat162 b2 = __floats2bfloat162_rn(acc[2 * j], acc[2 * j + 1]);
-          w[j] = *reinterpret_cast<uint32_t*>(&b2);
-        }
+        for (int j = 0; j < 4; ++j) w[j] = pack_half2<fmt_of<TOUT>>(acc[2 * j], acc[2 * j + 1]);
         *reinterpret_cast<uint4*>(o + g) = make_uint4(w[0], w[1], w[2], w[3]);
       } else {
         float* of = reinterpret_cast<float*>(o + g);
@@ -343,10 +348,7 @@ __global__ void __launch_bounds__(256, 2) first_conv1_3d_kernel(FirstConvArgs a)
             if (sizeof(TOUT) == 2) {
               uint32_t w[4];
 #pragma unroll
-              for (int j = 0; j < 4; ++j) {
-                __nv_bfloat162 b2 = __floats2bfloat162_rn(res[xi][2 * j], res[xi][2 * j + 1]);
-                w[j] = *reinterpret_cast<uint32_t*>(&b2);
-              }
+              for (int j = 0; j < 4; ++j) w[j] = pack_half2<fmt_of<TOUT>>(res[xi][2 * j], res[xi][2 * j + 1]);
               *reinterpret_cast<uint4*>(ov) = make_uint4(w[0], w[1], w[2], w[3]);
             } else {
               float* of = reinterpret_cast<float*>(ov);
@@ -466,10 +468,7 @@ __global__ void __launch_bounds__(256, 2) first_conv1_2d_kernel(FirstConvArgs a)
         if (sizeof(TOUT) == 2) {
           uint32_t pk[4];
 #pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            __nv_bfloat162 b2 = __floats2bfloat162_rn(acc[2 * j], acc[2 * j + 1]);
-            pk[j] = *reinterpret_cast<uint32_t*>(&b2);
-          }
+          for (int j = 0; j < 4; ++j) pk[j] = pack_half2<fmt_of<TOUT>>(acc[2 * j], acc[2 * j + 1]);
           *reinterpret_cast<uint4*>(o) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
         } else {
           float* of = reinterpret_cast<float*>(o);
@@ -521,8 +520,10 @@ int launch_first_conv(const FirstConvArgs& a, cudaStream_t stream) {
                     (a.kd == 1 || first_conv1_3d_smem(a.cout_pad) <= 100 * 1024);   // 3D: two blocks of it per SM
   const int groups = a.cout_pad / 8;
   if (fast && a.kd == 1 && a.D == 1 && (groups == 1 || groups == 2 || groups == 4 || groups == 8)) {
-    if (a.in_kind == 0 && a.esz == 2) launch_first_conv1_2d<uint8_t, __nv_bfloat16>(a, stream);
+    if (a.in_kind == 0 && a.esz == 2 && a.f16) launch_first_conv1_2d<uint8_t, __half>(a, stream);
+    else if (a.in_kind == 0 && a.esz == 2) launch_first_conv1_2d<uint8_t, __nv_bfloat16>(a, stream);
     else if (a.in_kind == 0 && a.esz == 4) launch_first_conv1_2d<uint8_t, float>(a, stream);
+    else if (a.in_kind == 1 && a.esz == 2 && a.f16) launch_first_conv1_2d<float, __half>(a, stream);
     else if (a.in_kind == 1 && a.esz == 2) launch_first_conv1_2d<float, __nv_bfloat16>(a, stream);
     else if (a.in_kind == 1 && a.esz == 4) launch_first_conv1_2d<float, float>(a, stream);
     else BIU_REQUIRE(false, "first_conv: bad in_kind/esz");
@@ -548,15 +549,19 @@ int launch_first_conv(const FirstConvArgs& a, cudaStream_t stream) {
       first_conv1_3d_kernel<TIN, TOUT><<<(int)rb3, 256, sm3, stream>>>(a);                               \
     }                                                                                                    \
   } while (0)
-    if (a.in_kind == 0 && a.esz == 2) BIU_FC1(uint8_t, __nv_bfloat16);
+    if (a.in_kind == 0 && a.esz == 2 && a.f16) BIU_FC1(uint8_t, __half);
+    else if (a.in_kind == 0 && a.esz == 2) BIU_FC1(uint8_t, __nv_bfloat16);
     else if (a.in_kind == 0 && a.esz == 4) BIU_FC1(uint8_t, float);
+    else if (a.in_kind == 1 && a.esz == 2 && a.f16) BIU_FC1(float, __half);
     else if (a.in_kind == 1 && a.esz == 2) BIU_FC1(float, __nv_bfloat16);
     else if (a.in_kind == 1 && a.esz == 4) BIU_FC1(float, float);
     else BIU_REQUIRE(false, "first_conv: bad in_kind/esz");
 #undef BIU_FC1
   }
+  else if (a.in_kind == 0 && a.esz == 2 && a.f16) BIU_FC(uint8_t, __half);
   else if (a.in_kind == 0 && a.esz == 2) BIU_FC(uint8_t, __nv_bfloat16);
   else if (a.in_kind == 0 && a.esz == 4) BIU_FC(uint8_t, float);
+  else if (a.in_kind == 1 && a.esz == 2 && a.f16) BIU_FC(float, __half);
   else if (a.in_kind == 1 && a.esz == 2) BIU_FC(float, __nv_bfloat16);
   else if (a.in_kind == 1 && a.esz == 4) BIU_FC(float, float);
   else BIU_REQUIRE(false, "first_conv: bad in_kind/esz");
@@ -625,7 +630,8 @@ int launch_pool2(const PoolArgs& a, cudaStream_t stream) {
   long long blocks = ceil_div_ll((long long)a.B * (a.dims == 3 ? a.D / 2 : a.D) * oh * ow * (a.c / vec), 256);
   if (blocks > 148LL * 16) blocks = 148LL * 16;
   if (blocks < 1) blocks = 1;
-  if (a.esz == 2) pool2_kernel<__nv_bfloat16, 8><<<(int)blocks, 256, 0, stream>>>(a);
+  if (a.esz == 2 && a.f16) pool2_kernel<__half, 8><<<(int)blocks, 256, 0, stream>>>(a);
+  else if (a.esz == 2) pool2_kernel<__nv_bfloat16, 8><<<(int)blocks, 256, 0, stream>>>(a);
   else pool2_kernel<float, 4><<<(int)blocks, 256, 0, stream>>>(a);
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
@@ -672,7 +678,8 @@ int launch_up_nearest(const UpNearestArgs& a, cudaStream_t stream) {
   long long blocks = (long long)a.B * a.D * a.H;             // one block iteration per input row
   if (blocks > 148LL * 16) blocks = 148LL * 16;
   if (blocks < 1) blocks = 1;
-  if (a.esz == 2) up_nearest_kernel<__nv_bfloat16, 8><<<(int)blocks, 256, 0, stream>>>(a);
+  if (a.esz == 2 && a.f16) up_nearest_kernel<__half, 8><<<(int)blocks, 256, 0, stream>>>(a);
+  else if (a.esz == 2) up_nearest_kernel<__nv_bfloat16, 8><<<(int)blocks, 256, 0, stream>>>(a);
   else up_nearest_kernel<float, 4><<<(int)blocks, 256, 0, stream>>>(a);
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
@@ -713,7 +720,8 @@ int launch_head(const HeadArgs& a, cudaStream_t stream) {
   long long blocks = ceil_div_ll(total, 256);
   if (blocks > 148LL * 16) blocks = 148LL * 16;
   if (blocks < 1) blocks = 1;
-  if (a.esz == 2) head_kernel<__nv_bfloat16><<<(int)blocks, 256, 0, stream>>>(a);
+  if (a.esz == 2 && a.f16) head_kernel<__half><<<(int)blocks, 256, 0, stream>>>(a);
+  else if (a.esz == 2) head_kernel<__nv_bfloat16><<<(int)blocks, 256, 0, stream>>>(a);
   else head_kernel<float><<<(int)blocks, 256, 0, stream>>>(a);
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
@@ -811,7 +819,8 @@ __global__ void __launch_bounds__(256) direct_conv_kernel(DirectConvArgs a) {
 int launch_direct_conv(const DirectConvArgs& a, cudaStream_t stream) {
   const long long npix = (long long)a.B * a.D * a.H * a.W;
   dim3 grid((unsigned)ceil_div_ll(npix, 64), (unsigned)ceil_div(a.cout, 64));
-  if (a.esz == 2) direct_conv_kernel<__nv_bfloat16><<<grid, 256, 0, stream>>>(a);
+  if (a.esz == 2 && a.f16) direct_conv_kernel<__half><<<grid, 256, 0, stream>>>(a);
+  else if (a.esz == 2) direct_conv_kernel<__nv_bfloat16><<<grid, 256, 0, stream>>>(a);
   else direct_conv_kernel<float><<<grid, 256, 0, stream>>>(a);
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
@@ -853,7 +862,8 @@ int launch_direct_up(const DirectUpArgs& a, cudaStream_t stream) {
   long long blocks = ceil_div_ll(total, 256);
   if (blocks > 148LL * 32) blocks = 148LL * 32;
   if (blocks < 1) blocks = 1;
-  if (a.esz == 2) direct_up_kernel<__nv_bfloat16><<<(int)blocks, 256, 0, stream>>>(a);
+  if (a.esz == 2 && a.f16) direct_up_kernel<__half><<<(int)blocks, 256, 0, stream>>>(a);
+  else if (a.esz == 2) direct_up_kernel<__nv_bfloat16><<<(int)blocks, 256, 0, stream>>>(a);
   else direct_up_kernel<float><<<(int)blocks, 256, 0, stream>>>(a);
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();

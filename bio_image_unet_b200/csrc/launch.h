@@ -10,11 +10,14 @@ extern unsigned long long g_launch_count;
 inline void count_launch(int n = 1) { g_launch_count += n; }
 
 // ---- tcgen05 implicit-GEMM convolution (conv_tc.cu) -------------------------------------------------------------
+// Every argument block below gives the activation storage as `esz` (bytes per element) and `f16`: with esz 2, 0 = bf16,
+// 1 = fp16 (2-byte elements, tensor-core operands of the same format); esz 4 = fp32 storage / tf32 operands.
 struct ConvTcArgs {
-  int esz;                      // 2 = bf16 operands, 4 = tf32 operands (fp32 storage)
+  int esz;                      // 2 = bf16 / fp16 operands, 4 = tf32 operands (fp32 storage)
+  int f16;
   const void* in;               // NHWC / NDHWC activations
   int in_ctot, in_coff;         // channel stride / offset of the source buffer
-  int cin;                      // logical input channels (multiple of 16 bf16 / 8 fp32)
+  int cin;                      // logical input channels (multiple of 16 bf16 / fp16, 8 fp32)
   int W, H, D, B;
   int kw, kh, kd;               // 3 or 1
   const void* wgt;              // packed [tap][n_total][cin]
@@ -54,7 +57,8 @@ int pick_ck(int cin, int esz);
 
 // ---- CUDA-core kernels (direct.cu): exact-fp32 path and shapes the tensor path cannot take ------------------------
 struct DirectConvArgs {
-  int esz;                      // activation storage: 2 = bf16, 4 = fp32
+  int esz;                      // activation storage: 2 = bf16 / fp16, 4 = fp32
+  int f16;
   const void* in;
   int in_ctot, in_coff, cin;
   int W, H, D, B;
@@ -71,7 +75,7 @@ struct DirectConvArgs {
 int launch_direct_conv(const DirectConvArgs& a, cudaStream_t stream);
 
 struct DirectUpArgs {           // ConvTranspose(k=2,s=2): fp32 weights [q][cin][cout], q = (az,ay,ax) bits
-  int esz;
+  int esz, f16;
   const void* in;
   int in_ctot, in_coff, cin;
   int W, H, D, B;
@@ -98,7 +102,7 @@ struct FirstConvArgs {          // planar u8 / f32 input with few channels -> NH
   float slope;
   const float* scale;
   const float* shift;
-  int esz;
+  int esz, f16;
   void* out;                    // NHWC, channels [coff, coff+cout_pad) written (pad = zeros)
   int out_ctot, out_coff, cout_pad;
   int round_tf32;
@@ -106,12 +110,13 @@ struct FirstConvArgs {          // planar u8 / f32 input with few channels -> NH
 int launch_first_conv(const FirstConvArgs& a, cudaStream_t stream);
 
 // First block of the 2D nets on the row kernel (conv_rows.cuh, first mode): uint8 tile in, NHWC features out; the three dx
-// taps are the GEMM's K, the dy taps are folded into N. bf16 / tf32 modes only (weights rounded like every other block's).
+// taps are the GEMM's K, the dy taps are folded into N. Tensor-core modes only (weights rounded like every other block's).
 struct FirstRowsArgs {
-  int esz;                      // 2 = bf16, 4 = tf32 storage
+  int esz;                      // 2 = bf16 / fp16, 4 = tf32 storage
+  int f16;
   const uint8_t* in;            // [B][H][W] uint8 (one channel)
   int W, H, B;
-  const void* wgt;              // [3 * n_total ((2 - dy), co)][16 bf16 | 8 tf32: (dx = 0..2, zeros)]
+  const void* wgt;              // [3 * n_total ((2 - dy), co)][16 bf16 / fp16 | 8 tf32: (dx = 0..2, zeros)]
   int n_total;                  // padded output channels: 16 or 32
   float slope;
   const float* scale;           // BatchNorm scale / 255 (the input rows hold the raw integers)
@@ -123,7 +128,7 @@ bool conv_first_rows_supported(const FirstRowsArgs& a);
 int launch_conv_first_rows(const FirstRowsArgs& a, cudaStream_t stream);
 
 struct PoolArgs {
-  int esz;
+  int esz, f16;
   const void* in;
   int in_ctot, in_coff, c;
   int W, H, D, B;               // input extents
@@ -136,7 +141,7 @@ struct PoolArgs {
 int launch_pool2(const PoolArgs& a, cudaStream_t stream);
 
 struct UpNearestArgs {          // nearest-neighbour x2 upsampling (multi_output_unet3d, use_interpolation=True)
-  int esz;
+  int esz, f16;
   const void* in;
   int in_ctot, in_coff, c;
   int W, H, D, B;               // input extents
@@ -147,7 +152,7 @@ struct UpNearestArgs {          // nearest-neighbour x2 upsampling (multi_output
 int launch_up_nearest(const UpNearestArgs& a, cudaStream_t stream);
 
 struct HeadArgs {               // 1x1 head + activation on NHWC features -> planar
-  int esz;
+  int esz, f16;
   const void* in;
   int in_ctot, in_coff, cin;
   long long npix_per_img;       // D*H*W

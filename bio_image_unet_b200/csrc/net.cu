@@ -33,6 +33,12 @@ static uint16_t host_bf16(float v) {
   u += 0x7FFFu + ((u >> 16) & 1u);   // round to nearest even
   return (uint16_t)(u >> 16);
 }
+static uint16_t host_fp16(float v) {
+  const __half_raw r = __float2half_rn(v);   // round to nearest even; beyond +-65504 -> +-inf
+  return r.x;
+}
+// weight element of a 2-byte precision mode
+static uint16_t host_2byte(const Net* n, float v) { return n->f16 ? host_fp16(v) : host_bf16(v); }
 
 struct Builder {
   Net* n;
@@ -103,7 +109,8 @@ int net_build(Net* n) {
   n->layers.clear(); n->bufs.clear(); n->ops.clear();
   Builder b{n};
   const int nf = n->nf;
-  n->esz = n->precision == PREC_BF16 ? 2 : 4;
+  n->f16 = n->precision == PREC_FP16 ? 1 : 0;
+  n->esz = (n->precision == PREC_BF16 || n->f16) ? 2 : 4;
   n->head_total = 0;
   for (int c : n->head_channels) n->head_total += c;
   BIU_REQUIRE(n->head_total >= 1 && n->head_total <= kMaxHead, "between 1 and %d output channels supported (got %d)",
@@ -389,7 +396,7 @@ int net_finalize(Net* n) {
         if (n->esz == 2) {
           std::vector<uint16_t> wp(cnt, 0);
           for (int co = 0; co < L.cout; ++co)
-            for (int ci = 0; ci < L.cin_phys; ++ci) wp[(size_t)co * L.cin_phys + ci] = host_bf16(wd[(size_t)ci * L.cout_pad + co]);
+            for (int ci = 0; ci < L.cin_phys; ++ci) wp[(size_t)co * L.cin_phys + ci] = host_2byte(n, wd[(size_t)ci * L.cout_pad + co]);
           uint16_t* d = nullptr;
           if (upload(n, wp, &d)) return -1;
           L.w_tc = d;
@@ -455,7 +462,7 @@ int net_finalize(Net* n) {
       if (upload(n, scale, &L.scale)) return -1;
       if (upload(n, shift, &L.shift)) return -1;
       // first block of a 2D net (one input channel): packing for the row kernel's first mode - the dx taps are the K
-      // dimension (zero padded to 16 bf16 / 8 tf32 elements), the dy taps are folded into N in the order dy = 2, 1, 0
+      // dimension (zero padded to 16 bf16 / fp16 or 8 tf32 elements), the dy taps are folded into N in the order dy = 2, 1, 0
       if (n->precision != PREC_FP32 && L.cin_log == 1 && L.kd == 1 && L.kw == 3 && L.kh == 3 &&
           (L.cout_pad == 16 || L.cout_pad == 32)) {
         const int kel = 32 / n->esz, nfold = 3 * L.cout_pad;
@@ -466,7 +473,7 @@ int net_finalize(Net* n) {
               wf[((size_t)(2 - dy) * L.cout_pad + co) * kel + dx] = w->data[(size_t)co * taps + dy * 3 + dx];
         if (n->esz == 2) {
           std::vector<uint16_t> wp(wf.size());
-          for (size_t i = 0; i < wf.size(); ++i) wp[i] = host_bf16(wf[i]);
+          for (size_t i = 0; i < wf.size(); ++i) wp[i] = host_2byte(n, wf[i]);
           uint16_t* d = nullptr;
           if (upload(n, wp, &d)) return -1;
           L.w_first = d;
@@ -488,7 +495,7 @@ int net_finalize(Net* n) {
             for (int co = 0; co < L.cout; ++co)
               for (int ci = 0; ci < L.cin_log; ++ci)
                 wp[((size_t)t * L.cout_pad + co) * L.cin_phys + phys[ci]] =
-                    host_bf16(w->data[((size_t)co * L.cin_log + ci) * taps + t]);
+                    host_2byte(n, w->data[((size_t)co * L.cin_log + ci) * taps + t]);
           uint16_t* d = nullptr;
           if (upload(n, wp, &d)) return -1;
           L.w_tc = d;
@@ -519,7 +526,7 @@ int net_finalize(Net* n) {
               }
           if (n->esz == 2) {
             std::vector<uint16_t> wp(wf.size());
-            for (size_t i = 0; i < wf.size(); ++i) wp[i] = host_bf16(wf[i]);
+            for (size_t i = 0; i < wf.size(); ++i) wp[i] = host_2byte(n, wf[i]);
             uint16_t* d = nullptr;
             if (upload(n, wp, &d)) return -1;
             L.w_fold = d;
@@ -544,7 +551,7 @@ int net_finalize(Net* n) {
                 }
             if (n->esz == 2) {
               std::vector<uint16_t> wp(wz.size());
-              for (size_t i = 0; i < wz.size(); ++i) wp[i] = host_bf16(wz[i]);
+              for (size_t i = 0; i < wz.size(); ++i) wp[i] = host_2byte(n, wz[i]);
               uint16_t* d = nullptr;
               if (upload(n, wp, &d)) return -1;
               L.w_fold_z = d;
@@ -584,7 +591,7 @@ int net_finalize(Net* n) {
             for (int co = 0; co < L.cout; ++co)
               for (int ci = 0; ci < L.cin_log; ++ci)
                 wp[((size_t)q * L.cout_pad + co) * L.cin_phys + ci] =
-                    host_bf16(w->data[((size_t)ci * L.cout + co) * L.nq + q]);
+                    host_2byte(n, w->data[((size_t)ci * L.cout + co) * L.nq + q]);
           uint16_t* d = nullptr;
           if (upload(n, wp, &d)) return -1;
           L.w_tc = d;
@@ -659,16 +666,13 @@ long long net_plan(Net* n, int B, int D, int H, int W) {
   return (long long)off;
 }
 
+template <int FMT>
 __global__ void max_join_kernel(const uint4* __restrict__ a, const uint4* __restrict__ b, uint4* __restrict__ out,
-                                long long nvec, int esz) {
+                                long long nvec) {
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += (long long)gridDim.x * blockDim.x) {
     uint4 x = a[i], y = b[i], r;
-    if (esz == 2) {
-      const __nv_bfloat162* xp = reinterpret_cast<const __nv_bfloat162*>(&x);
-      const __nv_bfloat162* yp = reinterpret_cast<const __nv_bfloat162*>(&y);
-      __nv_bfloat162* rp = reinterpret_cast<__nv_bfloat162*>(&r);
-#pragma unroll
-      for (int k = 0; k < 4; ++k) rp[k] = __hmax2(xp[k], yp[k]);
+    if (fmt_esz(FMT) == 2) {
+      r = make_uint4(max_half2<FMT>(x.x, y.x), max_half2<FMT>(x.y, y.y), max_half2<FMT>(x.z, y.z), max_half2<FMT>(x.w, y.w));
     } else {
       const float* xp = reinterpret_cast<const float*>(&x);
       const float* yp = reinterpret_cast<const float*>(&y);
@@ -885,8 +889,10 @@ __global__ void __launch_bounds__(256) up_bilinear_kernel(const T* __restrict__ 
 }
 
 // skip[pix][c] *= psi[pix] on one half of a concat buffer (AttentionBlock: out = skip_connection * psi)
+template <int FMT>
 __global__ void mul_psi_kernel(void* act, int ctot, int coff, int c, const float* __restrict__ psi, long long npix,
-                               int esz, int round_tf32) {
+                               int round_tf32) {
+  constexpr int esz = fmt_esz(FMT);
   const int vec = 16 / esz, cv = c / vec;
   const long long total = npix * cv;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
@@ -895,7 +901,14 @@ __global__ void mul_psi_kernel(void* act, int ctot, int coff, int c, const float
     const float s = __ldg(psi + pix);
     uint4* ptr = reinterpret_cast<uint4*>(reinterpret_cast<char*>(act) + ((pix * ctot + coff) * esz + (long long)v * 16));
     uint4 x = *ptr;
-    if (esz == 2) {
+    if (FMT == FMT_F16) {
+      __half2* xp = reinterpret_cast<__half2*>(&x);
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        float2 f = __half22float2(xp[k]);
+        xp[k] = __floats2half2_rn(f.x * s, f.y * s);
+      }
+    } else if (esz == 2) {
       __nv_bfloat162* xp = reinterpret_cast<__nv_bfloat162*>(&x);
 #pragma unroll
       for (int k = 0; k < 4; ++k) {
@@ -972,12 +985,12 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
         BIU_REQUIRE(a.in != nullptr, "network input pointer is null");
         a.cin = n->in_ch; a.W = w; a.H = h; a.D = d; a.B = shared > 0 ? n->B + shared : n->B; a.kd = L.kd;
         a.wgt = L.w_direct; a.cout = L.cout_pad; a.cout_real = L.cout; a.slope = L.slope; a.scale = L.scale; a.shift = L.shift;
-        a.esz = n->esz; a.out = shared > 0 ? ws + db->offset : dst_ptr(d, h, w); a.out_ctot = db->ctot; a.out_coff = o.dst_coff;
+        a.esz = n->esz; a.f16 = n->f16; a.out = shared > 0 ? ws + db->offset : dst_ptr(d, h, w); a.out_ctot = db->ctot; a.out_coff = o.dst_coff;
         a.cout_pad = L.cout_pad; a.round_tf32 = round_tf32;
         if (tc_allowed && in_kind == 0 && n->dims == 2 && a.D == 1 && L.w_first != nullptr) {
           FirstRowsArgs fr;
           memset(&fr, 0, sizeof(fr));
-          fr.esz = n->esz; fr.in = reinterpret_cast<const uint8_t*>(a.in); fr.W = a.W; fr.H = a.H; fr.B = a.B;
+          fr.esz = n->esz; fr.f16 = n->f16; fr.in = reinterpret_cast<const uint8_t*>(a.in); fr.W = a.W; fr.H = a.H; fr.B = a.B;
           fr.wgt = L.w_first; fr.n_total = L.cout_pad; fr.slope = L.slope; fr.scale = L.scale_first; fr.shift = L.shift;
           fr.out = a.out; fr.out_ctot = a.out_ctot; fr.out_coff = a.out_coff;
           if (conv_first_rows_supported(fr)) {
@@ -994,7 +1007,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
         const bool head = o.kind == OP_CONV_HEAD;
         ConvTcArgs a;
         memset(&a, 0, sizeof(a));
-        a.esz = n->esz; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.cin = L.cin_phys;
+        a.esz = n->esz; a.f16 = n->f16; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.cin = L.cin_phys;
         a.W = w; a.H = h; a.D = d; a.B = batch; a.kw = L.kw; a.kh = L.kh; a.kd = L.kd;
         a.wgt = L.w_tc; a.wgt_fold = L.w_fold; a.wgt_fold_z = L.w_fold_z; a.n_total = L.cout_pad; a.mode = head ? EPI_HEAD : EPI_CONV; a.slope = L.slope;
         a.scale = L.scale; a.shift = L.shift;
@@ -1055,7 +1068,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
               if (conv_tc_can_fuse_pool_xy(a)) {
                 zpairs = skip_pool = true;
                 memset(&zp, 0, sizeof(zp));
-                zp.esz = n->esz; zp.in = a.pool_out; zp.in_ctot = L.cout_pad; zp.in_coff = 0; zp.c = L.cout_pad;
+                zp.esz = n->esz; zp.f16 = n->f16; zp.in = a.pool_out; zp.in_ctot = L.cout_pad; zp.in_coff = 0; zp.c = L.cout_pad;
                 zp.W = w / 2; zp.H = h / 2; zp.D = d; zp.B = batch; zp.dims = 3; zp.mode = 2;
                 zp.out = ws + pb.offset; zp.out_ctot = pb.ctot; zp.out_coff = nx.dst_coff;
               } else {
@@ -1069,7 +1082,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
           n->op_kinds[op_index] += 16;
           DirectConvArgs da;
           memset(&da, 0, sizeof(da));
-          da.esz = n->esz; da.in = src; da.in_ctot = sb->ctot; da.in_coff = o.src_coff; da.cin = L.cin_phys;
+          da.esz = n->esz; da.f16 = n->f16; da.in = src; da.in_ctot = sb->ctot; da.in_coff = o.src_coff; da.cin = L.cin_phys;
           da.W = w; da.H = h; da.D = d; da.B = batch; da.kw = L.kw; da.kh = L.kh; da.kd = L.kd;
           da.wgt = L.w_direct; da.cout = L.cout_pad; da.slope = L.slope; da.scale = L.scale; da.shift = L.shift;
           da.round_tf32 = round_tf32;
@@ -1084,7 +1097,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
             if (int rc = launch_direct_conv(da, stream)) return rc;
             HeadArgs ha;
             memset(&ha, 0, sizeof(ha));
-            ha.esz = n->esz; ha.in = da.out; ha.in_ctot = scratch.ctot; ha.in_coff = 0; ha.cin = L.cout_pad;
+            ha.esz = n->esz; ha.f16 = n->f16; ha.in = da.out; ha.in_ctot = scratch.ctot; ha.in_coff = 0; ha.cin = L.cout_pad;
             ha.npix_per_img = (long long)d * h * w; ha.B = batch; ha.head_n = n->head_total;
             ha.w = n->head_w; ha.b = n->head_b;
             int row = 0;
@@ -1101,7 +1114,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
         const int od = n->dims == 3 ? 2 * d : d;
         ConvTcArgs a;
         memset(&a, 0, sizeof(a));
-        a.esz = n->esz; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.cin = L.cin_phys;
+        a.esz = n->esz; a.f16 = n->f16; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.cin = L.cin_phys;
         a.W = w; a.H = h; a.D = d; a.B = batch; a.kw = a.kh = a.kd = 1;
         a.wgt = L.w_tc; a.n_total = L.nq * L.cout_pad; a.mode = EPI_UP; a.slope = 1.f;
         a.scale = L.scale; a.shift = L.shift;
@@ -1113,7 +1126,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
           n->op_kinds[op_index] += 16;
           DirectUpArgs da;
           memset(&da, 0, sizeof(da));
-          da.esz = n->esz; da.in = src; da.in_ctot = sb->ctot; da.in_coff = o.src_coff; da.cin = L.cin_phys;
+          da.esz = n->esz; da.f16 = n->f16; da.in = src; da.in_ctot = sb->ctot; da.in_coff = o.src_coff; da.cin = L.cin_phys;
           da.W = w; da.H = h; da.D = d; da.B = batch; da.dims = n->dims; da.wgt = L.w_direct; da.bias = L.shift;
           da.cout = L.cout_pad; da.out = a.out; da.out_ctot = db->ctot; da.out_coff = o.dst_coff;
           da.round_tf32 = round_tf32;
@@ -1124,7 +1137,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
       case OP_POOL: {
         PoolArgs a;
         memset(&a, 0, sizeof(a));
-        a.esz = n->esz; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.c = o.c;
+        a.esz = n->esz; a.f16 = n->f16; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.c = o.c;
         a.W = w; a.H = h; a.D = d; a.B = batch; a.dims = n->dims; a.mode = o.pool_mode;
         a.out = dst_ptr(n->dims == 3 ? d / 2 : d, h / 2, w / 2); a.out_ctot = db->ctot; a.out_coff = o.dst_coff;
         if (int rc = launch_pool2(a, stream)) return rc;
@@ -1133,7 +1146,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
       case OP_UPNEAREST: {
         UpNearestArgs a;
         memset(&a, 0, sizeof(a));
-        a.esz = n->esz; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.c = o.c;
+        a.esz = n->esz; a.f16 = n->f16; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.c = o.c;
         a.W = w; a.H = h; a.D = d; a.B = batch; a.dims = n->dims;
         a.out = dst_ptr(n->dims == 3 ? 2 * d : d, 2 * h, 2 * w); a.out_ctot = db->ctot; a.out_coff = o.dst_coff;
         if (int rc = launch_up_nearest(a, stream)) return rc;
@@ -1144,7 +1157,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
         float* psi = reinterpret_cast<float*>(ws + db->offset);
         ConvTcArgs a;
         memset(&a, 0, sizeof(a));
-        a.esz = n->esz; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.cin = L.cin_phys;
+        a.esz = n->esz; a.f16 = n->f16; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.cin = L.cin_phys;
         a.W = w; a.H = h; a.D = d; a.B = batch; a.kw = a.kh = a.kd = 1;
         a.wgt = L.w_tc; a.n_total = L.cout_pad; a.mode = EPI_HEAD; a.slope = 0.f;
         a.scale = L.scale; a.shift = L.shift; a.out = nullptr;
@@ -1158,7 +1171,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
           const Buf& scratch = n->bufs[n->gate_scratch];
           DirectConvArgs da;
           memset(&da, 0, sizeof(da));
-          da.esz = n->esz; da.in = src; da.in_ctot = sb->ctot; da.in_coff = o.src_coff; da.cin = L.cin_phys;
+          da.esz = n->esz; da.f16 = n->f16; da.in = src; da.in_ctot = sb->ctot; da.in_coff = o.src_coff; da.cin = L.cin_phys;
           da.W = w; da.H = h; da.D = d; da.B = batch; da.kw = da.kh = da.kd = 1;
           da.wgt = L.w_direct; da.cout = L.cout_pad; da.slope = 0.f; da.scale = L.scale; da.shift = L.shift;
           da.round_tf32 = 0;
@@ -1166,7 +1179,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
           if (int rc = launch_direct_conv(da, stream)) return rc;
           HeadArgs ha;
           memset(&ha, 0, sizeof(ha));
-          ha.esz = n->esz; ha.in = da.out; ha.in_ctot = L.cout_pad; ha.in_coff = 0; ha.cin = L.cout_pad;
+          ha.esz = n->esz; ha.f16 = n->f16; ha.in = da.out; ha.in_ctot = L.cout_pad; ha.in_coff = 0; ha.cin = L.cout_pad;
           ha.npix_per_img = (long long)d * h * w; ha.B = batch; ha.head_n = 1;
           ha.w = L.gate_w; ha.b = L.gate_b; ha.act[0] = ACT_SIGMOID;
           ha.out_val = psi; ha.out_u8 = nullptr;
@@ -1180,9 +1193,10 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
         long long blocks = ceil_div_ll(npix * (o.c / vec), 256);
         if (blocks > 148 * 16) blocks = 148 * 16;
         if (blocks < 1) blocks = 1;
-        mul_psi_kernel<<<(int)blocks, 256, 0, stream>>>(ws + db->offset, db->ctot, o.dst_coff, o.c,
-                                                        reinterpret_cast<const float*>(ws + sb->offset), npix, n->esz,
-                                                        round_tf32);
+        float* psi = reinterpret_cast<float*>(ws + sb->offset);
+        if (n->f16) mul_psi_kernel<FMT_F16><<<(int)blocks, 256, 0, stream>>>(ws + db->offset, db->ctot, o.dst_coff, o.c, psi, npix, 0);
+        else if (n->esz == 2) mul_psi_kernel<FMT_BF16><<<(int)blocks, 256, 0, stream>>>(ws + db->offset, db->ctot, o.dst_coff, o.c, psi, npix, 0);
+        else mul_psi_kernel<FMT_TF32><<<(int)blocks, 256, 0, stream>>>(ws + db->offset, db->ctot, o.dst_coff, o.c, psi, npix, round_tf32);
         BIU_CHECK_CUDA(cudaGetLastError());
         count_launch();
         break;
@@ -1196,7 +1210,13 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
         const int blocks = n->B * (sb->ctot / G);
         const char* cur = ws + sb->offset + img * stream_img0(sb, 0);
         const char* prv = ws + sb->offset + img * stream_img0(sb, 1);
-        if (n->esz == 2) {
+        if (n->f16) {
+          if (smem > 48 * 1024)
+            BIU_CHECK_CUDA(cudaFuncSetAttribute(xcorr_join_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+          xcorr_join_kernel<__half><<<blocks, 256, smem, stream>>>(
+              reinterpret_cast<const __half*>(cur), reinterpret_cast<const __half*>(prv),
+              reinterpret_cast<__half*>(ws + db->offset), h, w, sb->ctot, G, 0);
+        } else if (n->esz == 2) {
           if (smem > 48 * 1024)
             BIU_CHECK_CUDA(cudaFuncSetAttribute(xcorr_join_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
           xcorr_join_kernel<__nv_bfloat16><<<blocks, 256, smem, stream>>>(
@@ -1220,7 +1240,11 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
         if (blocks > 148 * 16) blocks = 148 * 16;
         if (blocks < 1) blocks = 1;
         char* dst = ws + db->offset;
-        if (n->esz == 2)
+        if (n->f16)
+          up_trilinear_kernel<__half, 8><<<(int)blocks, 256, 0, stream>>>(
+              reinterpret_cast<const __half*>(src), sb->ctot, o.src_coff, o.c, batch, d, h, w,
+              reinterpret_cast<__half*>(dst), db->ctot, o.dst_coff, 0);
+        else if (n->esz == 2)
           up_trilinear_kernel<__nv_bfloat16, 8><<<(int)blocks, 256, 0, stream>>>(
               reinterpret_cast<const __nv_bfloat16*>(src), sb->ctot, o.src_coff, o.c, batch, d, h, w,
               reinterpret_cast<__nv_bfloat16*>(dst), db->ctot, o.dst_coff, 0);
@@ -1237,7 +1261,11 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
         int blocks = batch * (h + 1);                      // one block iteration per pair of output rows
         if (blocks > 148 * 8) blocks = 148 * 8;
         char* dst = ws + db->offset;
-        if (n->esz == 2)
+        if (n->f16)
+          up_bilinear_kernel<__half, 8><<<blocks, 256, 0, stream>>>(
+              reinterpret_cast<const __half*>(src), sb->ctot, o.src_coff, o.c, batch, h, w,
+              reinterpret_cast<__half*>(dst), db->ctot, o.dst_coff, 0);
+        else if (n->esz == 2)
           up_bilinear_kernel<__nv_bfloat16, 8><<<blocks, 256, 0, stream>>>(
               reinterpret_cast<const __nv_bfloat16*>(src), sb->ctot, o.src_coff, o.c, batch, h, w,
               reinterpret_cast<__nv_bfloat16*>(dst), db->ctot, o.dst_coff, 0);
@@ -1256,9 +1284,12 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
         long long blocks = ceil_div_ll(nvec, 256);
         if (blocks > 148 * 8) blocks = 148 * 8;
         if (blocks < 1) blocks = 1;
-        max_join_kernel<<<(int)blocks, 256, 0, stream>>>(reinterpret_cast<const uint4*>(ws + sb->offset + img * stream_img0(sb, 0)),
-                                                         reinterpret_cast<const uint4*>(ws + sb->offset + img * stream_img0(sb, 1)),
-                                                         reinterpret_cast<uint4*>(ws + db->offset), nvec, n->esz);
+        const uint4* xa = reinterpret_cast<const uint4*>(ws + sb->offset + img * stream_img0(sb, 0));
+        const uint4* xb = reinterpret_cast<const uint4*>(ws + sb->offset + img * stream_img0(sb, 1));
+        uint4* xo = reinterpret_cast<uint4*>(ws + db->offset);
+        if (n->f16) max_join_kernel<FMT_F16><<<(int)blocks, 256, 0, stream>>>(xa, xb, xo, nvec);
+        else if (n->esz == 2) max_join_kernel<FMT_BF16><<<(int)blocks, 256, 0, stream>>>(xa, xb, xo, nvec);
+        else max_join_kernel<FMT_TF32><<<(int)blocks, 256, 0, stream>>>(xa, xb, xo, nvec);
         BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
         break;

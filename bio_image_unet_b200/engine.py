@@ -14,7 +14,7 @@ from . import _lib
 KIND = {'unet2d': 0, 'siam2d': 1, 'unet3d': 2, 'mo3d': 3, 'unet2d_v0': 4, 'attunet2d': 5, 'mo2d': 6, 'nested2d': 7,
         'nested2d_3l': 8}
 KIND_2D = ('unet2d', 'siam2d', 'unet2d_v0', 'attunet2d', 'mo2d', 'nested2d', 'nested2d_3l')
-PRECISION = {'bf16': 0, 'tf32': 1, 'fp32': 2}
+PRECISION = {'bf16': 0, 'tf32': 1, 'fp32': 2, 'fp16': 3}
 SIAM_MODE = {'concat': 0, 'max': 1, 'control': 2, 'corr': 3}
 ACT = {None: 0, 'none': 0, 'sigmoid': 1, 'tanh': 2, 'relu': 3}
 HIST_BINS = 65536
@@ -34,14 +34,17 @@ class Engine:
 
     heads: list of (name, channels, activation) — a single ('', out_channels, 'sigmoid') entry for
     Unet / Siam_UNet / UNet3D, the ``output_heads`` dict entries for MultiOutputUnet3D.
+    precision: 'bf16' | 'fp16' (tcgen05 operands and stored activations in that format, fp32 accumulation and
+    BatchNorm / activation; fp16 keeps tf32's 10 mantissa bits, stores beyond +-65504 become +-inf) | 'tf32' (fp32
+    storage) | 'fp32' (CUDA-core kernels).
     """
 
     def __init__(self, kind, state_dict, n_filter, in_channels=1, heads=(('', 1, 'sigmoid'),), siam_mode='concat',
                  use_interpolation=False, precision='bf16', device='cuda:0'):
-        self.device = _require_cuda(device)
-        self.lib = _lib.load()
         if precision not in PRECISION:
             raise ValueError(f"precision must be one of {list(PRECISION)} (got {precision!r})")
+        self.device = _require_cuda(device)
+        self.lib = _lib.load()
         if kind == 'siam2d' and siam_mode not in SIAM_MODE:
             raise NotImplementedError('Unknown mode: {}'.format(siam_mode))   # siam_unet/siam_unet.py:124
         self.kind, self.precision = kind, precision
@@ -129,14 +132,15 @@ class Engine:
         d, h, w = self.tile
         dd = max(d >> level, 1) if self.kind in ('unet3d', 'mo3d') else 1
         hh, ww = h >> level, w >> level
-        esz = 2 if self.precision == 'bf16' else 4
+        esz = 2 if self.precision in ('bf16', 'fp16') else 4
         n = self.batch * dd * hh * ww * channels
         host = np.empty(n * esz, dtype=np.uint8)
         torch.cuda.synchronize(self.device)
         _lib.check(self.lib.biu_net_debug_copy(self.handle, name.encode(), _lib.ptr(self.workspace),
                                                host.ctypes.data_as(ctypes.c_void_p), host.nbytes))
         if esz == 2:
-            t = torch.from_numpy(host.view(np.int16).copy()).view(torch.bfloat16).float().numpy()
+            dt = torch.float16 if self.precision == 'fp16' else torch.bfloat16
+            t = torch.from_numpy(host.view(np.int16).copy()).view(dt).float().numpy()
         else:
             t = host.view(np.float32)
         return t.reshape(self.batch, dd, hh, ww, channels)

@@ -45,8 +45,10 @@ class Predict:
         ``deep_supervision`` the last supervision head ('<head>_4' / '<head>_3') is used, like the reference's
         ``train_mode=False`` (multi_output_unet/predict.py:90-94, multi_output_nested_unet.py:143-145).
     The reference runs the model in float16 on CUDA devices and stores the result patches as float16; here the
-    network runs in `precision` ('tf32' default) and the patches go through the same float16 rounding before the
-    margin-weighted stitch. Integer stacks (uint8 / uint16) are normalised on the device.
+    network runs in `precision` ('tf32' default | 'fp16' | 'bf16' | 'fp32', see unet.Predict) and the patches go
+    through the same float16 rounding before the margin-weighted stitch. precision='fp16' is the reference's own
+    arithmetic for this predictor: fp16 weights and activations, fp32 accumulation (the reference's float16
+    convolutions accumulate in fp32 as well). Integer stacks (uint8 / uint16) are normalised on the device.
     """
 
     def __init__(self, imgs, model_params, result_path=None, network=MultiOutputNestedUNet, max_patch_size=(1024, 1024),

@@ -16,7 +16,8 @@ from .multi_output_unet3d import MultiOutputUnet3D
 
 
 class Session:
-    """Reusable multi-output 3D predictor (checkpoint folded / packed once, workspace resident)."""
+    """Reusable multi-output 3D predictor (checkpoint folded / packed once, workspace resident).
+    precision: 'tf32' | 'fp16' | 'bf16' | 'fp32' (see unet.Predict)."""
 
     def __init__(self, model_params, max_patch_size=(64, 256, 256), overlap_factor=0.1, normalization_mode='single',
                  clip_threshold=(0., 99.98), device='cuda:0', precision='tf32', workspace_gb=24.0, dist=None):
@@ -172,7 +173,8 @@ class Predict:
 
     normalization_mode='single' follows the reference's formula; the reference itself fails there on numpy >= 2
     (``ndarray.ptp`` was removed, :111). Integer stacks (uint8 / uint16) are normalised on the device.
-    Engine-only keyword arguments: precision, workspace_gb, distributed (volumes are sharded over ranks).
+    Engine-only keyword arguments: precision ('tf32' | 'fp16' | 'bf16' | 'fp32', see unet.Predict), workspace_gb,
+    distributed (volumes are sharded over ranks).
     """
 
     def __init__(self, imgs, model_params, result_path=None, network=MultiOutputUnet3D,

@@ -23,7 +23,7 @@ def conv_block(dims, in_channels, out_channels, kernel_size=3, dropout=0., dilat
 class EngineModule(nn.Module):
     """Base class: lazily builds / rebuilds an Engine from the current parameters."""
 
-    precision = 'tf32'          # engine-only knob: 'bf16' | 'tf32' | 'fp32'
+    precision = 'tf32'          # engine-only knob: 'tf32' | 'fp16' | 'bf16' | 'fp32' (see unet.Predict)
 
     def _engine_spec(self):     # -> dict(kind=..., n_filter=..., in_channels=..., heads=[...], ...)
         raise NotImplementedError

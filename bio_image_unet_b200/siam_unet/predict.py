@@ -56,7 +56,8 @@ class _TiffSource:
 
 class Session:
     """Reusable Siamese predictor: checkpoint folded / packed once, weights and workspace resident on the device.
-    ``predict_stream`` runs pairs [lo, hi) of a page source through the three-stream pipeline."""
+    ``predict_stream`` runs pairs [lo, hi) of a page source through the three-stream pipeline.
+    precision: 'tf32' | 'fp16' | 'bf16' | 'fp32' (see unet.Predict)."""
 
     def __init__(self, model_params, resize_dim=(512, 512), invert=False, normalization_mode='single',
                  clip_threshold=(0.0, 99.98), add_tile=0, device='cuda:0', precision='tf32', workspace_gb=24.0):
@@ -248,7 +249,8 @@ class Predict:
     """Prediction of tif-movies with Siamese U-Net (constructor surface of siam_unet/predict.py:53-56).
 
     tif_file : str (an ndarray (T, H, W) is also accepted); resize_dim=None processes whole frames.
-    Engine-only keyword arguments: precision, workspace_gb, distributed, keep_intermediates (see unet.Predict).
+    Engine-only keyword arguments: precision ('tf32' | 'fp16' | 'bf16' | 'fp32'), workspace_gb, distributed,
+    keep_intermediates (see unet.Predict).
     """
 
     def __init__(self, tif_file, result_name, model_params, resize_dim=(512, 512), invert=False,

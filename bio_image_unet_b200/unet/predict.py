@@ -19,6 +19,7 @@ class Session:
     ``predict(frames)`` takes a host (F, H, W) uint8/uint16 stack (ideally pinned) and returns the stitched
     (F, C, H, W) uint8 result on the host; ``predict_device`` does the same for a stack already in HBM.
     ``Predict`` (the reference's constructor-runs-everything class) is a thin wrapper around this.
+    precision: 'tf32' | 'fp16' | 'bf16' | 'fp32' (see Predict).
     """
 
     KINDS = {'Unet': 'unet2d', 'AttentionUnet': 'attunet2d', 'Unet_v0': 'unet2d_v0'}
@@ -331,7 +332,9 @@ class Predict:
 
     Engine-only keyword arguments (defaults reproduce the reference's behaviour)
     ----------
-    precision : 'tf32' (default, sigmoid within 1e-3 of the fp32 reference) | 'bf16' (within 1e-2) | 'fp32'
+    precision : 'tf32' (default, sigmoid within 1e-3 of the fp32 reference) | 'fp16' (tf32-grade error at the bf16
+        speed; activations are stored as fp16, so values beyond +-65504 become +-inf as under the reference's
+        model.half()) | 'bf16' (within 1e-2) | 'fp32'
     workspace_gb : activation workspace budget used to pick the tile batch size
     keep_intermediates : keep the uint8 tiles / result tiles as attributes (test hook)
     mutate_input : the reference overwrites the caller's array with the normalised frames in 'single' mode

@@ -16,7 +16,8 @@ from .unet3d import UNet3D
 
 class Session:
     """Reusable 3D predictor: checkpoint folded / packed once; ``predict(vol)`` runs a (Z, X, Y) uint8 / uint16 host
-    volume through normalise -> split -> forward -> mod-3 stitch and returns the uint8 result (on rank 0)."""
+    volume through normalise -> split -> forward -> mod-3 stitch and returns the uint8 result (on rank 0).
+    precision: 'tf32' | 'fp16' | 'bf16' | 'fp32' (see unet.Predict)."""
 
     def __init__(self, model_params, resize_dim, invert=False, clip_threshold=(0., 99.8), add_patch=0, device='cuda:0',
                  precision='tf32', workspace_gb=24.0, dist=None):
@@ -184,7 +185,8 @@ class Predict:
     """Prediction of movies or 3D stacks with 3D U-Net (constructor surface of unet3d/predict.py:52-55).
 
     `normalization_mode` is accepted and unused, as in the reference: percentiles are always taken over the whole
-    volume (unet3d/predict.py:109-117). Engine-only keyword arguments as in unet.Predict; with `distributed=True`
+    volume (unet3d/predict.py:109-117). Engine-only keyword arguments as in unet.Predict (precision 'tf32' | 'fp16' |
+    'bf16' | 'fp32'); with `distributed=True`
     the z-rows of the patch grid are sharded over ranks: each rank uploads only its z-slab, the intensity histogram
     is all-reduced, boundary patches are exchanged point to point, every rank stitches the planes it owns and rank
     0 gathers the uint8 slabs (all device to device).

@@ -33,7 +33,8 @@ enum { BIU_NET_UNET2D = 0,   /* unet/unet.py:5 Unet */
        BIU_NET_NESTED2D_3L = 8 }; /* multi_output_nested_unet.py:151 MultiOutputNestedUNet_3Levels (3 pools) */
 enum { BIU_PREC_BF16 = 0,    /* bf16 operands on tcgen05, fp32 accumulate */
        BIU_PREC_TF32 = 1,    /* tf32 operands on tcgen05, fp32 storage */
-       BIU_PREC_FP32 = 2 };  /* fp32 CUDA-core kernels */
+       BIU_PREC_FP32 = 2,    /* fp32 CUDA-core kernels */
+       BIU_PREC_FP16 = 3 };  /* fp16 operands on tcgen05, fp32 accumulate, fp16 storage (beyond +-65504: +-inf) */
 enum { BIU_SIAM_CONCAT = 0, BIU_SIAM_MAX = 1, BIU_SIAM_CONTROL = 2, BIU_SIAM_CORR = 3 }; /* siam_unet.py:114-124 */
 enum { BIU_ACT_NONE = 0, BIU_ACT_SIGMOID = 1, BIU_ACT_TANH = 2, BIU_ACT_RELU = 3 };      /* multi_output_unet3d.py:97-104 */
 enum { BIU_PAD_REFLECT = 0,  /* unet/predict.py:163-168, unet3d/predict.py:134-137 */
@@ -85,7 +86,7 @@ int biu_net_set_fuse_pool(biu_net* net, int on);
  * form. Results are bit-identical; 21 % of the reference's FLOPs are not executed. */
 int biu_net_set_siam_shared(biu_net* net, int tiles_per_frame);
 /* Number of convolution / transposed-convolution / gate ops of the most recent biu_net_forward that a tensor-core
- * mode (bf16 / tf32) had to run on the CUDA-core kernels because the tile shape is outside what the tcgen05 kernels
+ * mode (bf16 / fp16 / tf32) had to run on the CUDA-core kernels because the tile shape is outside what the tcgen05 kernels
  * take (planes narrower than 8 px, ...). 0 in the exact-fp32 mode's sense of "as requested"; the Python Predict
  * classes turn a non-zero count into a RuntimeWarning (the result is the same, the speed is not). */
 int biu_net_fallback_ops(biu_net* net);
@@ -173,9 +174,11 @@ int biu_stitch_margin_f32(const float* tiles, const int* src_index, int T, int C
                           void* stream);
 
 /* ---- single layers (used by the parity tests; same kernels the network handle launches) ------------------- */
+/* Element code `esz` of the layer entry points: 2 = bf16 activations (and tcgen05 weights), 4 = fp32 storage / tf32
+ * math, BIU_ESZ_FP16 = fp16 activations / weights (2-byte elements). */
+enum { BIU_ESZ_FP16 = 3 };
 /* Conv(k in {1,3}, pad k/2) + per-channel scale/shift + LeakyReLU(slope) on tcgen05.
- * esz 2: bf16 activations/weights, 4: fp32 storage / tf32 math. in: NDHWC with channel stride in_ctot, offset
- * in_coff; wgt: [kd*kh*kw][cout][cin]; out: NDHWC (out_ctot/out_coff). */
+ * in: NDHWC with channel stride in_ctot, offset in_coff; wgt: [kd*kh*kw][cout][cin]; out: NDHWC (out_ctot/out_coff). */
 int biu_conv_tc(int esz, const void* in, int in_ctot, int in_coff, int cin, int B, int D, int H, int W, int kd,
                 int kh, int kw, const void* wgt, int cout, const float* scale, const float* shift, float slope,
                 void* out, int out_ctot, int out_coff, void* stream);
