@@ -19,7 +19,7 @@ import torch.nn.functional as F
 
 from bio_image_unet_b200 import _lib
 from oracle import models as omodels
-from tests import _golden, _parity_fp16
+from tests import _golden, _layer_ref, _parity_fp16
 from tests import test_gpu_baseline_sizes as sizes
 from tests import test_gpu_families as families
 from tests import test_gpu_unet as unet
@@ -190,6 +190,29 @@ def _sync_check():
     assert code.value == 0, f'device fault {hex(code.value)}'
 
 
+def _conv_tc_fp16(case, shift_gain=0.1, scale_gain=1.0):
+    torch.backends.cudnn.allow_tf32 = False
+    B, cin, cout, D, H, W, three = case
+    g = torch.Generator(device='cuda').manual_seed(11)
+    kd = 3 if three else 1
+    x = torch.randn((B, cin, D, H, W) if three else (B, cin, H, W), device='cuda', generator=g).half()
+    w = (torch.randn((cout, cin, kd, 3, 3) if three else (cout, cin, 3, 3), device='cuda', generator=g)
+         / (cin * 9 * kd) ** 0.5).half()
+    scale = (torch.rand(cout, device='cuda', generator=g) + 0.5) * scale_gain
+    shift = torch.randn(cout, device='cuda', generator=g) * shift_gain
+    wp = (w.permute(2, 3, 4, 0, 1) if three else w.permute(2, 3, 0, 1)).contiguous().view(kd * 9, cout, cin)
+    out = torch.zeros((B, D, H, W, cout) if three else (B, H, W, cout), device='cuda', dtype=torch.float16)
+    x_cl = _nhwc(x)
+    rc = _lib.load().biu_conv_tc(ESZ_FP16, _lib.ptr(x_cl), cin, 0, cin, B, D, H, W, kd, 3, 3, _lib.ptr(wp), cout,
+                                 _lib.ptr(scale), _lib.ptr(shift), 0.1, _lib.ptr(out), cout, 0, _lib.stream_ptr())
+    _lib.check(rc, 'biu_conv_tc')
+    _sync_check()
+    # fp32 accumulation of the same operands, one fp16 rounding (nearest even, beyond +-65504 +-inf) of the stored value
+    s, a = _layer_ref.conv_sums(_nhwc(x), w, 3 if three else 2)
+    lo, hi = _layer_ref.interval(s, a, scale, shift, 0.1, 'fp16', _layer_ref.C_GPU)
+    return out.float(), lo, hi
+
+
 @pytest.mark.parametrize('case', [
     # B, cin, cout, D, H, W, 3D
     (2, 64, 64, 1, 32, 32, False),      # halo kernel, 128B swizzle, CTA pairs
@@ -200,27 +223,17 @@ def _sync_check():
     (1, 32, 32, 8, 16, 16, True),       # 3D, 27 taps
 ])
 def test_conv_tc_fp16(case):
-    torch.backends.cudnn.allow_tf32 = False
-    B, cin, cout, D, H, W, three = case
-    g = torch.Generator(device='cuda').manual_seed(11)
-    kd = 3 if three else 1
-    x = torch.randn((B, cin, D, H, W) if three else (B, cin, H, W), device='cuda', generator=g).half()
-    w = (torch.randn((cout, cin, kd, 3, 3) if three else (cout, cin, 3, 3), device='cuda', generator=g)
-         / (cin * 9 * kd) ** 0.5).half()
-    scale = torch.rand(cout, device='cuda', generator=g) + 0.5
-    shift = torch.randn(cout, device='cuda', generator=g) * 0.1
-    wp = (w.permute(2, 3, 4, 0, 1) if three else w.permute(2, 3, 0, 1)).contiguous().view(kd * 9, cout, cin)
-    out = torch.zeros((B, D, H, W, cout) if three else (B, H, W, cout), device='cuda', dtype=torch.float16)
-    rc = _lib.load().biu_conv_tc(ESZ_FP16, _lib.ptr(_nhwc(x)), cin, 0, cin, B, D, H, W, kd, 3, 3, _lib.ptr(wp), cout,
-                                 _lib.ptr(scale), _lib.ptr(shift), 0.1, _lib.ptr(out), cout, 0, _lib.stream_ptr())
-    _lib.check(rc, 'biu_conv_tc')
-    _sync_check()
-    ref = F.conv3d(x.float(), w.float(), padding=1) if three else F.conv2d(x.float(), w.float(), padding=1)
-    bshape = (1, cout) + (1,) * (ref.dim() - 2)
-    ref = F.leaky_relu(ref * scale.view(bshape) + shift.view(bshape), 0.1)
-    got = _nchw(out.float())
-    # fp32 accumulation of the same operands, one fp16 rounding of the stored value (2^-11 relative)
-    assert torch.allclose(got, ref, rtol=2e-3, atol=2e-3), (got - ref).abs().max().item()
+    _layer_ref.check_interval(*_conv_tc_fp16(case), f'conv_tc fp16 {case}')
+
+
+@pytest.mark.parametrize('case', [(2, 64, 64, 1, 32, 32, False),     # halo kernel
+                                  (5, 512, 512, 1, 2, 2, False)])     # per-tap small-plane kernel
+def test_conv_tc_fp16_overflow_is_inf(case):
+    """DESIGN §5: fp16 stores do not saturate. A shift of about +-65000 and a scale of 2000 push part of the outputs
+    past +-65504: they must be +-inf exactly where the correctly rounded value is, and correctly rounded elsewhere."""
+    got, lo, hi = _conv_tc_fp16(case, shift_gain=40000.0, scale_gain=2000.0)
+    _layer_ref.check_interval(got, lo, hi, f'conv_tc fp16 overflow {case}')
+    assert bool(torch.isinf(got).any()) and bool(torch.isfinite(got).any()), 'the case must reach both sides of 65504'
 
 
 @pytest.mark.parametrize('dims,cin,cout', [(2, 64, 32), (2, 512, 256), (3, 32, 32)])
@@ -236,13 +249,17 @@ def test_up_tc_fp16(dims, cin, cout):
     wp = w.reshape(cin, cout, nq).permute(2, 1, 0).contiguous().view(nq * cout, cin)
     out = torch.zeros((B, 2 * D, 2 * H, 2 * W, cout) if dims == 3 else (B, 2 * H, 2 * W, cout), device='cuda',
                       dtype=torch.float16)
-    rc = _lib.load().biu_up_tc(ESZ_FP16, _lib.ptr(_nhwc(x)), cin, 0, cin, B, D, H, W, dims, _lib.ptr(wp), cout,
-                               _lib.ptr(bias.repeat(nq).contiguous()), _lib.ptr(out), cout, 0, _lib.stream_ptr())
+    # named, so that they outlive the launch: the caching allocator hands a freed temporary's memory to the next
+    # allocation, and a copy queued before the kernel would overwrite its input
+    x_cl = _nhwc(x)
+    bias_rep = bias.repeat(nq).contiguous()
+    rc = _lib.load().biu_up_tc(ESZ_FP16, _lib.ptr(x_cl), cin, 0, cin, B, D, H, W, dims, _lib.ptr(wp), cout,
+                               _lib.ptr(bias_rep), _lib.ptr(out), cout, 0, _lib.stream_ptr())
     _lib.check(rc, 'biu_up_tc')
     _sync_check()
-    ref = (F.conv_transpose3d if dims == 3 else F.conv_transpose2d)(x.float(), w.float(), bias, stride=2)
-    got = _nchw(out.float())
-    assert torch.allclose(got, ref, rtol=2e-3, atol=2e-3), (got - ref).abs().max().item()
+    s, a = _layer_ref.up_sums(_nhwc(x), w, dims)
+    lo, hi = _layer_ref.interval(s, a, torch.ones_like(bias), bias, 1.0, 'fp16', _layer_ref.C_GPU)
+    _layer_ref.check_interval(out.float(), lo, hi, f'up_tc fp16 {dims}D {cin}->{cout}')
 
 
 def test_conv_direct_fp16():
@@ -255,13 +272,14 @@ def test_conv_direct_fp16():
     shift = torch.randn(cout, device='cuda', generator=g) * 0.1
     wp = w.permute(2, 3, 1, 0).contiguous().view(9, cin, cout)
     out = torch.zeros(B, H, W, cout, device='cuda', dtype=torch.float16)
-    rc = _lib.load().biu_conv_direct(ESZ_FP16, _lib.ptr(_nhwc(x)), cin, 0, cin, B, 1, H, W, 1, 3, 3, _lib.ptr(wp), cout,
+    x_cl = _nhwc(x)
+    rc = _lib.load().biu_conv_direct(ESZ_FP16, _lib.ptr(x_cl), cin, 0, cin, B, 1, H, W, 1, 3, 3, _lib.ptr(wp), cout,
                                      _lib.ptr(scale), _lib.ptr(shift), 0.1, _lib.ptr(out), cout, 0, _lib.stream_ptr())
     _lib.check(rc, 'biu_conv_direct')
     _sync_check()
-    ref = F.leaky_relu(F.conv2d(x.float(), w, padding=1) * scale.view(1, -1, 1, 1) + shift.view(1, -1, 1, 1), 0.1)
-    got = _nchw(out.float())
-    assert torch.allclose(got, ref, rtol=2e-3, atol=2e-3), (got - ref).abs().max().item()
+    s, a = _layer_ref.conv_sums(_nhwc(x), w, 2)
+    lo, hi = _layer_ref.interval(s, a, scale, shift, 0.1, 'fp16', _layer_ref.C_GPU)
+    _layer_ref.check_interval(out.float(), lo, hi, 'conv_direct fp16')
 
 
 @pytest.mark.parametrize('dims,mode', [(2, 0), (3, 0), (3, 1)])
@@ -271,7 +289,8 @@ def test_pool2_fp16(dims, mode):
     x = torch.randn((B, C, D, H, W) if dims == 3 else (B, C, H, W), device='cuda', generator=g).half()
     out = torch.zeros((B, D // 2, H // 2, W // 2, C) if dims == 3 else (B, H // 2, W // 2, C), device='cuda',
                       dtype=torch.float16)
-    rc = _lib.load().biu_pool2(ESZ_FP16, _lib.ptr(_nhwc(x)), C, 0, C, B, D, H, W, dims, mode, _lib.ptr(out), C, 0,
+    x_cl = _nhwc(x)
+    rc = _lib.load().biu_pool2(ESZ_FP16, _lib.ptr(x_cl), C, 0, C, B, D, H, W, dims, mode, _lib.ptr(out), C, 0,
                                _lib.stream_ptr())
     _lib.check(rc, 'biu_pool2')
     _sync_check()

@@ -1,6 +1,7 @@
-"""Single-layer parity of the CUDA kernels (through the C-ABI) against plain PyTorch fp32 ops on the GPU.
+"""Single layers of the CUDA kernels (through the C-ABI) against the exact single-op reference of tests/_layer_ref.py.
 
-Tolerances: bf16 operands are rounded identically on both sides, so only the fp32 accumulation order differs.
+The operands are exactly representable on both sides, so every stored output must be the correctly rounded value of
+the float64 result, up to the fp32 accumulation allowance (pools: bit-identical).
 """
 import ctypes
 
@@ -9,6 +10,7 @@ import torch
 import torch.nn.functional as F
 
 from bio_image_unet_b200 import _lib
+from tests import _layer_ref as R
 
 pytestmark = pytest.mark.gpu
 
@@ -63,12 +65,9 @@ def _run_conv_tc(esz, B, cin, cout, D, H, W, k3d, seed, in_ctot=None, in_coff=0,
                          _lib.ptr(scale), _lib.ptr(shift), 0.1, _lib.ptr(out), out_ctot, out_coff, _lib.stream_ptr())
     _lib.check(rc, 'biu_conv_tc')
     _sync_check()
-    xs = x[:, in_coff:in_coff + cin].float()
-    ref = F.conv3d(xs, w.float(), padding=(kd // 2, 1, 1)) if dims3 else F.conv2d(xs, w.float(), padding=1)
-    bshape = (1, cout, 1, 1, 1) if dims3 else (1, cout, 1, 1)
-    ref = F.leaky_relu(ref * scale.view(bshape) + shift.view(bshape), 0.1)
-    got = _nchw(out.float())[:, out_coff:out_coff + cout]
-    return got, ref
+    s, a = R.conv_sums(x_cl[..., in_coff:in_coff + cin], w, 3 if dims3 else 2)
+    lo, hi = R.interval(s, a, scale, shift, 0.1, 'bf16' if esz == 2 else 'tf32', R.C_GPU)
+    return out[..., out_coff:out_coff + cout].float(), lo, hi
 
 
 CASES_BF16 = [
@@ -89,25 +88,19 @@ CASES_BF16 = [
 @pytest.mark.parametrize('case', CASES_BF16)
 def test_conv_tc_bf16(case):
     B, cin, cout, D, H, W, k3d = case
-    got, ref = _run_conv_tc(2, B, cin, cout, D, H, W, k3d, seed=1)
-    err = (got - ref).abs().max().item()
-    # output is rounded to bf16: relative 2^-9 of values of magnitude <~ 4
-    assert err < 4e-2, err
-    assert torch.allclose(got, ref, rtol=1e-2, atol=1e-2)
+    R.check_interval(*_run_conv_tc(2, B, cin, cout, D, H, W, k3d, seed=1), f'conv_tc bf16 {case}')
 
 
 def test_conv_tc_bf16_concat_offsets():
-    got, ref = _run_conv_tc(2, 2, 64, 32, 1, 32, 32, False, seed=2, in_ctot=128, in_coff=64, out_ctot=96, out_coff=32)
-    assert torch.allclose(got, ref, rtol=1e-2, atol=1e-2)
+    R.check_interval(*_run_conv_tc(2, 2, 64, 32, 1, 32, 32, False, seed=2, in_ctot=128, in_coff=64, out_ctot=96,
+                                   out_coff=32), 'conv_tc bf16 concat offsets')
 
 
 @pytest.mark.parametrize('case', [(2, 32, 32, 1, 32, 32, False), (1, 64, 128, 1, 16, 16, False),
                                   (1, 16, 16, 4, 8, 8, True), (2, 8, 16, 1, 16, 16, False)])
 def test_conv_tc_tf32(case):
     B, cin, cout, D, H, W, k3d = case
-    got, ref = _run_conv_tc(4, B, cin, cout, D, H, W, k3d, seed=3)
-    # outputs are rounded to tf32 (2^-11 relative)
-    assert torch.allclose(got, ref, rtol=2e-3, atol=2e-3), (got - ref).abs().max().item()
+    R.check_interval(*_run_conv_tc(4, B, cin, cout, D, H, W, k3d, seed=3), f'conv_tc tf32 {case}')
 
 
 @pytest.mark.parametrize('dims,cin,cout', [(2, 64, 32), (2, 512, 256), (3, 32, 32), (2, 32, 16)])
@@ -127,13 +120,14 @@ def test_up_tc(dims, cin, cout):
     bias_rep = bias.repeat(nq).contiguous()
     oshape = (B, 2 * D, 2 * H, 2 * W, cout) if dims == 3 else (B, 2 * H, 2 * W, cout)
     out = torch.zeros(oshape, device='cuda', dtype=torch.bfloat16)
-    rc = lib.biu_up_tc(2, _lib.ptr(_nhwc(x)), cin, 0, cin, B, D, H, W, dims, _lib.ptr(wp), cout, _lib.ptr(bias_rep),
+    x_cl = _nhwc(x)
+    rc = lib.biu_up_tc(2, _lib.ptr(x_cl), cin, 0, cin, B, D, H, W, dims, _lib.ptr(wp), cout, _lib.ptr(bias_rep),
                        _lib.ptr(out), cout, 0, _lib.stream_ptr())
     _lib.check(rc, 'biu_up_tc')
     _sync_check()
-    ref = (F.conv_transpose3d if dims == 3 else F.conv_transpose2d)(x.float(), w.float(), bias, stride=2)
-    got = _nchw(out.float())
-    assert torch.allclose(got, ref, rtol=1e-2, atol=1e-2), (got - ref).abs().max().item()
+    s, a = R.up_sums(_nhwc(x), w, dims)
+    lo, hi = R.interval(s, a, torch.ones_like(bias), bias, 1.0, 'bf16', R.C_GPU)
+    R.check_interval(out.float(), lo, hi, f'up_tc {dims}D {cin}->{cout}')
 
 
 @pytest.mark.parametrize('esz', [2, 4])
@@ -149,14 +143,15 @@ def test_conv_direct(esz):
     shift = torch.randn(cout, device='cuda', generator=g) * 0.1
     wp = w.permute(2, 3, 1, 0).contiguous().view(9, cin, cout)
     out = torch.zeros(B, H, W, cout, device='cuda', dtype=dt)
-    rc = lib.biu_conv_direct(esz, _lib.ptr(_nhwc(x)), cin, 0, cin, B, 1, H, W, 1, 3, 3, _lib.ptr(wp), cout,
+    x_cl = _nhwc(x)
+    rc = lib.biu_conv_direct(esz, _lib.ptr(x_cl), cin, 0, cin, B, 1, H, W, 1, 3, 3, _lib.ptr(wp), cout,
                              _lib.ptr(scale), _lib.ptr(shift), 0.1, _lib.ptr(out), cout, 0, _lib.stream_ptr())
     _lib.check(rc, 'biu_conv_direct')
     _sync_check()
-    ref = F.leaky_relu(F.conv2d(x.float(), w, padding=1) * scale.view(1, -1, 1, 1) + shift.view(1, -1, 1, 1), 0.1)
-    got = _nchw(out.float())
-    tol = 1e-2 if esz == 2 else 1e-5
-    assert torch.allclose(got, ref, rtol=tol, atol=tol), (got - ref).abs().max().item()
+    # CUDA-core kernel: fp32 weights, fmaf accumulation; biu_conv_direct stores fp32 unrounded in the 4-byte format
+    s, a = R.conv_sums(_nhwc(x), w, 2)
+    lo, hi = R.interval(s, a, scale, shift, 0.1, 'bf16' if esz == 2 else 'fp32', R.C_GPU)
+    R.check_interval(out.float(), lo, hi, f'conv_direct esz={esz}')
 
 
 @pytest.mark.parametrize('dims,mode', [(2, 0), (3, 0), (3, 1)])
@@ -168,7 +163,8 @@ def test_pool2(dims, mode):
     x = torch.randn(shape, device='cuda', generator=g).bfloat16()
     oshape = (B, D // 2, H // 2, W // 2, C) if dims == 3 else (B, H // 2, W // 2, C)
     out = torch.zeros(oshape, device='cuda', dtype=torch.bfloat16)
-    rc = lib.biu_pool2(2, _lib.ptr(_nhwc(x)), C, 0, C, B, D, H, W, dims, mode, _lib.ptr(out), C, 0, _lib.stream_ptr())
+    x_cl = _nhwc(x)
+    rc = lib.biu_pool2(2, _lib.ptr(x_cl), C, 0, C, B, D, H, W, dims, mode, _lib.ptr(out), C, 0, _lib.stream_ptr())
     _lib.check(rc, 'biu_pool2')
     _sync_check()
     if mode == 0:
