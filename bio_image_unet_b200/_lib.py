@@ -23,6 +23,7 @@ SIGNATURES = {
     'biu_net_debug_copy': (c_int, [_P, c_char_p, _P, _P, c_longlong]),
     'biu_net_set_force_direct': (c_int, [_P, c_int]),
     'biu_net_set_fuse_pool': (c_int, [_P, c_int]),
+    'biu_net_set_debug_stop': (c_int, [_P, c_int]),
     'biu_set_rows_kernel': (c_int, [c_int]),
     'biu_set_halo_cta2': (c_int, [c_int]),
     'biu_net_fallback_ops': (c_int, [_P]),

@@ -122,6 +122,12 @@ int biu_net_set_fuse_pool(biu_net* net, int on) {
   net->n->no_fuse = on ? 0 : 1;
   return 0;
 }
+int biu_net_set_debug_stop(biu_net* net, int last_op) {
+  BIU_REQUIRE(net && net->n, "null handle");
+  BIU_REQUIRE(last_op >= -1, "last_op must be -1 (off) or an op index (got %d)", last_op);
+  net->n->debug_stop = last_op;
+  return 0;
+}
 void biu_net_destroy(biu_net* net) {
   if (!net) return;
   if (net->n) net_destroy(net->n);

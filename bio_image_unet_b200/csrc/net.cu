@@ -943,10 +943,15 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
     }
   }
   n->op_kinds.assign(n->ops.size(), 0);
+  n->stopped = false;
   int op_index = -1;
   bool skip_pool = false;           // the previous convolution wrote the pooled tensor from its epilogue
   for (const Op& o : n->ops) {
     ++op_index;
+    // debug stop: the ops up to debug_stop ran exactly as in a full forward (fusion included: a pool fused into
+    // op debug_stop's epilogue has been written); nothing after it runs, so a test can read what op debug_stop wrote
+    // before a later op reuses the buffer
+    if (n->debug_stop >= 0 && op_index > n->debug_stop) { n->stopped = true; break; }
     if (n->profile && op_index > 0) BIU_CHECK_CUDA(cudaEventRecord(n->events[2 * op_index - 1], stream));
     if (n->profile) BIU_CHECK_CUDA(cudaEventRecord(n->events[2 * op_index], stream));
     n->op_kinds[op_index] = (int)o.kind;
@@ -1296,12 +1301,15 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
       }
     }
   }
-  if (n->profile && !n->ops.empty()) BIU_CHECK_CUDA(cudaEventRecord(n->events[2 * n->ops.size() - 1], stream));
+  if (n->profile && !n->ops.empty() && !n->stopped)
+    BIU_CHECK_CUDA(cudaEventRecord(n->events[2 * n->ops.size() - 1], stream));
   return 0;
 }
 
 int net_profile_read(Net* n, int max_ops, int* kinds, float* ms, int* n_ops) {
   BIU_REQUIRE(n->profile && n->events.size() >= 2 * n->ops.size(), "profiling was not enabled for the last forward");
+  BIU_REQUIRE(!n->stopped, "the last forward stopped after op %d (biu_net_set_debug_stop): the later ops have no "
+              "timings", n->debug_stop);
   const int cnt = (int)n->ops.size() < max_ops ? (int)n->ops.size() : max_ops;
   for (int i = 0; i < cnt; ++i) {
     BIU_CHECK_CUDA(cudaEventSynchronize(n->events[2 * i + 1]));

@@ -101,6 +101,8 @@ struct Net {
   int force_direct = 0;             // debugging: run every conv on the CUDA-core kernels
   int no_fuse = 0;                  // debugging: keep the max-pool as its own kernel
   int profile = 0;                  // bracket every op with CUDA events
+  int debug_stop = -1;              // test hook: >= 0 ends net_forward after that op (-1: run the whole program)
+  bool stopped = false;             // the last forward ended at debug_stop (its profile events are incomplete)
   std::vector<cudaEvent_t> events;  // 2 per op
   std::vector<int> op_kinds;        // kind (+16 if it ran on the CUDA-core fallback) of the last forward
 };

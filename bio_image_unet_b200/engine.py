@@ -127,13 +127,16 @@ class Engine:
                               f"unaffected.", RuntimeWarning, stacklevel=3)
         return val, u8
 
-    def debug_activation(self, name, channels, level):
-        """Test hook: NHWC activation buffer `name` as a float32 host array (batch, [d,] h, w, channels)."""
+    def debug_activation(self, name, channels, level, images=None):
+        """Test hook: NHWC activation buffer `name` as a float32 host array (images, [d,] h, w, channels). images
+        defaults to the batch; a twin-encoder buffer of Siam_UNet holds 2 * batch images ([current | previous]), or
+        batch + siam_shared with the shared encoder."""
+        images = self.batch if images is None else int(images)
         d, h, w = self.tile
         dd = max(d >> level, 1) if self.kind in ('unet3d', 'mo3d') else 1
         hh, ww = h >> level, w >> level
         esz = 2 if self.precision in ('bf16', 'fp16') else 4
-        n = self.batch * dd * hh * ww * channels
+        n = images * dd * hh * ww * channels
         host = np.empty(n * esz, dtype=np.uint8)
         torch.cuda.synchronize(self.device)
         _lib.check(self.lib.biu_net_debug_copy(self.handle, name.encode(), _lib.ptr(self.workspace),
@@ -143,7 +146,13 @@ class Engine:
             t = torch.from_numpy(host.view(np.int16).copy()).view(dt).float().numpy()
         else:
             t = host.view(np.float32)
-        return t.reshape(self.batch, dd, hh, ww, channels)
+        return t.reshape(images, dd, hh, ww, channels)
+
+    def set_debug_stop(self, last_op):
+        """Test hook: the following forwards return after op `last_op` of the layer program (-1: run all of it), so
+        that what that op wrote can be read before a later op reuses the buffer. out_val / out_u8 are not written by
+        a stopped forward, and read_profile() refuses it."""
+        _lib.check(self.lib.biu_net_set_debug_stop(self.handle, int(last_op)), 'biu_net_set_debug_stop')
 
     def set_profile(self, on):
         """Bracket every op of the following forwards with CUDA events (read them with read_profile())."""

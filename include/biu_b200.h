@@ -77,6 +77,10 @@ int biu_net_set_force_direct(biu_net* net, int on);
 /* Test hook: 0 = run MaxPool2d as its own kernel instead of fusing it into the preceding block's epilogue
  * (default 1; both give bit-identical activations). */
 int biu_net_set_fuse_pool(biu_net* net, int on);
+/* Test hook: last_op >= 0 makes the following biu_net_forward calls return after op `last_op` of the layer program
+ * (a pool fused into that op's epilogue is written, as in a full forward); later ops, out_val and out_u8 are not
+ * written, and biu_net_profile_read refuses such a forward. -1 (the default) runs the whole program. */
+int biu_net_set_debug_stop(biu_net* net, int last_op);
 /* Siam_UNet with per-frame ('single') normalisation (siam_unet/predict.py:102-136, siam_unet/siam_unet.py:85-112): frame t
  * is the current frame of pair t and the previous frame of pair t + 1 and its normalised tiles - hence its encoder
  * output - are the same in both. tiles_per_frame > 0 makes the following biu_net_plan(batch B, ...) / biu_net_forward

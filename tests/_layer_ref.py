@@ -29,6 +29,7 @@ Parameter folding mirrors net_finalize (bio_image_unet_b200/csrc/net.cu):
 Works on CPU and CUDA tensors alike (the GPU tests compute their references in float64 on the device).
 """
 import math
+import warnings
 
 import torch
 
@@ -248,3 +249,94 @@ def nearest_x2(x, dims):
     if dims == 2:
         return x.repeat_interleave(2, 1).repeat_interleave(2, 2)
     return x.repeat_interleave(2, 1).repeat_interleave(2, 2).repeat_interleave(2, 3)
+
+
+# ------------------------------------------------------------------------------------------------ Siam_UNet joins
+def siam_streams(emb, batch, shared):
+    """(current, previous) embeddings of a twin-encoder buffer emb (images, ..., C) as the engine addresses them
+    (stream_img0 in net.cu): [current (B) | previous (B)], or with the shared encoder previous = images [0, B) and
+    current = images [shared, shared + B)."""
+    if shared > 0:
+        return emb[shared:shared + batch], emb[:batch]
+    return emb[:batch], emb[batch:2 * batch]
+
+
+def max_join(cur, prev):
+    """torch.maximum of the two stored embeddings: bit-exact, the kernel takes the maximum of stored values."""
+    return torch.maximum(cur, prev)
+
+
+def xcorr_sums(cur, prev):
+    """Depth-wise cross-correlation of Siam_UNet mode='corr' (siam_unet.py:75-83) of channels-last embeddings cur, prev
+    (B, h, w, C): S = F.conv2d(cur, prev, groups=B*C, padding='same') in float64 as PyTorch computes it (for even
+    extents the extra padding is at the far end), A the same of |cur|, |prev|, and the number n of in-bounds taps of
+    every output (a 'same' convolution of ones). Channels-last float64 (B, h, w, C) results; n (1, h, w, 1)."""
+    f = torch.nn.functional
+    b, h, w, c = cur.shape
+    x = _cl_to_cf(cur.double()).reshape(1, b * c, h, w)
+    k = _cl_to_cf(prev.double()).reshape(b * c, 1, h, w)
+    one = torch.ones((1, 1, h, w), dtype=torch.float64, device=x.device)
+    with warnings.catch_warnings():      # even extents: PyTorch notes that it pads a copy of the input
+        warnings.simplefilter('ignore', UserWarning)
+        s = f.conv2d(x, k, groups=b * c, padding='same').reshape(b, c, h, w).movedim(1, -1)
+        a = f.conv2d(x.abs(), k.abs(), groups=b * c, padding='same').reshape(b, c, h, w).movedim(1, -1)
+        n = f.conv2d(one, one, padding='same').movedim(1, -1)
+    return s, a, n
+
+
+def xcorr_interval(s, a, n, fmt, c=1.0):
+    """[lo, hi] of the stored correlation: the kernel sums the n taps of an output one after the other with fmaf in
+    fp32 (n roundings), so it lies within gamma_n * A, gamma_n = n u / (1 - n u), u = 2^-24, of S; then one rounding
+    to the storage format (tf32 in tf32 mode, fp16 with its +-inf)."""
+    an = a * (n / (1.0 - n * 2.0 ** -24))
+    z = torch.zeros(s.shape[-1], dtype=torch.float32)
+    return interval(s, an, z + 1.0, z, 1.0, fmt, c)
+
+
+def xcorr_min_c(got, s, a, n, fmt, ladder=(0.0, 0.125, 0.25, 0.5, 1.0)):
+    """Smallest c of the ladder (in units of gamma_n * A) for which every stored correlation passes (inf: none)."""
+    got = got.to(s.device).float()
+    for c in ladder:
+        lo, hi = xcorr_interval(s, a, n, fmt, c)
+        if not bool(violations(got, lo, hi).any()):
+            return c
+    return math.inf
+
+
+# ------------------------------------------------------------------------------------------------ bilinear x2
+def bilinear_coord(n):
+    """The kernel's fp32 source coordinates (bilinear_coord in net.cu) of the 2n outputs of an extent n, align_corners
+    True: f = fp32(fp32(n - 1) / fp32(2n - 1)) * o in fp32, i0 = min(int(f), n - 1), i1 = min(i0 + 1, n - 1),
+    l1 = clamp(f - i0, 0, 1). PyTorch evaluates float32 up-sampling with the same expressions
+    (area_pixel_compute_scale / guard_index_and_lambda). Returns (i0, i1) int64 tensors and l1 float32."""
+    o = torch.arange(2 * n, dtype=torch.float32)
+    s = torch.tensor(float(n - 1), dtype=torch.float32) / torch.tensor(float(2 * n - 1), dtype=torch.float32)
+    f = s * o
+    i0 = torch.clamp(f.to(torch.int64), max=n - 1)
+    i1 = torch.clamp(i0 + 1, max=n - 1)
+    l1 = torch.clamp(f - i0.to(torch.float32), 0.0, 1.0)
+    return i0, i1, l1
+
+
+def _lerp_matrix(n, device):
+    """(2n, n) float64 matrix of the fp32 weights (1 - l1 in fp32, l1) at (i0, i1)."""
+    i0, i1, l1 = bilinear_coord(n)
+    m = torch.zeros((2 * n, n), dtype=torch.float64)
+    r = torch.arange(2 * n)
+    m[r, i0] += (1.0 - l1).double()
+    m[r, i1] += l1.double()
+    return m.to(device)
+
+
+def bilinear_x2(x):
+    """Bilinear x2 up-sampling with align_corners=True of a channels-last (N, H, W, C) tensor, in float64 with the
+    kernel's (and PyTorch float32's) fp32 coordinates and weights, and the matching |.|-sum for the allowance (the
+    weights are non-negative). F.interpolate on float64 would take float64 coordinates instead: at extent 64 they move
+    a weight by up to about 2^-17, more than the fp32 evaluation's own error, so they are not what the kernel is
+    held to. tests/test_layer_ref_host.py shows that this equals F.interpolate of float32 inputs."""
+    n, h, w, c = x.shape
+    mh, mw = _lerp_matrix(h, x.device), _lerp_matrix(w, x.device)
+    xd = x.double()
+    r = torch.einsum('yh,nhwc,xw->nyxc', mh, xd, mw)
+    a = torch.einsum('yh,nhwc,xw->nyxc', mh, xd.abs(), mw)
+    return r, a

@@ -2,6 +2,7 @@
 and each of the small kernel mistakes it is meant to catch fails it. Runs without a GPU."""
 import math
 
+import numpy as np
 import pytest
 import torch
 
@@ -193,3 +194,172 @@ def test_interval_keeps_infinities_of_fp16_overflow():
     R.check_interval(got, lo, hi, 'overflow')
     with pytest.raises(R.IntervalError):
         R.check_interval(torch.tensor([60000.0, 65504.0, -math.inf, 1.0]), lo, hi, 'saturated')
+
+
+# ------------------------------------------------------------------------------------------------ Siam_UNet joins
+def _twin_buffer(fmt, images, h=4, w=4, c=16, seed=5):
+    g = torch.Generator().manual_seed(seed)
+    return _operands(fmt, (images, h, w, c), g)
+
+
+@pytest.mark.parametrize('shared', [0, 2])
+def test_max_join_reference_and_planted_mistakes(shared):
+    """The engine's stream addressing (net.cu stream_img0) passes; a stream taken one image off, and min in place of
+    max, fail."""
+    B = 3
+    emb = _twin_buffer('bf16', B + shared if shared else 2 * B)
+    cur0 = shared if shared else 0
+    prev0 = 0 if shared else B
+    want = R.max_join(*R.siam_streams(emb, B, shared))
+    assert torch.equal(torch.maximum(emb[cur0:cur0 + B], emb[prev0:prev0 + B]), want)
+    off = cur0 - 1 if shared else cur0 + 1          # current stream addressed one image off
+    assert not torch.equal(torch.maximum(emb[off:off + B], emb[prev0:prev0 + B]), want)
+    assert not torch.equal(torch.minimum(emb[cur0:cur0 + B], emb[prev0:prev0 + B]), want)
+
+
+def _xcorr_emulate(cur, prev, fmt, near_pad=False, drop=None, trunc=False):
+    """xcorr_join_kernel: out[b, y, x, c] = sum over i, j of cur[b, y + i - pt, x + j - pl, c] * prev[b, i, j, c],
+    pt = (h - 1) // 2, pl = (w - 1) // 2, the in-bounds taps one after the other (i outer, j inner) with one fp32
+    rounding each (fmaf), then one rounding to the storage format. near_pad: pt = h // 2, pl = w // 2 (the extra pad
+    at the near end); drop = (i, j): that tap is left out; trunc: bf16 by truncation instead of rounding."""
+    b, h, w, c = cur.shape
+    pt, pl = (h // 2, w // 2) if near_pad else ((h - 1) // 2, (w - 1) // 2)
+    xp = torch.nn.functional.pad(cur.double(), (0, 0, pl, w - 1 - pl, pt, h - 1 - pt))
+    acc = torch.zeros(b, h, w, c, dtype=torch.float32)
+    for i in range(h):
+        for j in range(w):
+            if (i, j) == drop:
+                continue
+            p = xp[:, i:i + h, j:j + w, :] * prev[:, i:i + 1, j:j + 1, :].double()   # exact products
+            acc = (acc.double() + p).float()                                         # one rounding per tap
+    if trunc:
+        return (acc.view(torch.int32) & ~0xFFFF).view(torch.float32)
+    return R.round_to(acc, fmt)
+
+
+def _xcorr_check(got, cur, prev, fmt):
+    s, a, n = R.xcorr_sums(cur, prev)
+    lo, hi = R.xcorr_interval(s, a, n, fmt)
+    R.check_interval(got, lo, hi, f'xcorr {fmt}')
+
+
+@pytest.mark.parametrize('fmt', ['bf16', 'fp16', 'tf32', 'fp32'])
+@pytest.mark.parametrize('hw', [(4, 4), (5, 3), (6, 8)])
+def test_xcorr_reference_passes_the_kernel_emulation(fmt, hw):
+    h, w = hw
+    g = torch.Generator().manual_seed(h * 10 + w)
+    op = 'bf16' if fmt == 'fp32' else fmt
+    cur, prev = _operands(op, (2, h, w, 16), g), _operands(op, (2, h, w, 16), g)
+    _xcorr_check(_xcorr_emulate(cur, prev, fmt), cur, prev, fmt)
+    _, _, n = R.xcorr_sums(cur, prev)
+    # 'same' padding with the extra pad at the far end: for even extents the near corner sees more taps than the far
+    pt, pl = (h - 1) // 2, (w - 1) // 2
+    assert float(n.max()) == h * w
+    assert float(n[0, 0, 0, 0]) == (h - pt) * (w - pl) and float(n[0, -1, -1, 0]) == (pt + 1) * (pl + 1)
+
+
+@pytest.mark.parametrize('mistake', ['near_pad', 'drop_border_tap', 'swap', 'bf16_trunc'])
+def test_xcorr_reference_rejects_planted_mistakes(mistake):
+    fmt = 'bf16'
+    g = torch.Generator().manual_seed(9)
+    cur, prev = _operands(fmt, (2, 4, 6, 16), g), _operands(fmt, (2, 4, 6, 16), g)
+    if mistake == 'near_pad':              # even extents: the extra pad at the near end
+        got = _xcorr_emulate(cur, prev, fmt, near_pad=True)
+    elif mistake == 'drop_border_tap':     # the last tap of the correlation window left out
+        got = _xcorr_emulate(cur, prev, fmt, drop=(3, 5))
+    elif mistake == 'swap':                # cur and prev exchanged
+        got = _xcorr_emulate(prev, cur, fmt)
+    else:
+        got = _xcorr_emulate(cur, prev, fmt, trunc=True)
+    with pytest.raises(R.IntervalError):
+        _xcorr_check(got, cur, prev, fmt)
+
+
+def test_xcorr_reference_sees_one_dropped_tap_at_1024_taps():
+    """32 x 32 embeddings: every output sums up to 1024 taps, the allowance is gamma_1024 A, and one dropped product
+    still moves many outputs past it (tf32 storage, where no bf16 rounding hides the difference)."""
+    g = torch.Generator().manual_seed(4)
+    cur = _operands('tf32', (1, 32, 32, 4), g).abs()
+    prev = _operands('tf32', (1, 32, 32, 4), g).abs()
+    _xcorr_check(_xcorr_emulate(cur, prev, 'tf32'), cur, prev, 'tf32')
+    with pytest.raises(R.IntervalError):
+        _xcorr_check(_xcorr_emulate(cur, prev, 'tf32', drop=(16, 16)), cur, prev, 'tf32')
+
+
+# ------------------------------------------------------------------------------------------------ bilinear x2
+def test_bilinear_coordinates_match_pytorch_and_share_pairs():
+    """For every extent 1 ... 64: the kernel's fp32 coordinate rule gives bit for bit the weights of PyTorch's float32
+    F.interpolate(bilinear, align_corners=True), its (i0, i1) agree with the exact rule floor(o (n - 1) / (2n - 1)),
+    and output rows 2p - 1 and 2p always interpolate between the same two source rows p - 1 and p. So
+    up_bilinear_kernel's 2 x 2 path covers every output, and its per-pixel path is never taken."""
+    f = torch.nn.functional
+    for n in range(1, 65):
+        x = torch.eye(n, dtype=torch.float32).reshape(1, n, n, 1)          # channel c: one-hot source row c
+        y = f.interpolate(x, scale_factor=2, mode='bilinear', align_corners=True)[0, :, :, 0].t()
+        assert torch.equal(y.double(), R._lerp_matrix(n, 'cpu')), n
+        i0, i1, _ = R.bilinear_coord(n)
+        o = torch.arange(2 * n, dtype=torch.int64)
+        exact = torch.clamp((o * (n - 1)) // max(2 * n - 1, 1), max=n - 1)
+        assert torch.equal(i0, exact) and torch.equal(i1, torch.clamp(exact + 1, max=n - 1)), n
+        for p in range(1, n):
+            assert int(i0[2 * p - 1]) == int(i0[2 * p]) == p - 1 and int(i1[2 * p - 1]) == int(i1[2 * p]) == p, (n, p)
+
+
+def _bilinear_emulate(x, shift_src=False, copy_last_row=False):
+    """up_bilinear_kernel in fp32: coordinates f = fp32((n-1)/(2n-1)) * o, lerps h0 (w0 v00 + w1 v01) + h1 (...),
+    each product and sum rounded to fp32. shift_src: every source coordinate one pixel further (clamped);
+    copy_last_row: the last output row is a copy of the row before."""
+    def coords(n):
+        s = np.float32(n - 1) / np.float32(2 * n - 1)
+        out = []
+        for o in range(2 * n):
+            fo = np.float32(s * np.float32(o))
+            i0 = min(int(fo), n - 1)
+            l1 = np.float32(min(max(fo - np.float32(i0), np.float32(0)), np.float32(1)))
+            if shift_src:
+                i0 = min(i0 + 1, n - 1)
+            out.append((i0, min(i0 + 1, n - 1), float(np.float32(1) - l1), float(l1)))
+        return out
+    b, h, w, c = x.shape
+    ys, xs = coords(h), coords(w)
+    xf = x.float()
+    out = torch.empty(b, 2 * h, 2 * w, c, dtype=torch.float32)
+    for oy, (y0, y1, h0, h1) in enumerate(ys):
+        for ox, (x0, x1, w0, w1) in enumerate(xs):
+            t = xf[:, y0, x0] * w0 + xf[:, y0, x1] * w1
+            bt = xf[:, y1, x0] * w0 + xf[:, y1, x1] * w1
+            out[:, oy, ox] = t * h0 + bt * h1
+    if copy_last_row:
+        out[:, -1] = out[:, -2]
+    return out
+
+
+def _bilinear_check(got, x, fmt):
+    s, a = R.bilinear_x2(x)
+    z = torch.zeros(x.shape[-1])
+    lo, hi = R.interval(s, a, z + 1.0, z, 1.0, fmt, c=16.0)
+    R.check_interval(got, lo, hi, f'bilinear {fmt}')
+
+
+@pytest.mark.parametrize('fmt', ['bf16', 'fp16', 'tf32', 'fp32'])
+@pytest.mark.parametrize('hw', [(1, 2), (3, 5), (8, 12)])
+def test_bilinear_reference_passes_the_kernel_emulation(fmt, hw):
+    g = torch.Generator().manual_seed(hw[0] * 100 + hw[1])
+    x = _operands('bf16' if fmt == 'fp32' else fmt, (2, *hw, 16), g)
+    _bilinear_check(R.round_to(_bilinear_emulate(x), fmt), x, fmt)
+
+
+@pytest.mark.parametrize('mistake', ['align_corners_false', 'source_off_by_one', 'last_row_copied'])
+@pytest.mark.parametrize('fmt', ['bf16', 'tf32'])
+def test_bilinear_reference_rejects_planted_mistakes(mistake, fmt):
+    g = torch.Generator().manual_seed(2)
+    x = _operands(fmt, (2, 6, 10, 16), g)
+    if mistake == 'align_corners_false':
+        got = torch.nn.functional.interpolate(x.movedim(-1, 1), scale_factor=2, mode='bilinear',
+                                              align_corners=False).movedim(1, -1)
+    elif mistake == 'source_off_by_one':
+        got = _bilinear_emulate(x, shift_src=True)
+    else:
+        got = _bilinear_emulate(x, copy_last_row=True)
+    with pytest.raises(R.IntervalError):
+        _bilinear_check(R.round_to(got, fmt), x, fmt)
