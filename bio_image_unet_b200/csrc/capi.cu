@@ -21,12 +21,12 @@ unsigned long long g_launch_count = 0;
 
 using namespace biu;
 
-// `esz` of the layer entry points: 2 = bf16, 4 = fp32, BIU_ESZ_FP16 = fp16 -> storage bytes and fp16 flag
-static int layer_format(int esz, int* bytes, int* f16) {
+// `esz` of the layer entry points: 2 = bf16, BIU_ESZ_FP16 = fp16, 4 = fp32 -> ElemFmt. The tensor-core entry points take
+// fp32 storage as tf32 operands (fp32_fmt = FMT_TF32); the CUDA-core ones store it unrounded (FMT_F32).
+static int layer_format(int esz, int fp32_fmt, int* fmt) {
   BIU_REQUIRE(esz == 2 || esz == 4 || esz == BIU_ESZ_FP16, "unknown element code esz=%d (2 = bf16, %d = fp16, 4 = fp32)",
               esz, BIU_ESZ_FP16);
-  *bytes = esz == 4 ? 4 : 2;
-  *f16 = esz == BIU_ESZ_FP16 ? 1 : 0;
+  *fmt = esz == 4 ? fp32_fmt : (esz == BIU_ESZ_FP16 ? FMT_F16 : FMT_BF16);
   return 0;
 }
 
@@ -43,10 +43,12 @@ biu_net* biu_net_create(int kind, int n_filter, int in_channels, int n_heads, co
                         const int* head_acts, const char* const* head_names, int siam_mode, int use_interpolation,
                         int precision) {
   if (kind < 0 || kind > 8) { set_error("unknown network kind %d", kind); return nullptr; }
+  static_assert(BIU_PREC_BF16 == 0 && BIU_PREC_TF32 == 1 && BIU_PREC_FP32 == 2 && BIU_PREC_FP16 == 3, "prec_fmt order");
+  static const int prec_fmt[4] = {FMT_BF16, FMT_TF32, FMT_F32, FMT_F16};
   if (precision < 0 || precision > 3) { set_error("unknown precision %d", precision); return nullptr; }
   if (n_heads < 1 || !head_channels || !head_acts) { set_error("at least one output head is required"); return nullptr; }
   Net* n = new Net();
-  n->kind = kind; n->nf = n_filter; n->in_ch = in_channels; n->precision = precision;
+  n->kind = kind; n->nf = n_filter; n->in_ch = in_channels; n->fmt = prec_fmt[precision];
   n->siam_mode = siam_mode; n->use_interp = use_interpolation;
   for (int i = 0; i < n_heads; ++i) {
     n->head_channels.push_back(head_channels[i]);
@@ -198,7 +200,7 @@ int biu_conv_tc(int esz, const void* in, int in_ctot, int in_coff, int cin, int 
                 void* out, int out_ctot, int out_coff, void* stream) {
   ConvTcArgs a;
   memset(&a, 0, sizeof(a));
-  if (int rc = layer_format(esz, &a.esz, &a.f16)) return rc;
+  if (int rc = layer_format(esz, FMT_TF32, &a.fmt)) return rc;
   a.in = in; a.in_ctot = in_ctot; a.in_coff = in_coff; a.cin = cin;
   a.W = W; a.H = H; a.D = D; a.B = B; a.kw = kw; a.kh = kh; a.kd = kd;
   a.wgt = wgt; a.n_total = cout; a.mode = EPI_CONV; a.slope = slope; a.scale = scale; a.shift = shift;
@@ -209,7 +211,7 @@ int biu_up_tc(int esz, const void* in, int in_ctot, int in_coff, int cin, int B,
               const void* wgt, int cout, const float* bias_rep, void* out, int out_ctot, int out_coff, void* stream) {
   ConvTcArgs a;
   memset(&a, 0, sizeof(a));
-  if (int rc = layer_format(esz, &a.esz, &a.f16)) return rc;
+  if (int rc = layer_format(esz, FMT_TF32, &a.fmt)) return rc;
   a.in = in; a.in_ctot = in_ctot; a.in_coff = in_coff; a.cin = cin;
   a.W = W; a.H = H; a.D = D; a.B = B; a.kw = a.kh = a.kd = 1;
   a.wgt = wgt; a.n_total = (dims == 3 ? 8 : 4) * cout; a.mode = EPI_UP; a.slope = 1.f; a.scale = bias_rep;
@@ -221,7 +223,7 @@ int biu_conv_direct(int esz, const void* in, int in_ctot, int in_coff, int cin, 
                     void* out, int out_ctot, int out_coff, void* stream) {
   DirectConvArgs a;
   memset(&a, 0, sizeof(a));
-  if (int rc = layer_format(esz, &a.esz, &a.f16)) return rc;
+  if (int rc = layer_format(esz, FMT_F32, &a.fmt)) return rc;
   a.in = in; a.in_ctot = in_ctot; a.in_coff = in_coff; a.cin = cin;
   a.W = W; a.H = H; a.D = D; a.B = B; a.kw = kw; a.kh = kh; a.kd = kd;
   a.wgt = wgt; a.cout = cout; a.slope = slope; a.scale = scale; a.shift = shift;
@@ -232,7 +234,7 @@ int biu_pool2(int esz, const void* in, int in_ctot, int in_coff, int c, int B, i
               int mode, void* out, int out_ctot, int out_coff, void* stream) {
   PoolArgs a;
   memset(&a, 0, sizeof(a));
-  if (int rc = layer_format(esz, &a.esz, &a.f16)) return rc;
+  if (int rc = layer_format(esz, FMT_F32, &a.fmt)) return rc;
   a.in = in; a.in_ctot = in_ctot; a.in_coff = in_coff; a.c = c; a.W = W; a.H = H; a.D = D; a.B = B;
   a.dims = dims; a.mode = mode; a.out = out; a.out_ctot = out_ctot; a.out_coff = out_coff;
   return launch_pool2(a, (cudaStream_t)stream);

@@ -10,6 +10,7 @@
 #include <cuda_fp16.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <type_traits>
 
 namespace biu {
 
@@ -50,13 +51,34 @@ __host__ __device__ inline int ceil_div(int a, int b) { return (a + b - 1) / b; 
 __host__ __device__ inline long long ceil_div_ll(long long a, long long b) { return (a + b - 1) / b; }
 
 // ----------------------------------------------------------------------------------------------
-// Element formats of the activations and tcgen05 operands. bf16 and fp32 / tf32 are coded by their byte size (the `esz`
-// of the layer C-ABI, the template argument of the kernels); fp16 is a second 2-byte format with a code of its own.
+// Element formats of the activations and tcgen05 operands: the template argument of the kernels and the `fmt` of every
+// launcher argument block. The values of bf16, fp16 and tf32 are the element codes of the layer C-ABI. FMT_TF32 is fp32
+// storage rounded to tf32 (the tensor core's operand format); FMT_F32 is fp32 storage that is never rounded (the exact
+// fp32 mode, CUDA-core kernels only).
 // ----------------------------------------------------------------------------------------------
-enum ElemFmt { FMT_BF16 = 2, FMT_F16 = 3, FMT_TF32 = 4 };
-__host__ __device__ constexpr int fmt_esz(int fmt) { return fmt == FMT_TF32 ? 4 : 2; }
+enum ElemFmt { FMT_BF16 = 2, FMT_F16 = 3, FMT_TF32 = 4, FMT_F32 = 5 };
+__host__ __device__ constexpr int fmt_esz(int fmt) { return fmt == FMT_TF32 || fmt == FMT_F32 ? 4 : 2; }
 // A / B format field of the tcgen05 instruction descriptor (make_idesc)
 __host__ __device__ constexpr uint32_t fmt_idesc(int fmt) { return fmt == FMT_F16 ? 0u : (fmt == FMT_BF16 ? 1u : 2u); }
+
+// Storage type of a format: with_elem_type(fmt, f) calls f(ElemTag<T>{}) with T = __nv_bfloat16, __half or float, and
+// returns f's result (an error code). fmt_of<T> / ElemTag<T>::fmt is the tensor-core format of a storage type.
+template <typename T>
+constexpr int fmt_of = sizeof(T) == 4 ? FMT_TF32 : (std::is_same<T, __half>::value ? FMT_F16 : FMT_BF16);
+template <typename T> struct ElemTag {
+  using type = T;
+  static constexpr int fmt = fmt_of<T>;
+};
+template <typename F>
+int with_elem_type(int fmt, F&& f) {
+  switch (fmt) {
+    case FMT_BF16: return f(ElemTag<__nv_bfloat16>{});
+    case FMT_F16: return f(ElemTag<__half>{});
+    case FMT_TF32:
+    case FMT_F32: return f(ElemTag<float>{});
+  }
+  BIU_REQUIRE(false, "unknown element format %d", fmt);
+}
 
 #ifdef __CUDACC__
 

@@ -769,16 +769,6 @@ __global__ void __launch_bounds__(kHaloThreads, 1) conv_halo_kernel(const __grid
   if (warp == 1) { if (CTA2) tmem_dealloc2(tmem_base, ncols); else tmem_dealloc(tmem_base, ncols); }
 }
 
-// Host-side dispatch over the (k-steps per chunk, MMA tiles per work item) instantiations of one element format;
-// defined in conv_halo_bf16.cu / conv_halo_f16.cu / conv_halo_tf32.cu through BIU_DEFINE_HALO_DISPATCH so they compile in
-// parallel.
-int halo_dispatch_bf16(const CUtensorMap& tmA, const CUtensorMap& tmB, const ConvHaloParams& p, int grid, int smem,
-                       cudaStream_t stream);
-int halo_dispatch_f16(const CUtensorMap& tmA, const CUtensorMap& tmB, const ConvHaloParams& p, int grid, int smem,
-                      cudaStream_t stream);
-int halo_dispatch_tf32(const CUtensorMap& tmA, const CUtensorMap& tmB, const ConvHaloParams& p, int grid, int smem,
-                       cudaStream_t stream);
-
 #define BIU_HALO_LAUNCH(E, K, M)                                                                                  \
   do {                                                                                                             \
     if (p.cta2) {                                                                                                  \
@@ -811,19 +801,14 @@ int halo_dispatch_tf32(const CUtensorMap& tmA, const CUtensorMap& tmB, const Con
     if (p.mt == 8) BIU_HALO_LAUNCH(E, K, 8); else if (p.mt == 4) BIU_HALO_LAUNCH(E, K, 4);                          \
     else if (p.mt == 2) BIU_HALO_LAUNCH(E, K, 2); else BIU_HALO_LAUNCH(E, K, 1);                                    \
   } while (0)
-#define BIU_DEFINE_HALO_DISPATCH(NAME, E)                                                                          \
-  int NAME(const CUtensorMap& tmA, const CUtensorMap& tmB, const ConvHaloParams& p, int grid, int smem,            \
-           cudaStream_t stream) {                                                                                  \
-    const int ks = p.row_bytes / 32;                                                                               \
-    if (ks == 4) BIU_HALO_LAUNCH_M(E, 4); else if (ks == 2) BIU_HALO_LAUNCH_M(E, 2); else BIU_HALO_LAUNCH_M(E, 1); \
-    return 0;                                                                                                      \
-  }
-
-// Co-resident CTA pairs of the 2-CTA kernel with `smem` bytes of dynamic shared memory (0: no cluster launch possible).
-// The kernel is persistent with a static tile stride, so its grid must not exceed what is resident at once.
-int halo_max_pairs_bf16(int ks, int mt, int smem);
-int halo_max_pairs_f16(int ks, int mt, int smem);
-int halo_max_pairs_tf32(int ks, int mt, int smem);
+// Host-side dispatch over the (k-steps per chunk, MMA tiles per work item) instantiations of one element format.
+template <int FMT>
+int halo_dispatch(const CUtensorMap& tmA, const CUtensorMap& tmB, const ConvHaloParams& p, int grid, int smem,
+                  cudaStream_t stream) {
+  const int ks = p.row_bytes / 32;
+  if (ks == 4) BIU_HALO_LAUNCH_M(FMT, 4); else if (ks == 2) BIU_HALO_LAUNCH_M(FMT, 2); else BIU_HALO_LAUNCH_M(FMT, 1);
+  return 0;
+}
 
 #define BIU_HALO_PAIRS(E, K, M)                                                                                    \
   do {                                                                                                             \
@@ -848,10 +833,22 @@ int halo_max_pairs_tf32(int ks, int mt, int smem);
     if (mt == 8) BIU_HALO_PAIRS(E, K, 8); else if (mt == 4) BIU_HALO_PAIRS(E, K, 4);                                \
     else if (mt == 2) BIU_HALO_PAIRS(E, K, 2); else BIU_HALO_PAIRS(E, K, 1);                                        \
   } while (0)
-#define BIU_DEFINE_HALO_PAIRS(NAME, E)                                                                             \
-  int NAME(int ks, int mt, int smem) {                                                                             \
-    if (ks == 4) BIU_HALO_PAIRS_M(E, 4); else if (ks == 2) BIU_HALO_PAIRS_M(E, 2); else BIU_HALO_PAIRS_M(E, 1);     \
-    return 0;                                                                                                      \
-  }
+// Co-resident CTA pairs of the 2-CTA kernel with `smem` bytes of dynamic shared memory (0: no cluster launch possible).
+// The kernel is persistent with a static tile stride, so its grid must not exceed what is resident at once.
+template <int FMT>
+int halo_max_pairs(int ks, int mt, int smem) {
+  if (ks == 4) BIU_HALO_PAIRS_M(FMT, 4); else if (ks == 2) BIU_HALO_PAIRS_M(FMT, 2); else BIU_HALO_PAIRS_M(FMT, 1);
+  return 0;
+}
+
+// Each element format is instantiated in a translation unit of its own (conv_halo_bf16.cu / _f16.cu / _tf32.cu:
+// BIU_HALO_INSTANCES(, FMT)), so that they compile in parallel; every other unit only declares them.
+#define BIU_HALO_INSTANCES(EXTERN, E)                                                                                \
+  EXTERN template int halo_dispatch<E>(const CUtensorMap&, const CUtensorMap&, const ConvHaloParams&, int, int,      \
+                                       cudaStream_t);                                                                \
+  EXTERN template int halo_max_pairs<E>(int, int, int);
+BIU_HALO_INSTANCES(extern, FMT_BF16)
+BIU_HALO_INSTANCES(extern, FMT_F16)
+BIU_HALO_INSTANCES(extern, FMT_TF32)
 
 }  // namespace biu

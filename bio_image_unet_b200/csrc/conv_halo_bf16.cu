@@ -2,6 +2,5 @@
 #include <cstring>
 #include "conv_halo.cuh"
 namespace biu {
-BIU_DEFINE_HALO_DISPATCH(halo_dispatch_bf16, 2)
-BIU_DEFINE_HALO_PAIRS(halo_max_pairs_bf16, 2)
+BIU_HALO_INSTANCES(, FMT_BF16)
 }  // namespace biu

@@ -2,6 +2,5 @@
 #include <cstring>
 #include "conv_halo.cuh"
 namespace biu {
-BIU_DEFINE_HALO_DISPATCH(halo_dispatch_tf32, 4)
-BIU_DEFINE_HALO_PAIRS(halo_max_pairs_tf32, 4)
+BIU_HALO_INSTANCES(, FMT_TF32)
 }  // namespace biu

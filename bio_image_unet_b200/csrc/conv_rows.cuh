@@ -894,13 +894,6 @@ __global__ void __launch_bounds__(kRowsThreads, 1) conv_rows_kernel(const __grid
   if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
-int rows_dispatch_bf16(const CUtensorMap& tmA, const CUtensorMap& tmW, const ConvRowsParams& p, int grid, int smem,
-                       cudaStream_t stream);
-int rows_dispatch_f16(const CUtensorMap& tmA, const CUtensorMap& tmW, const ConvRowsParams& p, int grid, int smem,
-                      cudaStream_t stream);
-int rows_dispatch_tf32(const CUtensorMap& tmA, const CUtensorMap& tmW, const ConvRowsParams& p, int grid, int smem,
-                       cudaStream_t stream);
-
 #define BIU_ROWS_LAUNCH(E, K)                                                                                     \
   do {                                                                                                             \
     static int max_set = 0;                                                                                        \
@@ -911,12 +904,22 @@ int rows_dispatch_tf32(const CUtensorMap& tmA, const CUtensorMap& tmW, const Con
     }                                                                                                              \
     conv_rows_kernel<E, K><<<grid, kRowsThreads, smem, stream>>>(tmA, tmW, p);                                     \
   } while (0)
-#define BIU_DEFINE_ROWS_DISPATCH(NAME, E)                                                                          \
-  int NAME(const CUtensorMap& tmA, const CUtensorMap& tmW, const ConvRowsParams& p, int grid, int smem,            \
-           cudaStream_t stream) {                                                                                  \
-    const int ks = p.row_bytes / 32;                                                                               \
-    if (ks == 4) BIU_ROWS_LAUNCH(E, 4); else if (ks == 2) BIU_ROWS_LAUNCH(E, 2); else BIU_ROWS_LAUNCH(E, 1);       \
-    return 0;                                                                                                      \
-  }
+// Host-side dispatch over the k-steps per chunk of one element format.
+template <int FMT>
+int rows_dispatch(const CUtensorMap& tmA, const CUtensorMap& tmW, const ConvRowsParams& p, int grid, int smem,
+                  cudaStream_t stream) {
+  const int ks = p.row_bytes / 32;
+  if (ks == 4) BIU_ROWS_LAUNCH(FMT, 4); else if (ks == 2) BIU_ROWS_LAUNCH(FMT, 2); else BIU_ROWS_LAUNCH(FMT, 1);
+  return 0;
+}
+
+// Each element format is instantiated in a translation unit of its own (conv_rows_bf16.cu / _f16.cu / _tf32.cu:
+// BIU_ROWS_INSTANCES(, FMT)), so that they compile in parallel; every other unit only declares them.
+#define BIU_ROWS_INSTANCES(EXTERN, E)                                                                                \
+  EXTERN template int rows_dispatch<E>(const CUtensorMap&, const CUtensorMap&, const ConvRowsParams&, int, int,      \
+                                       cudaStream_t);
+BIU_ROWS_INSTANCES(extern, FMT_BF16)
+BIU_ROWS_INSTANCES(extern, FMT_F16)
+BIU_ROWS_INSTANCES(extern, FMT_TF32)
 
 }  // namespace biu

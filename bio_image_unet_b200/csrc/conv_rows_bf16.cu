@@ -1,5 +1,5 @@
 // bf16 instantiations of the row-streaming folded-tap convolution kernel (conv_rows.cuh)
 #include "conv_rows.cuh"
 namespace biu {
-BIU_DEFINE_ROWS_DISPATCH(rows_dispatch_bf16, 2)
+BIU_ROWS_INSTANCES(, FMT_BF16)
 }  // namespace biu

@@ -1,5 +1,5 @@
 // fp16 instantiations of the row-streaming folded-tap convolution kernel (conv_rows.cuh)
 #include "conv_rows.cuh"
 namespace biu {
-BIU_DEFINE_ROWS_DISPATCH(rows_dispatch_f16, FMT_F16)
+BIU_ROWS_INSTANCES(, FMT_F16)
 }  // namespace biu

@@ -1,5 +1,5 @@
 // tf32 (fp32 storage) instantiations of the row-streaming folded-tap convolution kernel (conv_rows.cuh)
 #include "conv_rows.cuh"
 namespace biu {
-BIU_DEFINE_ROWS_DISPATCH(rows_dispatch_tf32, 4)
+BIU_ROWS_INSTANCES(, FMT_TF32)
 }  // namespace biu

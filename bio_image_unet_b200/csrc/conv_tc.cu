@@ -47,13 +47,15 @@ void choose_box(int W, int H, int D, int B, int* lbw, int* lbh, int* lbd, int* l
   *lbw = lw; *lbh = lh; *lbd = ld; *lbb = lb;
 }
 
-static CUtensorMapDataType tma_dtype(int esz, int f16) {
-  return esz == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : (f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16);
+static CUtensorMapDataType tma_dtype(int fmt) {
+  return fmt == FMT_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
+                         : (fmt == FMT_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32);
 }
 
-static int encode_act_map(CUtensorMap* tm, const void* base, int esz, int f16, int C, int W, int H, int D, int B, int ctot,
+static int encode_act_map(CUtensorMap* tm, const void* base, int fmt, int C, int W, int H, int D, int B, int ctot,
                           int ck, int bw, int bh, int bd, int bb) {
   EncodeTiledFn enc = get_encode_fn();
+  const int esz = fmt_esz(fmt);
   BIU_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled entry point not available");
   cuuint64_t dims[5] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)D, (cuuint64_t)B};
   cuuint64_t strides[4] = {(cuuint64_t)ctot * esz, (cuuint64_t)W * ctot * esz, (cuuint64_t)H * W * ctot * esz,
@@ -63,7 +65,7 @@ static int encode_act_map(CUtensorMap* tm, const void* base, int esz, int f16, i
   const int rb = ck * esz;
   CUtensorMapSwizzle sw = rb == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
                                     : (rb == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
-  CUresult r = enc(tm, tma_dtype(esz, f16), 5,
+  CUresult r = enc(tm, tma_dtype(fmt), 5,
                    const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   BIU_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled(activations) failed with %d (C=%d W=%d H=%d D=%d B=%d ctot=%d ck=%d)",
@@ -71,9 +73,10 @@ static int encode_act_map(CUtensorMap* tm, const void* base, int esz, int f16, i
   return 0;
 }
 
-static int encode_wgt_map(CUtensorMap* tm, const void* base, int esz, int f16, int cin, int ntotal, int taps, int ck,
+static int encode_wgt_map(CUtensorMap* tm, const void* base, int fmt, int cin, int ntotal, int taps, int ck,
                           int n_blk) {
   EncodeTiledFn enc = get_encode_fn();
+  const int esz = fmt_esz(fmt);
   BIU_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled entry point not available");
   cuuint64_t dims[3] = {(cuuint64_t)cin, (cuuint64_t)ntotal, (cuuint64_t)taps};
   cuuint64_t strides[2] = {(cuuint64_t)cin * esz, (cuuint64_t)ntotal * cin * esz};
@@ -82,7 +85,7 @@ static int encode_wgt_map(CUtensorMap* tm, const void* base, int esz, int f16, i
   const int rb = ck * esz;
   CUtensorMapSwizzle sw = rb == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
                                     : (rb == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
-  CUresult r = enc(tm, tma_dtype(esz, f16), 3,
+  CUresult r = enc(tm, tma_dtype(fmt), 3,
                    const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   BIU_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled(weights) failed with %d (cin=%d n=%d taps=%d ck=%d nblk=%d)",
@@ -90,7 +93,8 @@ static int encode_wgt_map(CUtensorMap* tm, const void* base, int esz, int f16, i
   return 0;
 }
 
-int pick_ck(int cin, int esz) {
+int pick_ck(int cin, int fmt) {
+  const int esz = fmt_esz(fmt);
   const int cands[3] = {128 / esz, 64 / esz, 32 / esz};
   for (int i = 0; i < 3; ++i)
     if (cin % cands[i] == 0) return cands[i];
@@ -98,12 +102,12 @@ int pick_ck(int cin, int esz) {
 }
 
 bool conv_tc_supported(const ConvTcArgs& a) {
-  if (a.esz != 2 && a.esz != 4) return false;
-  if (a.f16 && a.esz != 2) return false;
-  if (pick_ck(a.cin, a.esz) == 0) return false;
+  if (a.fmt != FMT_BF16 && a.fmt != FMT_F16 && a.fmt != FMT_TF32) return false;
+  const int vec = 16 / fmt_esz(a.fmt);
+  if (pick_ck(a.cin, a.fmt) == 0) return false;
   if (a.n_total % 16 != 0) return false;
-  if (a.in_ctot % (16 / a.esz) != 0 || a.in_coff % (16 / a.esz) != 0) return false;
-  if (a.mode != EPI_HEAD && (a.out_ctot % (16 / a.esz) != 0 || a.out_coff % (16 / a.esz) != 0)) return false;
+  if (a.in_ctot % vec != 0 || a.in_coff % vec != 0) return false;
+  if (a.mode != EPI_HEAD && (a.out_ctot % vec != 0 || a.out_coff % vec != 0)) return false;
   if (a.mode == EPI_UP && a.up_cout % 16 != 0) return false;
   if (a.mode == EPI_HEAD && (a.n_total > 256 || a.head_n > kMaxHead)) return false;
   return true;
@@ -159,16 +163,17 @@ static HaloPlan plan_halo(const ConvTcArgs& a, int n_blk, bool cta2 = false) {
   HaloPlan pl{};
   pl.ok = false;
   if (!halo_shape_ok(a) || n_blk > 256) return pl;
+  const int esz = fmt_esz(a.fmt);
   if (cta2 && (n_blk % 32 != 0)) return pl;                // every CTA of a pair stages n_blk / 2 weight rows
   const int halo = a.kw == 3 ? 1 : 0;
   const int rows = 16 + 2 * halo;
   const int taps = halo ? 9 * a.kd : 1;
   // transposed-store staging of the epilogue: 32-channel chunks, conv / transposed conv into one pixel per thread
   const int stage_bytes = (n_blk % 32 == 0 && a.mode != EPI_HEAD && a.out != nullptr &&
-                           (a.mode != EPI_UP || a.up_cout % 32 == 0)) ? 8 * 1024 * a.esz : 0;
+                           (a.mode != EPI_UP || a.up_cout % 32 == 0)) ? 8 * 1024 * esz : 0;
   const int extra = (2 * a.n_total + (a.mode == EPI_HEAD ? a.head_n * n_blk : 0)) * 4 + 64 + stage_bytes;   // scale/shift/head
   const int budget = 225 * 1024 - extra;
-  const int ck0 = pick_ck(a.cin, a.esz);
+  const int ck0 = pick_ck(a.cin, a.fmt);
   int mt_max = 256 / n_blk;                                // two accumulator stages of mt * n_blk TMEM columns
   if (mt_max > 8) mt_max = 8;
   const int w8 = (a.W + 7) / 8;
@@ -182,12 +187,12 @@ static HaloPlan plan_halo(const ConvTcArgs& a, int n_blk, bool cta2 = false) {
   for (int abufs = 2; abufs >= 1; --abufs)
     for (int mt = mt_max; mt >= 1; mt >>= 1) {
       if (abufs == 2 && 2 * mt < mt_max) break;            // do not shrink tiles below half for the 2nd buffer
-      for (int ck = ck0; ck >= 32 / a.esz; ck >>= 1) {
+      for (int ck = ck0; ck >= 32 / esz; ck >>= 1) {
         if (a.cin % ck) continue;
 #ifdef BIU_DBG_KNOBS
         if (g_halo_force_ck > 0 && ck != g_halo_force_ck) continue;
 #endif
-        const int rb = ck * a.esz;
+        const int rb = ck * esz;
         const int chunks = a.cin / ck;
         const uint32_t tile = ((uint32_t)(a.kd * rows * (8 * mt + 2 * halo) * rb) + 1023u) & ~1023u;
         const uint32_t bst = ((uint32_t)((cta2 ? n_blk / 2 : n_blk) * rb) + 1023u) & ~1023u;
@@ -232,11 +237,11 @@ static bool halo_try_cta2(const ConvTcArgs& a, int n_blk, HaloPlan* out, int* pa
   if (per_block < 2 || (per_block & 1)) return false;
   static int cache[3][3][4];                               // [format][ks index][mt index] -> pairs + 1 for the largest smem seen
   static int cache_smem[3][3][4];
-  const int ks = pl.ck * a.esz / 32, ki = ks == 4 ? 2 : (ks == 2 ? 1 : 0), mi = pl.mt == 8 ? 3 : (pl.mt == 4 ? 2 : (pl.mt == 2 ? 1 : 0));
-  const int ei = a.esz == 4 ? 2 : (a.f16 ? 1 : 0);
+  const int ks = pl.ck * fmt_esz(a.fmt) / 32, ki = ks == 4 ? 2 : (ks == 2 ? 1 : 0), mi = pl.mt == 8 ? 3 : (pl.mt == 4 ? 2 : (pl.mt == 2 ? 1 : 0));
+  const int ei = a.fmt - FMT_BF16;                         // FMT_BF16 / FMT_F16 / FMT_TF32 -> 0 / 1 / 2
   if (cache[ei][ki][mi] == 0 || cache_smem[ei][ki][mi] < pl.smem) {
-    const int n = a.esz == 4 ? halo_max_pairs_tf32(ks, pl.mt, pl.smem)
-                             : (a.f16 ? halo_max_pairs_f16(ks, pl.mt, pl.smem) : halo_max_pairs_bf16(ks, pl.mt, pl.smem));
+    const int n =
+        with_elem_type(a.fmt, [&](auto tag) { return halo_max_pairs<decltype(tag)::fmt>(ks, pl.mt, pl.smem); });
     cache[ei][ki][mi] = n + 1;
     cache_smem[ei][ki][mi] = pl.smem;
   }
@@ -259,7 +264,7 @@ static int launch_conv_halo(const ConvTcArgs& a, int n_blk, const HaloPlan& pl, 
   p.nblk_inner = (p.n_blocks > 1 && !pl.b_resident && !pl.cta2) ? 1 : 0;
   p.kd = a.kd;
   p.halo = a.kw == 3 ? 1 : 0;
-  p.ck = pl.ck; p.cin_chunks = a.cin / pl.ck; p.row_bytes = pl.ck * a.esz;
+  p.ck = pl.ck; p.cin_chunks = a.cin / pl.ck; p.row_bytes = pl.ck * fmt_esz(a.fmt);
   p.n_blk = n_blk; p.n_total = a.n_total;
   p.a_bufs = pl.a_bufs; p.b_stages = pl.b_stages; p.a_buf_bytes = pl.a_buf_bytes; p.b_stage_bytes = pl.b_stage_bytes;
   p.b_resident = pl.b_resident;
@@ -277,10 +282,10 @@ static int launch_conv_halo(const ConvTcArgs& a, int n_blk, const HaloPlan& pl, 
 #endif
 
   CUtensorMap tmA, tmB;
-  const char* in_base = reinterpret_cast<const char*>(a.in) + (size_t)a.in_coff * a.esz;
-  if (int rc = encode_act_map(&tmA, in_base, a.esz, a.f16, a.cin, a.W, a.H, a.D, a.B, a.in_ctot, pl.ck, 8 * pl.mt + 2 * p.halo, 2, 1, 1))
+  const char* in_base = reinterpret_cast<const char*>(a.in) + (size_t)a.in_coff * fmt_esz(a.fmt);
+  if (int rc = encode_act_map(&tmA, in_base, a.fmt, a.cin, a.W, a.H, a.D, a.B, a.in_ctot, pl.ck, 8 * pl.mt + 2 * p.halo, 2, 1, 1))
     return rc;
-  if (int rc = encode_wgt_map(&tmB, a.wgt, a.esz, a.f16, a.cin, a.n_total, p.halo ? 9 * a.kd : 1, pl.ck, pl.cta2 ? n_blk / 2 : n_blk))
+  if (int rc = encode_wgt_map(&tmB, a.wgt, a.fmt, a.cin, a.n_total, p.halo ? 9 * a.kd : 1, pl.ck, pl.cta2 ? n_blk / 2 : n_blk))
     return rc;
   int grid = p.total_tiles < sm_count() ? p.total_tiles : sm_count();
   if (pl.cta2) {                                           // whole pairs, all of them resident at once
@@ -290,10 +295,9 @@ static int launch_conv_halo(const ConvTcArgs& a, int n_blk, const HaloPlan& pl, 
     grid = 2 * pairs;
   }
   BIU_REQUIRE(pl.mt == 1 || pl.mt == 2 || pl.mt == 4 || pl.mt == 8, "halo kernel: mt must be 1, 2, 4 or 8 (got %d)", pl.mt);
-  // the kernel instantiations live in their own translation units (conv_halo_bf16.cu / _f16.cu / _tf32.cu)
-  if (int rc = a.esz == 4 ? halo_dispatch_tf32(tmA, tmB, p, grid, pl.smem, stream)
-                          : (a.f16 ? halo_dispatch_f16(tmA, tmB, p, grid, pl.smem, stream)
-                                   : halo_dispatch_bf16(tmA, tmB, p, grid, pl.smem, stream)))
+  if (int rc = with_elem_type(a.fmt, [&](auto tag) {
+        return halo_dispatch<decltype(tag)::fmt>(tmA, tmB, p, grid, pl.smem, stream);
+      }))
     return rc;
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
@@ -332,22 +336,23 @@ static RowsPlan plan_rows(const ConvTcArgs& a) {
   if (a.mode != EPI_CONV && a.mode != EPI_HEAD) return pl;
   if (a.kw != 3 || a.kh != 3 || (a.kd != 1 && a.kd != 3)) return pl;
   // N of the folded MMA = 3 * Cout = 48 or 96; 192 (Cout = 64) for 2D bf16 / fp16 blocks: 8 TMEM slots, one pipeline
-  const bool wide = a.n_total == 64 && a.esz == 2 && a.kd == 1 && a.mode == EPI_CONV && !rows_no_wide();
+  const int esz = fmt_esz(a.fmt);
+  const bool wide = a.n_total == 64 && esz == 2 && a.kd == 1 && a.mode == EPI_CONV && !rows_no_wide();
   if (a.n_total != 16 && a.n_total != 32 && !wide) return pl;
   if (a.W < 128) return pl;                                  // one MMA tile = 128 consecutive pixels of a row
   if (a.mode == EPI_HEAD && a.out != nullptr) return pl;
   // fused max-pool: every plane is pooled in (y, x); 3D callers reduce the z pairs afterwards (conv_tc_can_fuse_pool_xy)
   if (a.pool_out != nullptr && ((a.H & 1) || (a.W & 1) || (a.kd == 3 && a.n_total > 32))) return pl;
   if (a.pool_out != nullptr && a.pool_3d) return pl;        // z pairs: plane mode only
-  const int ck = pick_ck(a.cin, a.esz);
+  const int ck = pick_ck(a.cin, a.fmt);
   if (ck == 0) return pl;
-  const int rb = ck * a.esz, chunks = a.cin / ck, nfold = 3 * a.n_total;
+  const int rb = ck * esz, chunks = a.cin / ck, nfold = 3 * a.n_total;
   pl.ck = ck;
   pl.w_tile_bytes = ((uint32_t)(nfold * rb) + 1023u) & ~1023u;
   pl.a_chunk_bytes = ((uint32_t)(kRowsPx * rb) + 1023u) & ~1023u;
   pl.cps = chunks;
   pl.a_slot_bytes = (uint32_t)chunks * pl.a_chunk_bytes;
-  const int px_bytes = a.n_total * a.esz;
+  const int px_bytes = a.n_total * esz;
   int stage_px = px_bytes < 64 ? px_bytes : 64;                                          // conv_rows.cuh: SB
   auto tail_of = [&](int spx) { return (2 * a.n_total + kMaxHead * a.n_total) * 4 + 16 * 32 * spx + 64; };   // scale/shift/heads + staging tiles
   const int wbytes = (int)(a.kd * 3 * chunks * pl.w_tile_bytes);
@@ -393,7 +398,7 @@ static int launch_conv_rows(const ConvTcArgs& a, const RowsPlan& pl, cudaStream_
     p.total_items = p.tiles_x * p.tiles_y * a.B;
   }
   p.kd = a.kd; p.w_taps = a.kd * 3;
-  p.ck = pl.ck; p.cin_chunks = nchunks > 0 ? nchunks : a.cin / pl.ck; p.row_bytes = pl.ck * a.esz;
+  p.ck = pl.ck; p.cin_chunks = nchunks > 0 ? nchunks : a.cin / pl.ck; p.row_bytes = pl.ck * fmt_esz(a.fmt);
   p.cin_chunk0 = chunk0; p.acc_mode = acc_mode; p.acc_scratch = reinterpret_cast<float*>(a.acc_scratch);
   p.cp = a.n_total;
   p.a_slots = pl.a_slots; p.a_slot_bytes = pl.a_slot_bytes; p.a_chunk_bytes = pl.a_chunk_bytes; p.cps = pl.cps; p.stage_px = pl.stage_px;
@@ -411,16 +416,16 @@ static int launch_conv_rows(const ConvTcArgs& a, const RowsPlan& pl, cudaStream_
   for (int i = 0; i < kMaxHead; ++i) p.head_act[i] = a.head_act[i];
   p.out_val = a.out_val; p.out_u8 = a.out_u8;
   CUtensorMap tmA, tmW;
-  const char* in_base = reinterpret_cast<const char*>(a.in) + (size_t)a.in_coff * a.esz;
-  if (int rc = pl.plane ? encode_act_map(&tmA, in_base, a.esz, a.f16, a.cin, a.W, a.H, a.D, a.B, a.in_ctot, pl.ck, 10, 18, 1, 1)
-                        : encode_act_map(&tmA, in_base, a.esz, a.f16, a.cin, a.W, a.H, a.D, a.B, a.in_ctot, pl.ck, kRowsPx, 1, 1, 1))
+  const char* in_base = reinterpret_cast<const char*>(a.in) + (size_t)a.in_coff * fmt_esz(a.fmt);
+  if (int rc = pl.plane ? encode_act_map(&tmA, in_base, a.fmt, a.cin, a.W, a.H, a.D, a.B, a.in_ctot, pl.ck, 10, 18, 1, 1)
+                        : encode_act_map(&tmA, in_base, a.fmt, a.cin, a.W, a.H, a.D, a.B, a.in_ctot, pl.ck, kRowsPx, 1, 1, 1))
     return rc;
-  if (int rc = encode_wgt_map(&tmW, pl.plane ? a.wgt_fold_z : a.wgt_fold, a.esz, a.f16, a.cin, 3 * a.n_total, a.kd * 3, pl.ck, 3 * a.n_total))
+  if (int rc = encode_wgt_map(&tmW, pl.plane ? a.wgt_fold_z : a.wgt_fold, a.fmt, a.cin, 3 * a.n_total, a.kd * 3, pl.ck, 3 * a.n_total))
     return rc;
   const int grid = p.total_items < sm_count_cached() ? p.total_items : sm_count_cached();
-  if (int rc = a.esz == 4 ? rows_dispatch_tf32(tmA, tmW, p, grid, pl.smem, stream)
-                          : (a.f16 ? rows_dispatch_f16(tmA, tmW, p, grid, pl.smem, stream)
-                                   : rows_dispatch_bf16(tmA, tmW, p, grid, pl.smem, stream)))
+  if (int rc = with_elem_type(a.fmt, [&](auto tag) {
+        return rows_dispatch<decltype(tag)::fmt>(tmA, tmW, p, grid, pl.smem, stream);
+      }))
     return rc;
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
@@ -438,7 +443,7 @@ static bool first_rows_enabled() {
 }
 bool conv_first_rows_supported(const FirstRowsArgs& a) {
   if (!first_rows_enabled() || rows_disabled() || halo_disabled()) return false;
-  if (a.wgt == nullptr || (a.n_total != 16 && a.n_total != 32) || (a.esz != 2 && a.esz != 4) || (a.f16 && a.esz != 2))
+  if (a.wgt == nullptr || (a.n_total != 16 && a.n_total != 32) || (a.fmt != FMT_BF16 && a.fmt != FMT_F16 && a.fmt != FMT_TF32))
     return false;
   return a.W >= 128 && a.H >= 1 && a.out_ctot % 8 == 0 && a.out_coff % 8 == 0;
 }
@@ -457,11 +462,11 @@ int launch_conv_first_rows(const FirstRowsArgs& a, cudaStream_t stream) {
   p.rblocks = (a.H + p.RB - 1) / p.RB;
   p.total_items = p.strips * p.rblocks * a.B;
   p.kd = 1; p.slot_px = 128; p.first = 1; p.first_in = a.in; p.w_taps = 1;
-  p.ck = rb / a.esz; p.cin_chunks = 1; p.row_bytes = rb; p.cps = 1;
+  p.ck = rb / fmt_esz(a.fmt); p.cin_chunks = 1; p.row_bytes = rb; p.cps = 1;
   p.cp = a.n_total;
   p.a_chunk_bytes = 128 * rb; p.a_slot_bytes = p.a_chunk_bytes;
   p.w_tile_bytes = ((uint32_t)(nfold * rb) + 1023u) & ~1023u;
-  const int px_bytes = a.n_total * a.esz;
+  const int px_bytes = a.n_total * fmt_esz(a.fmt);
   p.stage_px = px_bytes < 64 ? px_bytes : 64;
   const int tail = (2 * a.n_total + kMaxHead * a.n_total) * 4 + 16 * 32 * p.stage_px + 64;
   p.a_slots = kRowsMaxASlots;
@@ -471,11 +476,11 @@ int launch_conv_first_rows(const FirstRowsArgs& a, cudaStream_t stream) {
   p.mode = EPI_CONV; p.slope = a.slope; p.scale = a.scale; p.shift = a.shift;
   p.out = a.out; p.out_ctot = a.out_ctot; p.out_coff = a.out_coff;
   CUtensorMap tmW;
-  if (int rc = encode_wgt_map(&tmW, a.wgt, a.esz, a.f16, p.ck, nfold, 1, p.ck, nfold)) return rc;
+  if (int rc = encode_wgt_map(&tmW, a.wgt, a.fmt, p.ck, nfold, 1, p.ck, nfold)) return rc;
   const int grid = p.total_items < sm_count_cached() ? p.total_items : sm_count_cached();
-  if (int rc = a.esz == 4 ? rows_dispatch_tf32(tmW, tmW, p, grid, smem, stream)        // no activation map: the rows are
-                          : (a.f16 ? rows_dispatch_f16(tmW, tmW, p, grid, smem, stream)  // built in the kernel
-                                   : rows_dispatch_bf16(tmW, tmW, p, grid, smem, stream)))
+  if (int rc = with_elem_type(a.fmt, [&](auto tag) {      // no activation map: the rows are built in the kernel
+        return rows_dispatch<decltype(tag)::fmt>(tmW, tmW, p, grid, smem, stream);
+      }))
     return rc;
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
@@ -513,14 +518,15 @@ static RowsPlan plan_rows_plane(const ConvTcArgs& a, int chunks_limit = 0) {
   if (a.kw != 3 || a.kh != 3 || a.kd != 3 || a.D < 2) return pl;
   if (a.n_total != 16 && a.n_total != 32) return pl;
   if (a.W < 8 || a.H < 16) return pl;                        // tiny planes: the halo / per-tap kernels (wide ones try the row mode first)
-  const int ck = pick_ck(a.cin, a.esz);
+  const int ck = pick_ck(a.cin, a.fmt);
   if (ck == 0) return pl;
-  const int rb = ck * a.esz, chunks = chunks_limit > 0 ? chunks_limit : a.cin / ck, nfold = 3 * a.n_total;
+  const int esz = fmt_esz(a.fmt);
+  const int rb = ck * esz, chunks = chunks_limit > 0 ? chunks_limit : a.cin / ck, nfold = 3 * a.n_total;
   pl.plane = 1;
   pl.ck = ck;
   pl.w_tile_bytes = ((uint32_t)(nfold * rb) + 1023u) & ~1023u;
   pl.a_chunk_bytes = ((uint32_t)(180 * rb) + 1023u) & ~1023u;      // 18 x 10 halo tile of one plane and channel chunk
-  const int px_bytes = a.n_total * a.esz;
+  const int px_bytes = a.n_total * esz;
   pl.stage_px = px_bytes < 64 ? px_bytes : 64;
   const int tail = (2 * a.n_total + kMaxHead * a.n_total) * 4 + 16 * 32 * pl.stage_px + 64;
   const int wbytes = (int)(9 * chunks * pl.w_tile_bytes);
@@ -575,8 +581,8 @@ bool conv_tc_can_fuse_pool(const ConvTcArgs& a) {
 }
 
 int launch_conv_tc(const ConvTcArgs& a, cudaStream_t stream) {
-  BIU_REQUIRE(conv_tc_supported(a), "conv_tc: unsupported configuration (cin=%d n=%d esz=%d mode=%d)", a.cin,
-              a.n_total, a.esz, a.mode);
+  BIU_REQUIRE(conv_tc_supported(a), "conv_tc: unsupported configuration (cin=%d n=%d fmt=%d mode=%d)", a.cin,
+              a.n_total, a.fmt, a.mode);
   ConvTcParams p;
   memset(&p, 0, sizeof(p));
   p.W = a.W; p.H = a.H; p.D = a.D; p.B = a.B;
@@ -586,9 +592,9 @@ int launch_conv_tc(const ConvTcArgs& a, cudaStream_t stream) {
   p.tiles_d = ceil_div(a.D, 1 << p.lbd);
   p.tiles_b = ceil_div(a.B, 1 << p.lbb);
   p.kw = a.kw; p.kh = a.kh; p.kd = a.kd;
-  p.ck = pick_ck(a.cin, a.esz);
+  p.ck = pick_ck(a.cin, a.fmt);
   p.cin_chunks = a.cin / p.ck;
-  p.row_bytes = p.ck * a.esz;
+  p.row_bytes = p.ck * fmt_esz(a.fmt);
   {
     const RowsPlan pp = plan_rows_plane(a);
     {
@@ -608,7 +614,7 @@ int launch_conv_tc(const ConvTcArgs& a, cudaStream_t stream) {
     // K split: the nine-tap weights of all channel chunks do not fit beside a usable A ring (96 input channels: 162 KB).
     // Run the block as several launches over groups of chunks; the partial sums travel through an fp32 scratch.
     if (a.acc_scratch != nullptr && a.cin > 0 && a.mode == EPI_CONV) {
-      const int ck = pick_ck(a.cin, a.esz);
+      const int ck = pick_ck(a.cin, a.fmt);
       const int chunks = ck ? a.cin / ck : 0;
       const long long need = (long long)a.B * a.D * a.H * a.W * a.n_total * 4;
       int group = 0;
@@ -660,35 +666,24 @@ int launch_conv_tc(const ConvTcArgs& a, cudaStream_t stream) {
   const int smem = stages * stage_bytes + 1024;
 
   CUtensorMap tmA, tmB;
-  const char* in_base = reinterpret_cast<const char*>(a.in) + (size_t)a.in_coff * a.esz;
-  if (int rc = encode_act_map(&tmA, in_base, a.esz, a.f16, a.cin, a.W, a.H, a.D, a.B, a.in_ctot, p.ck, 1 << p.lbw,
+  const char* in_base = reinterpret_cast<const char*>(a.in) + (size_t)a.in_coff * fmt_esz(a.fmt);
+  if (int rc = encode_act_map(&tmA, in_base, a.fmt, a.cin, a.W, a.H, a.D, a.B, a.in_ctot, p.ck, 1 << p.lbw,
                               1 << p.lbh, 1 << p.lbd, 1 << p.lbb))
     return rc;
-  if (int rc = encode_wgt_map(&tmB, a.wgt, a.esz, a.f16, a.cin, a.n_total, a.kw * a.kh * a.kd, p.ck, n_blk)) return rc;
+  if (int rc = encode_wgt_map(&tmB, a.wgt, a.fmt, a.cin, a.n_total, a.kw * a.kh * a.kd, p.ck, n_blk)) return rc;
 
   dim3 grid(p.tiles_w * p.tiles_h * p.tiles_d * p.tiles_b, a.n_total / n_blk);
-  if (a.esz == 2 && a.f16) {
-    static int max_set = 0;
-    if (smem > max_set) {
-      BIU_CHECK_CUDA(cudaFuncSetAttribute(conv_tc_kernel<FMT_F16>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-      max_set = smem;
-    }
-    conv_tc_kernel<FMT_F16><<<grid, 192, smem, stream>>>(tmA, tmB, p);
-  } else if (a.esz == 2) {
-    static int max_set = 0;
-    if (smem > max_set) {
-      BIU_CHECK_CUDA(cudaFuncSetAttribute(conv_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-      max_set = smem;
-    }
-    conv_tc_kernel<2><<<grid, 192, smem, stream>>>(tmA, tmB, p);
-  } else {
-    static int max_set = 0;
-    if (smem > max_set) {
-      BIU_CHECK_CUDA(cudaFuncSetAttribute(conv_tc_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-      max_set = smem;
-    }
-    conv_tc_kernel<4><<<grid, 192, smem, stream>>>(tmA, tmB, p);
-  }
+  if (int rc = with_elem_type(a.fmt, [&](auto tag) {
+        constexpr int FMT = decltype(tag)::fmt;
+        static int max_set = 0;
+        if (smem > max_set) {
+          BIU_CHECK_CUDA(cudaFuncSetAttribute(conv_tc_kernel<FMT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+          max_set = smem;
+        }
+        conv_tc_kernel<FMT><<<grid, 192, smem, stream>>>(tmA, tmB, p);
+        return 0;
+      }))
+    return rc;
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
   return 0;

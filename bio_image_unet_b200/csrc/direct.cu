@@ -4,13 +4,7 @@
 #include "common.cuh"
 #include "launch.h"
 
-#include <type_traits>
-
 namespace biu {
-
-// element format of an activation storage type
-template <typename T>
-constexpr int fmt_of = sizeof(T) == 4 ? FMT_TF32 : (std::is_same<T, __half>::value ? FMT_F16 : FMT_BF16);
 
 template <typename T> __device__ __forceinline__ float ld_act(const T* p);
 template <> __device__ __forceinline__ float ld_act<float>(const float* p) { return __ldg(p); }
@@ -94,7 +88,7 @@ __global__ void __launch_bounds__(256) first_conv_kernel(FirstConvArgs a) {
     for (int j = 0; j < 8; ++j) {
       float t = fmaf(acc[j], s_scale[g * 8 + j], s_shift[g * 8 + j]);
       t = t > 0.f ? t : t * a.slope;
-      st_act<TOUT>(o + j, t, a.round_tf32);
+      st_act<TOUT>(o + j, t, a.fmt == FMT_TF32);
     }
   }
 }
@@ -169,7 +163,7 @@ __global__ void __launch_bounds__(256) first_conv1_kernel(FirstConvArgs a) {
         *reinterpret_cast<uint4*>(o + g) = make_uint4(w[0], w[1], w[2], w[3]);
       } else {
         float* of = reinterpret_cast<float*>(o + g);
-        if (a.round_tf32) {
+        if (a.fmt == FMT_TF32) {
 #pragma unroll
           for (int j = 0; j < 8; ++j) acc[j] = to_tf32(acc[j]);
         }
@@ -354,7 +348,7 @@ __global__ void __launch_bounds__(256, 2) first_conv1_3d_kernel(FirstConvArgs a)
               float* of = reinterpret_cast<float*>(ov);
               float v8[8];
 #pragma unroll
-              for (int j = 0; j < 8; ++j) v8[j] = a.round_tf32 ? to_tf32(res[xi][j]) : res[xi][j];
+              for (int j = 0; j < 8; ++j) v8[j] = a.fmt == FMT_TF32 ? to_tf32(res[xi][j]) : res[xi][j];
               *reinterpret_cast<float4*>(of) = make_float4(v8[0], v8[1], v8[2], v8[3]);
               *reinterpret_cast<float4*>(of + 4) = make_float4(v8[4], v8[5], v8[6], v8[7]);
             }
@@ -472,7 +466,7 @@ __global__ void __launch_bounds__(256, 2) first_conv1_2d_kernel(FirstConvArgs a)
           *reinterpret_cast<uint4*>(o) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
         } else {
           float* of = reinterpret_cast<float*>(o);
-          if (a.round_tf32) {
+          if (a.fmt == FMT_TF32) {
 #pragma unroll
             for (int j = 0; j < 8; ++j) acc[j] = to_tf32(acc[j]);
           }
@@ -509,63 +503,46 @@ int launch_first_conv(const FirstConvArgs& a, cudaStream_t stream) {
   long long blocks = ceil_div_ll(work, 256);
   if (blocks > 148LL * 8) blocks = 148LL * 8;
   if (blocks < 1) blocks = 1;
-#define BIU_FC(TIN, TOUT)                                                                                      \
-  do {                                                                                                         \
-    if (smem > 48 * 1024)                                                                                      \
-      BIU_CHECK_CUDA(cudaFuncSetAttribute(first_conv_kernel<TIN, TOUT>,                                        \
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));            \
-    first_conv_kernel<TIN, TOUT><<<(int)blocks, 256, smem, stream>>>(a);                                       \
-  } while (0)
   const bool fast = a.cin == 1 && a.out_ctot % 8 == 0 && a.out_coff % 8 == 0 && smem <= 48 * 1024 &&
                     (a.kd == 1 || first_conv1_3d_smem(a.cout_pad) <= 100 * 1024);   // 3D: two blocks of it per SM
   const int groups = a.cout_pad / 8;
-  if (fast && a.kd == 1 && a.D == 1 && (groups == 1 || groups == 2 || groups == 4 || groups == 8)) {
-    if (a.in_kind == 0 && a.esz == 2 && a.f16) launch_first_conv1_2d<uint8_t, __half>(a, stream);
-    else if (a.in_kind == 0 && a.esz == 2) launch_first_conv1_2d<uint8_t, __nv_bfloat16>(a, stream);
-    else if (a.in_kind == 0 && a.esz == 4) launch_first_conv1_2d<uint8_t, float>(a, stream);
-    else if (a.in_kind == 1 && a.esz == 2 && a.f16) launch_first_conv1_2d<float, __half>(a, stream);
-    else if (a.in_kind == 1 && a.esz == 2) launch_first_conv1_2d<float, __nv_bfloat16>(a, stream);
-    else if (a.in_kind == 1 && a.esz == 4) launch_first_conv1_2d<float, float>(a, stream);
-    else BIU_REQUIRE(false, "first_conv: bad in_kind/esz");
-  } else if (fast) {
-    long long fb = ceil_div_ll((long long)a.B * a.D * a.H * a.W, 256);
-    if (fb > 148LL * 16) fb = 148LL * 16;
-    if (fb < 1) fb = 1;
-    long long rb3 = (long long)a.B * ((a.D + kFc3ZC - 1) / kFc3ZC) * ((a.H + kFc3Rows - 1) / kFc3Rows) *
-                    ((a.W + kFc3Cols - 1) / kFc3Cols);                                 // tile columns (3D kernel)
-    if (rb3 > 148LL * 2) rb3 = 148LL * 2;
-    if (rb3 < 1) rb3 = 1;
-#define BIU_FC1(TIN, TOUT)                                                                               \
-  do {                                                                                                   \
-    if (a.kd == 1) first_conv1_kernel<TIN, TOUT, 9><<<(int)fb, 256, smem, stream>>>(a);                  \
-    else {                                                                                               \
-      static int attr_set = 0;                                                                          \
-      const int sm3 = (int)first_conv1_3d_smem(a.cout_pad);                                              \
-      if (sm3 > attr_set) {                                                                              \
-        BIU_CHECK_CUDA(cudaFuncSetAttribute(first_conv1_3d_kernel<TIN, TOUT>,                            \
-                                            cudaFuncAttributeMaxDynamicSharedMemorySize, sm3));          \
-        attr_set = sm3;                                                                                  \
-      }                                                                                                  \
-      first_conv1_3d_kernel<TIN, TOUT><<<(int)rb3, 256, sm3, stream>>>(a);                               \
-    }                                                                                                    \
-  } while (0)
-    if (a.in_kind == 0 && a.esz == 2 && a.f16) BIU_FC1(uint8_t, __half);
-    else if (a.in_kind == 0 && a.esz == 2) BIU_FC1(uint8_t, __nv_bfloat16);
-    else if (a.in_kind == 0 && a.esz == 4) BIU_FC1(uint8_t, float);
-    else if (a.in_kind == 1 && a.esz == 2 && a.f16) BIU_FC1(float, __half);
-    else if (a.in_kind == 1 && a.esz == 2) BIU_FC1(float, __nv_bfloat16);
-    else if (a.in_kind == 1 && a.esz == 4) BIU_FC1(float, float);
-    else BIU_REQUIRE(false, "first_conv: bad in_kind/esz");
-#undef BIU_FC1
-  }
-  else if (a.in_kind == 0 && a.esz == 2 && a.f16) BIU_FC(uint8_t, __half);
-  else if (a.in_kind == 0 && a.esz == 2) BIU_FC(uint8_t, __nv_bfloat16);
-  else if (a.in_kind == 0 && a.esz == 4) BIU_FC(uint8_t, float);
-  else if (a.in_kind == 1 && a.esz == 2 && a.f16) BIU_FC(float, __half);
-  else if (a.in_kind == 1 && a.esz == 2) BIU_FC(float, __nv_bfloat16);
-  else if (a.in_kind == 1 && a.esz == 4) BIU_FC(float, float);
-  else BIU_REQUIRE(false, "first_conv: bad in_kind/esz");
-#undef BIU_FC
+  const bool fast2d = fast && a.kd == 1 && a.D == 1 && (groups == 1 || groups == 2 || groups == 4 || groups == 8);
+  long long fb = ceil_div_ll((long long)a.B * a.D * a.H * a.W, 256);
+  if (fb > 148LL * 16) fb = 148LL * 16;
+  if (fb < 1) fb = 1;
+  long long rb3 = (long long)a.B * ((a.D + kFc3ZC - 1) / kFc3ZC) * ((a.H + kFc3Rows - 1) / kFc3Rows) *
+                  ((a.W + kFc3Cols - 1) / kFc3Cols);                                   // tile columns (3D kernel)
+  if (rb3 > 148LL * 2) rb3 = 148LL * 2;
+  if (rb3 < 1) rb3 = 1;
+  BIU_REQUIRE(a.in_kind == 0 || a.in_kind == 1, "first_conv: bad in_kind %d", a.in_kind);
+  const int rc = with_elem_type(a.fmt, [&](auto out_tag) {
+    using TOUT = typename decltype(out_tag)::type;
+    auto run = [&](auto in_tag) -> int {
+      using TIN = typename decltype(in_tag)::type;
+      if (fast2d) {
+        launch_first_conv1_2d<TIN, TOUT>(a, stream);
+      } else if (fast && a.kd == 1) {
+        first_conv1_kernel<TIN, TOUT, 9><<<(int)fb, 256, smem, stream>>>(a);
+      } else if (fast) {
+        static int attr_set = 0;
+        const int sm3 = (int)first_conv1_3d_smem(a.cout_pad);
+        if (sm3 > attr_set) {
+          BIU_CHECK_CUDA(cudaFuncSetAttribute(first_conv1_3d_kernel<TIN, TOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                              sm3));
+          attr_set = sm3;
+        }
+        first_conv1_3d_kernel<TIN, TOUT><<<(int)rb3, 256, sm3, stream>>>(a);
+      } else {
+        if (smem > 48 * 1024)
+          BIU_CHECK_CUDA(cudaFuncSetAttribute(first_conv_kernel<TIN, TOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                              (int)smem));
+        first_conv_kernel<TIN, TOUT><<<(int)blocks, 256, smem, stream>>>(a);
+      }
+      return 0;
+    };
+    return a.in_kind == 0 ? run(ElemTag<uint8_t>{}) : run(ElemTag<float>{});
+  });
+  if (rc) return rc;
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
   return 0;
@@ -622,7 +599,7 @@ __global__ void __launch_bounds__(256) pool2_kernel(PoolArgs a) {
 }
 
 int launch_pool2(const PoolArgs& a, cudaStream_t stream) {
-  const int vec = 16 / a.esz;
+  const int vec = 16 / fmt_esz(a.fmt);
   BIU_REQUIRE(a.c % vec == 0 && a.in_ctot % vec == 0 && a.in_coff % vec == 0 && a.out_ctot % vec == 0 &&
                   a.out_coff % vec == 0,
               "pool2: channel counts must be multiples of %d", vec);
@@ -630,9 +607,12 @@ int launch_pool2(const PoolArgs& a, cudaStream_t stream) {
   long long blocks = ceil_div_ll((long long)a.B * (a.dims == 3 ? a.D / 2 : a.D) * oh * ow * (a.c / vec), 256);
   if (blocks > 148LL * 16) blocks = 148LL * 16;
   if (blocks < 1) blocks = 1;
-  if (a.esz == 2 && a.f16) pool2_kernel<__half, 8><<<(int)blocks, 256, 0, stream>>>(a);
-  else if (a.esz == 2) pool2_kernel<__nv_bfloat16, 8><<<(int)blocks, 256, 0, stream>>>(a);
-  else pool2_kernel<float, 4><<<(int)blocks, 256, 0, stream>>>(a);
+  if (int rc = with_elem_type(a.fmt, [&](auto tag) {
+        using T = typename decltype(tag)::type;
+        pool2_kernel<T, 16 / sizeof(T)><<<(int)blocks, 256, 0, stream>>>(a);
+        return 0;
+      }))
+    return rc;
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
   return 0;
@@ -671,16 +651,19 @@ __global__ void __launch_bounds__(256) up_nearest_kernel(UpNearestArgs a) {
   }
 }
 int launch_up_nearest(const UpNearestArgs& a, cudaStream_t stream) {
-  const int vec = 16 / a.esz;
+  const int vec = 16 / fmt_esz(a.fmt);
   BIU_REQUIRE(a.c % vec == 0 && a.in_ctot % vec == 0 && a.in_coff % vec == 0 && a.out_ctot % vec == 0 &&
                   a.out_coff % vec == 0,
               "up_nearest: channel counts must be multiples of %d", vec);
   long long blocks = (long long)a.B * a.D * a.H;             // one block iteration per input row
   if (blocks > 148LL * 16) blocks = 148LL * 16;
   if (blocks < 1) blocks = 1;
-  if (a.esz == 2 && a.f16) up_nearest_kernel<__half, 8><<<(int)blocks, 256, 0, stream>>>(a);
-  else if (a.esz == 2) up_nearest_kernel<__nv_bfloat16, 8><<<(int)blocks, 256, 0, stream>>>(a);
-  else up_nearest_kernel<float, 4><<<(int)blocks, 256, 0, stream>>>(a);
+  if (int rc = with_elem_type(a.fmt, [&](auto tag) {
+        using T = typename decltype(tag)::type;
+        up_nearest_kernel<T, 16 / sizeof(T)><<<(int)blocks, 256, 0, stream>>>(a);
+        return 0;
+      }))
+    return rc;
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
   return 0;
@@ -720,9 +703,11 @@ int launch_head(const HeadArgs& a, cudaStream_t stream) {
   long long blocks = ceil_div_ll(total, 256);
   if (blocks > 148LL * 16) blocks = 148LL * 16;
   if (blocks < 1) blocks = 1;
-  if (a.esz == 2 && a.f16) head_kernel<__half><<<(int)blocks, 256, 0, stream>>>(a);
-  else if (a.esz == 2) head_kernel<__nv_bfloat16><<<(int)blocks, 256, 0, stream>>>(a);
-  else head_kernel<float><<<(int)blocks, 256, 0, stream>>>(a);
+  if (int rc = with_elem_type(a.fmt, [&](auto tag) {
+        head_kernel<typename decltype(tag)::type><<<(int)blocks, 256, 0, stream>>>(a);
+        return 0;
+      }))
+    return rc;
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
   return 0;
@@ -811,7 +796,7 @@ __global__ void __launch_bounds__(256) direct_conv_kernel(DirectConvArgs a) {
       float t = acc[i][j];
       t = fmaf(t, a.scale ? __ldg(a.scale + co) : 1.f, __ldg(a.shift + co));
       t = t > 0.f ? t : t * a.slope;
-      st_act<T>(out + pix * a.out_ctot + a.out_coff + co, t, a.round_tf32);
+      st_act<T>(out + pix * a.out_ctot + a.out_coff + co, t, a.fmt == FMT_TF32);
     }
   }
 }
@@ -819,9 +804,11 @@ __global__ void __launch_bounds__(256) direct_conv_kernel(DirectConvArgs a) {
 int launch_direct_conv(const DirectConvArgs& a, cudaStream_t stream) {
   const long long npix = (long long)a.B * a.D * a.H * a.W;
   dim3 grid((unsigned)ceil_div_ll(npix, 64), (unsigned)ceil_div(a.cout, 64));
-  if (a.esz == 2 && a.f16) direct_conv_kernel<__half><<<grid, 256, 0, stream>>>(a);
-  else if (a.esz == 2) direct_conv_kernel<__nv_bfloat16><<<grid, 256, 0, stream>>>(a);
-  else direct_conv_kernel<float><<<grid, 256, 0, stream>>>(a);
+  if (int rc = with_elem_type(a.fmt, [&](auto tag) {
+        direct_conv_kernel<typename decltype(tag)::type><<<grid, 256, 0, stream>>>(a);
+        return 0;
+      }))
+    return rc;
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
   return 0;
@@ -854,7 +841,7 @@ __global__ void __launch_bounds__(256) direct_up_kernel(DirectUpArgs a) {
     const int oW = 2 * a.W, oH = 2 * a.H, oD = a.dims == 3 ? 2 * a.D : a.D;
     const int oz = a.dims == 3 ? 2 * z + az : z;
     const long long op = (((long long)b * oD + oz) * oH + (2 * y + ay)) * oW + (2 * x + ax);
-    st_act<T>(out + op * a.out_ctot + a.out_coff + co, s, a.round_tf32);
+    st_act<T>(out + op * a.out_ctot + a.out_coff + co, s, a.fmt == FMT_TF32);
   }
 }
 int launch_direct_up(const DirectUpArgs& a, cudaStream_t stream) {
@@ -862,9 +849,11 @@ int launch_direct_up(const DirectUpArgs& a, cudaStream_t stream) {
   long long blocks = ceil_div_ll(total, 256);
   if (blocks > 148LL * 32) blocks = 148LL * 32;
   if (blocks < 1) blocks = 1;
-  if (a.esz == 2 && a.f16) direct_up_kernel<__half><<<(int)blocks, 256, 0, stream>>>(a);
-  else if (a.esz == 2) direct_up_kernel<__nv_bfloat16><<<(int)blocks, 256, 0, stream>>>(a);
-  else direct_up_kernel<float><<<(int)blocks, 256, 0, stream>>>(a);
+  if (int rc = with_elem_type(a.fmt, [&](auto tag) {
+        direct_up_kernel<typename decltype(tag)::type><<<(int)blocks, 256, 0, stream>>>(a);
+        return 0;
+      }))
+    return rc;
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
   return 0;

@@ -10,11 +10,12 @@ extern unsigned long long g_launch_count;
 inline void count_launch(int n = 1) { g_launch_count += n; }
 
 // ---- tcgen05 implicit-GEMM convolution (conv_tc.cu) -------------------------------------------------------------
-// Every argument block below gives the activation storage as `esz` (bytes per element) and `f16`: with esz 2, 0 = bf16,
-// 1 = fp16 (2-byte elements, tensor-core operands of the same format); esz 4 = fp32 storage / tf32 operands.
+// Every argument block below gives the activation storage as `fmt`, the ElemFmt code (common.cuh) that the kernels also
+// take as their template argument: FMT_BF16 / FMT_F16 (2-byte elements, tensor-core operands of the same format),
+// FMT_TF32 (fp32 storage rounded to tf32) or FMT_F32 (fp32 storage, never rounded: CUDA-core kernels only).
+// Byte sizes follow from fmt_esz(fmt).
 struct ConvTcArgs {
-  int esz;                      // 2 = bf16 / fp16 operands, 4 = tf32 operands (fp32 storage)
-  int f16;
+  int fmt;                      // FMT_BF16 / FMT_F16 / FMT_TF32
   const void* in;               // NHWC / NDHWC activations
   int in_ctot, in_coff;         // channel stride / offset of the source buffer
   int cin;                      // logical input channels (multiple of 16 bf16 / fp16, 8 fp32)
@@ -53,12 +54,11 @@ void conv_halo_set_cta2(int on);      // test hook: CTA pairs (tcgen05.mma.cta_g
 void conv_rows_set_enabled(int on);   // test hook: route narrow 3x3 blocks through the row-streaming kernel (default on)
 int launch_conv_tc(const ConvTcArgs& a, cudaStream_t stream);
 int read_device_fault(unsigned int* out);
-int pick_ck(int cin, int esz);
+int pick_ck(int cin, int fmt);
 
 // ---- CUDA-core kernels (direct.cu): exact-fp32 path and shapes the tensor path cannot take ------------------------
 struct DirectConvArgs {
-  int esz;                      // activation storage: 2 = bf16 / fp16, 4 = fp32
-  int f16;
+  int fmt;                      // FMT_TF32 rounds the stored fp32 activations to tf32 (so the tensor path can consume them)
   const void* in;
   int in_ctot, in_coff, cin;
   int W, H, D, B;
@@ -70,12 +70,11 @@ struct DirectConvArgs {
   const float* shift;           // [cout]
   void* out;
   int out_ctot, out_coff;
-  int round_tf32;               // round stored fp32 activations to tf32 (so the tensor path can consume them)
 };
 int launch_direct_conv(const DirectConvArgs& a, cudaStream_t stream);
 
 struct DirectUpArgs {           // ConvTranspose(k=2,s=2): fp32 weights [q][cin][cout], q = (az,ay,ax) bits
-  int esz, f16;
+  int fmt;
   const void* in;
   int in_ctot, in_coff, cin;
   int W, H, D, B;
@@ -85,7 +84,6 @@ struct DirectUpArgs {           // ConvTranspose(k=2,s=2): fp32 weights [q][cin]
   int cout;
   void* out;
   int out_ctot, out_coff;
-  int round_tf32;
 };
 int launch_direct_up(const DirectUpArgs& a, cudaStream_t stream);
 
@@ -102,18 +100,16 @@ struct FirstConvArgs {          // planar u8 / f32 input with few channels -> NH
   float slope;
   const float* scale;
   const float* shift;
-  int esz, f16;
+  int fmt;
   void* out;                    // NHWC, channels [coff, coff+cout_pad) written (pad = zeros)
   int out_ctot, out_coff, cout_pad;
-  int round_tf32;
 };
 int launch_first_conv(const FirstConvArgs& a, cudaStream_t stream);
 
 // First block of the 2D nets on the row kernel (conv_rows.cuh, first mode): uint8 tile in, NHWC features out; the three dx
 // taps are the GEMM's K, the dy taps are folded into N. Tensor-core modes only (weights rounded like every other block's).
 struct FirstRowsArgs {
-  int esz;                      // 2 = bf16 / fp16, 4 = tf32 storage
-  int f16;
+  int fmt;                      // FMT_BF16 / FMT_F16 / FMT_TF32
   const uint8_t* in;            // [B][H][W] uint8 (one channel)
   int W, H, B;
   const void* wgt;              // [3 * n_total ((2 - dy), co)][16 bf16 / fp16 | 8 tf32: (dx = 0..2, zeros)]
@@ -128,7 +124,7 @@ bool conv_first_rows_supported(const FirstRowsArgs& a);
 int launch_conv_first_rows(const FirstRowsArgs& a, cudaStream_t stream);
 
 struct PoolArgs {
-  int esz, f16;
+  int fmt;
   const void* in;
   int in_ctot, in_coff, c;
   int W, H, D, B;               // input extents
@@ -141,7 +137,7 @@ struct PoolArgs {
 int launch_pool2(const PoolArgs& a, cudaStream_t stream);
 
 struct UpNearestArgs {          // nearest-neighbour x2 upsampling (multi_output_unet3d, use_interpolation=True)
-  int esz, f16;
+  int fmt;
   const void* in;
   int in_ctot, in_coff, c;
   int W, H, D, B;               // input extents
@@ -152,7 +148,7 @@ struct UpNearestArgs {          // nearest-neighbour x2 upsampling (multi_output
 int launch_up_nearest(const UpNearestArgs& a, cudaStream_t stream);
 
 struct HeadArgs {               // 1x1 head + activation on NHWC features -> planar
-  int esz, f16;
+  int fmt;
   const void* in;
   int in_ctot, in_coff, cin;
   long long npix_per_img;       // D*H*W

@@ -37,8 +37,6 @@ static uint16_t host_fp16(float v) {
   const __half_raw r = __float2half_rn(v);   // round to nearest even; beyond +-65504 -> +-inf
   return r.x;
 }
-// weight element of a 2-byte precision mode
-static uint16_t host_2byte(const Net* n, float v) { return n->f16 ? host_fp16(v) : host_bf16(v); }
 
 struct Builder {
   Net* n;
@@ -109,8 +107,6 @@ int net_build(Net* n) {
   n->layers.clear(); n->bufs.clear(); n->ops.clear();
   Builder b{n};
   const int nf = n->nf;
-  n->f16 = n->precision == PREC_FP16 ? 1 : 0;
-  n->esz = (n->precision == PREC_BF16 || n->f16) ? 2 : 4;
   n->head_total = 0;
   for (int c : n->head_channels) n->head_total += c;
   BIU_REQUIRE(n->head_total >= 1 && n->head_total <= kMaxHead, "between 1 and %d output channels supported (got %d)",
@@ -143,7 +139,7 @@ int net_build(Net* n) {
     for (int l = 3; l >= 0; --l) {
       d_a[l] = b.buf("d" + std::to_string(2 * (3 - l) + 1), l, pad16(ch[l]));
       d_b[l] = (l > 0 || v0) ? b.buf("d" + std::to_string(2 * (3 - l) + 2), l, pad16(ch[l])) : -1;
-      if (att) psi[l] = b.buf("psi" + std::to_string(4 - l), l, 4 / n->esz);      // one float per pixel
+      if (att) psi[l] = b.buf("psi" + std::to_string(4 - l), l, 4 / fmt_esz(n->fmt));      // one float per pixel
     }
     if (att) gate_scratch = b.buf("gate_scratch", 0, pad16(nf / 2));              // CUDA-core fallback only
     n->gate_scratch = gate_scratch;
@@ -359,7 +355,48 @@ static int upload(Net* n, const std::vector<T>& h, T** dptr) {
   return 0;
 }
 
+// Tensor-core weights: `h` is laid out in the target order; it is converted to the net's format (bf16 / fp16, or fp32
+// rounded to tf32) and uploaded.
+static int upload_packed(Net* n, const std::vector<float>& h, void** dptr) {
+  if (n->fmt == FMT_TF32) {
+    std::vector<float> wp(h.size());
+    for (size_t i = 0; i < h.size(); ++i) wp[i] = host_round_tf32(h[i]);
+    float* d = nullptr;
+    if (upload(n, wp, &d)) return -1;
+    *dptr = d;
+    return 0;
+  }
+  BIU_REQUIRE(n->fmt == FMT_BF16 || n->fmt == FMT_F16, "no tensor-core weights in element format %d", n->fmt);
+  std::vector<uint16_t> wp(h.size());
+  for (size_t i = 0; i < h.size(); ++i) wp[i] = n->fmt == FMT_F16 ? host_fp16(h[i]) : host_bf16(h[i]);
+  uint16_t* d = nullptr;
+  if (upload(n, wp, &d)) return -1;
+  *dptr = d;
+  return 0;
+}
+
+// A convolution with bias followed by BatchNorm (eval), by state_dict prefixes.
+struct ConvBn {
+  const HostTensor *w, *bias, *g, *be, *mu, *var;
+};
+static bool find_conv_bn(Net* n, const std::string& conv, const std::string& bn, ConvBn* p) {
+  p->w = find_param(n, conv + ".weight");
+  p->bias = find_param(n, conv + ".bias");
+  p->g = find_param(n, bn + ".weight");
+  p->be = find_param(n, bn + ".bias");
+  p->mu = find_param(n, bn + ".running_mean");
+  p->var = find_param(n, bn + ".running_var");
+  return p->w && p->bias && p->g && p->be && p->mu && p->var;
+}
+// Output channel c of BN(conv(x) + b) = sc * conv(x) + shift, in float64: sc = g / sqrt(var + 1e-5),
+// shift = be + (b - mu) * sc.
+static void fold_bn(const ConvBn& p, int c, double* sc, double* shift) {
+  *sc = (double)p.g->data[c] / std::sqrt((double)p.var->data[c] + 1e-5);
+  *shift = (double)p.be->data[c] + ((double)p.bias->data[c] - (double)p.mu->data[c]) * *sc;
+}
+
 int net_finalize(Net* n) {
+  const bool tc = n->fmt != FMT_F32;          // the tensor-core modes pack weights for the tcgen05 kernels
   for (auto& L : n->layers) {
     const int taps = L.kd * L.kh * L.kw;
     if (L.is_gate) {
@@ -372,58 +409,37 @@ int net_finalize(Net* n) {
       std::vector<float> scale(L.cout_pad, 1.f), shift(L.cout_pad, 0.f);
       for (int s2 = 0; s2 < 2; ++s2) {
         const std::string base = L.name + br[s2];
-        const HostTensor* w = find_param(n, base + ".0.weight");
-        const HostTensor* bias = find_param(n, base + ".0.bias");
-        const HostTensor* g = find_param(n, base + ".1.weight");
-        const HostTensor* be = find_param(n, base + ".1.bias");
-        const HostTensor* mu = find_param(n, base + ".1.running_mean");
-        const HostTensor* var = find_param(n, base + ".1.running_var");
-        BIU_REQUIRE(w && bias && g && be && mu && var, "state_dict is missing parameters of '%s'", base.c_str());
-        BIU_REQUIRE((long long)w->data.size() == (long long)L.cout * c, "'%s.0.weight' has %lld elements, expected %lld",
-                    base.c_str(), (long long)w->data.size(), (long long)L.cout * c);
+        ConvBn p;
+        BIU_REQUIRE(find_conv_bn(n, base + ".0", base + ".1", &p), "state_dict is missing parameters of '%s'", base.c_str());
+        BIU_REQUIRE((long long)p.w->data.size() == (long long)L.cout * c, "'%s.0.weight' has %lld elements, expected %lld",
+                    base.c_str(), (long long)p.w->data.size(), (long long)L.cout * c);
         for (int co = 0; co < L.cout; ++co) {
-          const double sc = (double)g->data[co] / std::sqrt((double)var->data[co] + 1e-5);
-          shift[co] += (float)((double)be->data[co] + ((double)bias->data[co] - (double)mu->data[co]) * sc);
+          double sc, sh;
+          fold_bn(p, co, &sc, &sh);
+          shift[co] += (float)sh;
           for (int ci = 0; ci < c; ++ci)
-            wd[(size_t)(L.segs[s2].pstart + ci) * L.cout_pad + co] = (float)(sc * (double)w->data[(size_t)co * c + ci]);
+            wd[(size_t)(L.segs[s2].pstart + ci) * L.cout_pad + co] = (float)(sc * (double)p.w->data[(size_t)co * c + ci]);
         }
       }
       if (upload(n, wd, &L.w_direct)) return -1;
       if (upload(n, scale, &L.scale)) return -1;
       if (upload(n, shift, &L.shift)) return -1;
-      if (n->precision != PREC_FP32) {
-        const size_t cnt = (size_t)L.cout_pad * L.cin_phys;
-        if (n->esz == 2) {
-          std::vector<uint16_t> wp(cnt, 0);
-          for (int co = 0; co < L.cout; ++co)
-            for (int ci = 0; ci < L.cin_phys; ++ci) wp[(size_t)co * L.cin_phys + ci] = host_2byte(n, wd[(size_t)ci * L.cout_pad + co]);
-          uint16_t* d = nullptr;
-          if (upload(n, wp, &d)) return -1;
-          L.w_tc = d;
-        } else {
-          std::vector<float> wp(cnt, 0.f);
-          for (int co = 0; co < L.cout; ++co)
-            for (int ci = 0; ci < L.cin_phys; ++ci) wp[(size_t)co * L.cin_phys + ci] = host_round_tf32(wd[(size_t)ci * L.cout_pad + co]);
-          float* d = nullptr;
-          if (upload(n, wp, &d)) return -1;
-          L.w_tc = d;
-        }
+      if (tc) {
+        std::vector<float> wp((size_t)L.cout_pad * L.cin_phys, 0.f);
+        for (int co = 0; co < L.cout; ++co)
+          for (int ci = 0; ci < L.cin_phys; ++ci) wp[(size_t)co * L.cin_phys + ci] = wd[(size_t)ci * L.cout_pad + co];
+        if (int rc = upload_packed(n, wp, &L.w_tc)) return rc;
       }
       {
         const std::string base = L.name + ".psi";
-        const HostTensor* w = find_param(n, base + ".0.weight");
-        const HostTensor* bias = find_param(n, base + ".0.bias");
-        const HostTensor* g = find_param(n, base + ".1.weight");
-        const HostTensor* be = find_param(n, base + ".1.bias");
-        const HostTensor* mu = find_param(n, base + ".1.running_mean");
-        const HostTensor* var = find_param(n, base + ".1.running_var");
-        BIU_REQUIRE(w && bias && g && be && mu && var, "state_dict is missing parameters of '%s'", base.c_str());
-        BIU_REQUIRE((long long)w->data.size() == (long long)L.cout, "'%s.0.weight' has %lld elements, expected %d",
-                    base.c_str(), (long long)w->data.size(), L.cout);
-        const double sc = (double)g->data[0] / std::sqrt((double)var->data[0] + 1e-5);
-        std::vector<float> gw(L.cout_pad, 0.f), gb(1, 0.f);
-        for (int co = 0; co < L.cout; ++co) gw[co] = (float)(sc * (double)w->data[co]);
-        gb[0] = (float)((double)be->data[0] + ((double)bias->data[0] - (double)mu->data[0]) * sc);
+        ConvBn p;
+        BIU_REQUIRE(find_conv_bn(n, base + ".0", base + ".1", &p), "state_dict is missing parameters of '%s'", base.c_str());
+        BIU_REQUIRE((long long)p.w->data.size() == (long long)L.cout, "'%s.0.weight' has %lld elements, expected %d",
+                    base.c_str(), (long long)p.w->data.size(), L.cout);
+        double sc, sh;
+        fold_bn(p, 0, &sc, &sh);
+        std::vector<float> gw(L.cout_pad, 0.f), gb(1, (float)sh);
+        for (int co = 0; co < L.cout; ++co) gw[co] = (float)(sc * (double)p.w->data[co]);
         if (upload(n, gw, &L.gate_w)) return -1;
         if (upload(n, gb, &L.gate_b)) return -1;
       }
@@ -432,22 +448,19 @@ int net_finalize(Net* n) {
     if (!L.is_up) {
       const std::string ck = L.conv_key.empty() ? L.name + ".0" : L.conv_key;
       const std::string bk = L.bn_key.empty() ? L.name + ".1" : L.bn_key;
-      const HostTensor* w = find_param(n, ck + ".weight");
-      const HostTensor* bias = find_param(n, ck + ".bias");
-      const HostTensor* g = find_param(n, bk + ".weight");
-      const HostTensor* be = find_param(n, bk + ".bias");
-      const HostTensor* mu = find_param(n, bk + ".running_mean");
-      const HostTensor* var = find_param(n, bk + ".running_var");
-      BIU_REQUIRE(w && bias && g && be && mu && var, "state_dict is missing parameters of block '%s' / '%s'", ck.c_str(),
+      ConvBn p;
+      BIU_REQUIRE(find_conv_bn(n, ck, bk, &p), "state_dict is missing parameters of block '%s' / '%s'", ck.c_str(),
                   bk.c_str());
+      const HostTensor* w = p.w;
       BIU_REQUIRE((long long)w->data.size() == (long long)L.cout * L.cin_log * taps,
                   "'%s.weight' has %lld elements, expected %lld", ck.c_str(), (long long)w->data.size(),
                   (long long)L.cout * L.cin_log * taps);
       std::vector<float> scale(L.cout_pad, 0.f), shift(L.cout_pad, 0.f);
       for (int co = 0; co < L.cout; ++co) {
-        const double s = (double)g->data[co] / std::sqrt((double)var->data[co] + 1e-5);
-        scale[co] = (float)s;
-        shift[co] = (float)((double)be->data[co] + ((double)bias->data[co] - (double)mu->data[co]) * s);
+        double sc, sh;
+        fold_bn(p, co, &sc, &sh);
+        scale[co] = (float)sc;
+        shift[co] = (float)sh;
       }
       // physical channel of every logical input channel
       std::vector<int> phys(L.cin_log);
@@ -463,56 +476,28 @@ int net_finalize(Net* n) {
       if (upload(n, shift, &L.shift)) return -1;
       // first block of a 2D net (one input channel): packing for the row kernel's first mode - the dx taps are the K
       // dimension (zero padded to 16 bf16 / fp16 or 8 tf32 elements), the dy taps are folded into N in the order dy = 2, 1, 0
-      if (n->precision != PREC_FP32 && L.cin_log == 1 && L.kd == 1 && L.kw == 3 && L.kh == 3 &&
-          (L.cout_pad == 16 || L.cout_pad == 32)) {
-        const int kel = 32 / n->esz, nfold = 3 * L.cout_pad;
+      if (tc && L.cin_log == 1 && L.kd == 1 && L.kw == 3 && L.kh == 3 && (L.cout_pad == 16 || L.cout_pad == 32)) {
+        const int kel = 32 / fmt_esz(n->fmt), nfold = 3 * L.cout_pad;
         std::vector<float> wf((size_t)nfold * kel, 0.f);
         for (int dy = 0; dy < 3; ++dy)
           for (int dx = 0; dx < 3; ++dx)
             for (int co = 0; co < L.cout; ++co)
               wf[((size_t)(2 - dy) * L.cout_pad + co) * kel + dx] = w->data[(size_t)co * taps + dy * 3 + dx];
-        if (n->esz == 2) {
-          std::vector<uint16_t> wp(wf.size());
-          for (size_t i = 0; i < wf.size(); ++i) wp[i] = host_2byte(n, wf[i]);
-          uint16_t* d = nullptr;
-          if (upload(n, wp, &d)) return -1;
-          L.w_first = d;
-        } else {
-          for (auto& v : wf) v = host_round_tf32(v);
-          float* d = nullptr;
-          if (upload(n, wf, &d)) return -1;
-          L.w_first = d;
-        }
+        if (int rc = upload_packed(n, wf, &L.w_first)) return rc;
         std::vector<float> s255(L.cout_pad, 0.f);
         for (int co = 0; co < L.cout; ++co) s255[co] = scale[co] / 255.0f;
         if (upload(n, s255, &L.scale_first)) return -1;
       }
-      if (n->precision != PREC_FP32 && L.cin_phys % 16 == 0) {
-        const size_t cnt = (size_t)taps * L.cout_pad * L.cin_phys;
-        if (n->esz == 2) {
-          std::vector<uint16_t> wp(cnt, 0);
-          for (int t = 0; t < taps; ++t)
-            for (int co = 0; co < L.cout; ++co)
-              for (int ci = 0; ci < L.cin_log; ++ci)
-                wp[((size_t)t * L.cout_pad + co) * L.cin_phys + phys[ci]] =
-                    host_2byte(n, w->data[((size_t)co * L.cin_log + ci) * taps + t]);
-          uint16_t* d = nullptr;
-          if (upload(n, wp, &d)) return -1;
-          L.w_tc = d;
-        } else {
-          std::vector<float> wp(cnt, 0.f);
-          for (int t = 0; t < taps; ++t)
-            for (int co = 0; co < L.cout; ++co)
-              for (int ci = 0; ci < L.cin_log; ++ci)
-                wp[((size_t)t * L.cout_pad + co) * L.cin_phys + phys[ci]] =
-                    host_round_tf32(w->data[((size_t)co * L.cin_log + ci) * taps + t]);
-          float* d = nullptr;
-          if (upload(n, wp, &d)) return -1;
-          L.w_tc = d;
-        }
+      if (tc && L.cin_phys % 16 == 0) {
+        std::vector<float> wp((size_t)taps * L.cout_pad * L.cin_phys, 0.f);
+        for (int t = 0; t < taps; ++t)
+          for (int co = 0; co < L.cout; ++co)
+            for (int ci = 0; ci < L.cin_log; ++ci)
+              wp[((size_t)t * L.cout_pad + co) * L.cin_phys + phys[ci]] = w->data[((size_t)co * L.cin_log + ci) * taps + t];
+        if (int rc = upload_packed(n, wp, &L.w_tc)) return rc;
         // narrow blocks (Cout <= 32): second packing with the dy taps folded into the GEMM's N, in the order
         // dy = 2, 1, 0 = output rows r-1, r, r+1 of input row r (conv_rows.cuh)
-        if (L.kw == 3 && (L.cout_pad <= 32 || (L.cout_pad == 64 && L.kd == 1 && n->esz == 2))) {
+        if (L.kw == 3 && (L.cout_pad <= 32 || (L.cout_pad == 64 && L.kd == 1 && fmt_esz(n->fmt) == 2))) {
           const int tz = L.kd * 3, nfold = 3 * L.cout_pad;
           std::vector<float> wf((size_t)tz * nfold * L.cin_phys, 0.f);
           for (int dz = 0; dz < L.kd; ++dz)
@@ -524,18 +509,7 @@ int net_finalize(Net* n) {
                     wf[((size_t)(dz * 3 + dx) * nfold + (2 - dy) * L.cout_pad + co) * L.cin_phys + phys[ci]] =
                         w->data[((size_t)co * L.cin_log + ci) * taps + t];
               }
-          if (n->esz == 2) {
-            std::vector<uint16_t> wp(wf.size());
-            for (size_t i = 0; i < wf.size(); ++i) wp[i] = host_2byte(n, wf[i]);
-            uint16_t* d = nullptr;
-            if (upload(n, wp, &d)) return -1;
-            L.w_fold = d;
-          } else {
-            for (auto& v : wf) v = host_round_tf32(v);
-            float* d = nullptr;
-            if (upload(n, wf, &d)) return -1;
-            L.w_fold = d;
-          }
+          if (int rc = upload_packed(n, wf, &L.w_fold)) return rc;
           // 3D: third packing with the dz taps folded instead (planes narrower than 128 px: the row kernel's plane
           // mode streams the planes of a 16 x 8 tile), order dz = 2, 1, 0 = output planes z-1, z, z+1 of input plane z
           if (L.kd == 3 && L.cout_pad <= 32) {
@@ -549,18 +523,7 @@ int net_finalize(Net* n) {
                       wz[((size_t)(dy * 3 + dx) * nfold + (2 - dz) * L.cout_pad + co) * L.cin_phys + phys[ci]] =
                           w->data[((size_t)co * L.cin_log + ci) * taps + t];
                 }
-            if (n->esz == 2) {
-              std::vector<uint16_t> wp(wz.size());
-              for (size_t i = 0; i < wz.size(); ++i) wp[i] = host_2byte(n, wz[i]);
-              uint16_t* d = nullptr;
-              if (upload(n, wp, &d)) return -1;
-              L.w_fold_z = d;
-            } else {
-              for (auto& v : wz) v = host_round_tf32(v);
-              float* d = nullptr;
-              if (upload(n, wz, &d)) return -1;
-              L.w_fold_z = d;
-            }
+            if (int rc = upload_packed(n, wz, &L.w_fold_z)) return rc;
           }
         }
       }
@@ -583,29 +546,13 @@ int net_finalize(Net* n) {
       if (upload(n, wd, &L.w_direct)) return -1;
       if (upload(n, scale, &L.scale)) return -1;
       if (upload(n, shift, &L.shift)) return -1;
-      if (n->precision != PREC_FP32) {
-        const size_t cnt = (size_t)L.nq * L.cout_pad * L.cin_phys;
-        if (n->esz == 2) {
-          std::vector<uint16_t> wp(cnt, 0);
-          for (int q = 0; q < L.nq; ++q)
-            for (int co = 0; co < L.cout; ++co)
-              for (int ci = 0; ci < L.cin_log; ++ci)
-                wp[((size_t)q * L.cout_pad + co) * L.cin_phys + ci] =
-                    host_2byte(n, w->data[((size_t)ci * L.cout + co) * L.nq + q]);
-          uint16_t* d = nullptr;
-          if (upload(n, wp, &d)) return -1;
-          L.w_tc = d;
-        } else {
-          std::vector<float> wp(cnt, 0.f);
-          for (int q = 0; q < L.nq; ++q)
-            for (int co = 0; co < L.cout; ++co)
-              for (int ci = 0; ci < L.cin_log; ++ci)
-                wp[((size_t)q * L.cout_pad + co) * L.cin_phys + ci] =
-                    host_round_tf32(w->data[((size_t)ci * L.cout + co) * L.nq + q]);
-          float* d = nullptr;
-          if (upload(n, wp, &d)) return -1;
-          L.w_tc = d;
-        }
+      if (tc) {
+        std::vector<float> wp((size_t)L.nq * L.cout_pad * L.cin_phys, 0.f);
+        for (int q = 0; q < L.nq; ++q)
+          for (int co = 0; co < L.cout; ++co)
+            for (int ci = 0; ci < L.cin_log; ++ci)
+              wp[((size_t)q * L.cout_pad + co) * L.cin_phys + ci] = w->data[((size_t)ci * L.cout + co) * L.nq + q];
+        if (int rc = upload_packed(n, wp, &L.w_tc)) return rc;
       }
     }
   }
@@ -659,7 +606,7 @@ long long net_plan(Net* n, int B, int D, int H, int W) {
     level_dims(n, b.level, &d, &h, &w);
     b.offset = off;
     const size_t imgs = (b.batch_mul == 2 && n->siam_shared > 0) ? (size_t)B + n->siam_shared : (size_t)B * b.batch_mul;
-    size_t bytes = imgs * d * h * w * b.ctot * n->esz;
+    size_t bytes = imgs * d * h * w * b.ctot * fmt_esz(n->fmt);
     off += (bytes + 1023) & ~(size_t)1023;
   }
   n->ws_bytes = off;
@@ -933,8 +880,9 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
   BIU_REQUIRE(n->finalized, "network weights were not finalized");
   BIU_REQUIRE(n->B > 0, "biu_net_plan must be called before biu_net_forward");
   char* ws = reinterpret_cast<char*>(workspace);
-  const bool tc_allowed = n->precision != PREC_FP32 && !n->force_direct;
-  const int round_tf32 = n->precision == PREC_TF32 ? 1 : 0;
+  const bool tc_allowed = n->fmt != FMT_F32 && !n->force_direct;
+  const int esz = fmt_esz(n->fmt);
+  const int round_tf32 = n->fmt == FMT_TF32 ? 1 : 0;   // flag of the join and up-sampling kernels below
   if (n->profile && n->events.size() < 2 * n->ops.size()) {
     while (n->events.size() < 2 * n->ops.size()) {
       cudaEvent_t e;
@@ -969,12 +917,12 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
     const int batch = (o.batch_mul == 2 && shared > 0) ? n->B + shared : n->B * o.batch_mul;
     const Buf* sb = o.src >= 0 ? &n->bufs[o.src] : nullptr;
     const Buf* db = o.dst >= 0 ? &n->bufs[o.dst] : nullptr;
-    const size_t img_in = sb ? (size_t)d * h * w * sb->ctot * n->esz : 0;
+    const size_t img_in = sb ? (size_t)d * h * w * sb->ctot * esz : 0;
     // an op that covers both streams (batch_mul 2) starts at image 0 of the buffer
     const char* src = sb ? ws + sb->offset + (o.batch_mul == 2 ? 0 : stream_img0(sb, o.src_img0)) * img_in : nullptr;
     auto dst_ptr = [&](int dd, int hh, int ww) -> char* {
       return db ? ws + db->offset + (o.batch_mul == 2 ? 0 : stream_img0(db, o.dst_img0)) *
-                                        ((size_t)dd * hh * ww * db->ctot * n->esz) : nullptr;
+                                        ((size_t)dd * hh * ww * db->ctot * esz) : nullptr;
     };
     switch (o.kind) {
       case OP_FIRST: {
@@ -990,12 +938,12 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
         BIU_REQUIRE(a.in != nullptr, "network input pointer is null");
         a.cin = n->in_ch; a.W = w; a.H = h; a.D = d; a.B = shared > 0 ? n->B + shared : n->B; a.kd = L.kd;
         a.wgt = L.w_direct; a.cout = L.cout_pad; a.cout_real = L.cout; a.slope = L.slope; a.scale = L.scale; a.shift = L.shift;
-        a.esz = n->esz; a.f16 = n->f16; a.out = shared > 0 ? ws + db->offset : dst_ptr(d, h, w); a.out_ctot = db->ctot; a.out_coff = o.dst_coff;
-        a.cout_pad = L.cout_pad; a.round_tf32 = round_tf32;
+        a.fmt = n->fmt; a.out = shared > 0 ? ws + db->offset : dst_ptr(d, h, w); a.out_ctot = db->ctot; a.out_coff = o.dst_coff;
+        a.cout_pad = L.cout_pad;
         if (tc_allowed && in_kind == 0 && n->dims == 2 && a.D == 1 && L.w_first != nullptr) {
           FirstRowsArgs fr;
           memset(&fr, 0, sizeof(fr));
-          fr.esz = n->esz; fr.f16 = n->f16; fr.in = reinterpret_cast<const uint8_t*>(a.in); fr.W = a.W; fr.H = a.H; fr.B = a.B;
+          fr.fmt = n->fmt; fr.in = reinterpret_cast<const uint8_t*>(a.in); fr.W = a.W; fr.H = a.H; fr.B = a.B;
           fr.wgt = L.w_first; fr.n_total = L.cout_pad; fr.slope = L.slope; fr.scale = L.scale_first; fr.shift = L.shift;
           fr.out = a.out; fr.out_ctot = a.out_ctot; fr.out_coff = a.out_coff;
           if (conv_first_rows_supported(fr)) {
@@ -1012,7 +960,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
         const bool head = o.kind == OP_CONV_HEAD;
         ConvTcArgs a;
         memset(&a, 0, sizeof(a));
-        a.esz = n->esz; a.f16 = n->f16; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.cin = L.cin_phys;
+        a.fmt = n->fmt; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.cin = L.cin_phys;
         a.W = w; a.H = h; a.D = d; a.B = batch; a.kw = L.kw; a.kh = L.kh; a.kd = L.kd;
         a.wgt = L.w_tc; a.wgt_fold = L.w_fold; a.wgt_fold_z = L.w_fold_z; a.n_total = L.cout_pad; a.mode = head ? EPI_HEAD : EPI_CONV; a.slope = L.slope;
         a.scale = L.scale; a.shift = L.shift;
@@ -1023,7 +971,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
           int d0, h0, w0;
           level_dims(n, sc.level, &d0, &h0, &w0);
           a.acc_scratch = ws + sc.offset;
-          a.acc_scratch_bytes = (long long)n->B * sc.batch_mul * d0 * h0 * w0 * sc.ctot * n->esz;
+          a.acc_scratch_bytes = (long long)n->B * sc.batch_mul * d0 * h0 * w0 * sc.ctot * esz;
         }
         if (head) {
           a.head_n = n->head_total; a.head_w = n->head_w; a.head_b = n->head_b;
@@ -1073,7 +1021,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
               if (conv_tc_can_fuse_pool_xy(a)) {
                 zpairs = skip_pool = true;
                 memset(&zp, 0, sizeof(zp));
-                zp.esz = n->esz; zp.f16 = n->f16; zp.in = a.pool_out; zp.in_ctot = L.cout_pad; zp.in_coff = 0; zp.c = L.cout_pad;
+                zp.fmt = n->fmt; zp.in = a.pool_out; zp.in_ctot = L.cout_pad; zp.in_coff = 0; zp.c = L.cout_pad;
                 zp.W = w / 2; zp.H = h / 2; zp.D = d; zp.B = batch; zp.dims = 3; zp.mode = 2;
                 zp.out = ws + pb.offset; zp.out_ctot = pb.ctot; zp.out_coff = nx.dst_coff;
               } else {
@@ -1087,10 +1035,9 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
           n->op_kinds[op_index] += 16;
           DirectConvArgs da;
           memset(&da, 0, sizeof(da));
-          da.esz = n->esz; da.f16 = n->f16; da.in = src; da.in_ctot = sb->ctot; da.in_coff = o.src_coff; da.cin = L.cin_phys;
+          da.fmt = n->fmt; da.in = src; da.in_ctot = sb->ctot; da.in_coff = o.src_coff; da.cin = L.cin_phys;
           da.W = w; da.H = h; da.D = d; da.B = batch; da.kw = L.kw; da.kh = L.kh; da.kd = L.kd;
           da.wgt = L.w_direct; da.cout = L.cout_pad; da.slope = L.slope; da.scale = L.scale; da.shift = L.shift;
-          da.round_tf32 = round_tf32;
           if (!head) {
             da.out = dst_ptr(d, h, w); da.out_ctot = db->ctot; da.out_coff = o.dst_coff;
             if (int rc = launch_direct_conv(da, stream)) return rc;
@@ -1102,7 +1049,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
             if (int rc = launch_direct_conv(da, stream)) return rc;
             HeadArgs ha;
             memset(&ha, 0, sizeof(ha));
-            ha.esz = n->esz; ha.f16 = n->f16; ha.in = da.out; ha.in_ctot = scratch.ctot; ha.in_coff = 0; ha.cin = L.cout_pad;
+            ha.fmt = n->fmt; ha.in = da.out; ha.in_ctot = scratch.ctot; ha.in_coff = 0; ha.cin = L.cout_pad;
             ha.npix_per_img = (long long)d * h * w; ha.B = batch; ha.head_n = n->head_total;
             ha.w = n->head_w; ha.b = n->head_b;
             int row = 0;
@@ -1119,7 +1066,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
         const int od = n->dims == 3 ? 2 * d : d;
         ConvTcArgs a;
         memset(&a, 0, sizeof(a));
-        a.esz = n->esz; a.f16 = n->f16; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.cin = L.cin_phys;
+        a.fmt = n->fmt; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.cin = L.cin_phys;
         a.W = w; a.H = h; a.D = d; a.B = batch; a.kw = a.kh = a.kd = 1;
         a.wgt = L.w_tc; a.n_total = L.nq * L.cout_pad; a.mode = EPI_UP; a.slope = 1.f;
         a.scale = L.scale; a.shift = L.shift;
@@ -1131,10 +1078,9 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
           n->op_kinds[op_index] += 16;
           DirectUpArgs da;
           memset(&da, 0, sizeof(da));
-          da.esz = n->esz; da.f16 = n->f16; da.in = src; da.in_ctot = sb->ctot; da.in_coff = o.src_coff; da.cin = L.cin_phys;
+          da.fmt = n->fmt; da.in = src; da.in_ctot = sb->ctot; da.in_coff = o.src_coff; da.cin = L.cin_phys;
           da.W = w; da.H = h; da.D = d; da.B = batch; da.dims = n->dims; da.wgt = L.w_direct; da.bias = L.shift;
           da.cout = L.cout_pad; da.out = a.out; da.out_ctot = db->ctot; da.out_coff = o.dst_coff;
-          da.round_tf32 = round_tf32;
           if (int rc = launch_direct_up(da, stream)) return rc;
         }
         break;
@@ -1142,7 +1088,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
       case OP_POOL: {
         PoolArgs a;
         memset(&a, 0, sizeof(a));
-        a.esz = n->esz; a.f16 = n->f16; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.c = o.c;
+        a.fmt = n->fmt; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.c = o.c;
         a.W = w; a.H = h; a.D = d; a.B = batch; a.dims = n->dims; a.mode = o.pool_mode;
         a.out = dst_ptr(n->dims == 3 ? d / 2 : d, h / 2, w / 2); a.out_ctot = db->ctot; a.out_coff = o.dst_coff;
         if (int rc = launch_pool2(a, stream)) return rc;
@@ -1151,7 +1097,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
       case OP_UPNEAREST: {
         UpNearestArgs a;
         memset(&a, 0, sizeof(a));
-        a.esz = n->esz; a.f16 = n->f16; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.c = o.c;
+        a.fmt = n->fmt; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.c = o.c;
         a.W = w; a.H = h; a.D = d; a.B = batch; a.dims = n->dims;
         a.out = dst_ptr(n->dims == 3 ? 2 * d : d, 2 * h, 2 * w); a.out_ctot = db->ctot; a.out_coff = o.dst_coff;
         if (int rc = launch_up_nearest(a, stream)) return rc;
@@ -1162,7 +1108,7 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
         float* psi = reinterpret_cast<float*>(ws + db->offset);
         ConvTcArgs a;
         memset(&a, 0, sizeof(a));
-        a.esz = n->esz; a.f16 = n->f16; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.cin = L.cin_phys;
+        a.fmt = n->fmt; a.in = src; a.in_ctot = sb->ctot; a.in_coff = o.src_coff; a.cin = L.cin_phys;
         a.W = w; a.H = h; a.D = d; a.B = batch; a.kw = a.kh = a.kd = 1;
         a.wgt = L.w_tc; a.n_total = L.cout_pad; a.mode = EPI_HEAD; a.slope = 0.f;
         a.scale = L.scale; a.shift = L.shift; a.out = nullptr;
@@ -1176,15 +1122,16 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
           const Buf& scratch = n->bufs[n->gate_scratch];
           DirectConvArgs da;
           memset(&da, 0, sizeof(da));
-          da.esz = n->esz; da.f16 = n->f16; da.in = src; da.in_ctot = sb->ctot; da.in_coff = o.src_coff; da.cin = L.cin_phys;
+          // the gate's activation only feeds psi below and is read by no tensor-core kernel: fp32 stays unrounded
+          da.fmt = n->fmt == FMT_TF32 ? FMT_F32 : n->fmt;
+          da.in = src; da.in_ctot = sb->ctot; da.in_coff = o.src_coff; da.cin = L.cin_phys;
           da.W = w; da.H = h; da.D = d; da.B = batch; da.kw = da.kh = da.kd = 1;
           da.wgt = L.w_direct; da.cout = L.cout_pad; da.slope = 0.f; da.scale = L.scale; da.shift = L.shift;
-          da.round_tf32 = 0;
           da.out = ws + scratch.offset; da.out_ctot = L.cout_pad; da.out_coff = 0;
           if (int rc = launch_direct_conv(da, stream)) return rc;
           HeadArgs ha;
           memset(&ha, 0, sizeof(ha));
-          ha.esz = n->esz; ha.f16 = n->f16; ha.in = da.out; ha.in_ctot = L.cout_pad; ha.in_coff = 0; ha.cin = L.cout_pad;
+          ha.fmt = da.fmt; ha.in = da.out; ha.in_ctot = L.cout_pad; ha.in_coff = 0; ha.cin = L.cout_pad;
           ha.npix_per_img = (long long)d * h * w; ha.B = batch; ha.head_n = 1;
           ha.w = L.gate_w; ha.b = L.gate_b; ha.act[0] = ACT_SIGMOID;
           ha.out_val = psi; ha.out_u8 = nullptr;
@@ -1194,20 +1141,23 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
       }
       case OP_MULPSI: {
         const long long npix = (long long)batch * d * h * w;
-        const int vec = 16 / n->esz;
+        const int vec = 16 / esz;
         long long blocks = ceil_div_ll(npix * (o.c / vec), 256);
         if (blocks > 148 * 16) blocks = 148 * 16;
         if (blocks < 1) blocks = 1;
         float* psi = reinterpret_cast<float*>(ws + sb->offset);
-        if (n->f16) mul_psi_kernel<FMT_F16><<<(int)blocks, 256, 0, stream>>>(ws + db->offset, db->ctot, o.dst_coff, o.c, psi, npix, 0);
-        else if (n->esz == 2) mul_psi_kernel<FMT_BF16><<<(int)blocks, 256, 0, stream>>>(ws + db->offset, db->ctot, o.dst_coff, o.c, psi, npix, 0);
-        else mul_psi_kernel<FMT_TF32><<<(int)blocks, 256, 0, stream>>>(ws + db->offset, db->ctot, o.dst_coff, o.c, psi, npix, round_tf32);
+        if (int rc = with_elem_type(n->fmt, [&](auto tag) {
+              mul_psi_kernel<decltype(tag)::fmt><<<(int)blocks, 256, 0, stream>>>(
+                  ws + db->offset, db->ctot, o.dst_coff, o.c, psi, npix, round_tf32);
+              return 0;
+            }))
+          return rc;
         BIU_CHECK_CUDA(cudaGetLastError());
         count_launch();
         break;
       }
       case OP_XCORR: {
-        const size_t img = (size_t)d * h * w * sb->ctot * n->esz;
+        const size_t img = (size_t)d * h * w * sb->ctot * esz;
         int G = 8;
         while (G > 1 && (size_t)2 * h * w * G * sizeof(float) > 96 * 1024) G >>= 1;
         const size_t smem = (size_t)2 * h * w * G * sizeof(float);
@@ -1215,49 +1165,34 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
         const int blocks = n->B * (sb->ctot / G);
         const char* cur = ws + sb->offset + img * stream_img0(sb, 0);
         const char* prv = ws + sb->offset + img * stream_img0(sb, 1);
-        if (n->f16) {
-          if (smem > 48 * 1024)
-            BIU_CHECK_CUDA(cudaFuncSetAttribute(xcorr_join_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-          xcorr_join_kernel<__half><<<blocks, 256, smem, stream>>>(
-              reinterpret_cast<const __half*>(cur), reinterpret_cast<const __half*>(prv),
-              reinterpret_cast<__half*>(ws + db->offset), h, w, sb->ctot, G, 0);
-        } else if (n->esz == 2) {
-          if (smem > 48 * 1024)
-            BIU_CHECK_CUDA(cudaFuncSetAttribute(xcorr_join_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-          xcorr_join_kernel<__nv_bfloat16><<<blocks, 256, smem, stream>>>(
-              reinterpret_cast<const __nv_bfloat16*>(cur), reinterpret_cast<const __nv_bfloat16*>(prv),
-              reinterpret_cast<__nv_bfloat16*>(ws + db->offset), h, w, sb->ctot, G, 0);
-        } else {
-          if (smem > 48 * 1024)
-            BIU_CHECK_CUDA(cudaFuncSetAttribute(xcorr_join_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-          xcorr_join_kernel<float><<<blocks, 256, smem, stream>>>(reinterpret_cast<const float*>(cur),
-                                                                  reinterpret_cast<const float*>(prv),
-                                                                  reinterpret_cast<float*>(ws + db->offset), h, w,
-                                                                  sb->ctot, G, round_tf32);
-        }
+        if (int rc = with_elem_type(n->fmt, [&](auto tag) {
+              using T = typename decltype(tag)::type;
+              if (smem > 48 * 1024)
+                BIU_CHECK_CUDA(cudaFuncSetAttribute(xcorr_join_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+              xcorr_join_kernel<T><<<blocks, 256, smem, stream>>>(reinterpret_cast<const T*>(cur), reinterpret_cast<const T*>(prv),
+                                                                   reinterpret_cast<T*>(ws + db->offset), h, w, sb->ctot, G,
+                                                                   round_tf32);
+              return 0;
+            }))
+          return rc;
         BIU_CHECK_CUDA(cudaGetLastError());
         count_launch();
         break;
       }
       case OP_UPTRILINEAR: {
-        const long long total = (long long)batch * 8 * d * h * w * (o.c / (16 / n->esz));
+        const long long total = (long long)batch * 8 * d * h * w * (o.c / (16 / esz));
         long long blocks = ceil_div_ll(total, 256);
         if (blocks > 148 * 16) blocks = 148 * 16;
         if (blocks < 1) blocks = 1;
         char* dst = ws + db->offset;
-        if (n->f16)
-          up_trilinear_kernel<__half, 8><<<(int)blocks, 256, 0, stream>>>(
-              reinterpret_cast<const __half*>(src), sb->ctot, o.src_coff, o.c, batch, d, h, w,
-              reinterpret_cast<__half*>(dst), db->ctot, o.dst_coff, 0);
-        else if (n->esz == 2)
-          up_trilinear_kernel<__nv_bfloat16, 8><<<(int)blocks, 256, 0, stream>>>(
-              reinterpret_cast<const __nv_bfloat16*>(src), sb->ctot, o.src_coff, o.c, batch, d, h, w,
-              reinterpret_cast<__nv_bfloat16*>(dst), db->ctot, o.dst_coff, 0);
-        else
-          up_trilinear_kernel<float, 4><<<(int)blocks, 256, 0, stream>>>(reinterpret_cast<const float*>(src), sb->ctot,
-                                                                         o.src_coff, o.c, batch, d, h, w,
-                                                                         reinterpret_cast<float*>(dst), db->ctot,
-                                                                         o.dst_coff, round_tf32);
+        if (int rc = with_elem_type(n->fmt, [&](auto tag) {
+              using T = typename decltype(tag)::type;
+              up_trilinear_kernel<T, 16 / sizeof(T)><<<(int)blocks, 256, 0, stream>>>(
+                  reinterpret_cast<const T*>(src), sb->ctot, o.src_coff, o.c, batch, d, h, w, reinterpret_cast<T*>(dst), db->ctot,
+                  o.dst_coff, round_tf32);
+              return 0;
+            }))
+          return rc;
         BIU_CHECK_CUDA(cudaGetLastError());
         count_launch();
         break;
@@ -1266,25 +1201,20 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
         int blocks = batch * (h + 1);                      // one block iteration per pair of output rows
         if (blocks > 148 * 8) blocks = 148 * 8;
         char* dst = ws + db->offset;
-        if (n->f16)
-          up_bilinear_kernel<__half, 8><<<blocks, 256, 0, stream>>>(
-              reinterpret_cast<const __half*>(src), sb->ctot, o.src_coff, o.c, batch, h, w,
-              reinterpret_cast<__half*>(dst), db->ctot, o.dst_coff, 0);
-        else if (n->esz == 2)
-          up_bilinear_kernel<__nv_bfloat16, 8><<<blocks, 256, 0, stream>>>(
-              reinterpret_cast<const __nv_bfloat16*>(src), sb->ctot, o.src_coff, o.c, batch, h, w,
-              reinterpret_cast<__nv_bfloat16*>(dst), db->ctot, o.dst_coff, 0);
-        else
-          up_bilinear_kernel<float, 4><<<blocks, 256, 0, stream>>>(reinterpret_cast<const float*>(src), sb->ctot,
-                                                                   o.src_coff, o.c, batch, h, w,
-                                                                   reinterpret_cast<float*>(dst), db->ctot,
-                                                                   o.dst_coff, round_tf32);
+        if (int rc = with_elem_type(n->fmt, [&](auto tag) {
+              using T = typename decltype(tag)::type;
+              up_bilinear_kernel<T, 16 / sizeof(T)><<<blocks, 256, 0, stream>>>(
+                  reinterpret_cast<const T*>(src), sb->ctot, o.src_coff, o.c, batch, h, w, reinterpret_cast<T*>(dst), db->ctot,
+                  o.dst_coff, round_tf32);
+              return 0;
+            }))
+          return rc;
         BIU_CHECK_CUDA(cudaGetLastError());
         count_launch();
         break;
       }
       case OP_MAXJOIN: {
-        const size_t img = (size_t)d * h * w * sb->ctot * n->esz;
+        const size_t img = (size_t)d * h * w * sb->ctot * esz;
         const long long nvec = (long long)(img * n->B / 16);
         long long blocks = ceil_div_ll(nvec, 256);
         if (blocks > 148 * 8) blocks = 148 * 8;
@@ -1292,11 +1222,13 @@ int net_forward(Net* n, const void* in, int in_kind, const void* in2, float* out
         const uint4* xa = reinterpret_cast<const uint4*>(ws + sb->offset + img * stream_img0(sb, 0));
         const uint4* xb = reinterpret_cast<const uint4*>(ws + sb->offset + img * stream_img0(sb, 1));
         uint4* xo = reinterpret_cast<uint4*>(ws + db->offset);
-        if (n->f16) max_join_kernel<FMT_F16><<<(int)blocks, 256, 0, stream>>>(xa, xb, xo, nvec);
-        else if (n->esz == 2) max_join_kernel<FMT_BF16><<<(int)blocks, 256, 0, stream>>>(xa, xb, xo, nvec);
-        else max_join_kernel<FMT_TF32><<<(int)blocks, 256, 0, stream>>>(xa, xb, xo, nvec);
+        if (int rc = with_elem_type(n->fmt, [&](auto tag) {
+              max_join_kernel<decltype(tag)::fmt><<<(int)blocks, 256, 0, stream>>>(xa, xb, xo, nvec);
+              return 0;
+            }))
+          return rc;
         BIU_CHECK_CUDA(cudaGetLastError());
-  count_launch();
+        count_launch();
         break;
       }
     }
@@ -1326,7 +1258,7 @@ int net_debug_copy(Net* n, const char* buf_name, void* workspace, void* dst_host
       int d, h, w;
       level_dims(n, b.level, &d, &h, &w);
       const long long imgs = (b.batch_mul == 2 && n->siam_shared > 0) ? (long long)n->B + n->siam_shared : (long long)n->B * b.batch_mul;
-      long long bytes = imgs * d * h * w * b.ctot * n->esz;
+      long long bytes = imgs * d * h * w * b.ctot * fmt_esz(n->fmt);
       if (bytes > max_bytes) bytes = max_bytes;
       BIU_CHECK_CUDA(cudaMemcpy(dst_host, reinterpret_cast<char*>(workspace) + b.offset, bytes, cudaMemcpyDeviceToHost));
       return 0;

@@ -12,7 +12,6 @@ namespace biu {
 
 enum NetKind { NET_UNET2D = 0, NET_SIAM2D = 1, NET_UNET3D = 2, NET_MO3D = 3, NET_UNET2D_V0 = 4, NET_ATTUNET2D = 5, NET_MO2D = 6,
                NET_NESTED2D = 7, NET_NESTED2D_3L = 8 };
-enum Precision { PREC_BF16 = 0, PREC_TF32 = 1, PREC_FP32 = 2, PREC_FP16 = 3 };
 enum SiamMode { SIAM_CONCAT = 0, SIAM_MAX = 1, SIAM_CONTROL = 2, SIAM_CORR = 3 };
 
 struct HostTensor {
@@ -36,7 +35,7 @@ struct ConvLayer {     // one Conv+BN+LeakyReLU block, a transposed conv, or the
   float* gate_w = nullptr;   // is_gate: psi weights [cout_pad] and bias [1] (BatchNorm(1) folded)
   float* gate_b = nullptr;
   std::vector<Segment> segs;
-  void* w_tc = nullptr;      // packed [tap][n][cin_phys] bf16 / fp16 / tf32
+  void* w_tc = nullptr;      // packed [tap][n][cin_phys] in the net's format (bf16 / fp16 / tf32)
   void* w_fold = nullptr;    // narrow 3x3 blocks: [dz*3+dx][(2-dy)*cout_pad + co][cin_phys] for the row-streaming kernel
   void* w_fold_z = nullptr;  // narrow 3x3x3 blocks: [dy*3+dx][(2-dz)*cout_pad + co][cin_phys] for its plane mode (dz folded)
   float* w_direct = nullptr; // fp32 [tap or q][cin_phys][cout_pad]
@@ -67,8 +66,8 @@ struct Buf {
 };
 
 struct Net {
-  int kind = 0, dims = 2, nf = 32, in_ch = 1, precision = 0, esz = 2;
-  int f16 = 0;                      // 2-byte activations and weights are fp16 (PREC_FP16) instead of bf16
+  int kind = 0, dims = 2, nf = 32, in_ch = 1;
+  int fmt = 0;                      // ElemFmt (common.cuh) of the activations and tensor-core weights
   int siam_mode = 0, use_interp = 0;
   int levels = 4;
   std::vector<int> head_channels;   // per head

@@ -136,22 +136,32 @@ def test_bimodal_mask_iou(precision):
 
 
 def test_engine_tensor_path_matches_cuda_core_path():
-    """Same weights, tf32 storage: tcgen05 kernels vs the direct CUDA-core kernels on intermediate activations (cat4, mid2, d7)."""
+    """Same weights, tf32 storage: tcgen05 kernels vs the direct CUDA-core kernels on intermediate activations (cat4, mid2, d7).
+    Both paths store tf32-representable float32 values (low 13 mantissa bits zero); the 'fp32' mode does not round."""
     from bio_image_unet_b200.engine import Engine
     sd = stress_state_dict(32, seed=5)
     tiles = torch.randint(0, 256, (2, 1, 64, 64), dtype=torch.uint8, generator=torch.Generator().manual_seed(1)).cuda()
+    acts = [('d7', 32, 0), ('cat4', 64, 0), ('mid2', 512, 4)]
     eng = Engine('unet2d', sd, 32, 1, [('', 1, 'sigmoid')], precision='tf32', device='cuda:0')
     eng.plan(2, (64, 64))
     v_tc, _ = eng.forward(tiles, want_val=True)
-    a_tc = {n: eng.debug_activation(n, c, l) for n, c, l in [('d7', 32, 0), ('cat4', 64, 0), ('mid2', 512, 4)]}
+    a_tc = {n: eng.debug_activation(n, c, l) for n, c, l in acts}
     eng.set_force_direct(1)
     eng.plan(2, (64, 64))
     v_dc, _ = eng.forward(tiles, want_val=True)
-    a_dc = {n: eng.debug_activation(n, c, l) for n, c, l in [('d7', 32, 0), ('cat4', 64, 0), ('mid2', 512, 4)]}
+    a_dc = {n: eng.debug_activation(n, c, l) for n, c, l in acts}
+    eng.close()
     for n in a_tc:   # both paths round every stored activation to tf32; only the accumulation order differs
         rel = np.abs(a_tc[n] - a_dc[n]).max() / np.abs(a_dc[n]).max()
         assert rel < 1e-2, (n, rel)
+        for path, a in (('tcgen05', a_tc[n]), ('cuda-core', a_dc[n])):
+            assert not (a.view(np.uint32) & 0x1FFF).any(), (n, path, 'stores a value that is not tf32-representable')
     assert (v_tc - v_dc).abs().max().item() < 5e-2   # stress net, logit sigma ~13
+    eng = Engine('unet2d', sd, 32, 1, [('', 1, 'sigmoid')], precision='fp32', device='cuda:0')
+    eng.plan(2, (64, 64))
+    eng.forward(tiles, want_val=True)
+    for n, c, l in acts:
+        assert (eng.debug_activation(n, c, l).view(np.uint32) & 0x1FFF).any(), (n, 'fp32 mode rounded every value to tf32')
     eng.close()
 
 

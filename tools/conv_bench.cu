@@ -1,10 +1,12 @@
 // Single-layer timing harness for the tcgen05 convolution kernels (development aid, not part of the product).
-// Build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -DBIU_DBG_KNOBS -o tools/conv_bench tools/conv_bench.cu
+// Build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -DBIU_DBG_KNOBS -o tools/conv_bench tools/conv_bench.cu -lcuda
 // Usage: conv_bench [tiles]   -- times the cfg-2 Unet(32) layer shapes on `tiles` 512x512 tiles with every debug knob
 #include "../bio_image_unet_b200/csrc/conv_tc.cu"
 #include "../bio_image_unet_b200/csrc/conv_halo_bf16.cu"
+#include "../bio_image_unet_b200/csrc/conv_halo_f16.cu"
 #include "../bio_image_unet_b200/csrc/conv_halo_tf32.cu"
 #include "../bio_image_unet_b200/csrc/conv_rows_bf16.cu"
+#include "../bio_image_unet_b200/csrc/conv_rows_f16.cu"
 #include "../bio_image_unet_b200/csrc/conv_rows_tf32.cu"
 #include <vector>
 #include <cstdarg>
@@ -23,7 +25,7 @@ static float time_layer(const LayerCfg& L, int tiles, void* in, void* wgt, float
   const int H = 512 >> L.level, W = 512 >> L.level;
   ConvTcArgs a;
   memset(&a, 0, sizeof(a));
-  a.esz = 2; a.in = in; a.in_ctot = L.cin; a.in_coff = 0; a.cin = L.cin; a.W = W; a.H = H; a.D = 1; a.B = tiles;
+  a.fmt = FMT_BF16; a.in = in; a.in_ctot = L.cin; a.in_coff = 0; a.cin = L.cin; a.W = W; a.H = H; a.D = 1; a.B = tiles;
   if (!L.up) {
     a.kw = a.kh = 3; a.kd = 1; a.n_total = L.cout; a.mode = EPI_CONV; a.slope = 0.1f;
     a.out_ctot = L.cout;
