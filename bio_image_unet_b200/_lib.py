@@ -41,6 +41,11 @@ SIGNATURES = {
                                      c_int, c_int, c_int, c_int, _P, _P]),
     'biu_gather_tiles': (c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, c_int, c_int, c_int, c_int, c_int,
                                  c_int, _P, _P]),
+    'biu_gather_tiles_tta': (c_int, [_P, c_int, _P, c_longlong, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, c_int, c_int,
+                                     c_int, c_int, c_int, c_int, c_int, c_int, _P, _P]),
+    'biu_gather_tiles_f32_tta': (c_int, [_P, c_int, c_int, c_int, c_int, _P, _P, _P, c_int, c_int, c_int, c_int, c_int,
+                                         c_int, c_int, c_int, _P, _P]),
+    'biu_tta_accumulate': (c_int, [_P, c_longlong, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P]),
     'biu_stitch_mean_u8': (c_int, [_P, c_int, c_int, c_int, c_int, _P, _P, c_int, c_int, c_int, c_int, _P, _P]),
     'biu_stitch_mod3_u8': (c_int, [_P, c_int, c_int, c_int, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_int, _P,
                                    _P]),

@@ -178,6 +178,33 @@ int biu_gather_tiles_lut(const void* src, int dtype_bytes, const uint8_t* lut, l
   GatherArgs a{src, dtype_bytes, lut, lut_stride, F, Z, H, W, pad_mode, zs, ys, xs, nz, ny, nx, pd, ph, pw, dst};
   return launch_gather_tiles(a, (cudaStream_t)stream);
 }
+static int tta_code(int dims, int t, int* xform) {
+  BIU_REQUIRE(dims == 2 || dims == 3, "test-time augmentation: dims must be 2 or 3 (got %d)", dims);
+  BIU_REQUIRE(t >= 0 && t < 8, "test-time augmentation: transform code must be 0..7 (got %d)", t);
+  *xform = tta_xform(dims, t);
+  return 0;
+}
+int biu_gather_tiles_tta(const void* src, int dtype_bytes, const uint8_t* lut, long long lut_stride, int F, int Z, int H,
+                         int W, int pad_mode, const int* zs, const int* ys, const int* xs, int nz, int ny, int nx, int pd,
+                         int ph, int pw, int dims, int t, uint8_t* dst, void* stream) {
+  BIU_REQUIRE(dtype_bytes == 1 || (dtype_bytes == 2 && lut != nullptr),
+              "gather_tiles_tta: a uint8 source, or a uint8 / uint16 source and a table");
+  GatherArgs a{src, dtype_bytes, lut, lut_stride, F, Z, H, W, pad_mode, zs, ys, xs, nz, ny, nx, pd, ph, pw, dst, 0};
+  if (int rc = tta_code(dims, t, &a.xform)) return rc;
+  return launch_gather_tiles(a, (cudaStream_t)stream);
+}
+int biu_gather_tiles_f32_tta(const float* src, int F, int Z, int H, int W, const int* zs, const int* ys, const int* xs,
+                             int nz, int ny, int nx, int pd, int ph, int pw, int dims, int t, float* dst, void* stream) {
+  int xform = 0;
+  if (int rc = tta_code(dims, t, &xform)) return rc;
+  return launch_gather_tiles_f32(src, F, Z, H, W, zs, ys, xs, nz, ny, nx, pd, ph, pw, dst, (cudaStream_t)stream, xform);
+}
+int biu_tta_accumulate(const float* val, long long planes, int pd, int ph, int pw, int dims, int t, int pass, int passes,
+                       float* acc, uint8_t* out_u8, float* out_f32, void* stream) {
+  TtaAccArgs a{val, planes, pd, ph, pw, 0, pass, passes, acc, out_u8, out_f32};
+  if (int rc = tta_code(dims, t, &a.xform)) return rc;
+  return launch_tta_accumulate(a, (cudaStream_t)stream);
+}
 int biu_stitch_mean_u8(const uint8_t* tiles, int F, int C, int H, int W, const int* ys, const int* xs, int ny, int nx,
                        int ph, int pw, uint8_t* out, void* stream) {
   StitchMeanArgs a{tiles, F, C, H, W, ys, xs, ny, nx, ph, pw, out};

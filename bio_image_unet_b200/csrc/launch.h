@@ -182,8 +182,25 @@ struct GatherArgs {
   int nz, ny, nx;
   int pd, ph, pw;               // tile extents
   uint8_t* dst;                 // [F*nz*ny*nx][pd][ph][pw]
+  int xform;                    // test-time augmentation: XF_* bits, 0 = the tile as it is
 };
+// Transform of a tile's coordinates (test-time augmentation). The flips act first, the transpose (2D square tiles only)
+// last; the inverse transposes first. tta_xform maps the public code t (2D: bit 0 x, 1 y, 2 transpose; 3D: bit 0 x,
+// 1 y, 2 z) onto these bits.
+enum { XF_FLIP_X = 1, XF_FLIP_Y = 2, XF_FLIP_Z = 4, XF_TRANSPOSE = 8 };
+inline int tta_xform(int dims, int t) { return dims == 2 ? ((t & 3) | ((t & 4) ? XF_TRANSPOSE : 0)) : (t & 7); }
 int launch_gather_tiles(const GatherArgs& a, cudaStream_t stream);
+struct TtaAccArgs {             // one pass of the test-time augmentation merge
+  const float* val;             // [planes][pd][ph][pw]: the net's output on the transformed tiles
+  long long planes;             // tiles * channels
+  int pd, ph, pw;
+  int xform;                    // XF_* bits of the pass's transform; its inverse is applied on the read
+  int pass, passes;             // pass 0 writes acc, the last pass writes the mean to out_u8 / out_f32
+  float* acc;                   // [planes][pd][ph][pw] fp32 running sum in pass order
+  uint8_t* out_u8;              // trunc(mean * 255), the head epilogue's rule (may be null)
+  float* out_f32;               // mean (may be null)
+};
+int launch_tta_accumulate(const TtaAccArgs& a, cudaStream_t stream);
 struct StitchMeanArgs {         // unet/predict.py:204-229 == integer sum // count
   const uint8_t* tiles;         // [F][ny*nx][C][ph][pw]
   int F, C, H, W;               // output extents (already cropped to the image)
@@ -239,7 +256,8 @@ int launch_norm_lut_f32(const unsigned int* hist_bounds, const unsigned int* his
 int launch_apply_lut_f32(const void* img, int dtype_bytes, long long n_per_frame, int frames, const float* lut,
                          long long lut_stride, float* out, cudaStream_t stream);
 int launch_gather_tiles_f32(const float* src, int F, int Z, int H, int W, const int* zs, const int* ys, const int* xs,
-                            int nz, int ny, int nx, int pd, int ph, int pw, float* dst, cudaStream_t stream);
+                            int nz, int ny, int nx, int pd, int ph, int pw, float* dst, cudaStream_t stream,
+                            int xform = 0);
 
 
 

@@ -359,12 +359,14 @@ __device__ __forceinline__ int reflect_index(int i, int n) {
 // TSRC = uint8_t: plain copy of an already normalised stack. With a.lut the normalisation is fused in: the source is
 // the raw uint8 / uint16 stack and every value goes through the frame's look-up table on its way into the tile (the
 // normalised frame is then never written). V pixels per thread (16 when the tile width allows it): runs that lie inside
-// the source row and are 16-byte aligned move as whole vectors.
+// the source row and are 16-byte aligned move as whole vectors. Flips of a.xform (test-time augmentation) pick the
+// mirrored tile row / plane, and a mirrored x run is loaded as it lies in the source and reversed in registers.
 template <typename TSRC, int V>
 __global__ void __launch_bounds__(256) gather_tiles_kernel(GatherArgs a) {
   const long long tile_elems = (long long)a.pd * a.ph * a.pw;
   const long long total = (long long)a.F * a.nz * a.ny * a.nx * tile_elems;
   const TSRC* srcb = reinterpret_cast<const TSRC*>(a.src);
+  const bool fx = a.xform & XF_FLIP_X, fy = a.xform & XF_FLIP_Y, fz = a.xform & XF_FLIP_Z;
   for (long long idx = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * V; idx < total;
        idx += (long long)gridDim.x * blockDim.x * V) {
     long long r = idx;
@@ -375,13 +377,13 @@ __global__ void __launch_bounds__(256) gather_tiles_kernel(GatherArgs a) {
     const int iy = (int)(r % a.ny); r /= a.ny;
     const int iz = (int)(r % a.nz); r /= a.nz;
     const int f = (int)r;
-    int sz = a.zs[iz] + z, sy = a.ys[iy] + y;
+    int sz = a.zs[iz] + (fz ? a.pd - 1 - z : z), sy = a.ys[iy] + (fy ? a.ph - 1 - y : y);
     bool zero = false;
     if (sz >= a.Z) { if (a.pad_mode == 0) sz = reflect_index(sz, a.Z); else zero = true; }
     if (sy >= a.H) { if (a.pad_mode == 0) sy = reflect_index(sy, a.H); else zero = true; }
     const TSRC* row = srcb + (((long long)f * a.Z + sz) * a.H + sy) * a.W;
     const uint8_t* l = a.lut ? a.lut + (long long)f * a.lut_stride : nullptr;
-    const int sx0 = a.xs[ix] + x;
+    const int sx0 = a.xs[ix] + (fx ? a.pw - V - x : x);
     TSRC raw[V];
     bool zk[V];
     constexpr bool kVec = (V * sizeof(TSRC)) % 16 == 0;       // whole 16-byte vectors only (V = 4 runs stay scalar)
@@ -403,15 +405,97 @@ __global__ void __launch_bounds__(256) gather_tiles_kernel(GatherArgs a) {
     uint8_t v[V];
 #pragma unroll
     for (int k = 0; k < V; ++k) v[k] = zk[k] ? (uint8_t)0 : (l ? __ldg(l + raw[k]) : (uint8_t)raw[k]);
+    uint32_t* w = reinterpret_cast<uint32_t*>(v);
+    if (fx) {                                                  // reverse the V bytes: word order and bytes in a word
+      uint32_t rev[V / 4];
+#pragma unroll
+      for (int q = 0; q < V / 4; ++q) rev[q] = __byte_perm(w[V / 4 - 1 - q], 0, 0x0123);
+#pragma unroll
+      for (int q = 0; q < V / 4; ++q) w[q] = rev[q];
+    }
     if (V == 16) *reinterpret_cast<uint4*>(a.dst + idx) = *reinterpret_cast<uint4*>(v);
     else *reinterpret_cast<uchar4*>(a.dst + idx) = *reinterpret_cast<uchar4*>(v);
   }
+}
+
+// Value of tile source pixel (f, sz, sy, sx) after the far-end padding; uint8 tiles go through the table when there is one.
+template <typename TSRC, typename TDST>
+__device__ __forceinline__ TDST gather_at(const GatherArgs& a, int f, int sz, int sy, int sx) {
+  bool zero = false;
+  if (sz >= a.Z) { if (a.pad_mode == 0) sz = reflect_index(sz, a.Z); else zero = true; }
+  if (sy >= a.H) { if (a.pad_mode == 0) sy = reflect_index(sy, a.H); else zero = true; }
+  if (sx >= a.W) { if (a.pad_mode == 0) sx = reflect_index(sx, a.W); else zero = true; }
+  if (zero) return (TDST)0;
+  const TSRC raw = __ldg(reinterpret_cast<const TSRC*>(a.src) + (((long long)f * a.Z + sz) * a.H + sy) * a.W + sx);
+  if constexpr (sizeof(TDST) == 4) {
+    return raw;
+  } else {
+    return a.lut ? __ldg(a.lut + (long long)f * a.lut_stride + raw) : (uint8_t)raw;
+  }
+}
+
+// Transposed 2D tiles (XF_TRANSPOSE, ph == pw = P, pd == 1): out[i][j] = tile[fy ? P-1-j : j][fx ? P-1-i : i]. A block
+// moves 32 x 32 squares: it reads the source square row by row into shared memory and writes it out column by column,
+// so that both the global reads and the global writes of a warp are runs of consecutive pixels.
+template <typename TSRC, typename TDST>
+__global__ void __launch_bounds__(256) gather_tiles_transposed_kernel(GatherArgs a, TDST* __restrict__ dst) {
+  __shared__ TDST sh[32][33];
+  const int P = a.pw, nsq = (P + 31) / 32;
+  const bool fx = a.xform & XF_FLIP_X, fy = a.xform & XF_FLIP_Y;
+  const long long total = (long long)a.F * a.nz * a.ny * a.nx * nsq * nsq;
+  for (long long sq = blockIdx.x; sq < total; sq += gridDim.x) {
+    long long r = sq;
+    const int oj0 = (int)(r % nsq) * 32; r /= nsq;
+    const int oi0 = (int)(r % nsq) * 32; r /= nsq;
+    const long long n = r;
+    const int ix = (int)(r % a.nx); r /= a.nx;
+    const int iy = (int)(r % a.ny); r /= a.ny;
+    const int iz = (int)(r % a.nz); r /= a.nz;
+    const int f = (int)r;
+    for (int rr = threadIdx.y; rr < 32; rr += blockDim.y) {   // sh[rr][c] = out[oi0 + c][oj0 + rr]
+      const int i = oi0 + threadIdx.x, j = oj0 + rr;
+      if (i < P && j < P)
+        sh[rr][threadIdx.x] = gather_at<TSRC, TDST>(a, f, a.zs[iz], a.ys[iy] + (fy ? P - 1 - j : j),
+                                                    a.xs[ix] + (fx ? P - 1 - i : i));
+    }
+    __syncthreads();
+    for (int c = threadIdx.y; c < 32; c += blockDim.y) {
+      const int i = oi0 + c, j = oj0 + threadIdx.x;
+      if (i < P && j < P) dst[n * P * P + (long long)i * P + j] = sh[threadIdx.x][c];
+    }
+    __syncthreads();
+  }
+}
+
+template <typename TSRC, typename TDST>
+static void launch_gather_transposed(const GatherArgs& a, TDST* dst, cudaStream_t stream) {
+  const int nsq = (a.pw + 31) / 32;
+  long long blocks = (long long)a.F * a.nz * a.ny * a.nx * nsq * nsq;
+  if (blocks > 148LL * 16) blocks = 148LL * 16;
+  if (blocks < 1) blocks = 1;
+  gather_tiles_transposed_kernel<TSRC, TDST><<<(int)blocks, dim3(32, 8), 0, stream>>>(a, dst);
+}
+
+static int check_xform(const GatherArgs& a) {
+  BIU_REQUIRE(a.xform >= 0 && a.xform <= (XF_FLIP_X | XF_FLIP_Y | XF_FLIP_Z | XF_TRANSPOSE), "gather: bad transform %d",
+              a.xform);
+  BIU_REQUIRE(!(a.xform & XF_TRANSPOSE) || (a.ph == a.pw && a.pd == 1 && !(a.xform & XF_FLIP_Z)),
+              "gather: a transposed tile must be a square 2D tile (got %d x %d x %d)", a.pd, a.ph, a.pw);
+  return 0;
 }
 
 int launch_gather_tiles(const GatherArgs& a, cudaStream_t stream) {
   BIU_REQUIRE(a.pw % 4 == 0, "gather_tiles: tile width must be a multiple of 4 (got %d)", a.pw);
   BIU_REQUIRE(a.src_bytes == 1 || (a.src_bytes == 2 && a.lut != nullptr),
               "gather_tiles: a uint16 source needs the look-up table of the fused normalisation");
+  if (int rc = check_xform(a)) return rc;
+  if (a.xform & XF_TRANSPOSE) {
+    if (a.src_bytes == 2) launch_gather_transposed<uint16_t, uint8_t>(a, a.dst, stream);
+    else launch_gather_transposed<uint8_t, uint8_t>(a, a.dst, stream);
+    BIU_CHECK_CUDA(cudaGetLastError());
+    count_launch();
+    return 0;
+  }
   const int v = (a.pw % 16 == 0) ? 16 : 4;
   const long long total = (long long)a.F * a.nz * a.ny * a.nx * a.pd * a.ph * a.pw / v;
   long long blocks = ceil_div_ll(total, 256);
@@ -424,6 +508,77 @@ int launch_gather_tiles(const GatherArgs& a, cudaStream_t stream) {
     if (v == 16) gather_tiles_kernel<uint8_t, 16><<<(int)blocks, 256, 0, stream>>>(a);
     else gather_tiles_kernel<uint8_t, 4><<<(int)blocks, 256, 0, stream>>>(a);
   }
+  BIU_CHECK_CUDA(cudaGetLastError());
+  count_launch();
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Test-time augmentation merge: pass p of K adds the inverse-transformed output of the net on the transformed tiles
+// into the fp32 running sum, acc = ((v_0 + v_1) + ...) in pass order; pass 0 writes acc and the last pass writes
+// mean = acc * (1/K) (exact, K is a power of two) as float32 and / or as uint8 with the head epilogue's truncating
+// trunc(mean * 255). Gather formulation (every output element is written by one thread), no atomics: deterministic.
+// A block handles a 32 x 32 square of one output plane; for a transposed pass the square of val is staged in shared
+// memory so that reads and writes are both runs along x.
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) tta_accumulate_kernel(TtaAccArgs a) {
+  __shared__ float sh[32][33];
+  const bool fx = a.xform & XF_FLIP_X, fy = a.xform & XF_FLIP_Y, fz = a.xform & XF_FLIP_Z;
+  const bool tr = a.xform & XF_TRANSPOSE;
+  const int nsy = (a.ph + 31) / 32, nsx = (a.pw + 31) / 32;
+  const long long total = a.planes * a.pd * nsy * nsx;
+  const long long plane_elems = (long long)a.ph * a.pw;
+  const bool first = a.pass == 0, last = a.pass == a.passes - 1;
+  const float inv_k = 1.0f / (float)a.passes;
+  for (long long sq = blockIdx.x; sq < total; sq += gridDim.x) {
+    long long r = sq;
+    const int x0 = (int)(r % nsx) * 32; r /= nsx;
+    const int y0 = (int)(r % nsy) * 32; r /= nsy;
+    const int z = (int)(r % a.pd); r /= a.pd;
+    const long long p = r;
+    const long long obase = (p * a.pd + z) * plane_elems;
+    const float* vplane = a.val + (p * a.pd + (fz ? a.pd - 1 - z : z)) * plane_elems;
+    if (tr) {                                            // out[y][x] = val[fx ? P-1-x : x][fy ? P-1-y : y]
+      for (int rr = threadIdx.y; rr < 32; rr += blockDim.y) {
+        const int x = x0 + rr, y = y0 + threadIdx.x;       // sh[rr][c] = out[y0 + c][x0 + rr]
+        if (x < a.pw && y < a.ph)
+          sh[rr][threadIdx.x] = __ldg(vplane + (long long)(fx ? a.pw - 1 - x : x) * a.pw + (fy ? a.ph - 1 - y : y));
+      }
+      __syncthreads();
+    }
+    for (int rr = threadIdx.y; rr < 32; rr += blockDim.y) {
+      const int y = y0 + rr, x = x0 + threadIdx.x;
+      if (y >= a.ph || x >= a.pw) continue;
+      const float v = tr ? sh[threadIdx.x][rr]
+                         : __ldg(vplane + (long long)(fy ? a.ph - 1 - y : y) * a.pw + (fx ? a.pw - 1 - x : x));
+      const long long o = obase + (long long)y * a.pw + x;
+      const float s = first ? v : __fadd_rn(a.acc[o], v);
+      if (!last) {
+        a.acc[o] = s;
+      } else {
+        const float m = __fmul_rn(s, inv_k);
+        if (a.out_f32) a.out_f32[o] = m;
+        if (a.out_u8) a.out_u8[o] = (uint8_t)(m * 255.0f);   // as the head epilogues (unet/predict.py:200)
+      }
+    }
+    if (tr) __syncthreads();
+  }
+}
+
+int launch_tta_accumulate(const TtaAccArgs& a, cudaStream_t stream) {
+  BIU_REQUIRE(a.passes >= 1 && a.pass >= 0 && a.pass < a.passes, "tta_accumulate: pass %d of %d", a.pass, a.passes);
+  BIU_REQUIRE((a.passes & (a.passes - 1)) == 0, "tta_accumulate: the pass count must be a power of two (got %d)",
+              a.passes);
+  BIU_REQUIRE(a.xform >= 0 && a.xform <= (XF_FLIP_X | XF_FLIP_Y | XF_FLIP_Z | XF_TRANSPOSE), "tta_accumulate: bad transform");
+  BIU_REQUIRE(!(a.xform & XF_TRANSPOSE) || (a.ph == a.pw && a.pd == 1 && !(a.xform & XF_FLIP_Z)),
+              "tta_accumulate: a transposed tile must be a square 2D tile");
+  BIU_REQUIRE(a.pass == a.passes - 1 ? (a.out_u8 || a.out_f32) : a.acc != nullptr,
+              "tta_accumulate: the last pass needs an output, the others the accumulator");
+  const long long total = a.planes * a.pd * ((a.ph + 31) / 32) * ((a.pw + 31) / 32);
+  long long blocks = total;
+  if (blocks > 148LL * 16) blocks = 148LL * 16;
+  if (blocks < 1) blocks = 1;
+  tta_accumulate_kernel<<<(int)blocks, dim3(32, 8), 0, stream>>>(a);
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
   return 0;
@@ -837,13 +992,15 @@ int launch_apply_lut_f32(const void* img, int dtype_bytes, long long n_per_frame
   return 0;
 }
 
-// float32 patch gather, patches always inside the volume (patch = min(volume, max_patch), :129-131)
+// float32 patch gather, patches always inside the volume (patch = min(volume, max_patch), :129-131). Flips of `xform`
+// (test-time augmentation) as in gather_tiles_kernel; a float4 run of a mirrored row is reversed in registers.
 __global__ void __launch_bounds__(256) gather_tiles_f32_kernel(const float* __restrict__ src, int F, int Z, int H, int W,
                                                                const int* __restrict__ zs, const int* __restrict__ ys,
                                                                const int* __restrict__ xs, int nz, int ny, int nx, int pd,
-                                                               int ph, int pw, float* __restrict__ dst) {
+                                                               int ph, int pw, float* __restrict__ dst, int xform) {
   // 4 consecutive x per thread (pw is a multiple of 4: patch extents are multiples of 8 / 16)
   const long long total = (long long)F * nz * ny * nx * pd * ph * pw;
+  const bool fx = xform & XF_FLIP_X, fy = xform & XF_FLIP_Y, fz = xform & XF_FLIP_Z;
   for (long long idx = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 4; idx < total;
        idx += (long long)gridDim.x * blockDim.x * 4) {
     long long r = idx;
@@ -854,11 +1011,11 @@ __global__ void __launch_bounds__(256) gather_tiles_f32_kernel(const float* __re
     const int iy = (int)(r % ny); r /= ny;
     const int iz = (int)(r % nz); r /= nz;
     const int f = (int)r;
-    int zz = zs[iz] + z, yy = ys[iy] + y;
+    int zz = zs[iz] + (fz ? pd - 1 - z : z), yy = ys[iy] + (fy ? ph - 1 - y : y);
     if (zz >= Z) zz = reflect_index(zz, Z);      // np.pad(..., 'reflect') at the far end (multi_output_unet/predict.py:172),
     if (yy >= H) yy = reflect_index(yy, H);      // periodic like numpy's when the pad exceeds the extent
     const float* row = src + (((long long)f * Z + zz) * H + yy) * W;
-    const int sx0 = xs[ix] + x;
+    const int sx0 = xs[ix] + (fx ? pw - 4 - x : x);
     float v[4];
     if (sx0 + 4 <= W && ((reinterpret_cast<uintptr_t>(row + sx0) & 15) == 0)) {
       *reinterpret_cast<float4*>(v) = __ldg(reinterpret_cast<const float4*>(row + sx0));
@@ -870,17 +1027,28 @@ __global__ void __launch_bounds__(256) gather_tiles_f32_kernel(const float* __re
         v[q] = __ldg(row + xx);
       }
     }
+    if (fx) { float t0 = v[0], t1 = v[1]; v[0] = v[3]; v[1] = v[2]; v[2] = t1; v[3] = t0; }
     *reinterpret_cast<float4*>(dst + idx) = *reinterpret_cast<float4*>(v);
   }
 }
 int launch_gather_tiles_f32(const float* src, int F, int Z, int H, int W, const int* zs, const int* ys, const int* xs,
-                            int nz, int ny, int nx, int pd, int ph, int pw, float* dst, cudaStream_t stream) {
+                            int nz, int ny, int nx, int pd, int ph, int pw, float* dst, cudaStream_t stream, int xform) {
   BIU_REQUIRE(pw % 4 == 0, "gather_tiles_f32: patch width must be a multiple of 4 (got %d)", pw);
+  if (xform & XF_TRANSPOSE) {
+    GatherArgs a{src, 4, nullptr, 0, F, Z, H, W, 0, zs, ys, xs, nz, ny, nx, pd, ph, pw, nullptr, xform};
+    if (int rc = check_xform(a)) return rc;
+    launch_gather_transposed<float, float>(a, dst, stream);
+    BIU_CHECK_CUDA(cudaGetLastError());
+    count_launch();
+    return 0;
+  }
+  BIU_REQUIRE(xform >= 0 && xform <= (XF_FLIP_X | XF_FLIP_Y | XF_FLIP_Z), "gather_tiles_f32: bad transform %d", xform);
   const long long total = (long long)F * nz * ny * nx * pd * ph * pw / 4;
   long long blocks = ceil_div_ll(total, 256);
   if (blocks > 148LL * 32) blocks = 148LL * 32;
   if (blocks < 1) blocks = 1;
-  gather_tiles_f32_kernel<<<(int)blocks, 256, 0, stream>>>(src, F, Z, H, W, zs, ys, xs, nz, ny, nx, pd, ph, pw, dst);
+  gather_tiles_f32_kernel<<<(int)blocks, 256, 0, stream>>>(src, F, Z, H, W, zs, ys, xs, nz, ny, nx, pd, ph, pw, dst,
+                                                           xform);
   BIU_CHECK_CUDA(cudaGetLastError());
   count_launch();
   return 0;

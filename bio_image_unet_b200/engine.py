@@ -302,6 +302,58 @@ def gather_tiles_lut(raw, lut, zs, ys, xs, tile, pad_mode):
     return out
 
 
+def gather_tiles_tta(src, zs, ys, xs, tile, pad_mode, dims, t, lut=None):
+    """gather_tiles (src uint8, lut None) or gather_tiles_lut (raw uint8 / uint16 stack and its tables) producing the
+    tiles under test-time augmentation transform t (2D, dims 2: bit 0 flips x, 1 flips y, 2 transposes; 3D: bits 0-2
+    flip x, y, z). t = 0 gives the plain tiles."""
+    lib = _lib.load()
+    f, z, h, w = src.shape
+    pd, ph, pw = tile
+    dev = src.device
+    assert src.is_contiguous() and src.dtype in (torch.uint8, torch.uint16)
+    dzs, dys, dxs = _dev_i32(zs, dev), _dev_i32(ys, dev), _dev_i32(xs, dev)
+    out = torch.empty((f * len(zs) * len(ys) * len(xs), pd, ph, pw), dtype=torch.uint8, device=dev)
+    stride = 0 if lut is None or lut.shape[0] == 1 else HIST_BINS
+    with torch.cuda.device(dev):
+        _lib.check(lib.biu_gather_tiles_tta(_lib.ptr(src), src.element_size(), _lib.ptr(lut), stride, f, z, h, w,
+                                            int(pad_mode), _lib.ptr(dzs), _lib.ptr(dys), _lib.ptr(dxs), len(zs), len(ys),
+                                            len(xs), pd, ph, pw, int(dims), int(t), _lib.ptr(out), _lib.stream_ptr()),
+                   'biu_gather_tiles_tta')
+    return out
+
+
+def gather_tiles_f32_tta(src, zs, ys, xs, tile, dims, t):
+    """gather_tiles_f32 producing the patches under transform t (see gather_tiles_tta)."""
+    lib = _lib.load()
+    f, z, h, w = src.shape
+    pd, ph, pw = tile
+    dev = src.device
+    assert src.is_contiguous() and src.dtype == torch.float32
+    dzs, dys, dxs = _dev_i32(zs, dev), _dev_i32(ys, dev), _dev_i32(xs, dev)
+    out = torch.empty((f * len(zs) * len(ys) * len(xs), pd, ph, pw), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.biu_gather_tiles_f32_tta(_lib.ptr(src), f, z, h, w, _lib.ptr(dzs), _lib.ptr(dys), _lib.ptr(dxs),
+                                                len(zs), len(ys), len(xs), pd, ph, pw, int(dims), int(t), _lib.ptr(out),
+                                                _lib.stream_ptr()), 'biu_gather_tiles_f32_tta')
+    return out
+
+
+def tta_accumulate(val, acc, dims, t, p, passes, out_u8=None, out_f32=None):
+    """Pass p of `passes` of the test-time augmentation merge. val: (n, C, [d,] h, w) float32 output of the net on
+    the tiles of transform t; acc: fp32 buffer of val's shape (the running sum of T^-1(val) in pass order; written by
+    pass 0, not needed when passes == 1). The last pass writes the mean to out_f32 and / or trunc(mean * 255) to
+    out_u8 (tensors of val's shape)."""
+    lib = _lib.load()
+    assert val.is_contiguous() and val.dtype == torch.float32
+    for o in (acc, out_u8, out_f32):
+        assert o is None or (o.is_contiguous() and o.shape == val.shape)
+    pd = val.shape[2] if val.dim() == 5 else 1
+    with torch.cuda.device(val.device):
+        _lib.check(lib.biu_tta_accumulate(_lib.ptr(val), val.shape[0] * val.shape[1], pd, val.shape[-2], val.shape[-1],
+                                          int(dims), int(t), int(p), int(passes), _lib.ptr(acc), _lib.ptr(out_u8),
+                                          _lib.ptr(out_f32), _lib.stream_ptr()), 'biu_tta_accumulate')
+
+
 def stitch_mean_u8(tiles, frames, channels, out_hw, ys, xs, tile_hw):
     """tiles (F*ny*nx, C, ph, pw) uint8 -> (F, C, H, W) uint8, sum // count over covering tiles."""
     lib = _lib.load()

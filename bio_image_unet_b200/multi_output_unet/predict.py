@@ -49,13 +49,17 @@ class Predict:
     through the same float16 rounding before the margin-weighted stitch. precision='fp16' is the reference's own
     arithmetic for this predictor: fp16 weights and activations, fp32 accumulation (the reference's float16
     convolutions accumulate in fp32 as well). Integer stacks (uint8 / uint16) are normalised on the device.
+    tta (engine-only): None (default) | 'flips' (4 forwards per patch) | 'dihedral' (square patches: 8) - the head
+    outputs of the flipped / rotated patches are mapped back and averaged in fp32 on the device; the mean goes through
+    the float16 rounding and the margin-weighted stitch like an ordinary patch. It takes one more float32 buffer of
+    all result patches.
     """
 
     def __init__(self, imgs, model_params, result_path=None, network=MultiOutputNestedUNet, max_patch_size=(1024, 1024),
                  batch_size=1, normalization_mode='single', clip_threshold=(0., 99.98), add_tile=0,
                  compress_tif=False, show_progress=True, device: Union[torch.device, str] = 'auto',
                  progress_notifier: ProgressNotifier = ProgressNotifier.progress_notifier_tqdm(), *,
-                 precision='tf32', workspace_gb=24.0, keep_intermediates=False):
+                 precision='tf32', workspace_gb=24.0, keep_intermediates=False, tta=None):
         self.device = get_device() if device == 'auto' else torch.device(device)
         if isinstance(imgs, str):
             imgs = tiff.imread(imgs)
@@ -82,6 +86,9 @@ class Predict:
             self.imgs_shape = imgs.shape
         if imgs.dtype not in (np.uint8, np.uint16):
             raise TypeError(f'bio_image_unet_b200 normalises uint8 / uint16 stacks on the device; got {imgs.dtype}')
+        (self.patch_size, self.N_x, self.N_y, self.X_start, self.Y_start, self._wx, self._wy) = grid(
+            self.imgs_shape, max_patch_size, add_tile)
+        self.tta = P.tta_codes(tta, 2, self.patch_size)
 
         self.model_params = torch.load(model_params, map_location='cpu')
         heads = self.model_params['output_heads']
@@ -94,8 +101,6 @@ class Predict:
                              [(k + suffix, heads[k]['channels'], heads[k].get('activation')
                                if heads[k].get('activation') in ('sigmoid', 'tanh', 'relu') else None)
                               for k in self.target_keys], precision=precision, device=self.device)
-        (self.patch_size, self.N_x, self.N_y, self.X_start, self.Y_start, self._wx, self._wy) = grid(
-            self.imgs_shape, max_patch_size, add_tile)
         self.N_per_img = self.N_x * self.N_y
         self.N = self.N_per_img * self.imgs_shape[0]
 
@@ -134,18 +139,25 @@ class Predict:
         n_win = len(self._wx) * len(self._wy)
         patches = P.E.gather_tiles_f32(norm, [0], self._wx, self._wy, (1, ph, pw)).reshape(t * n_win, 1, ph, pw)
         tile_batch = P.pick_tile_batch(self.engine, (ph, pw), patches.shape[0], int(workspace_gb * 2 ** 30))
-        vals = []
-        it = range(0, patches.shape[0], tile_batch)
-        if self.show_progress and progress_notifier is not None:
-            it = progress_notifier.iterator(it)
-        for b0 in it:
-            tl = patches[b0:b0 + tile_batch]
-            cnt = tl.shape[0]
-            if cnt < tile_batch:
-                tl = torch.cat((tl, torch.zeros((tile_batch - cnt, *tl.shape[1:]), dtype=tl.dtype, device=dev)))
-            v, _ = self.engine.forward(tl.contiguous(), want_val=True, want_u8=False)
-            vals.append(v[:cnt])
-        vals = vals[0] if len(vals) == 1 else torch.cat(vals)                     # (P, head_total, ph, pw) float32
+        if self.tta is not None:       # mean over the transforms of every patch (float32), stitched like a patch
+            vals = P.run_tiles_tta(
+                lambda t: patches if t == 0 else P.E.gather_tiles_f32_tta(norm, [0], self._wx, self._wy, (1, ph, pw), 2,
+                                                                          t).reshape(-1, 1, ph, pw),
+                lambda tl, on_val: P.run_tiles(self.engine, tl, tile_batch, on_val=on_val),
+                patches.shape[0], self.tta, 2, out_dtype=torch.float32)
+        else:
+            vals = []
+            it = range(0, patches.shape[0], tile_batch)
+            if self.show_progress and progress_notifier is not None:
+                it = progress_notifier.iterator(it)
+            for b0 in it:
+                tl = patches[b0:b0 + tile_batch]
+                cnt = tl.shape[0]
+                if cnt < tile_batch:
+                    tl = torch.cat((tl, torch.zeros((tile_batch - cnt, *tl.shape[1:]), dtype=tl.dtype, device=dev)))
+                v, _ = self.engine.forward(tl.contiguous(), want_val=True, want_u8=False)
+                vals.append(v[:cnt])
+            vals = vals[0] if len(vals) == 1 else torch.cat(vals)                     # (P, head_total, ph, pw) float32
         # stitch per head (the hole value is the mean of that head's float16 patches, :279)
         idx = (np.arange(t)[:, None, None] * self.N_per_img + np.arange(self.N_x)[None, :, None] * self.N_y +
                np.arange(self.N_y)[None, None, :]).astype(np.int32)

@@ -17,12 +17,13 @@ from .multi_output_unet3d import MultiOutputUnet3D
 
 class Session:
     """Reusable multi-output 3D predictor (checkpoint folded / packed once, workspace resident).
-    precision: 'tf32' | 'fp16' | 'bf16' | 'fp32' (see unet.Predict)."""
+    precision: 'tf32' | 'fp16' | 'bf16' | 'fp32' (see unet.Predict); tta: None | 'flips' (see Predict)."""
 
     def __init__(self, model_params, max_patch_size=(64, 256, 256), overlap_factor=0.1, normalization_mode='single',
-                 clip_threshold=(0., 99.98), device='cuda:0', precision='tf32', workspace_gb=24.0, dist=None):
+                 clip_threshold=(0., 99.98), device='cuda:0', precision='tf32', workspace_gb=24.0, dist=None, tta=None):
         if normalization_mode not in ('single', 'first', 'all'):
             raise ValueError(f'Invalid normalization mode: {normalization_mode}')
+        self.tta = P.tta_codes(tta, 3, max_patch_size)
         params = torch.load(model_params, map_location='cpu') if isinstance(model_params, str) else model_params
         self.device = torch.device(device)
         self.max_patch_size, self.overlap_factor = max_patch_size, overlap_factor
@@ -37,7 +38,9 @@ class Session:
                              use_interpolation=params.get('use_interpolation', True), precision=precision,
                              device=self.device)
         self.tile_batch = None
-        self._planner = P.BatchPlanner(self.engine, self.workspace_bytes)
+        head_total = sum(self.output_heads[k]['channels'] for k in self.target_keys)
+        self._planner = P.BatchPlanner(self.engine, self.workspace_bytes,
+                                       lambda tile: P.tta_extra_bytes(tta, head_total, tile, in_bytes=4))
         self._out = P.PinnedOut()
         self._host_out, self._s_out = None, None
 
@@ -118,17 +121,31 @@ class Session:
             kept_p, kept_r = [], []
             for s in it:
                 e = min(s + vols_per_chunk, hi - lo)
-                patches = P.E.gather_tiles_f32(norm[s:e], self.Z_start, self.Y_start, self.X_start, self.patch_size)
-                patches = patches.reshape(-1, 1, *self.patch_size)
-                vals = []
-                for b0 in range(0, patches.shape[0], tile_batch):
-                    t = patches[b0:b0 + tile_batch]
-                    cnt = t.shape[0]
-                    if cnt < tile_batch:
-                        t = torch.cat((t, torch.zeros((tile_batch - cnt, *t.shape[1:]), dtype=t.dtype, device=dev)))
-                    v, _ = self.engine.forward(t.contiguous(), want_val=True, want_u8=False)
-                    vals.append(v[:cnt])
-                vals = vals[0] if len(vals) == 1 else torch.cat(vals)         # (n, head_total, pd, ph, pw)
+                if self.tta is None:
+                    patches = P.E.gather_tiles_f32(norm[s:e], self.Z_start, self.Y_start, self.X_start, self.patch_size)
+                    patches = patches.reshape(-1, 1, *self.patch_size)
+                    vals = []
+                    for b0 in range(0, patches.shape[0], tile_batch):
+                        t = patches[b0:b0 + tile_batch]
+                        cnt = t.shape[0]
+                        if cnt < tile_batch:
+                            t = torch.cat((t, torch.zeros((tile_batch - cnt, *t.shape[1:]), dtype=t.dtype, device=dev)))
+                        v, _ = self.engine.forward(t.contiguous(), want_val=True, want_u8=False)
+                        vals.append(v[:cnt])
+                    vals = vals[0] if len(vals) == 1 else torch.cat(vals)         # (n, head_total, pd, ph, pw)
+                else:       # mean over the 8 flips of every patch, merged on the device before the ramp blend
+                    plain = {}
+
+                    def gather(t):
+                        tl = P.E.gather_tiles_f32_tta(norm[s:e], self.Z_start, self.Y_start, self.X_start,
+                                                      self.patch_size, 3, t).reshape(-1, 1, *self.patch_size)
+                        if t == 0:
+                            plain['patches'] = tl
+                        return tl
+                    vals = P.run_tiles_tta(
+                        gather, lambda tl, on_val: P.run_tiles(self.engine, tl, tile_batch, on_val=on_val),
+                        (e - s) * self.N_per_vol, self.tta, 3, out_dtype=torch.float32)
+                    patches = plain['patches']
                 st = P.E.stitch_ramp_f32(vals, e - s, head_total, (d_img, h_img, w_img), self.Z_start, self.Y_start,
                                          self.X_start, self.patch_size, 16)
                 if on_device:
@@ -174,7 +191,9 @@ class Predict:
     normalization_mode='single' follows the reference's formula; the reference itself fails there on numpy >= 2
     (``ndarray.ptp`` was removed, :111). Integer stacks (uint8 / uint16) are normalised on the device.
     Engine-only keyword arguments: precision ('tf32' | 'fp16' | 'bf16' | 'fp32', see unet.Predict), workspace_gb,
-    distributed (volumes are sharded over ranks).
+    distributed (volumes are sharded over ranks), tta: None (default) or 'flips' - every patch also runs flipped along
+    every combination of z, y and x (8 forwards per patch); the head outputs are flipped back and averaged in fp32 on
+    the device before the ramp blend. About 8x the time of a plain prediction; memory stays within `workspace_gb`.
     """
 
     def __init__(self, imgs, model_params, result_path=None, network=MultiOutputUnet3D,
@@ -182,7 +201,8 @@ class Predict:
                  clip_threshold=(0., 99.98), add_tile=0, compress_tif=False, show_progress=True,
                  device: Union[torch.device, str] = 'auto',
                  progress_notifier: ProgressNotifier = ProgressNotifier.progress_notifier_tqdm(), *,
-                 precision='tf32', workspace_gb=24.0, distributed=False, keep_intermediates=False):
+                 precision='tf32', workspace_gb=24.0, distributed=False, keep_intermediates=False, tta=None):
+        P.tta_codes(tta, 3, max_patch_size)
         self.dist = DistContext(distributed)
         if device == 'auto':
             self.device = self.dist.device() if self.dist.active else get_device()
@@ -210,7 +230,7 @@ class Predict:
 
         self.model_params = torch.load(model_params, map_location='cpu')
         ses = Session(self.model_params, max_patch_size, overlap_factor, normalization_mode, clip_threshold,
-                      self.device, precision, workspace_gb, self.dist)
+                      self.device, precision, workspace_gb, self.dist, tta=tta)
         self.target_keys = ses.target_keys
         result = ses.predict(imgs, keep=keep_intermediates, progress_notifier=progress_notifier,
                              show_progress=show_progress)

@@ -79,8 +79,50 @@ class Normalizer2D:
         return E.apply_lut(frames_dev, lut)
 
 
-def run_tiles(eng, tiles, tile_batch, prev_tiles=None, want_val=False):
-    """Forward all tiles in batches of the planned size (the tail batch is zero-padded)."""
+TTA_MODES = (None, 'flips', 'dihedral')
+
+
+def tta_codes(tta, dims, tile):
+    """Transform codes of a predictor's `tta` setting, checked before any device work: None (no augmentation),
+    'flips' (2D: the 4 flips of y and x, t = 0..3; 3D: the 8 flips of z, y and x, t = 0..7) or 'dihedral' (2D square
+    tiles: all 8 symmetries of the square, t = 0..7; bit 2 transposes after the flips)."""
+    if tta is None:
+        return None
+    if not isinstance(tta, str) or tta not in TTA_MODES:
+        raise ValueError(f"tta must be one of {list(TTA_MODES)} (got {tta!r})")
+    if tta == 'flips':
+        return list(range(4 if dims == 2 else 8))
+    if dims != 2:
+        raise ValueError("tta='dihedral' needs 2D tiles: the 3D predictors take tta='flips' or None")
+    if int(tile[-1]) != int(tile[-2]):
+        raise ValueError(f"tta='dihedral' transposes tiles and needs square ones (got {tuple(tile)})")
+    return list(range(8))
+
+
+def tta_extra_bytes(tta, channels, tile, in_bytes=1):
+    """Device bytes per tile that test-time augmentation adds to a batch: the float output of the forward, the fp32
+    running sum and the transformed input tile."""
+    if tta is None:
+        return 0
+    px = int(np.prod(tile))
+    return 8 * int(channels) * px + int(in_bytes) * px
+
+
+def run_tiles(eng, tiles, tile_batch, prev_tiles=None, want_val=False, on_val=None):
+    """Forward all tiles in batches of the planned size (the tail batch is zero-padded). With `on_val` every batch's
+    float output is handed to on_val(start, val) instead of being returned, and no uint8 result is made."""
+    if on_val is not None:
+        for s in range(0, tiles.shape[0], tile_batch):
+            t = tiles[s:s + tile_batch]
+            p = None if prev_tiles is None else prev_tiles[s:s + tile_batch]
+            cnt = t.shape[0]
+            if cnt < tile_batch:
+                pad = torch.zeros((tile_batch - cnt, *t.shape[1:]), dtype=t.dtype, device=t.device)
+                t = torch.cat((t, pad))
+                p = None if p is None else torch.cat((p, pad))
+            val, _ = eng.forward(t.contiguous(), None if p is None else p.contiguous(), want_val=True, want_u8=False)
+            on_val(s, val[:cnt])
+        return None, None
     n = tiles.shape[0]
     outs_u8, outs_val = [], []
     for s in range(0, n, tile_batch):
@@ -114,17 +156,18 @@ class BatchPlanner:
     the planned batch (padding a 25-tile image to a 200-tile batch would cost 8x), and is never re-made for the
     shorter tail chunk of a movie (run_tiles pads that one)."""
 
-    def __init__(self, engine, workspace_bytes):
+    def __init__(self, engine, workspace_bytes, extra_per_tile=None):
         self.engine, self.workspace_bytes = engine, workspace_bytes
         self.tile, self.budget_batch, self.tile_batch = None, None, None
         self.plan_kwargs = {}                      # e.g. siam_shared=tiles per frame (Engine.plan)
+        self.extra_per_tile = extra_per_tile       # tile -> bytes per tile outside the workspace (test-time augmentation)
 
     def budget(self, tile):
         """Largest tile batch the workspace budget holds for this tile size."""
         tile = tuple(int(v) for v in tile)
         key = (tile, tuple(sorted(self.plan_kwargs.items())))
         if self.tile != key:
-            per_tile = self.engine.plan(1, tile)
+            per_tile = self.engine.plan(1, tile) + (self.extra_per_tile(tile) if self.extra_per_tile else 0)
             self.budget_batch = int(max(1, self.workspace_bytes // max(per_tile, 1)))
             self.tile, self.tile_batch = key, None
         return self.budget_batch
@@ -139,10 +182,11 @@ class BatchPlanner:
         return self.tile_batch
 
 
-def run_tiles_shared(eng, tiles_u, tile_batch, n_per):
+def run_tiles_shared(eng, tiles_u, tile_batch, n_per, on_val=None):
     """Siam_UNet with the shared twin encoder: tiles_u = [tiles of the previous frame of the first pair | tiles of the
     current frames] (n_pairs + n_per tiles); pair j = (previous tile j, current tile j + n_per). Batches of `tile_batch`
-    pairs take the contiguous slice of tile_batch + n_per unique tiles they need (the tail batch is zero-padded)."""
+    pairs take the contiguous slice of tile_batch + n_per unique tiles they need (the tail batch is zero-padded).
+    With `on_val` the float output of every batch goes to on_val(start pair, val) instead (as in run_tiles)."""
     n_pairs = tiles_u.shape[0] - n_per
     outs = []
     for s in range(0, n_pairs, tile_batch):
@@ -150,9 +194,39 @@ def run_tiles_shared(eng, tiles_u, tile_batch, n_per):
         t = tiles_u[s:s + cnt + n_per]
         if cnt < tile_batch:
             t = torch.cat((t, torch.zeros((tile_batch - cnt, *t.shape[1:]), dtype=t.dtype, device=t.device)))
-        _, u8 = eng.forward(t.contiguous(), None, want_val=False, want_u8=True)
-        outs.append(u8[:cnt])
+        val, u8 = eng.forward(t.contiguous(), None, want_val=on_val is not None, want_u8=on_val is None)
+        if on_val is not None:
+            on_val(s, val[:cnt])
+        else:
+            outs.append(u8[:cnt])
+    if on_val is not None:
+        return None
     return outs[0] if len(outs) == 1 else torch.cat(outs)
+
+
+def run_tiles_tta(gather, run, n, codes, dims, out_dtype=torch.uint8):
+    """Test-time augmentation of one chunk of `n` result tiles. For every transform code t of `codes`, in ascending
+    order: gather(t) makes the chunk's input tiles under T_t, run(tiles, on_val) runs the same forwards as a plain
+    prediction (run_tiles / run_tiles_shared with on_val), and every batch's float output goes through T_t^-1 into one
+    fp32 running sum of the chunk. The last pass writes the mean as the uint8 result tiles (trunc(mean * 255), as the
+    head does without augmentation) or as float32 (out_dtype). Plans, tile batches and stitches are those of a plain
+    prediction; the cost is len(codes) forwards per tile."""
+    k = len(codes)
+    bufs = {}
+
+    for p, t in enumerate(codes):
+        def on_val(s, val, p=p, t=t):
+            if not bufs:
+                shape = (n, *val.shape[1:])
+                bufs['out'] = torch.empty(shape, dtype=out_dtype, device=val.device)
+                bufs['acc'] = torch.empty(shape, dtype=torch.float32, device=val.device) if k > 1 else None
+            cnt = val.shape[0]
+            acc = None if bufs['acc'] is None else bufs['acc'][s:s + cnt]
+            out = bufs['out'][s:s + cnt]
+            E.tta_accumulate(val, acc, dims, t, p, k, out_u8=out if out_dtype == torch.uint8 else None,
+                             out_f32=out if out_dtype == torch.float32 else None)
+        run(gather(t), on_val)
+    return bufs['out']
 
 
 def pick_tile_batch(eng, tile, total_tiles, budget_bytes):
@@ -171,19 +245,34 @@ def check_starts(starts, tile, extent):
                              f'(image smaller than resize_dim with add_tile > 0)')
 
 
-def predict_frames_2d(eng, norm_u8, resize_dim, add_tile, out_channels, tile_batch, pad_mode=0, raw=None, lut=None):
+def predict_frames_2d(eng, norm_u8, resize_dim, add_tile, out_channels, tile_batch, pad_mode=0, raw=None, lut=None,
+                      tta=None):
     """norm_u8: (F, H, W) uint8 device tensor (already normalised) - or None with `raw` (the uint8 / uint16 stack) and
     `lut` (its normalisation tables): the normalisation is then fused into the tile gather and the normalised stack
-    is never written. Returns ((F, C, H, W) uint8 device tensor, grid, tiles, result_tiles)."""
+    is never written. tta: transform codes of test-time augmentation (tta_codes) or None. Returns ((F, C, H, W) uint8
+    device tensor, grid, tiles, result_tiles); with tta, `tiles` are the plain (t = 0) tiles."""
     f, h, w = (norm_u8 if norm_u8 is not None else raw).shape
     th, tw = resize_dim
     n_x, n_y, xs, ys = tiling.grid_2d(h, w, resize_dim, add_tile)
     check_starts(xs, th, h)
     check_starts(ys, tw, w)
-    if norm_u8 is not None:
+    if tta is not None:
+        src = (norm_u8 if norm_u8 is not None else raw).view(f, 1, h, w)
+        plain = {}
+
+        def gather(t):
+            tl = E.gather_tiles_tta(src, [0], xs, ys, (1, th, tw), pad_mode, 2, t, lut=None if norm_u8 is not None else lut)
+            if t == 0:
+                plain['tiles'] = tl
+            return tl
+        res_u8 = run_tiles_tta(gather, lambda tl, on_val: run_tiles(eng, tl, tile_batch, on_val=on_val),
+                               f * n_x * n_y, tta, 2)
+        tiles = plain['tiles']
+    elif norm_u8 is not None:
         tiles = E.gather_tiles(norm_u8.view(f, 1, h, w), [0], xs, ys, (1, th, tw), pad_mode)  # (F*N, 1, th, tw)
+        res_u8, _ = run_tiles(eng, tiles, tile_batch)
     else:
         tiles = E.gather_tiles_lut(raw.view(f, 1, h, w), lut, [0], xs, ys, (1, th, tw), pad_mode)
-    res_u8, _ = run_tiles(eng, tiles, tile_batch)
+        res_u8, _ = run_tiles(eng, tiles, tile_batch)
     out = E.stitch_mean_u8(res_u8, f, out_channels, (h, w), xs, ys, (th, tw))
     return out, (n_x, n_y, xs, ys), tiles, res_u8

@@ -57,12 +57,16 @@ class _TiffSource:
 class Session:
     """Reusable Siamese predictor: checkpoint folded / packed once, weights and workspace resident on the device.
     ``predict_stream`` runs pairs [lo, hi) of a page source through the three-stream pipeline.
-    precision: 'tf32' | 'fp16' | 'bf16' | 'fp32' (see unet.Predict)."""
+    precision: 'tf32' | 'fp16' | 'bf16' | 'fp32', tta: None | 'flips' | 'dihedral' (see unet.Predict; both frames of
+    a pair get the same transform)."""
 
     def __init__(self, model_params, resize_dim=(512, 512), invert=False, normalization_mode='single',
-                 clip_threshold=(0.0, 99.98), add_tile=0, device='cuda:0', precision='tf32', workspace_gb=24.0):
+                 clip_threshold=(0.0, 99.98), add_tile=0, device='cuda:0', precision='tf32', workspace_gb=24.0,
+                 tta=None):
         if normalization_mode not in ('single', 'first', 'all'):
             raise ValueError(f'normalization_mode {normalization_mode} not valid!')
+        P.tta_codes(tta, 2, resize_dim if resize_dim is not None else (1, 1))   # whole frames: checked per frame size
+        self.tta_mode = tta
         params = torch.load(model_params, map_location='cpu') if isinstance(model_params, str) else model_params
         self.device = torch.device(device)
         self.resize_dim, self.add_tile, self.invert = resize_dim, add_tile, invert
@@ -71,7 +75,8 @@ class Session:
         self.engine = Engine('siam2d', params['state_dict'], params['n_filter'], 1, [('', 1, 'sigmoid')],
                              siam_mode=params['mode'], precision=precision, device=self.device)
         self.tile_batch = None
-        self._planner = P.BatchPlanner(self.engine, self.workspace_bytes)
+        self._planner = P.BatchPlanner(self.engine, self.workspace_bytes,
+                                       lambda tile: P.tta_extra_bytes(tta, 1, tile, in_bytes=2))
         # per-frame normalisation + a join that uses the previous frame: frame t's encoder pass serves pair t (as the
         # current frame) and pair t + 1 (as the previous one) - it runs once (biu_net_set_siam_shared)
         self.shared_encoder = normalization_mode == 'single' and params['mode'] != 'control'
@@ -112,6 +117,7 @@ class Session:
         k, h, w = frames.shape
         rd, n_x, n_y, xs, ys = self.grid(h, w)
         th, tw = rd
+        tta = P.tta_codes(self.tta_mode, 2, rd)
         n_pairs = int(c_sel.shape[0])
         q_lo, q_hi = self.clip_threshold
         hist = P.E.histogram(frames)
@@ -122,9 +128,23 @@ class Session:
             P.check_starts(xs, th, h)
             P.check_starts(ys, tw, w)
             lut, _ = P.E.norm_lut(hist, hist, k, q_lo, q_hi, self.invert)
-            tiles_u = P.E.gather_tiles_lut(frames.contiguous().view(k, 1, h, w), lut, [0], xs, ys, (1, th, tw), 1)
             n_per = n_x * n_y
-            res_u8 = P.run_tiles_shared(self.engine, tiles_u, self.tile_batch, n_per)
+            if tta is None:
+                tiles_u = P.E.gather_tiles_lut(frames.contiguous().view(k, 1, h, w), lut, [0], xs, ys, (1, th, tw), 1)
+                res_u8 = P.run_tiles_shared(self.engine, tiles_u, self.tile_batch, n_per)
+            else:       # every unique tile of a pass carries the same transform: the shared encoder runs as it is
+                plain = {}
+
+                def gather(t):
+                    tl = P.E.gather_tiles_tta(frames.contiguous().view(k, 1, h, w), [0], xs, ys, (1, th, tw), 1, 2, t,
+                                              lut=lut)
+                    if t == 0:
+                        plain['tiles'] = tl
+                    return tl
+                res_u8 = P.run_tiles_tta(
+                    gather, lambda tl, on_val: P.run_tiles_shared(self.engine, tl, self.tile_batch, n_per, on_val=on_val),
+                    n_pairs * n_per, tta, 2)
+                tiles_u = plain['tiles']
             st = P.E.stitch_mean_u8(res_u8, n_pairs, 1, (h, w), xs, ys, (th, tw))
             self.last = dict(tiles_cur=tiles_u[n_per:], tiles_prev=tiles_u[:n_pairs * n_per], result_tiles=res_u8) if keep else {}
             return st
@@ -140,9 +160,24 @@ class Session:
             norm_cur = P.E.apply_lut(_take(frames, c_sel), lut)
         P.check_starts(xs, th, h)
         P.check_starts(ys, tw, w)
-        tiles_cur = P.E.gather_tiles(norm_cur.view(n_pairs, 1, h, w), [0], xs, ys, (1, th, tw), 1)      # zero padding
-        tiles_prev = P.E.gather_tiles(norm_prev.view(n_pairs, 1, h, w), [0], xs, ys, (1, th, tw), 1)
-        res_u8, _ = P.run_tiles(self.engine, tiles_cur, self.tile_batch, prev_tiles=tiles_prev)
+        if tta is None:
+            tiles_cur = P.E.gather_tiles(norm_cur.view(n_pairs, 1, h, w), [0], xs, ys, (1, th, tw), 1)      # zero padding
+            tiles_prev = P.E.gather_tiles(norm_prev.view(n_pairs, 1, h, w), [0], xs, ys, (1, th, tw), 1)
+            res_u8, _ = P.run_tiles(self.engine, tiles_cur, self.tile_batch, prev_tiles=tiles_prev)
+        else:           # both frames of a pair get the same transform
+            plain = {}
+
+            def gather(t):
+                tl = tuple(P.E.gather_tiles_tta(nf.view(n_pairs, 1, h, w), [0], xs, ys, (1, th, tw), 1, 2, t)
+                           for nf in (norm_cur, norm_prev))
+                if t == 0:
+                    plain['tiles'] = tl
+                return tl
+            res_u8 = P.run_tiles_tta(
+                gather, lambda tl, on_val: P.run_tiles(self.engine, tl[0], self.tile_batch, prev_tiles=tl[1],
+                                                       on_val=on_val),
+                n_pairs * n_x * n_y, tta, 2)
+            tiles_cur, tiles_prev = plain['tiles']
         st = P.E.stitch_mean_u8(res_u8, n_pairs, 1, (h, w), xs, ys, (th, tw))
         self.last = dict(tiles_cur=tiles_cur, tiles_prev=tiles_prev, result_tiles=res_u8) if keep else {}
         return st
@@ -250,14 +285,16 @@ class Predict:
 
     tif_file : str (an ndarray (T, H, W) is also accepted); resize_dim=None processes whole frames.
     Engine-only keyword arguments: precision ('tf32' | 'fp16' | 'bf16' | 'fp32'), workspace_gb, distributed,
-    keep_intermediates (see unet.Predict).
+    keep_intermediates, tta (None | 'flips' | 'dihedral'; see unet.Predict). With tta both frames of a pair get the
+    same flip / rotation, and the shared-encoder mode stays shared.
     """
 
     def __init__(self, tif_file, result_name, model_params, resize_dim=(512, 512), invert=False,
                  normalization_mode='single', clip_threshold=(0.0, 99.98), add_tile=0, normalize_result=False,
                  show_progress=True, device: Union[torch.device, str] = 'auto',
                  progress_notifier: ProgressNotifier = ProgressNotifier.progress_notifier_tqdm(), *,
-                 precision='tf32', workspace_gb=24.0, distributed=False, keep_intermediates=False):
+                 precision='tf32', workspace_gb=24.0, distributed=False, keep_intermediates=False, tta=None):
+        P.tta_codes(tta, 2, resize_dim if resize_dim is not None else (1, 1))
         self.dist = DistContext(distributed)
         if device == 'auto':
             self.device = self.dist.device() if self.dist.active else get_device()
@@ -278,7 +315,7 @@ class Predict:
         # load model
         self.model_params = torch.load(model_params, map_location='cpu')
         self.session = Session(self.model_params, resize_dim, invert, normalization_mode, clip_threshold, add_tile,
-                               self.device, precision, workspace_gb)
+                               self.device, precision, workspace_gb, tta=tta)
 
         if isinstance(tif_file, str):
             source = _TiffSource(tif_file)

@@ -156,6 +156,25 @@ int biu_gather_tiles_lut(const void* src, int dtype_bytes, const uint8_t* lut, l
                          int W, int pad_mode, const int* zs, const int* ys, const int* xs, int nz, int ny, int nx, int pd,
                          int ph, int pw, uint8_t* dst, void* stream);
 
+/* ---- test-time augmentation (engine-only, replaces nothing in the reference) ---------------------------------
+ * Transform code t of a tile: 2D (dims 2): bit 0 flips x, bit 1 flips y, bit 2 transposes after the flips (square tiles
+ * only); 3D (dims 3): bits 0, 1, 2 flip x, y, z. The transform acts on the tile after the far-end padding, and t = 0 is
+ * the plain tile. */
+/* biu_gather_tiles / biu_gather_tiles_lut producing T_t(tile): a uint8 source (lut NULL) or a uint8 / uint16 source
+ * with its normalisation tables. */
+int biu_gather_tiles_tta(const void* src, int dtype_bytes, const uint8_t* lut, long long lut_stride, int F, int Z, int H,
+                         int W, int pad_mode, const int* zs, const int* ys, const int* xs, int nz, int ny, int nx, int pd,
+                         int ph, int pw, int dims, int t, uint8_t* dst, void* stream);
+/* biu_gather_tiles_f32 producing T_t(patch). */
+int biu_gather_tiles_f32_tta(const float* src, int F, int Z, int H, int W, const int* zs, const int* ys, const int* xs,
+                             int nz, int ny, int nx, int pd, int ph, int pw, int dims, int t, float* dst, void* stream);
+/* Pass `pass` of `passes` (a power of two) of the merge: val [planes][pd][ph][pw] is the net's float output on the tiles
+ * of transform t; acc (same shape, fp32) = sum in pass order of T_t^-1(val). Pass 0 writes acc, the last pass writes
+ * mean = acc * (1 / passes) to out_f32 and / or out_u8 = trunc(mean * 255) (the rule of biu_net_forward's out_u8) and
+ * leaves acc as it was. Deterministic (no atomics). */
+int biu_tta_accumulate(const float* val, long long planes, int pd, int ph, int pw, int dims, int t, int pass, int passes,
+                       float* acc, uint8_t* out_u8, float* out_f32, void* stream);
+
 /* ---- stitching: replaces Predict.__stitch -------------------------------------------------------------------*/
 /* unet/predict.py:204-229, siam_unet/predict.py:217-240: uint8(nanmean) == sum // count.
  * tiles [F][ny*nx][C][ph][pw] -> out [F][C][H][W] */
