@@ -49,6 +49,8 @@ SIGNATURES = {
     'biu_stitch_mean_u8': (c_int, [_P, c_int, c_int, c_int, c_int, _P, _P, c_int, c_int, c_int, c_int, _P, _P]),
     'biu_stitch_mod3_u8': (c_int, [_P, c_int, c_int, c_int, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_int, _P,
                                    _P]),
+    'biu_stitch_weighted_u8': (c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, c_int, c_int, c_int, c_int,
+                                       c_int, c_int, _P, _P, _P, _P, _P]),
     'biu_stitch_ramp_f32': (c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, c_int, c_int, c_int, c_int,
                                     c_int, c_int, c_int, _P, _P]),
     'biu_normalize_f32_scratch_bytes': (ctypes.c_longlong, [ctypes.c_longlong, c_int]),

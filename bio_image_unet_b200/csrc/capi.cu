@@ -215,6 +215,12 @@ int biu_stitch_mod3_u8(const uint8_t* tiles, int Z, int H, int W, const int* zs,
   StitchMod3Args a{tiles, Z, H, W, zs, ys, xs, nz, ny, nx, pd, ph, pw, out};
   return launch_stitch_mod3(a, (cudaStream_t)stream);
 }
+int biu_stitch_weighted_u8(const uint8_t* tiles, int F, int C, int Z, int H, int W, const int* zs, const int* ys,
+                           const int* xs, int nz, int ny, int nx, int pd, int ph, int pw, const int* w_d, const int* w_h,
+                           const int* w_w, uint8_t* out, void* stream) {
+  StitchWeightedArgs a{tiles, F, C, Z, H, W, zs, ys, xs, nz, ny, nx, pd, ph, pw, w_d, w_h, w_w, out};
+  return launch_stitch_weighted(a, (cudaStream_t)stream);
+}
 int biu_stitch_ramp_f32(const float* tiles, int V, int C, int Z, int H, int W, const int* zs, const int* ys,
                         const int* xs, int nz, int ny, int nx, int pd, int ph, int pw, int margin, float* out,
                         void* stream) {

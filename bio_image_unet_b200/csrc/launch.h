@@ -217,6 +217,15 @@ struct StitchMod3Args {         // unet3d/predict.py:173-195
   uint8_t* out;                 // [Z][H][W]
 };
 int launch_stitch_mod3(const StitchMod3Args& a, cudaStream_t stream);
+struct StitchWeightedArgs {     // engine-only: (sum w * v) // (sum w), w = w_d[tz] * w_h[ty] * w_w[tx]
+  const uint8_t* tiles;         // [F][nz*ny*nx][C][pd][ph][pw]
+  int F, C, Z, H, W;            // output extents; starts may be negative and tiles may reach past the output
+  const int* zs; const int* ys; const int* xs;
+  int nz, ny, nx, pd, ph, pw;
+  const int* w_d; const int* w_h; const int* w_w;   // device int32 tables of pd / ph / pw entries in [0, 1024]
+  uint8_t* out;                 // [F][C][Z][H][W]
+};
+int launch_stitch_weighted(const StitchWeightedArgs& a, cudaStream_t stream);
 struct StitchRampArgs {         // multi_output_unet3d/predict.py:203-307
   const float* tiles;           // [V][nz*ny*nx][C][pd][ph][pw]
   int V, C, Z, H, W;

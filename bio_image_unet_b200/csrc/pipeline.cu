@@ -742,6 +742,102 @@ int launch_stitch_mod3(const StitchMod3Args& a, cudaStream_t stream) {
 }
 
 // ------------------------------------------------------------------------------------------------
+// Weighted overlap stitch (engine-only, no reference counterpart): out = (sum w * v) // (sum w) over the tiles covering
+// an element, w = w_d[tz] * w_h[ty] * w_w[tx] (each table entry in [0, 1024], so w <= 2^30 and w * v < 2^38), in exact
+// unsigned 64-bit integer arithmetic: the result does not depend on the order of the sum. Gather form of
+// stitch_mean_kernel (16 output elements per thread, one 16-byte load per covering tile where aligned, no atomics).
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) stitch_weighted_kernel(StitchWeightedArgs a) {
+  extern __shared__ unsigned int s_w[];                // [pd] w_d | [ph] w_h | [pw] w_w
+  unsigned int* s_wd = s_w;
+  unsigned int* s_wh = s_w + a.pd;
+  unsigned int* s_ww = s_wh + a.ph;
+  for (int i = threadIdx.x; i < a.pd + a.ph + a.pw; i += blockDim.x)
+    s_w[i] = (unsigned int)__ldg(i < a.pd ? a.w_d + i : (i < a.pd + a.ph ? a.w_h + (i - a.pd) : a.w_w + (i - a.pd - a.ph)));
+  __syncthreads();
+  const int W16 = (a.W + 15) / 16;
+  const int ntiles = a.nz * a.ny * a.nx;
+  const long long total = (long long)a.F * a.C * a.Z * a.H * W16;
+  for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
+       idx += (long long)gridDim.x * blockDim.x) {
+    long long r = idx;
+    const int x16 = (int)(r % W16) * 16; r /= W16;
+    const int y = (int)(r % a.H); r /= a.H;
+    const int z = (int)(r % a.Z); r /= a.Z;
+    const int c = (int)(r % a.C); r /= a.C;
+    const int f = (int)r;
+    unsigned long long num[16], den[16];
+#pragma unroll
+    for (int q = 0; q < 16; ++q) { num[q] = 0; den[q] = 0; }
+    for (int i = 0; i < a.nz; ++i) {
+      const int tz = z - a.zs[i];
+      if (tz < 0 || tz >= a.pd) continue;
+      for (int j = 0; j < a.ny; ++j) {
+        const int ty = y - a.ys[j];
+        if (ty < 0 || ty >= a.ph) continue;
+        const unsigned int wzy = s_wd[tz] * s_wh[ty];   // <= 2^20: the tile row's factor
+        for (int k = 0; k < a.nx; ++k) {
+          const int tx0 = x16 - a.xs[k];
+          if (tx0 <= -16 || tx0 >= a.pw) continue;
+          const long long n = (long long)f * ntiles + (i * a.ny + j) * a.nx + k;
+          const uint8_t* t = a.tiles + (((n * a.C + c) * a.pd + tz) * a.ph + ty) * a.pw;
+          if (tx0 >= 0 && tx0 + 16 <= a.pw && ((reinterpret_cast<uintptr_t>(t + tx0) & 15) == 0)) {
+            const uint4 v4 = __ldg(reinterpret_cast<const uint4*>(t + tx0));
+            const uint8_t* e = reinterpret_cast<const uint8_t*>(&v4);
+#pragma unroll
+            for (int q = 0; q < 16; ++q) {
+              const unsigned int w = wzy * s_ww[tx0 + q];
+              num[q] += (unsigned long long)w * e[q];
+              den[q] += w;
+            }
+          } else {
+#pragma unroll
+            for (int q = 0; q < 16; ++q) {
+              const int tx = tx0 + q;
+              if (tx >= 0 && tx < a.pw) {
+                const unsigned int w = wzy * s_ww[tx];
+                num[q] += (unsigned long long)w * __ldg(t + tx);
+                den[q] += w;
+              }
+            }
+          }
+        }
+      }
+    }
+    uint8_t o16[16];
+#pragma unroll
+    for (int q = 0; q < 16; ++q)                       // no covering tile, or zero weight: 0
+      o16[q] = den[q] ? (uint8_t)(num[q] / den[q]) : (uint8_t)0;
+    uint8_t* o = a.out + ((((long long)f * a.C + c) * a.Z + z) * a.H + y) * a.W + x16;
+    if (x16 + 16 <= a.W && ((reinterpret_cast<uintptr_t>(o) & 15) == 0)) {
+      *reinterpret_cast<uint4*>(o) = *reinterpret_cast<uint4*>(o16);
+    } else {
+#pragma unroll
+      for (int q = 0; q < 16; ++q)
+        if (x16 + q < a.W) o[q] = o16[q];
+    }
+  }
+}
+int launch_stitch_weighted(const StitchWeightedArgs& a, cudaStream_t stream) {
+  BIU_REQUIRE(a.tiles && a.out && a.zs && a.ys && a.xs && a.w_d && a.w_h && a.w_w, "stitch_weighted: null pointer");
+  BIU_REQUIRE(a.F > 0 && a.C > 0 && a.Z > 0 && a.H > 0 && a.W > 0, "stitch_weighted: bad output extents F=%d C=%d Z=%d H=%d W=%d",
+              a.F, a.C, a.Z, a.H, a.W);
+  BIU_REQUIRE(a.nz > 0 && a.ny > 0 && a.nx > 0 && a.pd > 0 && a.ph > 0 && a.pw > 0,
+              "stitch_weighted: bad grid %dx%dx%d or tile %dx%dx%d", a.nz, a.ny, a.nx, a.pd, a.ph, a.pw);
+  const long long table_bytes = 4LL * (a.pd + a.ph + a.pw);
+  BIU_REQUIRE(table_bytes <= 48 * 1024, "stitch_weighted: tile extents %d + %d + %d exceed the shared-memory tables",
+              a.pd, a.ph, a.pw);
+  const long long total = (long long)a.F * a.C * a.Z * a.H * ((a.W + 15) / 16);
+  long long blocks = ceil_div_ll(total, 256);
+  if (blocks > 148LL * 32) blocks = 148LL * 32;
+  if (blocks < 1) blocks = 1;
+  stitch_weighted_kernel<<<(int)blocks, 256, (size_t)table_bytes, stream>>>(a);
+  BIU_CHECK_CUDA(cudaGetLastError());
+  count_launch();
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
 // Multi-output 3D blend (multi_output_unet3d/predict.py:203-307, blend_margin rules as written):
 // weight starts at 1; z rule, then y rule, then x rule overwrite (not multiply); the "far side" ramps all
 // land on index 0 with final value (margin-1)/margin. Accumulation order = patch order z -> y -> x in fp32.

@@ -379,6 +379,33 @@ def stitch_mod3_u8(tiles, out_zhw, zs, ys, xs, tile):
     return out
 
 
+def stitch_weighted_u8(tiles, frames, channels, out_zhw, zs, ys, xs, tile, w_d, w_h, w_w):
+    """Engine-only weighted stitch: tiles (F*nz*ny*nx, C, pd, ph, pw) uint8 -> (F, C, Z, H, W) uint8,
+    out = (sum w * v) // (sum w) over the covering tiles, w = w_d[tz] * w_h[ty] * w_w[tx], in exact integer arithmetic
+    (0 where nothing covers an element). Starts may be negative; w_d / w_h / w_w have pd / ph / pw entries in [0, 1024]."""
+    lib = _lib.load()
+    dev = tiles.device
+    pd, ph, pw = (int(v) for v in tile)
+    tables = []
+    for name, tab, n in (('w_d', w_d, pd), ('w_h', w_h, ph), ('w_w', w_w, pw)):
+        tab = [int(v) for v in tab]
+        if len(tab) != n:
+            raise ValueError(f'{name} has {len(tab)} entries for a tile axis of {n}')
+        if min(tab) < 0 or max(tab) > 1024:
+            raise ValueError(f'{name} entries must lie in [0, 1024]')
+        tables.append(_dev_i32(tab, dev))
+    assert tiles.is_contiguous() and tiles.dtype == torch.uint8
+    assert tiles.numel() == frames * len(zs) * len(ys) * len(xs) * channels * pd * ph * pw, (tiles.shape, tile)
+    dzs, dys, dxs = _dev_i32(zs, dev), _dev_i32(ys, dev), _dev_i32(xs, dev)
+    out = torch.empty((frames, channels, *out_zhw), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.biu_stitch_weighted_u8(_lib.ptr(tiles), frames, channels, out_zhw[0], out_zhw[1], out_zhw[2],
+                                              _lib.ptr(dzs), _lib.ptr(dys), _lib.ptr(dxs), len(zs), len(ys), len(xs),
+                                              pd, ph, pw, *(_lib.ptr(t) for t in tables), _lib.ptr(out),
+                                              _lib.stream_ptr()), 'biu_stitch_weighted_u8')
+    return out
+
+
 def stitch_ramp_f32(tiles, vols, channels, out_zhw, zs, ys, xs, tile, margin=16):
     lib = _lib.load()
     dev = tiles.device

@@ -3,6 +3,8 @@
 Reference: unet/predict.py:115-229 (and the per-pair variant siam_unet/predict.py:125-240). All heavy steps run
 as CUDA kernels through the C-ABI; this module only sequences them and does the (tiny) index arithmetic.
 """
+import functools
+
 import numpy as np
 import torch
 
@@ -97,6 +99,42 @@ def tta_codes(tta, dims, tile):
     if int(tile[-1]) != int(tile[-2]):
         raise ValueError(f"tta='dihedral' transposes tiles and needs square ones (got {tuple(tile)})")
     return list(range(8))
+
+
+BLEND_MODES = (None, 'gaussian')
+
+
+def blend_mode(blend):
+    """A predictor's `blend` setting, checked before any device work: None (the reference's stitch) or 'gaussian'
+    (overlapping tiles weighted by blend_tables, exact integer weighted mean of the uint8 result tiles)."""
+    if blend is None:
+        return None
+    if not isinstance(blend, str) or blend not in BLEND_MODES:
+        raise ValueError(f"blend must be one of {list(BLEND_MODES)} (got {blend!r})")
+    return blend
+
+
+@functools.lru_cache(maxsize=None)
+def _gaussian_table(n):
+    return tuple(int(v) for v in tiling.gaussian_weights(n))
+
+
+def blend_tables(tile):
+    """Per-axis weight tables (w_d, w_h, w_w) of blend='gaussian' for a 2D (th, tw) tile (w_d = [1]) or a 3D
+    (pd, ph, pw) patch."""
+    tile = tuple(int(v) for v in tile)
+    return ((1,) if len(tile) == 2 else _gaussian_table(tile[0])), _gaussian_table(tile[-2]), _gaussian_table(tile[-1])
+
+
+def stitch_2d(res_u8, frames, channels, out_hw, xs, ys, tile_hw, blend=None):
+    """Stitch of the (frames * N, C, th, tw) uint8 result tiles of a 2D grid (xs: starts along rows, ys: along
+    columns) into (frames, C, H, W): the reference's mean (blend None) or the weighted stitch of blend='gaussian'.
+    One tile per frame (Siam_UNet on whole frames) has nothing to blend: both give the tile itself."""
+    if blend is None or len(xs) * len(ys) == 1:
+        return E.stitch_mean_u8(res_u8, frames, channels, out_hw, xs, ys, tile_hw)
+    out = E.stitch_weighted_u8(res_u8, frames, channels, (1, *out_hw), [0], xs, ys, (1, *tile_hw),
+                               *blend_tables(tile_hw))
+    return out.view(frames, channels, *out_hw)
 
 
 def tta_extra_bytes(tta, channels, tile, in_bytes=1):
@@ -246,11 +284,12 @@ def check_starts(starts, tile, extent):
 
 
 def predict_frames_2d(eng, norm_u8, resize_dim, add_tile, out_channels, tile_batch, pad_mode=0, raw=None, lut=None,
-                      tta=None):
+                      tta=None, blend=None):
     """norm_u8: (F, H, W) uint8 device tensor (already normalised) - or None with `raw` (the uint8 / uint16 stack) and
     `lut` (its normalisation tables): the normalisation is then fused into the tile gather and the normalised stack
-    is never written. tta: transform codes of test-time augmentation (tta_codes) or None. Returns ((F, C, H, W) uint8
-    device tensor, grid, tiles, result_tiles); with tta, `tiles` are the plain (t = 0) tiles."""
+    is never written. tta: transform codes of test-time augmentation (tta_codes) or None; blend: blend_mode() value.
+    Returns ((F, C, H, W) uint8 device tensor, grid, tiles, result_tiles); with tta, `tiles` are the plain (t = 0)
+    tiles."""
     f, h, w = (norm_u8 if norm_u8 is not None else raw).shape
     th, tw = resize_dim
     n_x, n_y, xs, ys = tiling.grid_2d(h, w, resize_dim, add_tile)
@@ -274,5 +313,5 @@ def predict_frames_2d(eng, norm_u8, resize_dim, add_tile, out_channels, tile_bat
     else:
         tiles = E.gather_tiles_lut(raw.view(f, 1, h, w), lut, [0], xs, ys, (1, th, tw), pad_mode)
         res_u8, _ = run_tiles(eng, tiles, tile_batch)
-    out = E.stitch_mean_u8(res_u8, f, out_channels, (h, w), xs, ys, (th, tw))
+    out = stitch_2d(res_u8, f, out_channels, (h, w), xs, ys, (th, tw), blend)
     return out, (n_x, n_y, xs, ys), tiles, res_u8

@@ -58,14 +58,15 @@ class Session:
     """Reusable Siamese predictor: checkpoint folded / packed once, weights and workspace resident on the device.
     ``predict_stream`` runs pairs [lo, hi) of a page source through the three-stream pipeline.
     precision: 'tf32' | 'fp16' | 'bf16' | 'fp32', tta: None | 'flips' | 'dihedral' (see unet.Predict; both frames of
-    a pair get the same transform)."""
+    a pair get the same transform), blend: None | 'gaussian' (see unet.Predict)."""
 
     def __init__(self, model_params, resize_dim=(512, 512), invert=False, normalization_mode='single',
                  clip_threshold=(0.0, 99.98), add_tile=0, device='cuda:0', precision='tf32', workspace_gb=24.0,
-                 tta=None):
+                 tta=None, blend=None):
         if normalization_mode not in ('single', 'first', 'all'):
             raise ValueError(f'normalization_mode {normalization_mode} not valid!')
         P.tta_codes(tta, 2, resize_dim if resize_dim is not None else (1, 1))   # whole frames: checked per frame size
+        self.blend = P.blend_mode(blend)
         self.tta_mode = tta
         params = torch.load(model_params, map_location='cpu') if isinstance(model_params, str) else model_params
         self.device = torch.device(device)
@@ -145,7 +146,7 @@ class Session:
                     gather, lambda tl, on_val: P.run_tiles_shared(self.engine, tl, self.tile_batch, n_per, on_val=on_val),
                     n_pairs * n_per, tta, 2)
                 tiles_u = plain['tiles']
-            st = P.E.stitch_mean_u8(res_u8, n_pairs, 1, (h, w), xs, ys, (th, tw))
+            st = P.stitch_2d(res_u8, n_pairs, 1, (h, w), xs, ys, (th, tw), self.blend)
             self.last = dict(tiles_cur=tiles_u[n_per:], tiles_prev=tiles_u[:n_pairs * n_per], result_tiles=res_u8) if keep else {}
             return st
         if self.normalization_mode == 'single':       # each frame on its own statistics (:128-136)
@@ -178,7 +179,7 @@ class Session:
                                                        on_val=on_val),
                 n_pairs * n_x * n_y, tta, 2)
             tiles_cur, tiles_prev = plain['tiles']
-        st = P.E.stitch_mean_u8(res_u8, n_pairs, 1, (h, w), xs, ys, (th, tw))
+        st = P.stitch_2d(res_u8, n_pairs, 1, (h, w), xs, ys, (th, tw), self.blend)
         self.last = dict(tiles_cur=tiles_cur, tiles_prev=tiles_prev, result_tiles=res_u8) if keep else {}
         return st
 
@@ -286,15 +287,18 @@ class Predict:
     tif_file : str (an ndarray (T, H, W) is also accepted); resize_dim=None processes whole frames.
     Engine-only keyword arguments: precision ('tf32' | 'fp16' | 'bf16' | 'fp32'), workspace_gb, distributed,
     keep_intermediates, tta (None | 'flips' | 'dihedral'; see unet.Predict). With tta both frames of a pair get the
-    same flip / rotation, and the shared-encoder mode stays shared.
+    same flip / rotation, and the shared-encoder mode stays shared. blend (None | 'gaussian'; see unet.Predict): with
+    resize_dim=None every frame is one tile, so there is nothing to blend and the result is the same.
     """
 
     def __init__(self, tif_file, result_name, model_params, resize_dim=(512, 512), invert=False,
                  normalization_mode='single', clip_threshold=(0.0, 99.98), add_tile=0, normalize_result=False,
                  show_progress=True, device: Union[torch.device, str] = 'auto',
                  progress_notifier: ProgressNotifier = ProgressNotifier.progress_notifier_tqdm(), *,
-                 precision='tf32', workspace_gb=24.0, distributed=False, keep_intermediates=False, tta=None):
+                 precision='tf32', workspace_gb=24.0, distributed=False, keep_intermediates=False, tta=None,
+                 blend=None):
         P.tta_codes(tta, 2, resize_dim if resize_dim is not None else (1, 1))
+        P.blend_mode(blend)
         self.dist = DistContext(distributed)
         if device == 'auto':
             self.device = self.dist.device() if self.dist.active else get_device()
@@ -315,7 +319,7 @@ class Predict:
         # load model
         self.model_params = torch.load(model_params, map_location='cpu')
         self.session = Session(self.model_params, resize_dim, invert, normalization_mode, clip_threshold, add_tile,
-                               self.device, precision, workspace_gb, tta=tta)
+                               self.device, precision, workspace_gb, tta=tta, blend=blend)
 
         if isinstance(tif_file, str):
             source = _TiffSource(tif_file)

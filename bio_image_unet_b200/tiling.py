@@ -42,6 +42,19 @@ def strided_starts(extent, patch, overlap_factor):
     return starts
 
 
+def gaussian_weights(n):
+    """Centre-weighted blend table of a tile axis of length n >= 1 (engine-only `blend='gaussian'`), in float64:
+    sigma = n / 8, g(i) = 1024 * exp(-(i - (n - 1) / 2)^2 / (2 sigma^2)), w(i) = max(1, floor(g(i) + 0.5)) as int32.
+    Symmetric (w(i) = w(n - 1 - i)), every value in [1, 1024]; n = 1 gives [1024]."""
+    n = int(n)
+    if n < 1:
+        raise ValueError(f'a tile axis has at least one element (got {n})')
+    i = np.arange(n, dtype=np.float64)
+    sigma = n / 8
+    g = 1024.0 * np.exp(-(i - (n - 1) / 2) ** 2 / (2 * sigma ** 2))
+    return np.maximum(1, np.floor(g + 0.5)).astype(np.int32)
+
+
 def shard_range(n_items, rank, world_size):
     """Contiguous, balanced [start, stop) slice of n_items for `rank` (frames / z-rows of patches / volumes)."""
     base, rem = divmod(n_items, world_size)

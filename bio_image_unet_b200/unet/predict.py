@@ -19,17 +19,19 @@ class Session:
     ``predict(frames)`` takes a host (F, H, W) uint8/uint16 stack (ideally pinned) and returns the stitched
     (F, C, H, W) uint8 result on the host; ``predict_device`` does the same for a stack already in HBM.
     ``Predict`` (the reference's constructor-runs-everything class) is a thin wrapper around this.
-    precision: 'tf32' | 'fp16' | 'bf16' | 'fp32', tta: None | 'flips' | 'dihedral' (see Predict).
+    precision: 'tf32' | 'fp16' | 'bf16' | 'fp32', tta: None | 'flips' | 'dihedral', blend: None | 'gaussian' (see
+    Predict).
     """
 
     KINDS = {'Unet': 'unet2d', 'AttentionUnet': 'attunet2d', 'Unet_v0': 'unet2d_v0'}
 
     def __init__(self, model_params, resize_dim=(512, 512), invert=False, normalization_mode='single',
                  clip_threshold=(0., 99.8), add_tile=0, device='cuda:0', precision='tf32', workspace_gb=24.0,
-                 network='Unet', tta=None):
+                 network='Unet', tta=None, blend=None):
         if normalization_mode not in ('single', 'first', 'all'):
             raise ValueError(f'normalization_mode {normalization_mode} not valid!')
         self.tta = P.tta_codes(tta, 2, resize_dim)
+        self.blend = P.blend_mode(blend)
         params = torch.load(model_params, map_location='cpu') if isinstance(model_params, str) else model_params
         self.device = torch.device(device)
         self.resize_dim, self.add_tile, self.invert = tuple(resize_dim), add_tile, invert
@@ -113,7 +115,8 @@ class Session:
         if frames_dev.dtype == torch.float32 or want_norm:
             norm = self.normalise_device(frames_dev, lut)
             out, grid, tiles, res_tiles = P.predict_frames_2d(self.engine, norm, self.resize_dim, self.add_tile,
-                                                              self.out_channels, self.tile_batch, tta=self.tta)
+                                                              self.out_channels, self.tile_batch, tta=self.tta,
+                                                              blend=self.blend)
             if frames_dev.dtype == torch.float32:      # what the reference stores back into a float stack (:131)
                 norm = self.last_norm_f32
         else:
@@ -121,7 +124,7 @@ class Session:
             out, grid, tiles, res_tiles = P.predict_frames_2d(self.engine, None, self.resize_dim, self.add_tile,
                                                               self.out_channels, self.tile_batch,
                                                               raw=frames_dev.contiguous(), lut=self.lut_device(frames_dev, lut),
-                                                              tta=self.tta)
+                                                              tta=self.tta, blend=self.blend)
         self.last = dict(grid=grid, norm=norm, tiles=tiles if keep else None, result_tiles=res_tiles if keep else None)
         return out
 
@@ -348,6 +351,10 @@ class Predict:
         rotations of the square (8 forwards). Each output is mapped back onto the tile, the float outputs are averaged
         in fp32 on the device, and the mean is quantised to uint8 once before the usual stitch. Costs about 4x / 8x
         the time of a plain prediction; tiles per forward and device memory stay within `workspace_gb`.
+    blend : overlap stitch. None (default): the reference's mean of the overlapping tiles. 'gaussian': every tile's
+        uint8 result is weighted by a centre-peaked Gaussian (sigma = tile / 8 per axis, tiling.gaussian_weights), so
+        that pixels near a tile border, where the net saw the least context, count least; out = (sum w * v) // (sum w)
+        in exact integer arithmetic. Composes with `tta` (the averaged tiles are blended).
     """
 
     def __init__(self, imgs, result_name, model_params, network='Unet', resize_dim=(512, 512),
@@ -355,8 +362,9 @@ class Predict:
                  normalize_result=False, show_progress=True, device: Union[torch.device, str] = 'auto',
                  progress_notifier: ProgressNotifier = ProgressNotifier.progress_notifier_tqdm(), *,
                  precision='tf32', workspace_gb=24.0, mutate_input=True, distributed=False,
-                 keep_intermediates=False, tta=None):
+                 keep_intermediates=False, tta=None, blend=None):
         P.tta_codes(tta, 2, resize_dim)
+        P.blend_mode(blend)
         self.dist = DistContext(distributed)
         self._keep = {'patches': [], 'result_patches': []} if keep_intermediates else None
         if device == 'auto':
@@ -400,7 +408,7 @@ class Predict:
             raise RuntimeError("shape '[1, %d, %d, %d]' is invalid for input of size %d" % (
                 self.model_params['in_channels'], resize_dim[0], resize_dim[1], resize_dim[0] * resize_dim[1]))
         self.session = Session(self.model_params, resize_dim, invert, normalization_mode, clip_threshold, add_tile,
-                               self.device, precision, workspace_gb, network=name, tta=tta)
+                               self.device, precision, workspace_gb, network=name, tta=tta, blend=blend)
 
         # frames of this rank
         t_total = self.imgs_shape[0]

@@ -17,17 +17,20 @@ from .unet3d import UNet3D
 class Session:
     """Reusable 3D predictor: checkpoint folded / packed once; ``predict(vol)`` runs a (Z, X, Y) uint8 / uint16 host
     volume through normalise -> split -> forward -> mod-3 stitch and returns the uint8 result (on rank 0).
-    precision: 'tf32' | 'fp16' | 'bf16' | 'fp32' (see unet.Predict); tta: None | 'flips' (see Predict)."""
+    precision: 'tf32' | 'fp16' | 'bf16' | 'fp32' (see unet.Predict); tta: None | 'flips', blend: None | 'gaussian'
+    (see Predict)."""
 
     def __init__(self, model_params, resize_dim, invert=False, clip_threshold=(0., 99.8), add_patch=0, device='cuda:0',
-                 precision='tf32', workspace_gb=24.0, dist=None, tta=None):
+                 precision='tf32', workspace_gb=24.0, dist=None, tta=None, blend=None):
         if len(resize_dim) != 3:
             raise IndexError('tuple index out of range')      # the reference indexes resize_dim[2] (:123)
         self.tta = P.tta_codes(tta, 3, resize_dim)
+        self.blend = P.blend_mode(blend)
         params = torch.load(model_params, map_location='cpu') if isinstance(model_params, str) else model_params
         self.device = torch.device(device)
         self.resize_dim, self.invert, self.clip_threshold, self.add_patch = resize_dim, invert, clip_threshold, add_patch
         self.workspace_bytes = int(workspace_gb * 2 ** 30)
+        self.out_channels = params['out_channels']
         self.dist = dist if dist is not None else DistContext(False)
         self.engine = Engine('unet3d', params['state_dict'], params['n_filter'], params['in_channels'],
                              [('', params['out_channels'], 'sigmoid')],
@@ -67,6 +70,17 @@ class Session:
                               n, self.tta, 3)
         return plain['patches'], res
 
+    def _stitch(self, tiles, n_planes, zs_local, patch):
+        """Output planes [own_lo, own_lo + n_planes) from the uint8 result patches of consecutive z-rows whose starts,
+        relative to own_lo, are zs_local (negative for rows that begin below): the reference's mod-3 rule, or the
+        weighted stitch of blend='gaussian' (which does not depend on the patch order)."""
+        x, y = self.vol_shape[1], self.vol_shape[2]
+        if self.blend is None:
+            return P.E.stitch_mod3_u8(tiles, (n_planes, x, y), zs_local, self.X_start, self.Y_start, patch)
+        st = P.E.stitch_weighted_u8(tiles.contiguous(), 1, self.out_channels, (n_planes, x, y), zs_local, self.X_start,
+                                    self.Y_start, patch, *P.blend_tables(patch))
+        return st.view(n_planes, x, y)
+
     def _predict_pipelined(self, vol_dev, lut, zs, patch, shape, n_xy, groups=4):
         """Single process, host result wanted: the z-rows of the patch grid run in `groups` groups from the far end of
         the volume towards z = 0 (tiling.zslab_plan with the groups as virtual ranks: a group borrows only from groups
@@ -97,8 +111,7 @@ class Session:
                 extra = [zi for s in sorted(plans[g]['borrow']) for zi in plans[g]['borrow'][s]]
                 st_rows = list(range(lo, hi)) + extra
                 tiles = res.reshape(n, d, h, w) if not extra else torch.cat([res_rows[zi] for zi in st_rows])
-                st = P.E.stitch_mod3_u8(tiles, (own_hi - own_lo, x, y), [zs[zi] - own_lo for zi in st_rows],
-                                        self.X_start, self.Y_start, (d, h, w))
+                st = self._stitch(tiles, own_hi - own_lo, [zs[zi] - own_lo for zi in st_rows], (d, h, w))
                 ev = torch.cuda.Event()
                 ev.record(cur)
                 with torch.cuda.stream(self._s_out):
@@ -187,8 +200,7 @@ class Session:
             assert extra_rows == list(range(r_hi, r_hi + len(extra_rows)))
             tiles = torch.cat([res_local] + [t for _, t in recvs]) if recvs else res_local
             st_rows = list(range(r_lo, r_hi + len(extra_rows)))
-            st = P.E.stitch_mod3_u8(tiles, (own_hi - own_lo, x, y), [zs[zi] - own_lo for zi in st_rows], self.X_start,
-                                    self.Y_start, (d, h, w))
+            st = self._stitch(tiles, own_hi - own_lo, [zs[zi] - own_lo for zi in st_rows], (d, h, w))
         else:
             st = torch.zeros((0, x, y), dtype=torch.uint8, device=dev)
         if keep:       # test hook: what the reference's __split / __predict return (gathered on rank 0)
@@ -215,15 +227,22 @@ class Predict:
     tta (engine-only): None (default) or 'flips': the net also runs on the patches flipped along every combination of
     z, y and x (8 forwards per patch); the outputs are flipped back, averaged in fp32 on the device and quantised to
     uint8 once before the mod-3 stitch. About 8x the time of a plain prediction; memory stays within `workspace_gb`.
+
+    blend (engine-only): None (default, the reference's mod-3 stitch) or 'gaussian': the overlapping uint8 result
+    patches are merged as (sum w * v) // (sum w) with w = w_d[tz] * w_h[ty] * w_w[tx], Gaussian tables with sigma =
+    patch / 8 per axis (tiling.gaussian_weights), so that voxels near a patch border count least. Exact integer
+    arithmetic: sharding and z-row groups do not change a byte. Composes with `tta`.
     """
 
     def __init__(self, vol, result_name, model_params, network=UNet3D, resize_dim=(512, 512),
                  invert=False, normalization_mode='single', clip_threshold=(0., 99.8), add_patch=0,
                  normalize_result=False, progress_bar=True, device: Union[torch.device, str] = 'auto',
                  progress_notifier: ProgressNotifier = ProgressNotifier.progress_notifier_tqdm(), *,
-                 precision='tf32', workspace_gb=24.0, distributed=False, keep_intermediates=False, tta=None):
+                 precision='tf32', workspace_gb=24.0, distributed=False, keep_intermediates=False, tta=None,
+                 blend=None):
         if len(resize_dim) == 3:
             P.tta_codes(tta, 3, resize_dim)
+        P.blend_mode(blend)
         if isinstance(vol, str):
             vol = tiff.imread(vol)
         self.dist = DistContext(distributed)
@@ -247,7 +266,7 @@ class Predict:
 
         self.model_params = torch.load(model_params, map_location='cpu')
         ses = Session(self.model_params, resize_dim, invert, clip_threshold, add_patch, self.device, precision,
-                      workspace_gb, self.dist, tta=tta)
+                      workspace_gb, self.dist, tta=tta, blend=blend)
         print('Predicting data ...') if self.progress_bar and self.dist.rank == 0 else None
         vol_result = ses.predict(vol, keep=keep_intermediates)
         for k in ('N_z', 'N_x', 'N_y', 'Z_start', 'X_start', 'Y_start', 'N'):

@@ -183,6 +183,16 @@ int biu_stitch_mean_u8(const uint8_t* tiles, int F, int C, int H, int W, const i
 /* unet3d/predict.py:173-195: three slots, patch n -> slot n % 3, last writer wins, nanmean, uint8. */
 int biu_stitch_mod3_u8(const uint8_t* tiles, int Z, int H, int W, const int* zs, const int* ys, const int* xs, int nz,
                        int ny, int nx, int pd, int ph, int pw, uint8_t* out, void* stream);
+/* Engine-only (replaces nothing in the reference): weighted overlap stitch of uint8 result tiles,
+ *   out[f][c][z][y][x] = (sum w * v) // (sum w)   (0 where no tile covers the element or sum w = 0)
+ * over every tile n covering the element, v = its value there, w = w_d[tz] * w_h[ty] * w_w[tx] at the in-tile position
+ * (tz, ty, tx). Exact unsigned 64-bit integer sums and floor division: the result does not depend on the order of the
+ * tiles. w_d / w_h / w_w: device int32 tables of pd / ph / pw entries, each in [0, 1024]. tiles
+ * [F][nz*ny*nx][C][pd][ph][pw] -> out [F][C][Z][H][W]; starts may be negative and tiles may reach past the output.
+ * 2D: nz = pd = Z = 1, zs = {0}, w_d = {1}. */
+int biu_stitch_weighted_u8(const uint8_t* tiles, int F, int C, int Z, int H, int W, const int* zs, const int* ys,
+                           const int* xs, int nz, int ny, int nx, int pd, int ph, int pw, const int* w_d, const int* w_h,
+                           const int* w_w, uint8_t* out, void* stream);
 /* multi_output_unet3d/predict.py:203-307: ramp-weighted blend, tiles [V][nz*ny*nx][C][pd][ph][pw] float32. */
 int biu_stitch_ramp_f32(const float* tiles, int V, int C, int Z, int H, int W, const int* zs, const int* ys,
                         const int* xs, int nz, int ny, int nx, int pd, int ph, int pw, int margin, float* out,
