@@ -137,27 +137,15 @@ class Predict:
         del frames
         # split: every sliding window (reflect padding at the far end when the image is smaller than the patch)
         n_win = len(self._wx) * len(self._wy)
-        patches = P.E.gather_tiles_f32(norm, [0], self._wx, self._wy, (1, ph, pw)).reshape(t * n_win, 1, ph, pw)
-        tile_batch = P.pick_tile_batch(self.engine, (ph, pw), patches.shape[0], int(workspace_gb * 2 ** 30))
-        if self.tta is not None:       # mean over the transforms of every patch (float32), stitched like a patch
-            vals = P.run_tiles_tta(
-                lambda t: patches if t == 0 else P.E.gather_tiles_f32_tta(norm, [0], self._wx, self._wy, (1, ph, pw), 2,
-                                                                          t).reshape(-1, 1, ph, pw),
-                lambda tl, on_val: P.run_tiles(self.engine, tl, tile_batch, on_val=on_val),
-                patches.shape[0], self.tta, 2, out_dtype=torch.float32)
-        else:
-            vals = []
-            it = range(0, patches.shape[0], tile_batch)
-            if self.show_progress and progress_notifier is not None:
-                it = progress_notifier.iterator(it)
-            for b0 in it:
-                tl = patches[b0:b0 + tile_batch]
-                cnt = tl.shape[0]
-                if cnt < tile_batch:
-                    tl = torch.cat((tl, torch.zeros((tile_batch - cnt, *tl.shape[1:]), dtype=tl.dtype, device=dev)))
-                v, _ = self.engine.forward(tl.contiguous(), want_val=True, want_u8=False)
-                vals.append(v[:cnt])
-            vals = vals[0] if len(vals) == 1 else torch.cat(vals)                     # (P, head_total, ph, pw) float32
+        tile_batch = P.pick_tile_batch(self.engine, (ph, pw), t * n_win, int(workspace_gb * 2 ** 30))
+        progress = progress_notifier.iterator if (self.tta is None and self.show_progress and
+                                                  progress_notifier is not None) else None
+        # (P, head_total, ph, pw) float32; with tta the mean over the transforms of every patch, stitched like a patch
+        vals, patches = P.predict_tiles(
+            lambda k: P.E.gather_tiles_f32_tta(norm, [0], self._wx, self._wy, (1, ph, pw), 2, k).reshape(-1, 1, ph, pw),
+            lambda tl, on_val: P.run_tiles(self.engine, tl, tile_batch, want_val=True, want_u8=False, on_val=on_val,
+                                           progress=progress),
+            t * n_win, self.tta, 2, out_dtype=torch.float32)
         # stitch per head (the hole value is the mean of that head's float16 patches, :279)
         idx = (np.arange(t)[:, None, None] * self.N_per_img + np.arange(self.N_x)[None, :, None] * self.N_y +
                np.arange(self.N_y)[None, None, :]).astype(np.int32)

@@ -41,7 +41,7 @@ class Session:
         head_total = sum(self.output_heads[k]['channels'] for k in self.target_keys)
         self._planner = P.BatchPlanner(self.engine, self.workspace_bytes,
                                        lambda tile: P.tta_extra_bytes(tta, head_total, tile, in_bytes=4))
-        self._out = P.PinnedOut()
+        self._pin = P.PinnedPool()
         self._host_out, self._s_out = None, None
 
     def _plan(self, tile, n_tiles):
@@ -121,31 +121,13 @@ class Session:
             kept_p, kept_r = [], []
             for s in it:
                 e = min(s + vols_per_chunk, hi - lo)
-                if self.tta is None:
-                    patches = P.E.gather_tiles_f32(norm[s:e], self.Z_start, self.Y_start, self.X_start, self.patch_size)
-                    patches = patches.reshape(-1, 1, *self.patch_size)
-                    vals = []
-                    for b0 in range(0, patches.shape[0], tile_batch):
-                        t = patches[b0:b0 + tile_batch]
-                        cnt = t.shape[0]
-                        if cnt < tile_batch:
-                            t = torch.cat((t, torch.zeros((tile_batch - cnt, *t.shape[1:]), dtype=t.dtype, device=dev)))
-                        v, _ = self.engine.forward(t.contiguous(), want_val=True, want_u8=False)
-                        vals.append(v[:cnt])
-                    vals = vals[0] if len(vals) == 1 else torch.cat(vals)         # (n, head_total, pd, ph, pw)
-                else:       # mean over the 8 flips of every patch, merged on the device before the ramp blend
-                    plain = {}
-
-                    def gather(t):
-                        tl = P.E.gather_tiles_f32_tta(norm[s:e], self.Z_start, self.Y_start, self.X_start,
-                                                      self.patch_size, 3, t).reshape(-1, 1, *self.patch_size)
-                        if t == 0:
-                            plain['patches'] = tl
-                        return tl
-                    vals = P.run_tiles_tta(
-                        gather, lambda tl, on_val: P.run_tiles(self.engine, tl, tile_batch, on_val=on_val),
-                        (e - s) * self.N_per_vol, self.tta, 3, out_dtype=torch.float32)
-                    patches = plain['patches']
+                # (n, head_total, pd, ph, pw); with tta the mean over the 8 flips, merged before the ramp blend
+                vals, patches = P.predict_tiles(
+                    lambda t: P.E.gather_tiles_f32_tta(norm[s:e], self.Z_start, self.Y_start, self.X_start,
+                                                       self.patch_size, 3, t).reshape(-1, 1, *self.patch_size),
+                    lambda tl, on_val: P.run_tiles(self.engine, tl, tile_batch, want_val=True, want_u8=False,
+                                                   on_val=on_val),
+                    (e - s) * self.N_per_vol, self.tta, 3, out_dtype=torch.float32)
                 st = P.E.stitch_ramp_f32(vals, e - s, head_total, (d_img, h_img, w_img), self.Z_start, self.Y_start,
                                          self.X_start, self.patch_size, 16)
                 if on_device:
@@ -167,7 +149,7 @@ class Session:
             full = self.dist.gather_slabs(out_local, self.dist.shards(n_vol))
             if not to_host:
                 return full                  # (N, head_total, D, H, W) float32 device tensor (rank 0)
-            full = None if full is None else self._out.fetch(full)
+            full = None if full is None else self._pin.fetch('out', full)
         else:
             if self._s_out is not None:
                 self._s_out.synchronize()

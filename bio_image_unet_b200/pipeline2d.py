@@ -29,56 +29,30 @@ def to_device_stack(frames_np, device):
     return host.to(device, non_blocking=True)
 
 
-class PinnedOut:
-    """Reusable pinned host buffer for the final D2H copy of a result (grown on demand)."""
+class PinnedPool:
+    """Reusable pinned host buffers, one per key, grown on demand. A view stays valid until the next call that uses
+    the same key."""
 
     def __init__(self):
-        self.buf = None
+        self.bufs = {}
 
-    def view(self, shape, dtype):
-        """Pinned host tensor of the given shape (the buffer is reused by the next call)."""
-        n = int(np.prod(shape)) * torch.empty((), dtype=dtype).element_size()
-        if self.buf is None or self.buf.numel() < n:
-            self.buf = torch.empty(n, dtype=torch.uint8, pin_memory=True)
-        return self.buf[:n].view(dtype).view(*shape)
+    def view(self, key, shape, dtype):
+        """Pinned host tensor of the given shape and dtype."""
+        n = int(np.prod(shape)) * dtype.itemsize
+        buf = self.bufs.get(key)
+        if buf is None or buf.numel() < n:
+            buf = self.bufs[key] = torch.empty(n, dtype=torch.uint8, pin_memory=True)
+        return buf[:n].view(dtype).view(*shape)
 
-    def fetch(self, t):
-        n = t.numel() * t.element_size()
-        if self.buf is None or self.buf.numel() < n:
-            self.buf = torch.empty(n, dtype=torch.uint8, pin_memory=True)
-        host = self.buf[:n].view(t.dtype).view(t.shape)
+    def fetch(self, key, t):
+        """Device tensor `t` copied to the host: a numpy view of the pinned buffer of `key`."""
+        host = self.view(key, t.shape, t.dtype)
         host.copy_(t, non_blocking=True)
         torch.cuda.current_stream(t.device).synchronize()
         return host.numpy()
 
-
-class Normalizer2D:
-    """Percentile normalisation of a (F, H, W) integer stack to uint8 on the device
-    (unet/predict.py:122-150). ``stats_reduce`` lets the multi-GPU driver all-reduce the stack-wide histogram."""
-
-    def __init__(self, mode, clip_threshold, invert, stats_reduce=None, first_frame_hist=None):
-        if mode not in ('single', 'first', 'all'):
-            raise ValueError(f'normalization_mode {mode} not valid!')
-        self.mode, self.clip, self.invert = mode, clip_threshold, invert
-        self.stats_reduce = stats_reduce
-        self.first_frame_hist = first_frame_hist
-        self.params = None
-
-    def __call__(self, frames_dev):
-        f = frames_dev.shape[0]
-        hist = E.histogram(frames_dev)
-        if self.mode == 'single':
-            lut, self.params = E.norm_lut(hist, hist, f, self.clip[0], self.clip[1], self.invert)
-        else:
-            total = E.hist_sum(hist)
-            if self.stats_reduce is not None:
-                total = self.stats_reduce(total)
-            if self.mode == 'all':
-                bounds = total
-            else:
-                bounds = self.first_frame_hist(hist) if self.first_frame_hist is not None else hist[0:1].contiguous()
-            lut, self.params = E.norm_lut(bounds, total, 1, self.clip[0], self.clip[1], self.invert)
-        return E.apply_lut(frames_dev, lut)
+    def close(self):
+        self.bufs = {}
 
 
 TTA_MODES = (None, 'flips', 'dihedral')
@@ -146,39 +120,42 @@ def tta_extra_bytes(tta, channels, tile, in_bytes=1):
     return 8 * int(channels) * px + int(in_bytes) * px
 
 
-def run_tiles(eng, tiles, tile_batch, prev_tiles=None, want_val=False, on_val=None):
-    """Forward all tiles in batches of the planned size (the tail batch is zero-padded). With `on_val` every batch's
-    float output is handed to on_val(start, val) instead of being returned, and no uint8 result is made."""
+def _joined(outs):
+    return None if not outs else outs[0] if len(outs) == 1 else torch.cat(outs)
+
+
+def run_tiles(eng, tiles, tile_batch, prev_tiles=None, n_per=0, want_val=False, want_u8=True, on_val=None,
+              progress=None):
+    """Forward all tiles in batches of the planned `tile_batch` results (the tail batch is zero-padded) and return
+    the (uint8, float) outputs of the head, trimmed to the tiles; an output that is not wanted is None. With `on_val`
+    every batch's float output goes to on_val(start, val) instead: no uint8 output is made and both returned are None.
+
+    prev_tiles: the second input of a two-input Siam_UNet, sliced like `tiles`. n_per: Siam_UNet with the shared twin
+    encoder, n_per tiles per frame - tiles = [tiles of the previous frame of the first pair | tiles of the current
+    frames], pair j = (tile j, tile j + n_per), so len(tiles) - n_per results, and the batch starting at pair s takes
+    the unique tiles tiles[s : s + cnt + n_per]. progress: wraps the iterator over the batch starts."""
     if on_val is not None:
-        for s in range(0, tiles.shape[0], tile_batch):
-            t = tiles[s:s + tile_batch]
-            p = None if prev_tiles is None else prev_tiles[s:s + tile_batch]
-            cnt = t.shape[0]
-            if cnt < tile_batch:
-                pad = torch.zeros((tile_batch - cnt, *t.shape[1:]), dtype=t.dtype, device=t.device)
-                t = torch.cat((t, pad))
-                p = None if p is None else torch.cat((p, pad))
-            val, _ = eng.forward(t.contiguous(), None if p is None else p.contiguous(), want_val=True, want_u8=False)
-            on_val(s, val[:cnt])
-        return None, None
-    n = tiles.shape[0]
+        want_val, want_u8 = True, False
+    n = tiles.shape[0] - n_per
+    starts = range(0, n, tile_batch)
     outs_u8, outs_val = [], []
-    for s in range(0, n, tile_batch):
-        t = tiles[s:s + tile_batch]
-        p = None if prev_tiles is None else prev_tiles[s:s + tile_batch]
-        cnt = t.shape[0]
+    for s in (starts if progress is None else progress(starts)):
+        cnt = min(tile_batch, n - s)
+        t = tiles[s:s + cnt + n_per]
+        p = None if prev_tiles is None else prev_tiles[s:s + cnt]
         if cnt < tile_batch:
             pad = torch.zeros((tile_batch - cnt, *t.shape[1:]), dtype=t.dtype, device=t.device)
             t = torch.cat((t, pad))
-            if p is not None:
-                p = torch.cat((p, pad))
-        val, u8 = eng.forward(t.contiguous(), None if p is None else p.contiguous(), want_val=want_val, want_u8=True)
-        outs_u8.append(u8[:cnt])
+            p = None if p is None else torch.cat((p, pad))
+        val, u8 = eng.forward(t.contiguous(), None if p is None else p.contiguous(), want_val=want_val, want_u8=want_u8)
+        if on_val is not None:
+            on_val(s, val[:cnt])
+            continue
+        if want_u8:
+            outs_u8.append(u8[:cnt])
         if want_val:
             outs_val.append(val[:cnt])
-    u8 = outs_u8[0] if len(outs_u8) == 1 else torch.cat(outs_u8)
-    val = None if not want_val else (outs_val[0] if len(outs_val) == 1 else torch.cat(outs_val))
-    return u8, val
+    return _joined(outs_u8), _joined(outs_val)
 
 
 def even_batch(total_tiles, budget_batch):
@@ -220,38 +197,23 @@ class BatchPlanner:
         return self.tile_batch
 
 
-def run_tiles_shared(eng, tiles_u, tile_batch, n_per, on_val=None):
-    """Siam_UNet with the shared twin encoder: tiles_u = [tiles of the previous frame of the first pair | tiles of the
-    current frames] (n_pairs + n_per tiles); pair j = (previous tile j, current tile j + n_per). Batches of `tile_batch`
-    pairs take the contiguous slice of tile_batch + n_per unique tiles they need (the tail batch is zero-padded).
-    With `on_val` the float output of every batch goes to on_val(start pair, val) instead (as in run_tiles)."""
-    n_pairs = tiles_u.shape[0] - n_per
-    outs = []
-    for s in range(0, n_pairs, tile_batch):
-        cnt = min(tile_batch, n_pairs - s)
-        t = tiles_u[s:s + cnt + n_per]
-        if cnt < tile_batch:
-            t = torch.cat((t, torch.zeros((tile_batch - cnt, *t.shape[1:]), dtype=t.dtype, device=t.device)))
-        val, u8 = eng.forward(t.contiguous(), None, want_val=on_val is not None, want_u8=on_val is None)
-        if on_val is not None:
-            on_val(s, val[:cnt])
-        else:
-            outs.append(u8[:cnt])
-    if on_val is not None:
-        return None
-    return outs[0] if len(outs) == 1 else torch.cat(outs)
+def predict_tiles(gather, run, n, codes, dims, out_dtype=torch.uint8):
+    """Result tiles of one chunk of `n` tiles and the chunk's plain input tiles: (result, gather(0)). gather(t) makes
+    the input tiles under transform t (t = 0: the plain tiles); run(tiles, on_val) is run_tiles on them, returning
+    its (uint8, float) outputs.
 
-
-def run_tiles_tta(gather, run, n, codes, dims, out_dtype=torch.uint8):
-    """Test-time augmentation of one chunk of `n` result tiles. For every transform code t of `codes`, in ascending
-    order: gather(t) makes the chunk's input tiles under T_t, run(tiles, on_val) runs the same forwards as a plain
-    prediction (run_tiles / run_tiles_shared with on_val), and every batch's float output goes through T_t^-1 into one
-    fp32 running sum of the chunk. The last pass writes the mean as the uint8 result tiles (trunc(mean * 255), as the
-    head does without augmentation) or as float32 (out_dtype). Plans, tile batches and stitches are those of a plain
-    prediction; the cost is len(codes) forwards per tile."""
+    codes None: the plain tiles run once, and the result is the head's own output - its uint8, or its float output
+    for out_dtype float32. Otherwise test-time augmentation: for every transform code t of `codes`, in ascending
+    order, the same forwards as a plain prediction run on gather(t), and every batch's float output goes through
+    T_t^-1 into one fp32 running sum of the chunk. The last pass writes the mean as uint8 (trunc(mean * 255), as the
+    head does) or as float32 (out_dtype). Plans, tile batches and stitches are those of a plain prediction; the cost
+    is len(codes) forwards per tile."""
+    if codes is None:
+        plain = gather(0)
+        u8, val = run(plain, None)
+        return (u8 if out_dtype == torch.uint8 else val), plain
     k = len(codes)
     bufs = {}
-
     for p, t in enumerate(codes):
         def on_val(s, val, p=p, t=t):
             if not bufs:
@@ -263,8 +225,11 @@ def run_tiles_tta(gather, run, n, codes, dims, out_dtype=torch.uint8):
             out = bufs['out'][s:s + cnt]
             E.tta_accumulate(val, acc, dims, t, p, k, out_u8=out if out_dtype == torch.uint8 else None,
                              out_f32=out if out_dtype == torch.float32 else None)
-        run(gather(t), on_val)
-    return bufs['out']
+        tiles = gather(t)
+        if t == 0:
+            plain = tiles
+        run(tiles, on_val)
+    return bufs['out'], plain
 
 
 def pick_tile_batch(eng, tile, total_tiles, budget_bytes):
@@ -283,35 +248,21 @@ def check_starts(starts, tile, extent):
                              f'(image smaller than resize_dim with add_tile > 0)')
 
 
-def predict_frames_2d(eng, norm_u8, resize_dim, add_tile, out_channels, tile_batch, pad_mode=0, raw=None, lut=None,
-                      tta=None, blend=None):
-    """norm_u8: (F, H, W) uint8 device tensor (already normalised) - or None with `raw` (the uint8 / uint16 stack) and
-    `lut` (its normalisation tables): the normalisation is then fused into the tile gather and the normalised stack
-    is never written. tta: transform codes of test-time augmentation (tta_codes) or None; blend: blend_mode() value.
-    Returns ((F, C, H, W) uint8 device tensor, grid, tiles, result_tiles); with tta, `tiles` are the plain (t = 0)
-    tiles."""
-    f, h, w = (norm_u8 if norm_u8 is not None else raw).shape
+def predict_frames_2d(eng, frames, resize_dim, add_tile, out_channels, tile_batch, lut=None, pad_mode=0, tta=None,
+                      blend=None):
+    """frames: (F, H, W) contiguous device stack, already normalised to uint8 - or, with `lut` (its normalisation
+    tables), the raw uint8 / uint16 stack: the normalisation is then fused into the tile gather and the normalised
+    stack is never written. tta: transform codes of test-time augmentation (tta_codes) or None; blend: blend_mode()
+    value. Returns ((F, C, H, W) uint8 device tensor, grid, tiles, result_tiles); `tiles` are the plain (t = 0)
+    (F*N, 1, th, tw) tiles."""
+    f, h, w = frames.shape
     th, tw = resize_dim
     n_x, n_y, xs, ys = tiling.grid_2d(h, w, resize_dim, add_tile)
     check_starts(xs, th, h)
     check_starts(ys, tw, w)
-    if tta is not None:
-        src = (norm_u8 if norm_u8 is not None else raw).view(f, 1, h, w)
-        plain = {}
-
-        def gather(t):
-            tl = E.gather_tiles_tta(src, [0], xs, ys, (1, th, tw), pad_mode, 2, t, lut=None if norm_u8 is not None else lut)
-            if t == 0:
-                plain['tiles'] = tl
-            return tl
-        res_u8 = run_tiles_tta(gather, lambda tl, on_val: run_tiles(eng, tl, tile_batch, on_val=on_val),
-                               f * n_x * n_y, tta, 2)
-        tiles = plain['tiles']
-    elif norm_u8 is not None:
-        tiles = E.gather_tiles(norm_u8.view(f, 1, h, w), [0], xs, ys, (1, th, tw), pad_mode)  # (F*N, 1, th, tw)
-        res_u8, _ = run_tiles(eng, tiles, tile_batch)
-    else:
-        tiles = E.gather_tiles_lut(raw.view(f, 1, h, w), lut, [0], xs, ys, (1, th, tw), pad_mode)
-        res_u8, _ = run_tiles(eng, tiles, tile_batch)
+    src = frames.view(f, 1, h, w)
+    res_u8, tiles = predict_tiles(lambda t: E.gather_tiles_tta(src, [0], xs, ys, (1, th, tw), pad_mode, 2, t, lut=lut),
+                                  lambda tl, on_val: run_tiles(eng, tl, tile_batch, on_val=on_val),
+                                  f * n_x * n_y, tta, 2)
     out = stitch_2d(res_u8, f, out_channels, (h, w), xs, ys, (th, tw), blend)
     return out, (n_x, n_y, xs, ys), tiles, res_u8

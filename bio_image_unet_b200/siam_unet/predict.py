@@ -82,7 +82,7 @@ class Session:
         # current frame) and pair t + 1 (as the previous one) - it runs once (biu_net_set_siam_shared)
         self.shared_encoder = normalization_mode == 'single' and params['mode'] != 'control'
         self.siam_mode = params['mode']
-        self._pin, self._streams, self._dev_in = {}, None, None
+        self._pin, self._streams, self._dev_in = P.PinnedPool(), None, None
         self.last = {}
 
     # ---- geometry / planning ---------------------------------------------------------------------------------
@@ -130,22 +130,12 @@ class Session:
             P.check_starts(ys, tw, w)
             lut, _ = P.E.norm_lut(hist, hist, k, q_lo, q_hi, self.invert)
             n_per = n_x * n_y
-            if tta is None:
-                tiles_u = P.E.gather_tiles_lut(frames.contiguous().view(k, 1, h, w), lut, [0], xs, ys, (1, th, tw), 1)
-                res_u8 = P.run_tiles_shared(self.engine, tiles_u, self.tile_batch, n_per)
-            else:       # every unique tile of a pass carries the same transform: the shared encoder runs as it is
-                plain = {}
-
-                def gather(t):
-                    tl = P.E.gather_tiles_tta(frames.contiguous().view(k, 1, h, w), [0], xs, ys, (1, th, tw), 1, 2, t,
-                                              lut=lut)
-                    if t == 0:
-                        plain['tiles'] = tl
-                    return tl
-                res_u8 = P.run_tiles_tta(
-                    gather, lambda tl, on_val: P.run_tiles_shared(self.engine, tl, self.tile_batch, n_per, on_val=on_val),
-                    n_pairs * n_per, tta, 2)
-                tiles_u = plain['tiles']
+            src = frames.contiguous().view(k, 1, h, w)
+            # with tta every unique tile of a pass carries the same transform: the shared encoder runs as it is
+            res_u8, tiles_u = P.predict_tiles(
+                lambda t: P.E.gather_tiles_tta(src, [0], xs, ys, (1, th, tw), 1, 2, t, lut=lut),
+                lambda tl, on_val: P.run_tiles(self.engine, tl, self.tile_batch, n_per=n_per, on_val=on_val),
+                n_pairs * n_per, tta, 2)
             st = P.stitch_2d(res_u8, n_pairs, 1, (h, w), xs, ys, (th, tw), self.blend)
             self.last = dict(tiles_cur=tiles_u[n_per:], tiles_prev=tiles_u[:n_pairs * n_per], result_tiles=res_u8) if keep else {}
             return st
@@ -161,37 +151,17 @@ class Session:
             norm_cur = P.E.apply_lut(_take(frames, c_sel), lut)
         P.check_starts(xs, th, h)
         P.check_starts(ys, tw, w)
-        if tta is None:
-            tiles_cur = P.E.gather_tiles(norm_cur.view(n_pairs, 1, h, w), [0], xs, ys, (1, th, tw), 1)      # zero padding
-            tiles_prev = P.E.gather_tiles(norm_prev.view(n_pairs, 1, h, w), [0], xs, ys, (1, th, tw), 1)
-            res_u8, _ = P.run_tiles(self.engine, tiles_cur, self.tile_batch, prev_tiles=tiles_prev)
-        else:           # both frames of a pair get the same transform
-            plain = {}
-
-            def gather(t):
-                tl = tuple(P.E.gather_tiles_tta(nf.view(n_pairs, 1, h, w), [0], xs, ys, (1, th, tw), 1, 2, t)
-                           for nf in (norm_cur, norm_prev))
-                if t == 0:
-                    plain['tiles'] = tl
-                return tl
-            res_u8 = P.run_tiles_tta(
-                gather, lambda tl, on_val: P.run_tiles(self.engine, tl[0], self.tile_batch, prev_tiles=tl[1],
-                                                       on_val=on_val),
-                n_pairs * n_x * n_y, tta, 2)
-            tiles_cur, tiles_prev = plain['tiles']
+        # zero padding; with tta both frames of a pair get the same transform
+        res_u8, (tiles_cur, tiles_prev) = P.predict_tiles(
+            lambda t: tuple(P.E.gather_tiles_tta(nf.view(n_pairs, 1, h, w), [0], xs, ys, (1, th, tw), 1, 2, t)
+                            for nf in (norm_cur, norm_prev)),
+            lambda tl, on_val: P.run_tiles(self.engine, tl[0], self.tile_batch, prev_tiles=tl[1], on_val=on_val),
+            n_pairs * n_x * n_y, tta, 2)
         st = P.stitch_2d(res_u8, n_pairs, 1, (h, w), xs, ys, (th, tw), self.blend)
         self.last = dict(tiles_cur=tiles_cur, tiles_prev=tiles_prev, result_tiles=res_u8) if keep else {}
         return st
 
     # ---- the streaming pipeline --------------------------------------------------------------------------------
-    def _pinned(self, key, shape, dtype):
-        n = int(np.prod(shape))
-        buf = self._pin.get(key)
-        if buf is None or buf.numel() < n or buf.dtype != dtype:
-            buf = torch.empty(n, dtype=dtype, pin_memory=True)
-            self._pin[key] = buf
-        return buf[:n].view(*shape)
-
     def predict_stream(self, source, lo, hi, sink, chunk_pairs=None, keep=None, progress=None, out_dev=None):
         """Pairs [lo, hi) of `source` (an object with n / shape / dtype / read_into(dst, frame_indices)) through the
         device; `sink(first_pair, frames_u8)` receives the stitched (n, H, W) uint8 pages of each chunk in order (a
@@ -221,8 +191,8 @@ class Session:
             if self._dev_in is None or self._dev_in[0] != key:
                 self._dev_in = (key, [torch.empty((kmax, h, w), dtype=tdtype, device=dev) for _ in range(2)])
             dev_in = self._dev_in[1]
-            stage = [self._pinned(f'stage{b}', (kmax, h, w), tdtype) for b in range(2)]
-            outb = [self._pinned(f'out{b}', (chunk_pairs, h, w), torch.uint8) for b in range(2)]
+            stage = [self._pin.view(f'stage{b}', (kmax, h, w), tdtype) for b in range(2)]
+            outb = [self._pin.view(f'out{b}', (chunk_pairs, h, w), torch.uint8) for b in range(2)]
             ev_in = [torch.cuda.Event() for _ in range(2)]
             ev_done = [torch.cuda.Event() for _ in range(2)]
             ev_out = [torch.cuda.Event() for _ in range(2)]
@@ -278,7 +248,8 @@ class Session:
         if self.engine is not None:
             self.engine.close()
             self.engine = None
-        self._pin, self._dev_in = {}, None
+        self._pin.close()
+        self._dev_in = None
 
 
 class Predict:

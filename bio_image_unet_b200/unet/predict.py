@@ -47,7 +47,7 @@ class Session:
                                        lambda tile: P.tta_extra_bytes(tta, self.out_channels, tile))
         self.fixed_lut = None          # set by Predict for 'first' / 'all' (stack-wide statistics incl. other ranks)
         self.last = {}
-        self._pin, self._streams, self._dev_in = {}, None, None
+        self._pin, self._streams, self._dev_in = P.PinnedPool(), None, None
         self._comm_stream, self._d2h_stream, self._slab, self._full, self.comm = None, None, None, None, {}
 
     def _ensure_plan(self, total_tiles):
@@ -113,33 +113,21 @@ class Session:
             self._ensure_plan(f * n_x * n_y)
         want_norm = keep if want_norm is None else want_norm
         if frames_dev.dtype == torch.float32 or want_norm:
-            norm = self.normalise_device(frames_dev, lut)
-            out, grid, tiles, res_tiles = P.predict_frames_2d(self.engine, norm, self.resize_dim, self.add_tile,
-                                                              self.out_channels, self.tile_batch, tta=self.tta,
-                                                              blend=self.blend)
+            src = norm = self.normalise_device(frames_dev, lut)
+            lut = None
             if frames_dev.dtype == torch.float32:      # what the reference stores back into a float stack (:131)
                 norm = self.last_norm_f32
         else:
-            norm = None
-            out, grid, tiles, res_tiles = P.predict_frames_2d(self.engine, None, self.resize_dim, self.add_tile,
-                                                              self.out_channels, self.tile_batch,
-                                                              raw=frames_dev.contiguous(), lut=self.lut_device(frames_dev, lut),
-                                                              tta=self.tta, blend=self.blend)
+            norm, src, lut = None, frames_dev.contiguous(), self.lut_device(frames_dev, lut)
+        out, grid, tiles, res_tiles = P.predict_frames_2d(self.engine, src, self.resize_dim, self.add_tile,
+                                                          self.out_channels, self.tile_batch, lut=lut, tta=self.tta,
+                                                          blend=self.blend)
         self.last = dict(grid=grid, norm=norm, tiles=tiles if keep else None, result_tiles=res_tiles if keep else None)
         return out
 
     def predict(self, frames):
         """Host stack in, host result out (H2D and D2H inside, pipelined against the compute)."""
         return self.predict_movie(frames)[0]
-
-    def _pinned(self, key, shape, dtype):
-        """Reusable pinned host buffer (grown on demand)."""
-        n = int(np.prod(shape))
-        buf = self._pin.get(key)
-        if buf is None or buf.numel() < n or buf.dtype != dtype:
-            buf = torch.empty(n, dtype=dtype, pin_memory=True)
-            self._pin[key] = buf
-        return buf[:n].view(*shape)
 
     def predict_movie(self, frames, chunk_frames=None, want_norm=False, out_dev=None):
         """Pipelined prediction of a host (F, H, W) uint8/uint16 stack (numpy array or torch tensor, ideally
@@ -179,14 +167,14 @@ class Session:
             cur = torch.cuda.current_stream(dev)
             for st in self._streams:
                 st.wait_stream(cur)
-            out_host = self._pinned('out', (f, self.out_channels, h, w), torch.uint8) if out_dev is None else None
-            norm_host = self._pinned('norm', (f, h, w), torch.float32 if is_float else torch.uint8) if want_norm else None
+            out_host = self._pin.view('out', (f, self.out_channels, h, w), torch.uint8) if out_dev is None else None
+            norm_host = self._pin.view('norm', (f, h, w), torch.float32 if is_float else torch.uint8) if want_norm else None
             pinned_in = resident or host.is_pinned()
             key = (chunk_frames, h, w, host.dtype)
             if not resident and (self._dev_in is None or self._dev_in[0] != key):
                 self._dev_in = (key, [torch.empty((chunk_frames, h, w), dtype=host.dtype, device=dev) for _ in range(2)])
             dev_in = None if resident else self._dev_in[1]
-            stage = None if pinned_in else [self._pinned(f'stage{b}', (chunk_frames, h, w), host.dtype) for b in range(2)]
+            stage = None if pinned_in else [self._pin.view(f'stage{b}', (chunk_frames, h, w), host.dtype) for b in range(2)]
             ev_in = [torch.cuda.Event() for _ in range(2)]
             ev_done = [torch.cuda.Event() for _ in range(2)]
             for i, s0 in enumerate(range(0, f, chunk_frames)):
@@ -271,7 +259,7 @@ class Session:
                 if self._full is None or tuple(self._full.shape) != (n_total, c, h, w):
                     self._full = torch.empty((n_total, c, h, w), dtype=torch.uint8, device=dev) if ctx.multi else None
                 full = self._full if ctx.multi else slab
-            out_host = self._pinned('out_full', (n_total, c, h, w), torch.uint8) if (to_host and ctx.rank == 0) else None
+            out_host = self._pin.view('out_full', (n_total, c, h, w), torch.uint8) if (to_host and ctx.rank == 0) else None
             t_ev = []
             for j in range(segments):
                 a, b = P.tiling.shard_range(f, j, segments)
@@ -317,7 +305,8 @@ class Session:
         if self.engine is not None:
             self.engine.close()
             self.engine = None
-        self._pin, self._dev_in, self._slab, self._full = {}, None, None, None
+        self._pin.close()
+        self._dev_in, self._slab, self._full = None, None, None
 
 
 class Predict:

@@ -40,7 +40,7 @@ class Session:
         self._planner = P.BatchPlanner(self.engine, self.workspace_bytes,
                                        lambda tile: P.tta_extra_bytes(tta, params['out_channels'], tile))
         self.exchanged_bytes = 0
-        self._out = P.PinnedOut()
+        self._pin = P.PinnedPool()
         self._s_out = None
 
     def _plan(self, tile, n_tiles):
@@ -51,24 +51,13 @@ class Session:
         """uint8 result patches (n, 1, d, h, w) of the patch rows starting at `zs` of the (1, Z, X, Y) raw slab `src`
         (normalisation fused into the gather), and the plain uint8 patches; with test-time augmentation the result is
         the mean over the flips, merged on the device before the one uint8 quantisation."""
-        d, h, w = patch
         n = len(zs) * len(self.X_start) * len(self.Y_start)
-        if self.tta is None:
-            patches = P.E.gather_tiles_lut(src, lut, zs, self.X_start, self.Y_start, patch, 0)
-            tile_batch = self._plan(patch, n)
-            res, _ = P.run_tiles(self.engine, patches.reshape(n, 1, d, h, w), tile_batch)
-            return patches, res
         tile_batch = self._plan(patch, n)
-        plain = {}
-
-        def gather(t):
-            tl = P.E.gather_tiles_tta(src, zs, self.X_start, self.Y_start, patch, 0, 3, t, lut=lut)
-            if t == 0:
-                plain['patches'] = tl
-            return tl.reshape(n, 1, d, h, w)
-        res = P.run_tiles_tta(gather, lambda tl, on_val: P.run_tiles(self.engine, tl, tile_batch, on_val=on_val),
-                              n, self.tta, 3)
-        return plain['patches'], res
+        res, patches = P.predict_tiles(
+            lambda t: P.E.gather_tiles_tta(src, zs, self.X_start, self.Y_start, patch, 0, 3, t, lut=lut),
+            lambda tl, on_val: P.run_tiles(self.engine, tl.reshape(n, 1, *patch), tile_batch, on_val=on_val),
+            n, self.tta, 3)
+        return patches, res
 
     def _stitch(self, tiles, n_planes, zs_local, patch):
         """Output planes [own_lo, own_lo + n_planes) from the uint8 result patches of consecutive z-rows whose starts,
@@ -90,7 +79,7 @@ class Session:
         z, x, y = shape
         dev = self.device
         plans = tiling.zslab_plan(zs, d, z, min(groups, self.N_z))
-        out_host = self._out.view((z, x, y), torch.uint8)
+        out_host = self._pin.view('out', (z, x, y), torch.uint8)
         if self._s_out is None:
             self._s_out = torch.cuda.Stream(dev)
         cur = torch.cuda.current_stream(dev)
@@ -211,7 +200,7 @@ class Session:
         full = ctx.gather_slabs(st, [p['own'] for p in plans], n_total=z) if ctx.multi else st
         if full is None or not to_host:
             return full
-        return self._out.fetch(full)      # view of a pinned buffer that the next call reuses
+        return self._pin.fetch('out', full)      # view of a pinned buffer that the next call reuses
 
 
 class Predict:

@@ -170,10 +170,13 @@ def test_unet_decomposes(precision, network, tta):
 
 
 @pytest.mark.parametrize('precision', PRECISIONS)
-@pytest.mark.parametrize('shared', [True, False])
-def test_siam_decomposes(precision, shared):
+@pytest.mark.parametrize('siam_path', ['shared_encoder', 'two_input'])
+def test_siam_decomposes(precision, siam_path):
+    """Both Siam_UNet paths: the shared twin encoder ('concat' in 'single' mode, batches of unique tiles through
+    run_tiles with n_per) and the two-input network ('control')."""
     from bio_image_unet_b200.siam_unet import Session
     from bio_image_unet_b200.siam_unet.siam_unet import Siam_UNet
+    shared = siam_path == 'shared_encoder'
     torch.manual_seed(2)
     mode = 'concat' if shared else 'control'
     ck = {'state_dict': Siam_UNet(n_filter=8, mode=mode).eval().state_dict(), 'n_filter': 8, 'mode': mode}
@@ -198,8 +201,8 @@ def test_siam_decomposes(precision, shared):
         acc = None
         for t in codes:
             vals = []
-            P.run_tiles_shared(ses.engine, T(tiles_u, 2, t).contiguous(), ses.tile_batch, n_per,
-                               on_val=lambda s, v: vals.append(v.clone()))
+            P.run_tiles(ses.engine, T(tiles_u, 2, t).contiguous(), ses.tile_batch, n_per=n_per,
+                        on_val=lambda s, v: vals.append(v.clone()))
             v = T_inv(torch.cat(vals), 2, t)
             acc = v if acc is None else acc + v
     else:

@@ -3,8 +3,9 @@
 
 For every config the same Session runs the modes tta=None, 'flips' and (2D) 'dihedral' in alternation, `--reps` times
 each: device-resident and end-to-end rates, and the device time of the TTA gather and merge launches, taken from CUDA
-events around every call of engine.gather_tiles_tta / engine.tta_accumulate, as a share of the step. The card's name,
-power limit and SM clock are read in the same call. One JSON line per config and mode.
+events around every call of engine.gather_tiles_tta / engine.tta_accumulate in the TTA modes, as a share of the step
+(tta=None gathers through the same entry point with transform 0, which is no TTA work). The card's name, power limit
+and SM clock are read in the same call. One JSON line per config and mode.
 
     python tools/bench_tta.py [--configs 1,2,4] [--frames 32] [--reps 2] [--out DIR]
 """
@@ -25,10 +26,13 @@ from bio_image_unet_b200 import pipeline2d as P  # noqa: E402
 from bio_image_unet_b200.dist import DistContext  # noqa: E402
 
 _EVENTS = []
+_TTA_ON = [False]          # set while the session runs a TTA mode
 
 
 def _timed(fn):
     def wrap(*a, **k):
+        if not _TTA_ON[0]:
+            return fn(*a, **k)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         r = fn(*a, **k)
@@ -53,6 +57,7 @@ def set_tta(ses, mode, dims, channels):
     """Switch an existing Session's tta mode (re-plans on the next call)."""
     tile = ses.resize_dim
     ses.tta = P.tta_codes(mode, dims, tile)
+    _TTA_ON[0] = ses.tta is not None
     ses._planner.extra_per_tile = lambda t: P.tta_extra_bytes(mode, channels, t)
     ses._planner.tile = None
     ses._planner.tile_batch = None
